@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload cfg1|cfg2|cfg3|cfg4] [--precision tf32|fp32] [--variant softmax|contrast]
+                    [--dump-outputs DIR]
 
 One "step" = one GE2E forward + backward (grads to E, w, b) over one synthetic batch.
   value  device-resident inputs, the C-ABI calls of K consecutive steps captured in ONE CUDA graph
@@ -25,6 +26,9 @@ N=1 runs cfg3 (the config the metric is quoted on).  N>1 runs cfg4 (N=8192, M=16
 ranks (strong scaling: total work fixed); every rank checks its shard of the result against the single-GPU
 plan on the same batch (parity_check, non-zero exit on failure) and rank 0 times cfg4 unsharded on its own
 GPU so the line carries its own 1-GPU denominator (scaling_efficiency_same_workload).
+--dump-outputs DIR writes what the K-th (last) timed step returned to its caller -- loss, dw, db and dE, float32 --
+as DIR/<name>.npy (a sampled dE comes with its row indices, dE_rows.npy).  The batches are seeded and w = 10, b = -5, so the same arguments give the same inputs and two
+builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -78,6 +82,35 @@ def make_batch(N, M, D, seed=0):
     g = torch.Generator().manual_seed(seed)
     x = torch.randn(N * M, D, generator=g)
     return (x / x.norm(dim=1, keepdim=True)).reshape(N, M, D).contiguous()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_row_ids(U, D):
+    """Utterance rows of dE that --dump-outputs writes: all U when they fit 64 MB (less 1 MB kept for the
+    scalars and the row indices), else a fixed seeded sample (numpy default_rng(0)), sorted.  cfg4's dE is 134 MB."""
+    cap = (DUMP_BYTES - (1 << 20)) // (4 * D)
+    if U <= cap:
+        return np.arange(U)
+    return np.sort(np.random.default_rng(0).choice(U, cap, replace=False))
+
+
+def write_outputs(out_dir, outputs, N, M, D):
+    """outputs: name -> float32 host array, dE as the [rows, D] rows of dump_row_ids.  Writes out_dir/<name>.npy:
+    dE as [N, M, D] when it holds every row, else its rows plus their indices into [N * M, D] as dE_rows.npy
+    (float64, exact).  Returns what the JSON line records."""
+    rows = outputs["dE"].shape[0]
+    if rows == N * M:
+        outputs = dict(outputs, dE=outputs["dE"].reshape(N, M, D))
+    else:
+        outputs = dict(outputs, dE_rows=dump_row_ids(N * M, D).astype(np.float64))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return {"dir": os.path.abspath(out_dir), "shapes": {k: list(a.shape) for k, a in outputs.items()},
+            "dE_rows": "all" if rows == N * M else
+                       f"{rows} of {N * M} utterance rows of dE as [N * M, D], indices in dE_rows.npy (dump_row_ids)"}
 
 
 class ClockSampler(threading.Thread):
@@ -421,6 +454,11 @@ def run_ours(args):
         ms = [ms_med] * args.steps
         clocks = sampler.finish()
         extra["replays_ms"] = [round(x, 6) for x in replays]
+        if args.dump_outputs:
+            # the plan's buffers hold the last timed step (batch (K - 1) % n_rot); later measurements reuse them
+            ids = torch.from_numpy(dump_row_ids(U, D)).to(dev)
+            outputs = {"loss": plan.loss.cpu().numpy(), "dw": plan.dw.cpu().numpy(), "db": plan.db.cpu().numpy(),
+                       "dE": plan.dE.reshape(U, D)[ids].cpu().numpy()}
         g1 = plan.capture(E, w, b)
         launches = plan.launches_per_step * args.steps
         extra["ms_per_step_l2_flushed"] = float(np.median(timed_steps(g1.replay, args.steps, args.warmup, flush)))
@@ -679,6 +717,16 @@ def run_ours(args):
             t = torch.tensor([ev0.elapsed_time(ev1)], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = [t.item() / args.steps] * args.steps
+            if args.dump_outputs:
+                # loss / dw / db are global; every rank holds its speakers' rows of dE and sends rank 0 the sampled ones
+                ids = dump_row_ids(U, D)
+                lo = off * M
+                mine = torch.from_numpy(ids[(ids >= lo) & (ids < lo + n_local * M)] - lo).to(dev)
+                parts = [None] * world if rank == 0 else None
+                dist.gather_object(splan.dE.reshape(-1, D)[mine].cpu().numpy(), parts, dst=0)
+                if rank == 0:
+                    outputs = {"loss": splan.loss.cpu().numpy(), "dw": splan.dw.cpu().numpy(),
+                               "db": splan.db.cpu().numpy(), "dE": np.concatenate(parts)}
             splan.step(shards[0], w, b)                     # same batch as the checks below
             torch.cuda.synchronize()
             extra["sharded_loss_check"] = {"graph_plan": splan.loss.item()}
@@ -840,6 +888,8 @@ def run_ours(args):
     if cpu_val is not None:
         line["cpu_baseline"] = {"value": cpu_val, "unit": UNIT, "cores": cpu_info["cores"], "kind": cpu_info["kind"],
                                 "sample": cpu_sample_text(cpu_info, N, M)}
+    if args.dump_outputs:
+        line["outputs"] = write_outputs(args.dump_outputs, outputs, N, M, D)
     line.update(extra)
     print(json.dumps(line))
     _leave(world)
@@ -883,7 +933,14 @@ def main():
     ap.add_argument("--workload", default=None, choices=sorted(WORKLOADS))
     ap.add_argument("--precision", default="tf32", choices=["tf32", "fp32", "fp32_simt", "fp32_split", "f16"])
     ap.add_argument("--variant", default="softmax", choices=["softmax", "contrast"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write loss, dw, db and dE of the last one as DIR/<name>.npy (float32; "
+                         "dE rows sampled to keep the total under 64 MB, their indices in dE_rows.npy)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or os.environ.get("GE2E_BENCH_SHARDED_EAGER") == "1"):
+        ap.error("--dump-outputs writes the outputs of the CUDA-graph timed path of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)
