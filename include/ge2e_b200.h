@@ -58,7 +58,9 @@ enum ge2e_variant { GE2E_SOFTMAX = 0, GE2E_CONTRAST = 1 }; /* paper eq. (6) / eq
  *            softmax probabilities are normalised by a forward launch before the step kernel cuts them into
  *            planes.  Softmax variant, D = 128 or 256, shapes of the tensor-core path only; unlike GE2E_TF32
  *            this is a demand: an uncovered (shape, variant) returns GE2E_ERR_UNSUPPORTED -- ask
- *            ge2e_b200_path() first and fall back to GE2E_FP32. */
+ *            ge2e_b200_path() first and fall back to GE2E_FP32.  The planes are written by kernels that read E
+ *            16 bytes at a time: E (and dE) must be 16-byte aligned, else GE2E_ERR_UNSUPPORTED (copy an E that
+ *            sits at an odd offset of its allocation into fresh storage first). */
 /* GE2E_F16:  the hi plane of GE2E_FP32_SPLIT alone: fp16 operands carry the same 11-bit mantissa as TF32 (the
  *            stated tolerance stays 2e-3) at twice its MMA rate, one MMA per product; same kernels, same
  *            row-closing order and the same shape rules as GE2E_FP32_SPLIT (a demand, too).  It pays where the MMAs
@@ -75,8 +77,15 @@ unsigned long long ge2e_b200_launch_count(void);
  * fp16 planes (GE2E_FP32_SPLIT), 3 = tcgen05 one fp16 plane (GE2E_F16); the last two answer
  * GE2E_ERR_UNSUPPORTED when the shape / variant is not covered.
  * GE2E_TF32 is a permission, not a demand: shapes the tensor-core path does not cover run on
- * the (more accurate) SIMT kernels.  Negative = bad variant / precision. */
+ * the (more accurate) SIMT kernels.  Negative = bad variant / precision.  The answer depends on the shape
+ * only: the plane precisions (2, 3) also need a 16-byte-aligned E (see GE2E_FP32_SPLIT). */
 int ge2e_b200_path(int n_local, int n_total, int M, int D, int variant, int precision);
+/* Largest M (utterances per speaker) whose backward runs at embedding width D, on every path and alignment;
+ * 0 for an unsupported D.  The backward's last stage keeps a speaker's 2 M + 2 rows in 200 KB of shared memory:
+ * 199 at D = 128, 99 at D = 256, 49 at D = 512, 24 at D = 1024.  ge2e_b200_forward_backward and
+ * ge2e_b200_backward refuse a larger M with GE2E_ERR_UNSUPPORTED before launching anything; a forward alone
+ * may still run such a shape.  Host only, no GPU needed. */
+int ge2e_b200_max_utterances(int D);
 /* Debug: while device_buf is non-NULL the tensor-core kernels run an instrumented instantiation that
  * stamps %globaltimer at its pipeline events into device_buf[grid][3 roles (TMA, MMA, epilogue)][64];
  * NULL switches it off.  kernel: -1 = all, 0 = forward-rows kernel, 1 = step kernel; | 0x100 = also one

@@ -23,8 +23,12 @@ def _unit(x):
 
 
 def _unit_bwd(dxh, xh, n):
+    """F.cosine_similarity's gradient of x / max(|x|, delta): clamped value, unclamped derivative x / |x|
+    (see ge2e_oracle._unit_bwd): (dxh - xh (xh . dxh) s) / max(|x|, delta), s = max(|x|, delta) / |x|, 0 at x = 0."""
     proj = (xh * dxh).sum(-1, keepdim=True)
-    return torch.where(n >= COS_DELTA, (dxh - xh * proj) / n.clamp_min(COS_DELTA), dxh / COS_DELTA)
+    nc = n.clamp_min(COS_DELTA)
+    s = torch.where(n > 0, nc / torch.where(n > 0, n, torch.ones_like(n)), torch.zeros_like(n))
+    return (dxh - xh * (proj * s)) / nc
 
 
 def forward_backward(E, w=10.0, b=-5.0, eps=1e-6, variant="softmax", g=1.0, chunk=8192):

@@ -32,6 +32,18 @@ def resolve_precision(name: str, n_local: int, n_total: int, M: int, D: int, var
         return TF32           # shapes the fp16-operand kernels do not cover: the TF32 permission
     return PRECISIONS[name]
 
+def check_backward_shape(M: int, D: int) -> None:
+    """ValueError (before anything is launched) for an M whose backward the kernels cannot run at width D."""
+    m = lib().ge2e_b200_max_utterances(D)
+    if M > m:
+        raise ValueError(f"the GE2E backward supports at most {m} utterances per speaker at D = {D} (got M = {M}); "
+                         "its last stage keeps a speaker's 2 M + 2 rows in 200 KB of shared memory")
+
+
+def planes_need_copy(ptr: int, precision: int) -> bool:
+    """The fp16-plane precisions read E 16 bytes at a time: an E at an odd offset of its allocation is copied."""
+    return precision in (FP32_SPLIT, F16) and ptr % 16 != 0
+
 # name -> (restype, argtypes); kept in the order of include/ge2e_b200.h
 PROTOTYPES = {
     "ge2e_b200_version": (C.c_int, []),
@@ -39,6 +51,7 @@ PROTOTYPES = {
     "ge2e_b200_last_cuda_error": (C.c_int, []),
     "ge2e_b200_launch_count": (C.c_ulonglong, []),
     "ge2e_b200_path": (C.c_int, [C.c_int] * 6),
+    "ge2e_b200_max_utterances": (C.c_int, [C.c_int]),
     "ge2e_b200_debug_trace": (None, [C.c_void_p, C.c_int]),
     "ge2e_b200_debug_stamps": (None, [C.c_void_p]),
     "ge2e_b200_debug_hybrid": (None, [C.c_int]),

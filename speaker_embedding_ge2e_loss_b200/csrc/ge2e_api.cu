@@ -89,6 +89,8 @@ int ge2e_b200_path(int n_local, int n_total, int M, int D, int variant, int prec
   return on_tc(n_local, n_total, M, D, variant, precision) ? 1 : 0;
 }
 
+int ge2e_b200_max_utterances(int D) { return finalize_max_rows(D); }
+
 int ge2e_b200_check_device(void) {
   int dev = 0, major = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return GE2E_ERR_DEVICE;
@@ -327,6 +329,7 @@ int ge2e_b200_backward_indexed(const float* E, const int32_t* row_index, const f
                                float* dE_hat, float* dC_hat, float* accum, float* dE, void* workspace,
                                size_t workspace_bytes, ge2e_stream_t stream) {
   if (!accum) return GE2E_ERR_ARGUMENT;
+  if (M > finalize_max_rows(D)) return GE2E_ERR_UNSUPPORTED;     // before the rows kernels run
   // row_scale is meaningful only where the forward produced it
   const float* scale = tc_softmax_step(N, N, M, D, variant, precision) ? row_scale : nullptr;
   int rc = ge2e_b200_bwd_rows(e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, scale, N, N, 0, M, D, w, b, eps,
@@ -459,6 +462,8 @@ int ge2e_b200_forward_backward(const float* E, const int32_t* row_index, int N, 
   int rc = check_shape(N, N, 0, M, D);
   if (rc != GE2E_OK) return rc;
   if ((rc = check_enum(variant, precision)) != GE2E_OK) return rc;
+  // refused before any launch: never a forward that ran and a finalize that cannot
+  if (M > finalize_max_rows(D)) return GE2E_ERR_UNSUPPORTED;
   if (use_small_step(N, M, D, variant, precision)) {
     if (!workspace || workspace_bytes < small_step_workspace_bytes(N, M, D)) return GE2E_ERR_WORKSPACE;
     if (variant == GE2E_CONTRAST && !row_kstar) return GE2E_ERR_ARGUMENT;

@@ -37,6 +37,16 @@ void count_launch(int n = 1);
     GE2E_CUDA_TRY(cudaGetLastError());         \
   } while (0)
 
+// Backward of x -> x_hat = x / max(|x|, delta) as F.cosine_similarity differentiates it: the norm's VALUE is
+// clamped but its derivative x / |x| is kept, so
+//   dx = (dx_hat - x_hat (x_hat . dx_hat) s) / max(|x|, delta),   s = max(|x|, delta) / |x|
+// s = 1 above the clamp (the usual Jacobian), delta / |x| below it, 0 at x = 0 (where x_hat = 0).  Callers
+// scale their projection x_hat . dx_hat by s.  Below the clamp n is 0 or a normal float (n^2 would underflow
+// first), so the approximate division is safe there and keeps the IEEE division's slow path out of the kernels.
+__device__ __forceinline__ float clamp_proj_scale(float n) {
+  return n >= kCosDelta ? 1.f : (n > 0.f ? __fdividef(kCosDelta, n) : 0.f);
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -134,6 +144,8 @@ int simt_fwd_rows(const RowsArgs& a, float* row_stat, int32_t* row_kstar, float*
 int simt_bwd_rows(const RowsArgs& a, const float* row_stat, const int32_t* row_kstar,
                   const float* row_aux, const float* grad_out, float* dE_hat, float* dC_hat_partial,
                   float* dwdb_accum, cudaStream_t st);
+// largest M whose backward finalize runs at width D (0: D unsupported); see ge2e_b200_max_utterances
+int finalize_max_rows(int D);
 int simt_bwd_finalize(const float* E, const int32_t* row_index, const float* dE_hat, const float* dC_hat_local,
                       const float* cos_diag, const float* row_stat, const float* row_aux,
                       const float* row_scale /* nullable: dE_hat row r is g * row_scale[r] * dE_hat[r] */,

@@ -741,7 +741,7 @@ __device__ __forceinline__ void finalize_body(const float* __restrict__ E, const
   }
   __syncthreads();
 
-  // centroid Jacobian: dc = (dC_hat - c_hat (c_hat . dC_hat)) / |c|   (or dC_hat / delta)
+  // centroid Jacobian: dc = (dC_hat - c_hat (c_hat . dC_hat) s) / max(|c|, delta)   (clamp_proj_scale)
   const float fm = (float)M;
   {
     float n2 = 0.f, pr = 0.f;
@@ -755,15 +755,15 @@ __device__ __forceinline__ void finalize_body(const float* __restrict__ E, const
     if (tid == 0) { s_bc[0] = n2t; s_bc[1] = prt; }
     __syncthreads();
     const float nc = sqrtf(s_bc[0]);
-    const bool ok = nc >= kCosDelta;
     const float inv = 1.f / fmaxf(nc, kCosDelta);
-    const float proj = s_bc[1] * inv;            // c_hat . dC_hat
+    float proj = s_bc[1] * inv;                  // c_hat . dC_hat
+    if (nc < kCosDelta) proj *= clamp_proj_scale(nc);
     for (int d = tid; d < Dp; d += kThreads) {
       float v = 0.f;
       if (d < D) {
         const float dch = REUSE_E ? __ldcg(dC_hat + (size_t)j * D + d) : dC_hat[(size_t)j * D + d];
         const float ch = (sS[d] / fm) * inv;
-        v = (ok ? (dch - ch * proj) * inv : dch * inv) / fm;
+        v = (dch - ch * proj) * inv / fm;
       }
       sB[d] = v;
     }
@@ -787,7 +787,6 @@ __device__ __forceinline__ void finalize_body(const float* __restrict__ E, const
     }
     ne2 = warp_sum(ne2); nu2 = warp_sum(nu2); eu = warp_sum(eu); eg = warp_sum(eg) * gsc;
     const float ne = sqrtf(ne2), nu = sqrtf(nu2);
-    const bool ok_e = ne >= kCosDelta, ok_u = nu >= kCosDelta;
     const float inv_ne = 1.f / fmaxf(ne, kCosDelta), inv_nu = 1.f / fmaxf(nu, kCosDelta);
     const float cdv = eu * inv_ne * inv_nu;       // e_hat . u_hat (== cos_diag)
     // diagonal element of w*G
@@ -801,8 +800,10 @@ __device__ __forceinline__ void finalize_body(const float* __restrict__ E, const
     }
     const float dd = w * Gd;
     // d e_hat = dE_hat_offdiag + dd * u_hat ;  d u_hat = dd * e_hat
-    const float proj_e = eg * inv_ne + dd * cdv;  // e_hat . d e_hat
-    const float proj_u = dd * cdv;                // u_hat . d u_hat
+    float proj_e = eg * inv_ne + dd * cdv;        // e_hat . d e_hat
+    float proj_u = dd * cdv;                      // u_hat . d u_hat
+    if (ne < kCosDelta) proj_e *= clamp_proj_scale(ne);   // warp-uniform, rare
+    if (nu < kCosDelta) proj_u *= clamp_proj_scale(nu);
     for (int d = lane << 2; d < Dp; d += 128) {
       const float4 e = *reinterpret_cast<const float4*>(&sE[(size_t)i * Dp + d]);
       const float4 s = *reinterpret_cast<const float4*>(&sS[d]);
@@ -815,8 +816,8 @@ __device__ __forceinline__ void finalize_body(const float* __restrict__ E, const
         const float uh = ((sv[t] - ev[t]) / m1) * inv_nu;
         const float deh = gg[t] * gsc + dd * uh;
         const float duh = dd * eh;
-        de[t] = ok_e ? (deh - eh * proj_e) * inv_ne : deh * inv_ne;
-        du[t] = ok_u ? (duh - uh * proj_u) * inv_nu : duh * inv_nu;
+        de[t] = (deh - eh * proj_e) * inv_ne;
+        du[t] = (duh - uh * proj_u) * inv_nu;
       }
       // each (i, d) slot is read and then overwritten by the same single lane: no cross-lane hazard
       // (and no __syncwarp here: for D < 128 only some lanes enter this loop)
@@ -901,7 +902,7 @@ finalize_warp_kernel(const float* __restrict__ E, const float* __restrict__ dE_h
       }
   }
   const float inv_m = 1.f / (float)M, inv_m1 = 1.f / (float)(M - 1);
-  // centroid Jacobian: bc = dc_j / M with dc = (dC_hat - c_hat (c_hat . dC_hat)) / |c|  (or dC_hat / delta)
+  // centroid Jacobian: bc = dc_j / M with dc = (dC_hat - c_hat (c_hat . dC_hat) s) / max(|c|, delta)  (clamp_proj_scale)
   float4 bc[KCH];
   {
     float4 dch[KCH];
@@ -914,11 +915,11 @@ finalize_warp_kernel(const float* __restrict__ E, const float* __restrict__ dE_h
     }
     ss = warp_sum(ss); pr = warp_sum(pr);
     const float nc = sqrtf(ss) * inv_m;
-    const bool ok = nc >= kCosDelta;
     const float inv = 1.f / fmaxf(nc, kCosDelta);
-    const float proj = (pr * inv_m) * inv;          // c_hat . dC_hat
+    float proj = (pr * inv_m) * inv;                // c_hat . dC_hat
+    if (nc < kCosDelta) proj *= clamp_proj_scale(nc);   // warp-uniform, rare
     const float k1 = inv * inv_m;                   // dC_hat coefficient
-    const float k2 = ok ? proj * inv * inv * inv_m * inv_m : 0.f;   // coefficient of s (c_hat = s inv / M)
+    const float k2 = proj * inv * inv * inv_m * inv_m;              // coefficient of s (c_hat = s inv / M)
 #pragma unroll
     for (int c = 0; c < KCH; ++c) {
       bc[c].x = dch[c].x * k1 - s[c].x * k2; bc[c].y = dch[c].y * k1 - s[c].y * k2;
@@ -961,7 +962,6 @@ finalize_warp_kernel(const float* __restrict__ E, const float* __restrict__ dE_h
       if (i0 + r < M) {
         const int row = j * M + i0 + r;
         const float ne = sqrtf(ne2[r]), nu = sqrtf(nd2[r]) * inv_m1;
-        const bool ok_e = ne >= kCosDelta, ok_u = nu >= kCosDelta;
         const float inv_ne = 1.f / fmaxf(ne, kCosDelta), inv_nu = 1.f / fmaxf(nu, kCosDelta);
         const float cdv = (ed[r] * inv_m1) * inv_ne * inv_nu;       // e_hat . u_hat
         float Gd;                                                   // diagonal element of G
@@ -973,16 +973,18 @@ finalize_warp_kernel(const float* __restrict__ E, const float* __restrict__ dE_h
         }
         const float dd = w * Gd;
         const float gsc = row_scale != nullptr ? g * __ldcg(row_scale + row) : 1.f;   // un-normalised dE_hat rows
-        const float proj_e = eg[r] * gsc * inv_ne + dd * cdv;       // e_hat . d e_hat
-        const float proj_u = dd * cdv;                              // u_hat . d u_hat
-        // d e_hat = gv + dd u_hat, d u_hat = dd e_hat; Jacobians of the two normalisations:
-        //   de = (deh - e_hat proj_e) / |e|  ->  gv inv_ne + d (dd inv_nu inv_m1 inv_ne) - e (proj_e inv_ne^2)
-        //   du = (duh - u_hat proj_u) / |u|  ->  e (dd inv_ne inv_nu) - d (proj_u inv_nu^2 inv_m1)
+        float proj_e = eg[r] * gsc * inv_ne + dd * cdv;             // e_hat . d e_hat
+        float proj_u = dd * cdv;                                    // u_hat . d u_hat
+        if (ne < kCosDelta) proj_e *= clamp_proj_scale(ne);         // warp-uniform, rare
+        if (nu < kCosDelta) proj_u *= clamp_proj_scale(nu);
+        // d e_hat = gv + dd u_hat, d u_hat = dd e_hat; Jacobians of the two normalisations (inv_x = 1 / max(|x|, delta)):
+        //   de = (deh - e_hat proj_e) inv_ne  ->  gv inv_ne + d (dd inv_nu inv_m1 inv_ne) - e (proj_e inv_ne^2)
+        //   du = (duh - u_hat proj_u) inv_nu  ->  e (dd inv_ne inv_nu) - d (proj_u inv_nu^2 inv_m1)
         const float r_ag = inv_ne * gsc;
         const float r_ad = dd * inv_nu * inv_m1 * inv_ne;
-        const float r_ae = ok_e ? -proj_e * inv_ne * inv_ne : 0.f;
+        const float r_ae = -proj_e * inv_ne * inv_ne;
         const float r_be = dd * inv_ne * inv_nu;
-        const float r_bd = ok_u ? -proj_u * inv_nu * inv_nu * inv_m1 : 0.f;
+        const float r_bd = -proj_u * inv_nu * inv_nu * inv_m1;
         if (lane == i0 + r) { a_g = r_ag; a_e = r_ae; a_d = r_ad; b_e = r_be; b_d = r_bd; }
 #pragma unroll
         for (int c = 0; c < KCH; ++c) {
@@ -1108,7 +1110,7 @@ finalize_reg_kernel(const float* __restrict__ E, const float* __restrict__ dE_ha
     t_ed = reduce16_transposed(q, lane);
   }
   const float inv_m = 1.f / (float)M, inv_m1 = 1.f / (float)(M - 1);
-  // centroid Jacobian: bc = dc_j / M with dc = (dC_hat - c_hat (c_hat . dC_hat)) / |c|  (or dC_hat / delta)
+  // centroid Jacobian: bc = dc_j / M with dc = (dC_hat - c_hat (c_hat . dC_hat) s) / max(|c|, delta)  (clamp_proj_scale)
   float4 bc[KCH];
   {
     float4 dch[KCH];
@@ -1121,11 +1123,11 @@ finalize_reg_kernel(const float* __restrict__ E, const float* __restrict__ dE_ha
     }
     ss = warp_sum(ss); pr = warp_sum(pr);
     const float nc = sqrtf(ss) * inv_m;
-    const bool ok = nc >= kCosDelta;
     const float inv = 1.f / fmaxf(nc, kCosDelta);
-    const float proj = (pr * inv_m) * inv;          // c_hat . dC_hat
+    float proj = (pr * inv_m) * inv;                // c_hat . dC_hat
+    if (nc < kCosDelta) proj *= clamp_proj_scale(nc);   // warp-uniform, rare
     const float k1 = inv * inv_m;
-    const float k2 = ok ? proj * inv * inv * inv_m * inv_m : 0.f;
+    const float k2 = proj * inv * inv * inv_m * inv_m;
 #pragma unroll
     for (int c = 0; c < KCH; ++c) {
       bc[c].x = dch[c].x * k1 - s[c].x * k2; bc[c].y = dch[c].y * k1 - s[c].y * k2;
@@ -1138,7 +1140,6 @@ finalize_reg_kernel(const float* __restrict__ E, const float* __restrict__ dE_ha
   {
     const int row = j * M + min(my_row, M - 1);
     const float ne = sqrtf(t_ne2), nu = sqrtf(t_nd2) * inv_m1;
-    const bool ok_e = ne >= kCosDelta, ok_u = nu >= kCosDelta;
     const float inv_ne = 1.f / fmaxf(ne, kCosDelta), inv_nu = 1.f / fmaxf(nu, kCosDelta);
     const float cdv = (t_ed * inv_m1) * inv_ne * inv_nu;          // e_hat . u_hat
     float Gd;                                                     // diagonal element of G
@@ -1154,9 +1155,14 @@ finalize_reg_kernel(const float* __restrict__ E, const float* __restrict__ dE_ha
     const float proj_u = dd * cdv;                                // u_hat . d u_hat
     a_g = inv_ne * gsc;
     a_d = dd * inv_nu * inv_m1 * inv_ne;
-    a_e = ok_e ? -proj_e * inv_ne * inv_ne : 0.f;
+    a_e = -proj_e * inv_ne * inv_ne;
     b_e = dd * inv_ne * inv_nu;
-    b_d = ok_u ? -proj_u * inv_nu * inv_nu * inv_m1 : 0.f;
+    b_d = -proj_u * inv_nu * inv_nu * inv_m1;
+    // rows at or below the clamp (rare; lanes past row M - 1 hold no row): projections scaled by clamp_proj_scale
+    if (__any_sync(0xffffffffu, my_row < M && (ne < kCosDelta || nu < kCosDelta))) {
+      a_e *= clamp_proj_scale(ne);
+      b_d *= clamp_proj_scale(nu);
+    }
   }
   float4 sd[KCH];
 #pragma unroll
@@ -1308,6 +1314,17 @@ int rows_per_cta(int D) { return kWarps * (D <= 256 ? 4 : (D <= 512 ? 2 : 1)); }
 // ------------------------------------------------------------------------------------------
 // launchers
 // ------------------------------------------------------------------------------------------
+// The generic prep / finalize kernels hold a speaker's rows in shared memory: (M + 1) and (2 M + 2) rows of Dp
+// floats.  The warp kernels that take over for D = 128 / 256 / 512 with aligned rows cover M <= 32 in finalize,
+// which is inside this bound at every D they serve, so the bound is the backward's envelope.
+constexpr size_t kGenericSmemCap = 200 * 1024;
+
+int finalize_max_rows(int D) {
+  if (D < 1 || D > 1024) return 0;
+  const size_t row = (size_t)((D + 3) & ~3) * sizeof(float);
+  return (int)(kGenericSmemCap / row / 2) - 1;
+}
+
 bool warp_path_ok(int D, std::initializer_list<const void*> ptrs) {
   if (D != 128 && D != 256 && D != 512) return false;
   for (const void* q : ptrs)
@@ -1373,7 +1390,7 @@ int simt_prep(const float* E, const int32_t* row_index, int n_local, int M, int 
   if (prec >= 2) return GE2E_ERR_UNSUPPORTED;     // the fp16 planes are written by the warp kernels only
   const int Dp = (D + 3) & ~3;
   const size_t smem = (size_t)(M + 1) * Dp * sizeof(float);
-  if (smem > 200 * 1024) return GE2E_ERR_UNSUPPORTED;
+  if (smem > kGenericSmemCap) return GE2E_ERR_UNSUPPORTED;
   if (round_tf32_) {
     int rc = set_smem(prep_kernel<true>, smem);
     if (rc != GE2E_OK) return rc;
@@ -1453,8 +1470,8 @@ int simt_bwd_finalize(const float* E, const int32_t* row_index, const float* dE_
     return GE2E_OK;
   }
   const int Dp = (D + 3) & ~3;
+  if (M > finalize_max_rows(D)) return GE2E_ERR_UNSUPPORTED;
   const size_t smem = (size_t)(2 * M + 2) * Dp * sizeof(float);
-  if (smem > 200 * 1024) return GE2E_ERR_UNSUPPORTED;
   int rc = set_smem(finalize_kernel, smem);
   if (rc != GE2E_OK) return rc;
   finalize_kernel<<<n_local, kThreads, smem, st>>>(E, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux, row_scale, M, D,
@@ -1549,7 +1566,7 @@ small_step_kernel(const SmallParams p) {
   __shared__ float s_cd[32];
   __shared__ __align__(8) unsigned long long s_bar;   // bulk-copy completion (stage 2 operands)
   __shared__ float s_ine[16], s_inu[16], s_aux[16];   // fast path: 1/|e|, 1/|u|, 1 - p_jj per row of the speaker
-  __shared__ int s_ok[16];                            // fast path: bit 0 |e| >= delta, bit 1 |u| >= delta
+  __shared__ float s_pe[16], s_pu[16];                // fast path: clamp_proj_scale of |e|, |u|
   constexpr int R4 = MR / 4;                          // rows per thread where the block splits into 4 row groups
   const int j = blockIdx.x, N = gridDim.x, M = p.M, D = p.D, Dp = p.Dp;
   const int Np = (N + 3) & ~3;
@@ -1651,7 +1668,7 @@ small_step_kernel(const SmallParams p) {
       if (hl == 0) {
         s_cd[hw] = cosd; p.cos_diag[(size_t)j * M + hw] = cosd;
         s_ine[hw] = inv_ne; s_inu[hw] = inv_nu;
-        s_ok[hw] = (ne >= kCosDelta ? 1 : 0) | (nu >= kCosDelta ? 2 : 0);
+        s_pe[hw] = clamp_proj_scale(ne); s_pu[hw] = clamp_proj_scale(nu);
       }
     }
   } else {
@@ -1948,7 +1965,6 @@ small_step_kernel(const SmallParams p) {
         for (int o = 8; o > 0; o >>= 1) eg += __shfl_xor_sync(0xffffffffu, eg, o);
         if (act) {
           const float inv_ne = s_ine[hw], inv_nu = s_inu[hw], cdv = s_cd[hw];
-          const bool ok_e = (s_ok[hw] & 1) != 0, ok_u = (s_ok[hw] & 2) != 0;
           float Gd;                                      // diagonal element of G
           if (VARIANT == GE2E_SOFTMAX) {
             Gd = -g * s_aux[hw];                         // g (p_jj - 1), accumulated off-diagonal in stage 2
@@ -1957,8 +1973,8 @@ small_step_kernel(const SmallParams p) {
             Gd = -g * sp * (1.f - sp);
           }
           const float dd = w * Gd;
-          const float proj_e = eg * inv_ne + dd * cdv;   // e_hat . d e_hat
-          const float proj_u = dd * cdv;                 // u_hat . d u_hat
+          const float proj_e = (eg * inv_ne + dd * cdv) * s_pe[hw];   // (e_hat . d e_hat) s_e
+          const float proj_u = (dd * cdv) * s_pu[hw];                 // (u_hat . d u_hat) s_u
           for (int c4 = hl; c4 < ncol4; c4 += 16) {
             const float4 e = reinterpret_cast<const float4*>(fE + (size_t)hw * Dp)[c4];
             const float4 sv = reinterpret_cast<const float4*>(fS)[c4];
@@ -1971,8 +1987,8 @@ small_step_kernel(const SmallParams p) {
               const float uh = ((ss[t] - ev[t]) * inv_m1) * inv_nu;
               const float deh = gg[t] + dd * uh;
               const float duh = dd * eh;
-              de[t] = ok_e ? (deh - eh * proj_e) * inv_ne : deh * inv_ne;
-              du[t] = ok_u ? (duh - uh * proj_u) * inv_nu : duh * inv_nu;
+              de[t] = (deh - eh * proj_e) * inv_ne;
+              du[t] = (duh - uh * proj_u) * inv_nu;
             }
             // each slot is read and then overwritten by the same lane
             reinterpret_cast<float4*>(fU + (size_t)hw * Dp)[c4] = make_float4(du[0], du[1], du[2], du[3]);
@@ -2033,7 +2049,7 @@ small_step_kernel(const SmallParams p) {
   GE2E_SMALL_STAMP(9);
   if (p.stop == 7) break;
   if (fast) {
-    // centroid Jacobian: d c = (dC_hat - c_hat (c_hat . dC_hat)) / |c|   (or dC_hat / delta), kept as d c / M
+    // centroid Jacobian: d c = (dC_hat - c_hat (c_hat . dC_hat) s) / max(|c|, delta)  (clamp_proj_scale), kept as d c / M
     const float dch = tid < D ? __ldcg(p.dC_hat + (size_t)j * D + tid) : 0.f;      // assembled at the L2 by all CTAs
     float prp = warp_sum(c_mine * dch);
     if (lane == 0) red[wid] = prp;
@@ -2044,8 +2060,8 @@ small_step_kernel(const SmallParams p) {
     if (tid < D) {
       const float nc = sqrtf(c_norm2);
       const float inv = 1.f / fmaxf(nc, kCosDelta);
-      const float proj = pr * inv;                   // c_hat . dC_hat
-      fB[tid] = (nc >= kCosDelta ? (dch - (c_mine * inv) * proj) * inv : dch * inv) / fm;
+      const float proj = pr * inv * clamp_proj_scale(nc);   // (c_hat . dC_hat) s
+      fB[tid] = (dch - (c_mine * inv) * proj) * inv / fm;
     }
     __syncthreads();
     for (int i = wid; i < M; i += kWarps) {           // fan-out of d c and of the leave-one-out centroids (s3:105-111)

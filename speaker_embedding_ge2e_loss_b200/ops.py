@@ -124,6 +124,8 @@ def _fwd_impl(E: Tensor, w: Tensor, b: Tensor, eps: float, variant: int, precisi
     are 1-element placeholders where the path does not use them."""
     _need_cuda(E, w, b)
     E, w, b = _f32c(E), _f32c(w), _f32c(b)
+    if _lib.planes_need_copy(E.data_ptr(), precision):
+        E = E.clone()
     if row_index is None:
         N, M, D = E.shape
     else:
@@ -180,6 +182,7 @@ def _bwd_impl(grad_out, E, w, b, e_hat, c_hat, cos_diag, row_stat, row_kstar, ro
     N, D = c_hat.shape
     U = e_hat.shape[0]
     M = U // N
+    _lib.check_backward_shape(M, D)
     dev = E.device
     with _on_device(dev):
         dE = torch.empty_like(E)
@@ -301,7 +304,7 @@ class _StepBufs:
 
 class _EagerPlan:
     __slots__ = ("N", "M", "D", "U", "variant", "precision", "device", "dev_index", "path", "fused", "ws_bytes", "free",
-                 "one", "free_on")
+                 "one", "free_on", "planes", "bwd_ok")
 
     def __init__(self, dev, N, M, D, variant, precision):
         self.N, self.M, self.D, self.U = N, M, D, N * M
@@ -310,6 +313,8 @@ class _EagerPlan:
         h = lib()
         self.path = h.ge2e_b200_path(N, N, M, D, variant, precision)
         self.fused = variant == _lib.SOFTMAX and self.path in (1, 2, 3)
+        self.planes = precision in (_lib.FP32_SPLIT, _lib.F16)
+        self.bwd_ok = M <= h.ge2e_b200_max_utterances(D)
         # the whole-step entry point (single-kernel step for reference-sized batches) may need more than the stages
         self.ws_bytes = max(h.ge2e_b200_workspace_bytes(N, N, M, D, variant, precision),
                             h.ge2e_b200_step_workspace_bytes(N, M, D, variant, precision))
@@ -405,7 +410,11 @@ class _GE2EEager(torch.autograd.Function):
                 raise ValueError(f"{U_} rows do not split into {speakers} speakers")
         dev = E.device
         plan = _eager_plan(dev, N, M, D, variant, precision)
+        if plan.planes and E.data_ptr() % 16:
+            E = E.clone()           # the fp16-plane kernels read E 16 bytes at a time
         want_grad = ctx.needs_input_grad[0] or ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
+        if want_grad and not plan.bwd_ok:
+            _lib.check_backward_shape(M, D)
         if want_grad:
             # A loss somebody will differentiate (s4:196 + s4:200): the WHOLE step now, with upstream gradient 1 --
             # one C call: one kernel for reference-sized batches, prep + ONE persistent step kernel + finalize on
@@ -512,6 +521,8 @@ def prep(E: Tensor, c_hat_local_out: Tensor, precision: int):
     all-gather buffer).  Returns (e_hat, cos_diag, accum)."""
     _need_cuda(E, c_hat_local_out)
     E = _f32c(E)
+    if _lib.planes_need_copy(E.data_ptr(), precision):
+        E = E.clone()
     _same_f32c(c_hat_local_out)
     n, M, D = E.shape
     dev = E.device

@@ -50,6 +50,7 @@ class GE2EPlan:
         self._ws = torch.zeros(max(nbytes, 1), dtype=torch.uint8, device=dev)   # zero once: the kernels restore it
         # 1: the reference-sized batch runs fwd+bwd as ONE kernel (ge2e_b200_forward_backward)
         self.single_kernel = lib().ge2e_b200_step_launches(N, M, D, self.variant, self.precision) == 1
+        self._bwd_ok = M <= lib().ge2e_b200_max_utterances(D)
         self._ws_bytes = nbytes
         self.loss, self.dw, self.db = self._accum[0], self._accum[1], self._accum[2]
         self._graph = None
@@ -58,6 +59,12 @@ class GE2EPlan:
         """Enqueue fwd (+ bwd) on the current stream.  Results land in .loss/.dE/.dw/.db."""
         assert E.is_cuda and E.dtype == torch.float32 and E.is_contiguous() and tuple(E.shape) == (self.N, self.M, self.D)
         h, N, M, D = lib(), self.N, self.M, self.D
+        if _lib.planes_need_copy(E.data_ptr(), self.precision):
+            # a plan copies nothing behind the caller's back (its steps are captured into graphs)
+            raise ValueError("GE2EPlan: the fp16-plane precisions need a 16-byte-aligned E; this one sits at an "
+                             "offset of its storage -- pass E.clone(), or build the plan with precision='fp32_simt'")
+        if backward and not self._bwd_ok:
+            _lib.check_backward_shape(M, D)
         stream = torch.cuda.current_stream(self.device).cuda_stream
         ws = self._ws.data_ptr() if self._ws_bytes else None
         if backward:
@@ -129,6 +136,7 @@ class ShardedGE2EPlan:
         self.variant = _lib.VARIANTS[variant]
         self.eps = float(eps)
         self.device = torch.device(device if device is not None else "cuda")
+        _lib.check_backward_shape(M, D)
         with torch.cuda.device(self.device):
             self.precision = _lib.resolve_precision(precision, n_local, n_total, M, D, self.variant)
         U, dev, f32 = n_local * M, self.device, torch.float32

@@ -47,3 +47,18 @@ def test_span_offsets_reproduce_reference_batches(name):
     got = np.stack([flat[o:o + span] for o in off]).reshape(N * M, L, mels)
     assert got.dtype == np.float32 and np.array_equal(got, z[name + "_batch"])
     assert off.dtype == np.int64 and off.flags["C_CONTIGUOUS"] and (off % mels == 0).all()
+
+
+def test_backward_envelope_query_and_refusal():
+    """ge2e_b200_max_utterances (host only): the backward keeps 2 M + 2 rows of D floats (D rounded up to 4) in
+    200 KB of shared memory; the Python layer refuses a larger M with a ValueError that names the limit."""
+    from speaker_embedding_ge2e_loss_b200 import _lib
+    h = _lib.lib()
+    for D, m in [(128, 199), (256, 99), (512, 49), (768, 32), (1000, 24), (1023, 24), (1024, 24), (1, 6399)]:
+        assert h.ge2e_b200_max_utterances(D) == m
+        Dp = (D + 3) // 4 * 4
+        assert (2 * m + 2) * Dp * 4 <= 200 * 1024 < (2 * m + 4) * Dp * 4
+    assert h.ge2e_b200_max_utterances(0) == 0 and h.ge2e_b200_max_utterances(1025) == 0
+    _lib.check_backward_shape(99, 256)
+    with pytest.raises(ValueError, match="at most 99 utterances per speaker at D = 256"):
+        _lib.check_backward_shape(100, 256)
