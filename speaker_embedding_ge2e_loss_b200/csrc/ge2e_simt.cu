@@ -209,6 +209,7 @@ __device__ __forceinline__ void put4(float* base, size_t row, int D, int col, fl
 constexpr int kPrepWarps = 4;
 constexpr int kRowBatch = 4;   // rows in flight per lane (KCH float4 loads each)
 constexpr int kRegRows = 16;   // register-resident variants hold up to this many rows per speaker
+constexpr int kRegBlocksPerSM = 4;   // register-resident variants: <= 128 registers, 16 warps resident per SM
 
 template <int KCH, int PREC>
 __global__ void __launch_bounds__(kPrepWarps * 32)
@@ -304,12 +305,14 @@ prep_warp_kernel(const float* __restrict__ E, const int32_t* __restrict__ idx, i
 }
 
 // ------------------------------------------------------------------------------------------
-// K1 (register-resident variant, M <= 16): as prep_warp_kernel, but every row of the speaker is
-// loaded ONCE, all loads in flight together (16 KCH 16-byte loads per lane), and kept in
-// registers.  The per-row sums go through a transposing butterfly (reduce16_transposed): lane l
-// ends up with the totals of row rev4(l & 15), so the square roots / reciprocals of all rows are
-// evaluated once, lane-parallel, instead of row after row by the whole warp.  With ~7 warps per
-// SM the kernel time is the latency of one warp's dependency chain; this is what keeps it short.
+// K1 (register-resident variant, M <= 16, D = 128 W): W warps per speaker, warp w of the speaker
+// owning the columns [128 w, 128 w + 128), so a lane holds one float4 of every row.  Every row is
+// loaded ONCE, all loads in flight together, and kept in registers.  The per-row sums go through a
+// transposing butterfly (reduce16_transposed): lane l ends up with the warp's partial of row
+// rev4(l & 15); the W partials are added through shared memory (speaker_sum), so the square roots
+// / reciprocals of all rows are evaluated once, lane-parallel, instead of row after row.  At cfg3
+// there are a few warps per scheduler and the kernel time is the latency of one warp's dependency
+// chain; splitting the columns over W warps halves that chain's loads and arithmetic at D = 256.
 // ------------------------------------------------------------------------------------------
 __host__ __device__ constexpr int rev4(int i) {
   return ((i & 1) << 3) | ((i & 2) << 1) | ((i & 4) >> 1) | ((i & 8) >> 3);
@@ -328,73 +331,81 @@ __device__ __forceinline__ float reduce16_transposed(const float (&v)[16], int l
   return e + __shfl_xor_sync(0xffffffffu, e, 16);
 }
 
-template <int KCH, int RR, int PREC>
-__global__ void __launch_bounds__(kPrepWarps * 32)
+// Speaker totals of Q quantities from the partials of the speaker's W warps (warps W s ... W s + W - 1 of the
+// block).  Lane l's x[q] is either a per-row partial of row rev4(l & 15) (reduce16_transposed) or a per-speaker
+// scalar (the same in every lane); either way lanes l and l + 16 agree, so 16 slots per quantity carry it.  The
+// partials are added in warp order: every warp of the speaker gets the same bits.  One named barrier per speaker,
+// so a speaker whose warps returned early holds up nobody.  W = 1 is a no-op.
+template <int W, int Q>
+__device__ __forceinline__ void speaker_sum(float (&x)[Q], float (*xch)[Q][16], int wid, int lane) {
+  if (W == 1) return;
+  if (lane < 16) {
+#pragma unroll
+    for (int q = 0; q < Q; ++q) xch[wid][q][lane] = x[q];
+  }
+  asm volatile("bar.sync %0, %1;" ::"r"(1 + wid / W), "r"(W * 32) : "memory");
+  const int first = wid - wid % W;
+#pragma unroll
+  for (int q = 0; q < Q; ++q) {
+    float t = xch[first][q][lane & 15];
+#pragma unroll
+    for (int w = 1; w < W; ++w) t += xch[first + w][q][lane & 15];
+    x[q] = t;
+  }
+}
+
+template <int W, int RR, int PREC>
+__global__ void __launch_bounds__(kPrepWarps * 32, kRegBlocksPerSM)
 prep_reg_kernel(const float* __restrict__ E, const int32_t* __restrict__ idx, int n_local, int M,
                 float* __restrict__ e_hat, float* __restrict__ c_hat, float* __restrict__ cos_diag,
                 float* __restrict__ accum) {
-  constexpr int D = KCH * 128, R = RR;     // rows held in registers (M <= R <= 16)
+  constexpr int D = W * 128, R = RR;       // rows held in registers (M <= R <= 16)
   static_assert(R <= 16, "reduce16_transposed handles 16 rows");
+  static_assert(kPrepWarps % W == 0, "a block holds whole speakers");
+  __shared__ float xch[kPrepWarps][4][16];
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  const int j = blockIdx.x * kPrepWarps + wid;
+  const int j = blockIdx.x * (kPrepWarps / W) + wid / W;
+  const int col = 128 * (wid % W) + 4 * lane;     // this lane's four columns of every row
   pdl_wait();        // before touching memory: the previous step's kernels may still read what this one writes
   pdl_trigger();     // the forward tensor-core kernel may set itself up while this grid runs
   if (blockIdx.x == 0 && threadIdx.x < 4 && accum != nullptr) accum[threadIdx.x] = 0.f;
-  if (j >= n_local) return;
-  float4 v[R][KCH];
+  if (j >= n_local) return;     // all W warps of the speaker
+  float4 v[R];
 #pragma unroll
-  for (int i = 0; i < R; ++i) {
-    const float4* rp = (i < M) ? reinterpret_cast<const float4*>(E + phys_row(idx, (size_t)j * M + i) * D) + lane : nullptr;
+  for (int i = 0; i < R; ++i)
+    v[i] = (i < M) ? __ldg(reinterpret_cast<const float4*>(E + phys_row(idx, (size_t)j * M + i) * D + col))
+                   : make_float4(0.f, 0.f, 0.f, 0.f);
+  float4 s = v[0];
 #pragma unroll
-    for (int c = 0; c < KCH; ++c) v[i][c] = (i < M) ? __ldg(rp + c * 32) : make_float4(0.f, 0.f, 0.f, 0.f);
-  }
-  float4 s[KCH];
-#pragma unroll
-  for (int c = 0; c < KCH; ++c) {
-    s[c] = v[0][c];
-#pragma unroll
-    for (int i = 1; i < R; ++i) { s[c].x += v[i][c].x; s[c].y += v[i][c].y; s[c].z += v[i][c].z; s[c].w += v[i][c].w; }
-  }
+  for (int i = 1; i < R; ++i) { s.x += v[i].x; s.y += v[i].y; s.z += v[i].z; s.w += v[i].w; }
   const float inv_m = 1.f / (float)M, inv_m1 = 1.f / (float)(M - 1);
-  float ss = 0.f;
-#pragma unroll
-  for (int c = 0; c < KCH; ++c) ss += dot4(s[c], s[c]);
-  ss = warp_sum(ss);
-  const float sc = inv_m / fmaxf(sqrtf(ss) * inv_m, kCosDelta);       // s3:37 + normalisation
-#pragma unroll
-  for (int c = 0; c < KCH; ++c)
-    put4<PREC>(c_hat, j, D, 4 * lane + 128 * c,
-               make_float4(s[c].x * sc, s[c].y * sc, s[c].z * sc, s[c].w * sc));
-  // |e|^2, |s - e|^2, e.(s - e) of every row (u = (s - e) / (M - 1): s3:105-111)
+  // |e|^2, |s - e|^2, e.(s - e) of every row (u = (s - e) / (M - 1): s3:105-111), and |s|^2
   float ne2[16], nd2[16], ed[16];
 #pragma unroll
   for (int i = R; i < 16; ++i) { ne2[i] = 0.f; nd2[i] = 0.f; ed[i] = 0.f; }
 #pragma unroll
   for (int i = 0; i < R; ++i) {
-    ne2[i] = 0.f; nd2[i] = 0.f; ed[i] = 0.f;
-#pragma unroll
-    for (int c = 0; c < KCH; ++c) {
-      const float4 e = v[i][c];
-      const float4 d = make_float4(s[c].x - e.x, s[c].y - e.y, s[c].z - e.z, s[c].w - e.w);
-      ne2[i] += dot4(e, e); nd2[i] += dot4(d, d); ed[i] += dot4(e, d);
-    }
+    const float4 e = v[i];
+    const float4 d = make_float4(s.x - e.x, s.y - e.y, s.z - e.z, s.w - e.w);
+    ne2[i] = dot4(e, e); nd2[i] = dot4(d, d); ed[i] = dot4(e, d);
   }
-  const float t_ne2 = reduce16_transposed(ne2, lane), t_nd2 = reduce16_transposed(nd2, lane);
-  const float t_ed = reduce16_transposed(ed, lane);
+  float t[4] = {reduce16_transposed(ne2, lane), reduce16_transposed(nd2, lane), reduce16_transposed(ed, lane),
+                warp_sum(dot4(s, s))};
+  speaker_sum<W>(t, xch, wid, lane);
+  const float sc = inv_m / fmaxf(sqrtf(t[3]) * inv_m, kCosDelta);       // s3:37 + normalisation
+  put4<PREC>(c_hat, j, D, col, make_float4(s.x * sc, s.y * sc, s.z * sc, s.w * sc));
   const int my_row = rev4(lane & 15);
-  const float inv_ne = 1.f / fmaxf(sqrtf(t_ne2), kCosDelta);
-  const float inv_nu = 1.f / fmaxf(sqrtf(t_nd2) * inv_m1, kCosDelta);
-  if (lane < 16 && my_row < M) cos_diag[(size_t)j * M + my_row] = (t_ed * inv_m1) * inv_ne * inv_nu;   // s3:57
+  const float inv_ne = 1.f / fmaxf(sqrtf(t[0]), kCosDelta);
+  const float inv_nu = 1.f / fmaxf(sqrtf(t[1]) * inv_m1, kCosDelta);
+  if (wid % W == 0 && lane < 16 && my_row < M)
+    cos_diag[(size_t)j * M + my_row] = (t[2] * inv_m1) * inv_ne * inv_nu;   // s3:57
 #pragma unroll
   for (int i = 0; i < R; ++i) {
     if (i < M) {      // warp-uniform
       const float k = __shfl_sync(0xffffffffu, inv_ne, rev4(i));
-#pragma unroll
-      for (int c = 0; c < KCH; ++c) {
-        float4 e = v[i][c];
-        e.x *= k; e.y *= k; e.z *= k; e.w *= k;
-        put4<PREC>(e_hat, (size_t)j * M + i, D, 4 * lane + 128 * c, e);
-      }
+      float4 e = v[i];
+      e.x *= k; e.y *= k; e.z *= k; e.w *= k;
+      put4<PREC>(e_hat, (size_t)j * M + i, D, col, e);
     }
   }
 }
@@ -1022,135 +1033,104 @@ finalize_warp_kernel(const float* __restrict__ E, const float* __restrict__ dE_h
 }
 
 // ------------------------------------------------------------------------------------------
-// K4 (register-resident variant, M <= 16): the speaker's E rows are loaded once (before the
-// programmatic-launch wait: E is not produced by the preceding grids) and stay in registers;
-// dE_hat rows are read twice (L2 / L1 hits).  Row sums through reduce16_transposed, the per-row
-// Jacobian coefficients are computed lane-parallel (lane l owns row rev4(l & 15)) and broadcast.
+// K4 (register-resident variant, M <= 16, D = 128 W): W warps per speaker, split over the columns as
+// in prep_reg_kernel.  The speaker's E rows are loaded once (before the programmatic-launch wait: E
+// is not produced by the preceding grids) and stay in registers; everything the preceding grids
+// produced (dE_hat rows, the dC_hat row, the row scalars) is requested right after the wait, in one
+// batch; dE_hat rows are read twice (L2 / L1 hits).  Row sums through reduce16_transposed and
+// speaker_sum, the per-row Jacobian coefficients are computed lane-parallel (lane l owns row
+// rev4(l & 15)) and broadcast; the column sums (s, sum_i du_i) never leave the warp.
 //   de_i = a_g gv_i + a_e e_i + a_d d_i ,  du_i = b_e e_i + b_d d_i ,  d_i = s - e_i
 //   dE_i = de_i + dc_j / M + (sum_i' du_i' - du_i) / (M - 1)
 // ------------------------------------------------------------------------------------------
-template <int KCH, int RR>
-__global__ void __launch_bounds__(kPrepWarps * 32)
+template <int W, int RR>
+__global__ void __launch_bounds__(kPrepWarps * 32, kRegBlocksPerSM)
 finalize_reg_kernel(const float* __restrict__ E, const float* __restrict__ dE_hat,
                     const float* __restrict__ dC_hat, const float* __restrict__ cos_diag,
                     const float* __restrict__ row_aux, const float* __restrict__ row_scale, int n_local, int M,
                     const float* __restrict__ wp, const float* __restrict__ bp, float eps, int variant,
                     const float* __restrict__ gp, float* __restrict__ dE, const int32_t* __restrict__ idx) {
-  constexpr int D = KCH * 128, R = RR;     // rows held in registers (M <= R <= 16)
+  constexpr int D = W * 128, R = RR;       // rows held in registers (M <= R <= 16)
   static_assert(R <= 16, "reduce16_transposed handles 16 rows");
+  static_assert(kPrepWarps % W == 0, "a block holds whole speakers");
+  __shared__ float xch[kPrepWarps][6][16];
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  const int j = blockIdx.x * kPrepWarps + wid;
+  const int j = blockIdx.x * (kPrepWarps / W) + wid / W;
+  const int col = 128 * (wid % W) + 4 * lane;     // this lane's four columns of every row
   const bool active = j < n_local;
-  float4 v[R][KCH];
+  float4 v[R];
   // the row index is an input of the whole op as well (never written by the preceding grids)
 #pragma unroll
-  for (int i = 0; i < R; ++i) {
-    const bool in = active && i < M;
-    const float4* rp = in ? reinterpret_cast<const float4*>(E + phys_row(idx, (size_t)j * M + i) * D) + lane : nullptr;
+  for (int i = 0; i < R; ++i)
+    v[i] = (active && i < M) ? __ldg(reinterpret_cast<const float4*>(E + phys_row(idx, (size_t)j * M + i) * D + col))
+                             : make_float4(0.f, 0.f, 0.f, 0.f);
+  // what depends on E alone runs before the wait: the column sum s and the partial row sums |e|^2, |s - e|^2,
+  // e.(s - e) and |s|^2 (t[1..4]); e.dE_hat and s.dC_hat (t[0], t[5]) follow it
+  float4 s = v[0];
 #pragma unroll
-    for (int c = 0; c < KCH; ++c) v[i][c] = in ? __ldg(rp + c * 32) : make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int i = 1; i < R; ++i) { s.x += v[i].x; s.y += v[i].y; s.z += v[i].z; s.w += v[i].w; }
+  float t[6];
+  {
+    float ne2[16], nd2[16], ed[16];
+#pragma unroll
+    for (int i = R; i < 16; ++i) { ne2[i] = 0.f; nd2[i] = 0.f; ed[i] = 0.f; }
+#pragma unroll
+    for (int i = 0; i < R; ++i) {
+      const float4 e = v[i];
+      const float4 d = make_float4(s.x - e.x, s.y - e.y, s.z - e.z, s.w - e.w);
+      ne2[i] = dot4(e, e); nd2[i] = dot4(d, d); ed[i] = dot4(e, d);
+    }
+    t[1] = reduce16_transposed(ne2, lane); t[2] = reduce16_transposed(nd2, lane); t[3] = reduce16_transposed(ed, lane);
+    t[4] = warp_sum(dot4(s, s));
   }
   pdl_wait();        // launched with the PDL attribute: dE_hat / dC_hat come from the preceding grids
   pdl_trigger();     // the next step's prep may be scheduled (it waits for this grid before touching memory)
-  if (!active) return;
+  if (!active) return;     // all W warps of the speaker
   const float w = __ldg(wp), b = __ldg(bp), g = __ldg(gp);
-  const float4* Gj = reinterpret_cast<const float4*>(dE_hat + (size_t)j * M * D) + lane;
-  float4 s[KCH];
-#pragma unroll
-  for (int c = 0; c < KCH; ++c) {
-    s[c] = v[0][c];
-#pragma unroll
-    for (int i = 1; i < R; ++i) { s[c].x += v[i][c].x; s[c].y += v[i][c].y; s[c].z += v[i][c].z; s[c].w += v[i][c].w; }
-  }
-  // row sums, one quantity at a time (16 live partials instead of 64: the rows already hold 128 registers)
-  float t_ne2, t_nd2, t_ed, t_eg;
+  const int my_row = rev4(lane & 15);
+  const int row = j * M + min(my_row, M - 1);     // lanes past row M - 1 hold no row
+  const float4 dch = __ldcg(reinterpret_cast<const float4*>(dC_hat + (size_t)j * D + col));
+  const float aux = variant == GE2E_SOFTMAX ? __ldcg(row_aux + row) : __ldg(cos_diag + row);
+  const float gsc = row_scale != nullptr ? g * __ldcg(row_scale + row) : 1.f;   // un-normalised dE_hat rows
+  const float* Gj = dE_hat + (size_t)j * M * D + col;
   {
-    float q[16];
+    float eg[16];
 #pragma unroll
-    for (int i = R; i < 16; ++i) q[i] = 0.f;
+    for (int i = R; i < 16; ++i) eg[i] = 0.f;
 #pragma unroll
-    for (int i = 0; i < R; ++i) {
-      if (i == R / 2) asm volatile("" ::: "memory");   // two batches of dE_hat loads: bounds the registers in flight
-      q[i] = 0.f;
-#pragma unroll
-      for (int c = 0; c < KCH; ++c) {
-        const float4 gv = (i < M) ? __ldg(Gj + (size_t)i * (D / 4) + c * 32) : make_float4(0.f, 0.f, 0.f, 0.f);
-        q[i] += dot4(v[i][c], gv);
-      }
-    }
-    t_eg = reduce16_transposed(q, lane);
-#pragma unroll
-    for (int i = 0; i < R; ++i) {
-      q[i] = 0.f;
-#pragma unroll
-      for (int c = 0; c < KCH; ++c) q[i] += dot4(v[i][c], v[i][c]);
-    }
-    t_ne2 = reduce16_transposed(q, lane);
-#pragma unroll
-    for (int i = 0; i < R; ++i) {
-      q[i] = 0.f;
-#pragma unroll
-      for (int c = 0; c < KCH; ++c) {
-        const float4 e = v[i][c];
-        const float4 d = make_float4(s[c].x - e.x, s[c].y - e.y, s[c].z - e.z, s[c].w - e.w);
-        q[i] += dot4(d, d);
-      }
-    }
-    t_nd2 = reduce16_transposed(q, lane);
-#pragma unroll
-    for (int i = 0; i < R; ++i) {
-      q[i] = 0.f;
-#pragma unroll
-      for (int c = 0; c < KCH; ++c) {
-        const float4 e = v[i][c];
-        const float4 d = make_float4(s[c].x - e.x, s[c].y - e.y, s[c].z - e.z, s[c].w - e.w);
-        q[i] += dot4(e, d);
-      }
-    }
-    t_ed = reduce16_transposed(q, lane);
+    for (int i = 0; i < R; ++i)
+      eg[i] = dot4(v[i], (i < M) ? __ldg(reinterpret_cast<const float4*>(Gj + (size_t)i * D)) : make_float4(0.f, 0.f, 0.f, 0.f));
+    t[0] = reduce16_transposed(eg, lane);
+    t[5] = warp_sum(dot4(s, dch));
   }
+  speaker_sum<W>(t, xch, wid, lane);
+  const float t_eg = t[0], t_ne2 = t[1], t_nd2 = t[2], t_ed = t[3];
   const float inv_m = 1.f / (float)M, inv_m1 = 1.f / (float)(M - 1);
   // centroid Jacobian: bc = dc_j / M with dc = (dC_hat - c_hat (c_hat . dC_hat) s) / max(|c|, delta)  (clamp_proj_scale)
-  float4 bc[KCH];
+  float4 bc;
   {
-    float4 dch[KCH];
-    float ss = 0.f, pr = 0.f;
-#pragma unroll
-    for (int c = 0; c < KCH; ++c) {
-      dch[c] = __ldcg(reinterpret_cast<const float4*>(dC_hat + (size_t)j * D) + lane + c * 32);
-      ss += dot4(s[c], s[c]);
-      pr += dot4(s[c], dch[c]);
-    }
-    ss = warp_sum(ss); pr = warp_sum(pr);
-    const float nc = sqrtf(ss) * inv_m;
+    const float nc = sqrtf(t[4]) * inv_m;
     const float inv = 1.f / fmaxf(nc, kCosDelta);
-    float proj = (pr * inv_m) * inv;                // c_hat . dC_hat
+    float proj = (t[5] * inv_m) * inv;              // c_hat . dC_hat
     if (nc < kCosDelta) proj *= clamp_proj_scale(nc);   // warp-uniform, rare
     const float k1 = inv * inv_m;
     const float k2 = proj * inv * inv * inv_m * inv_m;
-#pragma unroll
-    for (int c = 0; c < KCH; ++c) {
-      bc[c].x = dch[c].x * k1 - s[c].x * k2; bc[c].y = dch[c].y * k1 - s[c].y * k2;
-      bc[c].z = dch[c].z * k1 - s[c].z * k2; bc[c].w = dch[c].w * k1 - s[c].w * k2;
-    }
+    bc = make_float4(dch.x * k1 - s.x * k2, dch.y * k1 - s.y * k2, dch.z * k1 - s.z * k2, dch.w * k1 - s.w * k2);
   }
   // this lane's row
-  const int my_row = rev4(lane & 15);
   float a_g, a_e, a_d, b_e, b_d;
   {
-    const int row = j * M + min(my_row, M - 1);
     const float ne = sqrtf(t_ne2), nu = sqrtf(t_nd2) * inv_m1;
     const float inv_ne = 1.f / fmaxf(ne, kCosDelta), inv_nu = 1.f / fmaxf(nu, kCosDelta);
     const float cdv = (t_ed * inv_m1) * inv_ne * inv_nu;          // e_hat . u_hat
     float Gd;                                                     // diagonal element of G
     if (variant == GE2E_SOFTMAX) {
-      Gd = -g * __ldcg(row_aux + row);                            // g (p_jj - 1)
+      Gd = -g * aux;                                              // g (p_jj - 1)
     } else {
-      const float sp = 1.f / (1.f + expf(-fmaf(w, __ldg(cos_diag + row) + eps, b)));
+      const float sp = 1.f / (1.f + expf(-fmaf(w, aux + eps, b)));
       Gd = -g * sp * (1.f - sp);
     }
     const float dd = w * Gd;
-    const float gsc = row_scale != nullptr ? g * __ldcg(row_scale + row) : 1.f;   // un-normalised dE_hat rows
     const float proj_e = t_eg * gsc * inv_ne + dd * cdv;          // e_hat . d e_hat
     const float proj_u = dd * cdv;                                // u_hat . d u_hat
     a_g = inv_ne * gsc;
@@ -1164,45 +1144,32 @@ finalize_reg_kernel(const float* __restrict__ E, const float* __restrict__ dE_ha
       b_d *= clamp_proj_scale(nu);
     }
   }
-  float4 sd[KCH];
-#pragma unroll
-  for (int c = 0; c < KCH; ++c) sd[c] = make_float4(0.f, 0.f, 0.f, 0.f);
+  float4 sd = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
   for (int i = 0; i < R; ++i) {
     if (i < M) {
       const float r_be = __shfl_sync(0xffffffffu, b_e, rev4(i)), r_bd = __shfl_sync(0xffffffffu, b_d, rev4(i));
-#pragma unroll
-      for (int c = 0; c < KCH; ++c) {
-        const float4 e = v[i][c];
-        sd[c].x += r_be * e.x + r_bd * (s[c].x - e.x); sd[c].y += r_be * e.y + r_bd * (s[c].y - e.y);
-        sd[c].z += r_be * e.z + r_bd * (s[c].z - e.z); sd[c].w += r_be * e.w + r_bd * (s[c].w - e.w);
-      }
+      const float4 e = v[i];
+      sd.x += r_be * e.x + r_bd * (s.x - e.x); sd.y += r_be * e.y + r_bd * (s.y - e.y);
+      sd.z += r_be * e.z + r_bd * (s.z - e.z); sd.w += r_be * e.w + r_bd * (s.w - e.w);
     }
   }
+  // dE_i = a_g gv_i + a_e e_i + a_d d_i + bc + (sd - b_e e_i - b_d d_i) / (M - 1), with d_i = s - e_i, is
+  //   k_g gv_i + k_e e_i + k_s s + base:  three coefficients per row instead of five
+  const float k_s = a_d - b_d * inv_m1;
+  const float k_e = a_e - b_e * inv_m1 - k_s;
+  const float4 base = make_float4(fmaf(sd.x, inv_m1, bc.x), fmaf(sd.y, inv_m1, bc.y), fmaf(sd.z, inv_m1, bc.z),
+                                  fmaf(sd.w, inv_m1, bc.w));
 #pragma unroll
   for (int i = 0; i < R; ++i) {
     if (i < M) {
-      float4* Oi = reinterpret_cast<float4*>(dE + phys_row(idx, (size_t)j * M + i) * D) + lane;
-      const float r_ag = __shfl_sync(0xffffffffu, a_g, rev4(i)), r_ae = __shfl_sync(0xffffffffu, a_e, rev4(i));
-      const float r_ad = __shfl_sync(0xffffffffu, a_d, rev4(i)), r_be = __shfl_sync(0xffffffffu, b_e, rev4(i));
-      const float r_bd = __shfl_sync(0xffffffffu, b_d, rev4(i));
-#pragma unroll
-      for (int c = 0; c < KCH; ++c) {
-        const float4 e = v[i][c];
-        const float4 gv = __ldg(Gj + (size_t)i * (D / 4) + c * 32);
-        const float ev[4] = {e.x, e.y, e.z, e.w}, gg[4] = {gv.x, gv.y, gv.z, gv.w};
-        const float sv[4] = {s[c].x, s[c].y, s[c].z, s[c].w}, sdv[4] = {sd[c].x, sd[c].y, sd[c].z, sd[c].w};
-        const float bv[4] = {bc[c].x, bc[c].y, bc[c].z, bc[c].w};
-        float o[4];
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-          const float d = sv[t] - ev[t];
-          const float de = r_ag * gg[t] + r_ae * ev[t] + r_ad * d;
-          const float du = r_be * ev[t] + r_bd * d;
-          o[t] = de + bv[t] + (sdv[t] - du) * inv_m1;
-        }
-        Oi[c * 32] = make_float4(o[0], o[1], o[2], o[3]);
-      }
+      const float r_g = __shfl_sync(0xffffffffu, a_g, rev4(i)), r_e = __shfl_sync(0xffffffffu, k_e, rev4(i));
+      const float r_s = __shfl_sync(0xffffffffu, k_s, rev4(i));
+      const float4 e = v[i];
+      const float4 gv = __ldg(reinterpret_cast<const float4*>(Gj + (size_t)i * D));
+      const float4 o = make_float4(r_g * gv.x + r_e * e.x + fmaf(r_s, s.x, base.x), r_g * gv.y + r_e * e.y + fmaf(r_s, s.y, base.y),
+                                   r_g * gv.z + r_e * e.z + fmaf(r_s, s.z, base.z), r_g * gv.w + r_e * e.w + fmaf(r_s, s.w, base.w));
+      *reinterpret_cast<float4*>(dE + phys_row(idx, (size_t)j * M + i) * D + col) = o;
     }
   }
 }
@@ -1337,13 +1304,14 @@ void launch_prep_warp(const float* E, const int32_t* idx, int n_local, int M, in
                       float* cos_diag, float* accum, cudaStream_t st) {
   const int grid = (n_local + kPrepWarps - 1) / kPrepWarps;
   if (KCH <= 2 && M <= kRegRows) {
-    constexpr int K2 = KCH <= 2 ? KCH : 1;    // the register-resident variant is only instantiated for D <= 256
-    const dim3 g(grid), bl(kPrepWarps * 32);
+    // the register-resident variant: one warp per 128 columns, only instantiated for D <= 256
+    constexpr int W = KCH <= 2 ? KCH : 1, spb = kPrepWarps / W;
+    const dim3 g((n_local + spb - 1) / spb), bl(kPrepWarps * 32);
 #define GE2E_PREP_REG(RR)                                                                                          \
-  (prec == 3 ? launch_pdl(prep_reg_kernel<K2, RR, 3>, g, bl, 0, st, true, E, idx, n_local, M, e_hat, c_hat, cos_diag, accum) \
-   : prec == 2 ? launch_pdl(prep_reg_kernel<K2, RR, 2>, g, bl, 0, st, true, E, idx, n_local, M, e_hat, c_hat, cos_diag, accum) \
-   : prec == 1 ? launch_pdl(prep_reg_kernel<K2, RR, 1>, g, bl, 0, st, true, E, idx, n_local, M, e_hat, c_hat, cos_diag, accum) \
-               : launch_pdl(prep_reg_kernel<K2, RR, 0>, g, bl, 0, st, true, E, idx, n_local, M, e_hat, c_hat, cos_diag, accum))
+  (prec == 3 ? launch_pdl(prep_reg_kernel<W, RR, 3>, g, bl, 0, st, true, E, idx, n_local, M, e_hat, c_hat, cos_diag, accum) \
+   : prec == 2 ? launch_pdl(prep_reg_kernel<W, RR, 2>, g, bl, 0, st, true, E, idx, n_local, M, e_hat, c_hat, cos_diag, accum) \
+   : prec == 1 ? launch_pdl(prep_reg_kernel<W, RR, 1>, g, bl, 0, st, true, E, idx, n_local, M, e_hat, c_hat, cos_diag, accum) \
+               : launch_pdl(prep_reg_kernel<W, RR, 0>, g, bl, 0, st, true, E, idx, n_local, M, e_hat, c_hat, cos_diag, accum))
     if (M <= 4) GE2E_PREP_REG(4); else if (M <= 8) GE2E_PREP_REG(8); else if (M <= 12) GE2E_PREP_REG(12); else GE2E_PREP_REG(16);
 #undef GE2E_PREP_REG
     return;
@@ -1365,10 +1333,11 @@ void launch_finalize_warp(const float* E, const float* dE_hat, const float* dC_h
                           int variant, const float* g, float* dE, const int32_t* idx, bool pdl, cudaStream_t st) {
   const int grid = (n_local + kPrepWarps - 1) / kPrepWarps;
   if (KCH <= 2 && M <= kRegRows) {
-    constexpr int K2 = KCH <= 2 ? KCH : 1;
+    constexpr int W = KCH <= 2 ? KCH : 1, spb = kPrepWarps / W;
+    const dim3 gr((n_local + spb - 1) / spb), bl(kPrepWarps * 32);
 #define GE2E_FIN_REG(RR)                                                                                     \
-  launch_pdl(finalize_reg_kernel<K2, RR>, dim3(grid), dim3(kPrepWarps * 32), 0, st, pdl, E, dE_hat, dC_hat, cos_diag, \
-             row_aux, row_scale, n_local, M, w, b, eps, variant, g, dE, idx)
+  launch_pdl(finalize_reg_kernel<W, RR>, gr, bl, 0, st, pdl, E, dE_hat, dC_hat, cos_diag, row_aux, row_scale, n_local, M, \
+             w, b, eps, variant, g, dE, idx)
     if (M <= 4) GE2E_FIN_REG(4); else if (M <= 8) GE2E_FIN_REG(8); else if (M <= 12) GE2E_FIN_REG(12); else GE2E_FIN_REG(16);
 #undef GE2E_FIN_REG
     return;
