@@ -14,6 +14,7 @@
  *     memory; the library never allocates, frees or retains pointers => calls are
  *     CUDA-graph capturable.  All calls are asynchronous on `stream` and never synchronise.
  *   - fp32, row-major, contiguous.  Embeddings E[n_local, M, D]; U_local = n_local * M rows.
+ *     The _typed entry points also take E (and write dE) in bf16 / fp16: see ge2e_dtype.
  *   - w, b, grad_out are DEVICE scalars (no host sync to read nn.Parameters).
  *   - Return value: 0 on success, a negative ge2e_status otherwise (ge2e_b200_strerror).
  *   - Speaker sharding: a rank owns speakers [spk_offset, spk_offset + n_local) out of
@@ -59,13 +60,31 @@ enum ge2e_variant { GE2E_SOFTMAX = 0, GE2E_CONTRAST = 1 }; /* paper eq. (6) / eq
  *            planes.  Softmax variant, D = 128 or 256, shapes of the tensor-core path only; unlike GE2E_TF32
  *            this is a demand: an uncovered (shape, variant) returns GE2E_ERR_UNSUPPORTED -- ask
  *            ge2e_b200_path() first and fall back to GE2E_FP32.  The planes are written by kernels that read E
- *            16 bytes at a time: E (and dE) must be 16-byte aligned, else GE2E_ERR_UNSUPPORTED (copy an E that
+ *            16 bytes at a time: E (and dE) must be 16-byte aligned (8 bytes for bf16 / fp16), else GE2E_ERR_UNSUPPORTED (copy an E that
  *            sits at an odd offset of its allocation into fresh storage first). */
 /* GE2E_F16:  the hi plane of GE2E_FP32_SPLIT alone: fp16 operands carry the same 11-bit mantissa as TF32 (the
  *            stated tolerance stays 2e-3) at twice its MMA rate, one MMA per product; same kernels, same
  *            row-closing order and the same shape rules as GE2E_FP32_SPLIT (a demand, too).  It pays where the MMAs
  *            dominate (config 4 and its shards); at config 3 the extra forward launch costs more than it saves. */
 enum ge2e_precision { GE2E_FP32 = 0, GE2E_TF32 = 1, GE2E_FP32_SPLIT = 2, GE2E_F16 = 3 };
+
+/* Element type of the embeddings E and of their gradient dE (the e_dtype / de_dtype arguments of the _typed entry
+ * points; every other buffer of this ABI is fp32 or int32 whatever E is).
+ *   E    fp32, bf16 or fp16.  Each element is widened to fp32 exactly when it is loaded; every number after that
+ *        load (e_hat, c_hat, cos_diag, the row statistics, loss, dw, db, and dE before its final rounding) is the
+ *        one the fp32 call computes for E converted to fp32.  Which kernels run (ge2e_b200_path, the single-kernel
+ *        rule, the precisions) depends on the shape only, as for fp32.
+ *   dE   fp32 or E's own type (anything else: GE2E_ERR_ARGUMENT).  It is computed in fp32, multiplied by the upstream
+ *        gradient grad_out in fp32 and then rounded to its type exactly once (round to nearest even; an fp16 result
+ *        beyond its range becomes +-inf, which is what a dynamic loss scaler looks for).  Rounding before the
+ *        scaling would flush small fp16 gradients to zero before a loss scale could save them: a caller that runs
+ *        the step with grad_out = 1 and applies the real upstream gradient later (ge2e_b200_scale_grads_typed)
+ *        keeps dE in fp32 until then.
+ * Unknown codes return GE2E_ERR_ARGUMENT before anything is launched.  Alignment: rows of E / dE are read and
+ * written four elements at a time where they start at a multiple of four elements (16 bytes for fp32, 8 for the
+ * half types); other inputs take the scalar kernels, except under the plane precisions (GE2E_FP32_SPLIT,
+ * GE2E_F16), which need that alignment (GE2E_ERR_UNSUPPORTED otherwise). */
+enum ge2e_dtype { GE2E_DT_F32 = 0, GE2E_DT_BF16 = 1, GE2E_DT_F16 = 2 };
 
 int ge2e_b200_version(void);
 const char* ge2e_b200_strerror(int status);
@@ -282,6 +301,9 @@ int ge2e_b200_step_launches(int N, int M, int D, int variant, int precision);
  * dE_out[n] = g * dE_in[n], dwdb_out[2] = g * dwdb_in[2] -- one launch (`loss.backward()`, s4:200). */
 int ge2e_b200_scale_grads(const float* dE_in, float* dE_out, long long n, const float* dwdb_in, float* dwdb_out,
                           const float* grad_out, ge2e_stream_t stream);
+/* The same with dE_out of type de_dtype (ge2e_dtype): dE_in stays fp32, each g * dE_in[n] is rounded once. */
+int ge2e_b200_scale_grads_typed(const float* dE_in, void* dE_out, int de_dtype, long long n, const float* dwdb_in,
+                                float* dwdb_out, const float* grad_out, ge2e_stream_t stream);
 int ge2e_b200_forward_backward(const float* E, const int32_t* row_index, int N, int M, int D, const float* w,
                                const float* b, float eps, int variant, int precision, const float* grad_out,
                                float* e_hat, float* c_hat, float* cos_diag, float* row_stat, int32_t* row_kstar,
@@ -396,6 +418,35 @@ int ge2e_b200_backward_indexed(const float* E, const int32_t* row_index, const f
                                const float* grad_out, float* dE_hat, float* dC_hat, float* accum,
                                float* dE, void* workspace, size_t workspace_bytes,
                                ge2e_stream_t stream);
+
+/* ---- embeddings of another element type (ge2e_dtype) ------------------------------------
+ * The _indexed entry points (row_index nullable) with E of type e_dtype and dE of type de_dtype.  The plain and
+ * _indexed entry points are these with GE2E_DT_F32 for both.  All other buffers are fp32 / int32 as above. */
+int ge2e_b200_prep_typed(const void* E, int e_dtype, const int32_t* row_index, int n_local, int M, int D,
+                         int precision, float* e_hat, float* c_hat_local, float* cos_diag, float* accum,
+                         ge2e_stream_t stream);
+int ge2e_b200_bwd_finalize_typed(const void* E, int e_dtype, const int32_t* row_index, const float* dE_hat,
+                                 const float* dC_hat_local, const float* cos_diag, const float* row_stat,
+                                 const float* row_aux, const float* row_scale, int n_local, int M, int D,
+                                 const float* w, const float* b, float eps, int variant, const float* grad_out,
+                                 void* dE, int de_dtype, ge2e_stream_t stream);
+int ge2e_b200_forward_typed(const void* E, int e_dtype, const int32_t* row_index, int N, int M, int D,
+                            const float* w, const float* b, float eps, int variant, int precision, float* e_hat,
+                            float* c_hat, float* cos_diag, float* row_stat, int32_t* row_kstar, float* row_aux,
+                            float* accum, float* dE_hat, float* row_scale, void* workspace, size_t workspace_bytes,
+                            ge2e_stream_t stream);
+int ge2e_b200_backward_typed(const void* E, int e_dtype, const int32_t* row_index, const float* e_hat,
+                             const float* c_hat, const float* cos_diag, const float* row_stat,
+                             const int32_t* row_kstar, const float* row_aux, const float* row_scale, int N, int M,
+                             int D, const float* w, const float* b, float eps, int variant, int precision,
+                             const float* grad_out, float* dE_hat, float* dC_hat, float* accum, void* dE,
+                             int de_dtype, void* workspace, size_t workspace_bytes, ge2e_stream_t stream);
+int ge2e_b200_forward_backward_typed(const void* E, int e_dtype, const int32_t* row_index, int N, int M, int D,
+                                     const float* w, const float* b, float eps, int variant, int precision,
+                                     const float* grad_out, float* e_hat, float* c_hat, float* cos_diag,
+                                     float* row_stat, int32_t* row_kstar, float* row_aux, float* row_scale,
+                                     float* accum, float* dE_hat, float* dC_hat, void* dE, int de_dtype,
+                                     void* workspace, size_t workspace_bytes, ge2e_stream_t stream);
 
 /* ---- static helpers of the reference class (used by s5_eval_model.py:42-43) ----------- */
 

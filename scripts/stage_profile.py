@@ -1,7 +1,7 @@
 """Per-kernel time of the fwd+bwd step inside the CUDA graph that bench.py times.
 
     python scripts/stage_profile.py --out DIR [--workload cfg3] [--precision tf32] [--variant softmax]
-                                    [--steps 20] [--replays 5]
+                                    [--dtype float32|bfloat16|float16] [--steps 20] [--replays 5]
 
 The step is captured the way bench.py captures it: GE2EPlan.capture over batches rotated so that their
 total exceeds the 126 MB L2 (every step reads its E from HBM).  First the graph is replayed with the
@@ -13,7 +13,8 @@ dependent launch, so a kernel starts while its predecessor runs and waits inside
 predecessor's.  Each launch is therefore also given its exclusive time, end - max(start, end of the previous
 kernel), which is what it adds to the step; the exclusive times of a step and the gaps between its kernels
 add up to the step time.  The medians per kernel and per role go to DIR/stage_profile.json together with the
-GPU's name and power limit, read in the same run.
+GPU's name and power limit, read in the same run.  ``--dtype`` is the element type of the embeddings (and of dE):
+the plan is built with ``GE2EPlan(dtype=...)`` and the batches are converted once, before the capture.
 """
 from __future__ import annotations
 
@@ -73,6 +74,7 @@ def main():
     ap.add_argument("--workload", default="cfg3", choices=sorted(WORKLOADS))
     ap.add_argument("--precision", default="tf32")
     ap.add_argument("--variant", default="softmax", choices=["softmax", "contrast"])
+    ap.add_argument("--dtype", default="float32", choices=["float32", "bfloat16", "float16"])
     ap.add_argument("--steps", type=int, default=20, help="steps per graph replay")
     ap.add_argument("--replays", type=int, default=5)
     args = ap.parse_args()
@@ -83,11 +85,13 @@ def main():
     dev = torch.device("cuda:0")
     N, M, D = WORKLOADS[args.workload]
     U = N * M
-    n_rot = max(2, int(np.ceil(1.5 * 126e6 / (U * D * 4))))
-    batches = [make_batch(N, M, D, seed=i).to(dev) for i in range(n_rot)]
+    dtype = getattr(torch, args.dtype)
+    esize = torch.empty((), dtype=dtype).element_size()
+    n_rot = max(2, int(np.ceil(1.5 * 126e6 / (U * D * esize))))
+    batches = [make_batch(N, M, D, seed=i).to(dev, dtype) for i in range(n_rot)]
     w = torch.tensor(10.0, device=dev)
     b = torch.tensor(-5.0, device=dev)
-    plan = GE2EPlan(N, M, D, args.variant, args.precision, device=dev)
+    plan = GE2EPlan(N, M, D, args.variant, args.precision, device=dev, dtype=dtype)
     g = plan.capture(batches, w, b, steps=args.steps)
     for _ in range(2):
         g.replay()
@@ -134,12 +138,12 @@ def main():
         excl_role[role(name)].append(float(np.median(ex)) * per_step)
     res = {
         "workload": args.workload, "N": N, "M": M, "D": D, "precision": args.precision, "variant": args.variant,
-        "path": plan.path, "gpu": gpu_info(),
+        "dtype": args.dtype, "path": plan.path, "gpu": gpu_info(),
         "step_us": float(np.median(step_ms)) * 1e3, "step_us_replays": [round(x * 1e3, 2) for x in step_ms],
         "kernel_us_per_step": {k: round(sum(v), 3) for k, v in by_role.items()},
         "exclusive_us_per_step": {k: round(sum(v), 3) for k, v in excl_role.items()},
         "kernels": per_kernel,
-        "how": (f"GE2EPlan.capture of {args.steps} steps over {n_rot} rotating batches ({n_rot * U * D * 4 / 1e6:.0f} MB, "
+        "how": (f"GE2EPlan.capture of {args.steps} steps over {n_rot} rotating batches ({n_rot * U * D * esize / 1e6:.0f} MB, "
                 f"more than the L2); step_us = median over {args.replays} replays of CUDA-event time / steps, profiler "
                 f"off; kernel times from one torch.profiler run of {args.replays} more replays (CUDA activities), the "
                 "median duration (and median exclusive time) of each kernel times its launches per step, summed "
@@ -150,7 +154,7 @@ def main():
     path = os.path.join(args.out, "stage_profile.json")
     with open(path, "w") as f:
         json.dump(res, f, indent=1)
-    print(json.dumps({k: res[k] for k in ("workload", "precision", "variant", "gpu", "step_us", "kernel_us_per_step",
+    print(json.dumps({k: res[k] for k in ("workload", "precision", "variant", "dtype", "gpu", "step_us", "kernel_us_per_step",
                                           "exclusive_us_per_step", "step_us_outside_the_kernels")}))
     for k, v in sorted(per_kernel.items(), key=lambda kv: -kv[1]["median_us"] * kv[1]["launches"]):
         print(f"  {v['role']:9s} {v['median_us']:8.2f} us (exclusive {v['median_exclusive_us']:7.2f}) x {v['launches']:4d}  {k}")

@@ -19,6 +19,8 @@ VARIANTS = {"softmax": SOFTMAX, "contrast": CONTRAST}
 # "f16": the 2e-3 tolerance class with fp16 operands instead of TF32 (same 11-bit mantissa, twice the MMA rate:
 # GE2E_F16).  Opt-in: it wins only where the MMAs dominate (config 4 on one GPU: 1.12x, DESIGN 3.4).
 PRECISIONS = {"fp32": FP32, "tf32": TF32, "fp32_simt": FP32, "fp32_split": FP32_SPLIT, "tf32_mma": TF32, "f16": F16}
+# element type of E / dE (enum ge2e_dtype): only these two tensors may be bf16 / fp16, every other buffer is fp32
+DT_F32, DT_BF16, DT_F16 = 0, 1, 2
 
 
 def resolve_precision(name: str, n_local: int, n_total: int, M: int, D: int, variant: int) -> int:
@@ -40,9 +42,10 @@ def check_backward_shape(M: int, D: int) -> None:
                          "its last stage keeps a speaker's 2 M + 2 rows in 200 KB of shared memory")
 
 
-def planes_need_copy(ptr: int, precision: int) -> bool:
-    """The fp16-plane precisions read E 16 bytes at a time: an E at an odd offset of its allocation is copied."""
-    return precision in (FP32_SPLIT, F16) and ptr % 16 != 0
+def planes_need_copy(ptr: int, precision: int, element_size: int = 4) -> bool:
+    """The fp16-plane precisions read E four elements at a time (16 bytes for fp32, 8 for bf16 / fp16): an E at
+    another offset of its allocation is copied."""
+    return precision in (FP32_SPLIT, F16) and ptr % (4 * element_size) != 0
 
 # name -> (restype, argtypes); kept in the order of include/ge2e_b200.h
 PROTOTYPES = {
@@ -99,6 +102,7 @@ PROTOTYPES = {
     "ge2e_b200_step_workspace_bytes": (C.c_size_t, [C.c_int] * 5),
     "ge2e_b200_step_launches": (C.c_int, [C.c_int] * 5),
     "ge2e_b200_scale_grads": (C.c_int, [_f32p, _f32p, C.c_longlong, _f32p, _f32p, _f32p, _stream]),
+    "ge2e_b200_scale_grads_typed": (C.c_int, [_f32p, C.c_void_p, C.c_int, C.c_longlong, _f32p, _f32p, _f32p, _stream]),
     "ge2e_b200_forward_backward": (C.c_int, [_f32p, _i32p, C.c_int, C.c_int, C.c_int, _f32p, _f32p, C.c_float, C.c_int,
                                              C.c_int, _f32p, _f32p, _f32p, _f32p, _f32p, _i32p, _f32p, _f32p, _f32p,
                                              _f32p, _f32p, _f32p, C.c_void_p, C.c_size_t, _stream]),
@@ -112,6 +116,21 @@ PROTOTYPES = {
     "ge2e_b200_threshold_counts_scratch_bytes": (C.c_size_t, [C.c_int]),
     "ge2e_b200_threshold_counts": (C.c_int, [_f32p, C.c_int, C.c_int, _f32p, C.c_int, C.c_void_p, C.c_void_p,
                                              C.c_void_p, C.c_size_t, _stream]),
+    "ge2e_b200_prep_typed": (C.c_int, [C.c_void_p, C.c_int, _i32p, C.c_int, C.c_int, C.c_int, C.c_int, _f32p, _f32p,
+                                       _f32p, _f32p, _stream]),
+    "ge2e_b200_bwd_finalize_typed": (C.c_int, [C.c_void_p, C.c_int, _i32p, _f32p, _f32p, _f32p, _f32p, _f32p, _f32p,
+                                               C.c_int, C.c_int, C.c_int, _f32p, _f32p, C.c_float, C.c_int, _f32p,
+                                               C.c_void_p, C.c_int, _stream]),
+    "ge2e_b200_forward_typed": (C.c_int, [C.c_void_p, C.c_int, _i32p, C.c_int, C.c_int, C.c_int, _f32p, _f32p,
+                                          C.c_float, C.c_int, C.c_int, _f32p, _f32p, _f32p, _f32p, _i32p, _f32p, _f32p,
+                                          _f32p, _f32p, C.c_void_p, C.c_size_t, _stream]),
+    "ge2e_b200_backward_typed": (C.c_int, [C.c_void_p, C.c_int, _i32p, _f32p, _f32p, _f32p, _f32p, _i32p, _f32p, _f32p,
+                                           C.c_int, C.c_int, C.c_int, _f32p, _f32p, C.c_float, C.c_int, C.c_int, _f32p,
+                                           _f32p, _f32p, _f32p, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, _stream]),
+    "ge2e_b200_forward_backward_typed": (C.c_int, [C.c_void_p, C.c_int, _i32p, C.c_int, C.c_int, C.c_int, _f32p, _f32p,
+                                                   C.c_float, C.c_int, C.c_int, _f32p, _f32p, _f32p, _f32p, _f32p,
+                                                   _i32p, _f32p, _f32p, _f32p, _f32p, _f32p, C.c_void_p, C.c_int,
+                                                   C.c_void_p, C.c_size_t, _stream]),
     "ge2e_b200_centroids": (C.c_int, [_f32p, C.c_int, C.c_int, C.c_int, _f32p, _stream]),
     "ge2e_b200_utterance_centroids": (C.c_int, [_f32p, C.c_int, C.c_int, C.c_int, _f32p, _stream]),
     "ge2e_b200_normalize_rows": (C.c_int, [_f32p, C.c_int, C.c_int, _f32p, _stream]),

@@ -40,6 +40,13 @@ bool is_planes(int precision) { return precision == GE2E_FP32_SPLIT || precision
 // operand precision code of the tensor-core launchers (ge2e_common.cuh): 0 TF32, 1 split planes, 2 one plane
 int tc_prec(int precision) { return precision == GE2E_FP32_SPLIT ? 1 : (precision == GE2E_F16 ? 2 : 0); }
 
+// E is fp32 / bf16 / fp16; dE is fp32 or E's own type
+int check_dtypes(int e_dtype, int de_dtype) {
+  if (e_dtype != GE2E_DT_F32 && e_dtype != GE2E_DT_BF16 && e_dtype != GE2E_DT_F16) return GE2E_ERR_ARGUMENT;
+  if (de_dtype != GE2E_DT_F32 && de_dtype != e_dtype) return GE2E_ERR_ARGUMENT;
+  return GE2E_OK;
+}
+
 bool on_tc(int n_local, int n_total, int M, int D, int variant, int precision) {
   if (n_local <= 0 || n_total <= 0 || M < 2 || D <= 0) return false;
   if (precision == GE2E_TF32) return tc_supported(n_local, n_total, M, D, variant);
@@ -51,14 +58,14 @@ bool on_tc(int n_local, int n_total, int M, int D, int variant, int precision) {
 
 extern "C" {
 
-int ge2e_b200_version(void) { return 100; }
+int ge2e_b200_version(void) { return 101; }
 
 const char* ge2e_b200_strerror(int status) {
   switch (status) {
     case GE2E_OK: return "ok";
     case GE2E_ERR_SHAPE: return "bad shape: need n_local,n_total,D > 0, M >= 2, shard inside [0,n_total)";
     case GE2E_ERR_UNSUPPORTED: return "shape not supported by the requested precision path";
-    case GE2E_ERR_ARGUMENT: return "null pointer or unknown variant/precision";
+    case GE2E_ERR_ARGUMENT: return "null pointer or unknown variant/precision/dtype";
     case GE2E_ERR_WORKSPACE: return "workspace smaller than ge2e_b200_workspace_bytes()";
     case GE2E_ERR_DEVICE: return "current CUDA device is not compute capability 10.x (sm_100a build)";
     case GE2E_ERR_LAUNCH: return "CUDA launch or driver error (see ge2e_b200_last_cuda_error)";
@@ -104,19 +111,29 @@ size_t ge2e_b200_workspace_bytes(int n_local, int n_total, int M, int D, int var
   return 0;
 }
 
-int ge2e_b200_prep_indexed(const float* E, const int32_t* row_index, int n_local, int M, int D, int precision,
-                           float* e_hat, float* c_hat_local, float* cos_diag, float* accum,
-                           ge2e_stream_t stream) {
+int ge2e_b200_prep_typed(const void* E, int e_dtype, const int32_t* row_index, int n_local, int M, int D,
+                         int precision, float* e_hat, float* c_hat_local, float* cos_diag, float* accum,
+                         ge2e_stream_t stream) {
   if (!E || !e_hat || !c_hat_local || !cos_diag) return GE2E_ERR_ARGUMENT;
   int rc = check_shape(n_local, n_local, 0, M, D);
   if (rc != GE2E_OK) return rc;
   if ((rc = check_enum(GE2E_SOFTMAX, precision)) != GE2E_OK) return rc;
-  return simt_prep(E, row_index, n_local, M, D, precision, e_hat, c_hat_local, cos_diag, accum, (cudaStream_t)stream);
+  if ((rc = check_dtypes(e_dtype, GE2E_DT_F32)) != GE2E_OK) return rc;
+  return simt_prep(E, e_dtype, row_index, n_local, M, D, precision, e_hat, c_hat_local, cos_diag, accum,
+                   (cudaStream_t)stream);
+}
+
+int ge2e_b200_prep_indexed(const float* E, const int32_t* row_index, int n_local, int M, int D, int precision,
+                           float* e_hat, float* c_hat_local, float* cos_diag, float* accum,
+                           ge2e_stream_t stream) {
+  return ge2e_b200_prep_typed(E, GE2E_DT_F32, row_index, n_local, M, D, precision, e_hat, c_hat_local, cos_diag, accum,
+                              stream);
 }
 
 int ge2e_b200_prep(const float* E, int n_local, int M, int D, int precision, float* e_hat,
                    float* c_hat_local, float* cos_diag, float* accum, ge2e_stream_t stream) {
-  return ge2e_b200_prep_indexed(E, nullptr, n_local, M, D, precision, e_hat, c_hat_local, cos_diag, accum, stream);
+  return ge2e_b200_prep_typed(E, GE2E_DT_F32, nullptr, n_local, M, D, precision, e_hat, c_hat_local, cos_diag, accum,
+                              stream);
 }
 
 static int fwd_rows_impl(const float* e_hat, const float* c_hat_all, const float* cos_diag,
@@ -204,18 +221,20 @@ int ge2e_b200_bwd_rows(const float* e_hat, const float* c_hat_all, const float* 
                        (cudaStream_t)stream);
 }
 
-static int bwd_finalize_impl(const float* E, const int32_t* row_index, const float* dE_hat, const float* dC_hat_local,
-                           const float* cos_diag, const float* row_stat, const float* row_aux,
-                           const float* row_scale, int n_local, int M, int D, const float* w, const float* b, float eps,
-                           int variant, const float* grad_out, float* dE, bool pdl, ge2e_stream_t stream) {
+int ge2e_b200_bwd_finalize_typed(const void* E, int e_dtype, const int32_t* row_index, const float* dE_hat,
+                                 const float* dC_hat_local, const float* cos_diag, const float* row_stat,
+                                 const float* row_aux, const float* row_scale, int n_local, int M, int D,
+                                 const float* w, const float* b, float eps, int variant, const float* grad_out,
+                                 void* dE, int de_dtype, ge2e_stream_t stream) {
   if (!E || !dE_hat || !dC_hat_local || !cos_diag || !row_stat || !w || !b || !grad_out || !dE)
     return GE2E_ERR_ARGUMENT;
   if (variant == GE2E_SOFTMAX && !row_aux) return GE2E_ERR_ARGUMENT;
   int rc = check_shape(n_local, n_local, 0, M, D);
   if (rc != GE2E_OK) return rc;
   if ((rc = check_enum(variant, GE2E_FP32)) != GE2E_OK) return rc;
-  return simt_bwd_finalize(E, row_index, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux, row_scale, n_local, M, D, w,
-                           b, eps, variant, grad_out, dE, pdl, (cudaStream_t)stream);
+  if ((rc = check_dtypes(e_dtype, de_dtype)) != GE2E_OK) return rc;
+  return simt_bwd_finalize(E, e_dtype, row_index, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux, row_scale, n_local,
+                           M, D, w, b, eps, variant, grad_out, dE, de_dtype, true, (cudaStream_t)stream);
 }
 
 int ge2e_b200_bwd_finalize_indexed(const float* E, const int32_t* row_index, const float* dE_hat,
@@ -223,16 +242,16 @@ int ge2e_b200_bwd_finalize_indexed(const float* E, const int32_t* row_index, con
                                    const float* row_aux, const float* row_scale, int n_local, int M, int D,
                                    const float* w, const float* b, float eps, int variant, const float* grad_out,
                                    float* dE, ge2e_stream_t stream) {
-  return bwd_finalize_impl(E, row_index, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux, row_scale, n_local, M, D, w,
-                           b, eps, variant, grad_out, dE, true, stream);
+  return ge2e_b200_bwd_finalize_typed(E, GE2E_DT_F32, row_index, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux,
+                                      row_scale, n_local, M, D, w, b, eps, variant, grad_out, dE, GE2E_DT_F32, stream);
 }
 
 int ge2e_b200_bwd_finalize(const float* E, const float* dE_hat, const float* dC_hat_local,
                            const float* cos_diag, const float* row_stat, const float* row_aux,
                            const float* row_scale, int n_local, int M, int D, const float* w, const float* b,
                            float eps, int variant, const float* grad_out, float* dE, ge2e_stream_t stream) {
-  return bwd_finalize_impl(E, nullptr, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux, row_scale, n_local, M, D, w,
-                           b, eps, variant, grad_out, dE, true, stream);
+  return ge2e_b200_bwd_finalize_typed(E, GE2E_DT_F32, nullptr, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux,
+                                      row_scale, n_local, M, D, w, b, eps, variant, grad_out, dE, GE2E_DT_F32, stream);
 }
 
 int ge2e_b200_gather_spans(const float* bank, const long long* src_off, int rows, long long span, int offsets_aligned,
@@ -296,21 +315,32 @@ static bool tc_softmax_step(int n_local, int n_total, int M, int D, int variant,
   return variant == GE2E_SOFTMAX && on_tc(n_local, n_total, M, D, variant, precision);
 }
 
+int ge2e_b200_forward_typed(const void* E, int e_dtype, const int32_t* row_index, int N, int M, int D, const float* w,
+                            const float* b, float eps, int variant, int precision, float* e_hat, float* c_hat,
+                            float* cos_diag, float* row_stat, int32_t* row_kstar, float* row_aux, float* accum,
+                            float* dE_hat, float* row_scale, void* workspace, size_t workspace_bytes,
+                            ge2e_stream_t stream) {
+  if (!accum) return GE2E_ERR_ARGUMENT;
+  int rc = check_enum(variant, precision);
+  if (rc != GE2E_OK) return rc;
+  if ((rc = check_dtypes(e_dtype, GE2E_DT_F32)) != GE2E_OK) return rc;
+  // tensor-core path: prep and the rows kernel are adjacent in the stream, the second one is launched
+  // programmatically under the first one's tail
+  const bool tc = on_tc(N, N, M, D, variant, precision);
+  rc = ge2e_b200_prep_typed(E, e_dtype, row_index, N, M, D, precision, e_hat, c_hat, cos_diag, accum, stream);
+  if (rc != GE2E_OK) return rc;
+  return fwd_rows_impl(e_hat, c_hat, cos_diag, N, N, 0, M, D, w, b, eps, variant, precision, row_stat, row_kstar,
+                       row_aux, accum, nullptr, nullptr, dE_hat, row_scale, workspace, workspace_bytes, tc, stream);
+}
+
 int ge2e_b200_forward_indexed(const float* E, const int32_t* row_index, int N, int M, int D, const float* w,
                               const float* b, float eps, int variant, int precision, float* e_hat, float* c_hat,
                               float* cos_diag, float* row_stat, int32_t* row_kstar, float* row_aux, float* accum,
                               float* dE_hat, float* row_scale, void* workspace, size_t workspace_bytes,
                               ge2e_stream_t stream) {
-  if (!accum) return GE2E_ERR_ARGUMENT;
-  int rc = check_enum(variant, precision);
-  if (rc != GE2E_OK) return rc;
-  // tensor-core path: prep and the rows kernel are adjacent in the stream, the second one is launched
-  // programmatically under the first one's tail
-  const bool tc = on_tc(N, N, M, D, variant, precision);
-  rc = ge2e_b200_prep_indexed(E, row_index, N, M, D, precision, e_hat, c_hat, cos_diag, accum, stream);
-  if (rc != GE2E_OK) return rc;
-  return fwd_rows_impl(e_hat, c_hat, cos_diag, N, N, 0, M, D, w, b, eps, variant, precision, row_stat, row_kstar,
-                       row_aux, accum, nullptr, nullptr, dE_hat, row_scale, workspace, workspace_bytes, tc, stream);
+  return ge2e_b200_forward_typed(E, GE2E_DT_F32, row_index, N, M, D, w, b, eps, variant, precision, e_hat, c_hat,
+                                 cos_diag, row_stat, row_kstar, row_aux, accum, dE_hat, row_scale, workspace,
+                                 workspace_bytes, stream);
 }
 
 int ge2e_b200_forward(const float* E, int N, int M, int D, const float* w, const float* b, float eps,
@@ -322,13 +352,14 @@ int ge2e_b200_forward(const float* E, int N, int M, int D, const float* w, const
                                    stream);
 }
 
-int ge2e_b200_backward_indexed(const float* E, const int32_t* row_index, const float* e_hat, const float* c_hat,
-                               const float* cos_diag, const float* row_stat, const int32_t* row_kstar,
-                               const float* row_aux, const float* row_scale, int N, int M, int D, const float* w,
-                               const float* b, float eps, int variant, int precision, const float* grad_out,
-                               float* dE_hat, float* dC_hat, float* accum, float* dE, void* workspace,
-                               size_t workspace_bytes, ge2e_stream_t stream) {
+int ge2e_b200_backward_typed(const void* E, int e_dtype, const int32_t* row_index, const float* e_hat,
+                             const float* c_hat, const float* cos_diag, const float* row_stat, const int32_t* row_kstar,
+                             const float* row_aux, const float* row_scale, int N, int M, int D, const float* w,
+                             const float* b, float eps, int variant, int precision, const float* grad_out,
+                             float* dE_hat, float* dC_hat, float* accum, void* dE, int de_dtype, void* workspace,
+                             size_t workspace_bytes, ge2e_stream_t stream) {
   if (!accum) return GE2E_ERR_ARGUMENT;
+  if (check_dtypes(e_dtype, de_dtype) != GE2E_OK) return GE2E_ERR_ARGUMENT;
   if (M > finalize_max_rows(D)) return GE2E_ERR_UNSUPPORTED;     // before the rows kernels run
   // row_scale is meaningful only where the forward produced it
   const float* scale = tc_softmax_step(N, N, M, D, variant, precision) ? row_scale : nullptr;
@@ -337,8 +368,19 @@ int ge2e_b200_backward_indexed(const float* E, const int32_t* row_index, const f
                               workspace_bytes, stream);
   if (rc != GE2E_OK) return rc;
   // the finalize kernel directly follows the dC_hat tensor-core kernel: programmatic launch
-  return bwd_finalize_impl(E, row_index, dE_hat, dC_hat, cos_diag, row_stat, row_aux, scale, N, M, D, w, b, eps, variant,
-                           grad_out, dE, true, stream);
+  return ge2e_b200_bwd_finalize_typed(E, e_dtype, row_index, dE_hat, dC_hat, cos_diag, row_stat, row_aux, scale, N, M, D,
+                                      w, b, eps, variant, grad_out, dE, de_dtype, stream);
+}
+
+int ge2e_b200_backward_indexed(const float* E, const int32_t* row_index, const float* e_hat, const float* c_hat,
+                               const float* cos_diag, const float* row_stat, const int32_t* row_kstar,
+                               const float* row_aux, const float* row_scale, int N, int M, int D, const float* w,
+                               const float* b, float eps, int variant, int precision, const float* grad_out,
+                               float* dE_hat, float* dC_hat, float* accum, float* dE, void* workspace,
+                               size_t workspace_bytes, ge2e_stream_t stream) {
+  return ge2e_b200_backward_typed(E, GE2E_DT_F32, row_index, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux,
+                                  row_scale, N, M, D, w, b, eps, variant, precision, grad_out, dE_hat, dC_hat, accum, dE,
+                                  GE2E_DT_F32, workspace, workspace_bytes, stream);
 }
 
 int ge2e_b200_backward(const float* E, const float* e_hat, const float* c_hat, const float* cos_diag,
@@ -451,42 +493,60 @@ int ge2e_b200_step_launches(int N, int M, int D, int variant, int precision) {
   return use_small_step(N, M, D, variant, precision) ? 1 : 0;
 }
 
-int ge2e_b200_forward_backward(const float* E, const int32_t* row_index, int N, int M, int D, const float* w,
-                               const float* b, float eps, int variant, int precision, const float* grad_out,
-                               float* e_hat, float* c_hat, float* cos_diag, float* row_stat, int32_t* row_kstar,
-                               float* row_aux, float* row_scale, float* accum, float* dE_hat, float* dC_hat,
-                               float* dE, void* workspace, size_t workspace_bytes, ge2e_stream_t stream) {
+int ge2e_b200_forward_backward_typed(const void* E, int e_dtype, const int32_t* row_index, int N, int M, int D,
+                                     const float* w, const float* b, float eps, int variant, int precision,
+                                     const float* grad_out, float* e_hat, float* c_hat, float* cos_diag,
+                                     float* row_stat, int32_t* row_kstar, float* row_aux, float* row_scale,
+                                     float* accum, float* dE_hat, float* dC_hat, void* dE, int de_dtype,
+                                     void* workspace, size_t workspace_bytes, ge2e_stream_t stream) {
   if (!E || !w || !b || !grad_out || !e_hat || !c_hat || !cos_diag || !row_stat || !row_aux || !row_scale || !accum ||
       !dE_hat || !dC_hat || !dE)
     return GE2E_ERR_ARGUMENT;
   int rc = check_shape(N, N, 0, M, D);
   if (rc != GE2E_OK) return rc;
   if ((rc = check_enum(variant, precision)) != GE2E_OK) return rc;
+  if ((rc = check_dtypes(e_dtype, de_dtype)) != GE2E_OK) return rc;
   // refused before any launch: never a forward that ran and a finalize that cannot
   if (M > finalize_max_rows(D)) return GE2E_ERR_UNSUPPORTED;
   if (use_small_step(N, M, D, variant, precision)) {
     if (!workspace || workspace_bytes < small_step_workspace_bytes(N, M, D)) return GE2E_ERR_WORKSPACE;
     if (variant == GE2E_CONTRAST && !row_kstar) return GE2E_ERR_ARGUMENT;
-    return simt_small_step(E, row_index, N, M, D, w, b, eps, variant, grad_out, e_hat, c_hat, cos_diag, row_stat,
-                           row_kstar, row_aux, nullptr, accum, dE_hat, dC_hat, accum + 1, dE, workspace,
-                           (cudaStream_t)stream);
+    return simt_small_step(E, e_dtype, row_index, N, M, D, w, b, eps, variant, grad_out, e_hat, c_hat, cos_diag,
+                           row_stat, row_kstar, row_aux, nullptr, accum, dE_hat, dC_hat, accum + 1, dE, de_dtype,
+                           workspace, (cudaStream_t)stream);
   }
   // prep (zeroes accum) -> rows: every kernel is launched programmatically under its predecessor's tail
-  rc = ge2e_b200_prep_indexed(E, row_index, N, M, D, precision, e_hat, c_hat, cos_diag, accum, stream);
+  rc = ge2e_b200_prep_typed(E, e_dtype, row_index, N, M, D, precision, e_hat, c_hat, cos_diag, accum, stream);
   if (rc != GE2E_OK) return rc;
   rc = ge2e_b200_step_rows(e_hat, c_hat, cos_diag, N, N, 0, M, D, w, b, eps, variant, precision, grad_out, row_stat,
                            row_kstar, row_aux, row_scale, accum, dE_hat, dC_hat, workspace, workspace_bytes, stream);
   if (rc != GE2E_OK) return rc;
   const float* scale = tc_softmax_step(N, N, M, D, variant, precision) ? row_scale : nullptr;
-  return bwd_finalize_impl(E, row_index, dE_hat, dC_hat, cos_diag, row_stat, row_aux, scale, N, M, D, w, b, eps, variant,
-                           grad_out, dE, true, stream);
+  return ge2e_b200_bwd_finalize_typed(E, e_dtype, row_index, dE_hat, dC_hat, cos_diag, row_stat, row_aux, scale, N, M, D,
+                                      w, b, eps, variant, grad_out, dE, de_dtype, stream);
+}
+
+int ge2e_b200_forward_backward(const float* E, const int32_t* row_index, int N, int M, int D, const float* w,
+                               const float* b, float eps, int variant, int precision, const float* grad_out,
+                               float* e_hat, float* c_hat, float* cos_diag, float* row_stat, int32_t* row_kstar,
+                               float* row_aux, float* row_scale, float* accum, float* dE_hat, float* dC_hat,
+                               float* dE, void* workspace, size_t workspace_bytes, ge2e_stream_t stream) {
+  return ge2e_b200_forward_backward_typed(E, GE2E_DT_F32, row_index, N, M, D, w, b, eps, variant, precision, grad_out,
+                                          e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, row_scale, accum, dE_hat,
+                                          dC_hat, dE, GE2E_DT_F32, workspace, workspace_bytes, stream);
+}
+
+int ge2e_b200_scale_grads_typed(const float* dE_in, void* dE_out, int de_dtype, long long n, const float* dwdb_in,
+                                float* dwdb_out, const float* grad_out, ge2e_stream_t stream) {
+  if (!dE_in || !dE_out || !dwdb_in || !dwdb_out || !grad_out) return GE2E_ERR_ARGUMENT;
+  if (check_dtypes(de_dtype, de_dtype) != GE2E_OK) return GE2E_ERR_ARGUMENT;
+  if (n < 1) return GE2E_ERR_SHAPE;
+  return simt_scale_grads(dE_in, dE_out, de_dtype, n, dwdb_in, dwdb_out, grad_out, (cudaStream_t)stream);
 }
 
 int ge2e_b200_scale_grads(const float* dE_in, float* dE_out, long long n, const float* dwdb_in, float* dwdb_out,
                           const float* grad_out, ge2e_stream_t stream) {
-  if (!dE_in || !dE_out || !dwdb_in || !dwdb_out || !grad_out) return GE2E_ERR_ARGUMENT;
-  if (n < 1) return GE2E_ERR_SHAPE;
-  return simt_scale_grads(dE_in, dE_out, n, dwdb_in, dwdb_out, grad_out, (cudaStream_t)stream);
+  return ge2e_b200_scale_grads_typed(dE_in, dE_out, GE2E_DT_F32, n, dwdb_in, dwdb_out, grad_out, stream);
 }
 
 int ge2e_b200_centroids(const float* E, int N, int M, int D, float* C, ge2e_stream_t stream) {

@@ -135,9 +135,10 @@ struct RowsArgs {
 };
 
 // row_index (nullable): logical row r = [speaker][utterance] lives at physical row row_index[r] of E / dE
+// e_dt / de_dt: ge2e_dtype of E / dE (checked by the C ABI: dE is fp32 or E's type)
 // prec: 0 = fp32 operands as they are, 1 = rounded to TF32, 3 = the hi plane of 2 alone, 2 = two fp16 planes [rows][2][D] (hi, lo) in the
 // same allocation (D = 128 / 256 / 512 only)
-int simt_prep(const float* E, const int32_t* row_index, int n_local, int M, int D, int prec, float* e_hat,
+int simt_prep(const void* E, int e_dt, const int32_t* row_index, int n_local, int M, int D, int prec, float* e_hat,
               float* c_hat_local, float* cos_diag, float* accum, cudaStream_t st);
 int simt_fwd_rows(const RowsArgs& a, float* row_stat, int32_t* row_kstar, float* row_aux,
                   float* loss_accum, float* per_row_out, float* sim_out, cudaStream_t st);
@@ -146,22 +147,24 @@ int simt_bwd_rows(const RowsArgs& a, const float* row_stat, const int32_t* row_k
                   float* dwdb_accum, cudaStream_t st);
 // largest M whose backward finalize runs at width D (0: D unsupported); see ge2e_b200_max_utterances
 int finalize_max_rows(int D);
-int simt_bwd_finalize(const float* E, const int32_t* row_index, const float* dE_hat, const float* dC_hat_local,
+int simt_bwd_finalize(const void* E, int e_dt, const int32_t* row_index, const float* dE_hat, const float* dC_hat_local,
                       const float* cos_diag, const float* row_stat, const float* row_aux,
                       const float* row_scale /* nullable: dE_hat row r is g * row_scale[r] * dE_hat[r] */,
                       int n_local, int M, int D,
                       const float* w, const float* b, float eps, int variant,
-                      const float* grad_out, float* dE, bool pdl, cudaStream_t st);
+                      const float* grad_out, void* dE, int de_dt, bool pdl, cudaStream_t st);
 // fused single-kernel fwd+bwd step for small batches (ge2e_simt.cu)
 bool small_step_supported(int N, int M, int D);
 bool small_step_preferred(int N, int M, int D, int variant);   // supported AND faster than the pipeline
 size_t small_step_workspace_bytes(int N, int M, int D);
-int simt_small_step(const float* E, const int32_t* row_index, int N, int M, int D, const float* w, const float* b,
-                    float eps, int variant, const float* grad_out, float* e_hat, float* c_hat, float* cos_diag,
-                    float* row_stat, int32_t* row_kstar, float* row_aux, float* per_row, float* loss_accum,
-                    float* dE_hat, float* dC_hat, float* dwdb, float* dE, void* workspace, cudaStream_t st);
-int simt_scale_grads(const float* in, float* out, long long n, const float* dwdb_in, float* dwdb_out, const float* g,
-                     cudaStream_t st);
+int simt_small_step(const void* E, int e_dt, const int32_t* row_index, int N, int M, int D, const float* w,
+                    const float* b, float eps, int variant, const float* grad_out, float* e_hat, float* c_hat,
+                    float* cos_diag, float* row_stat, int32_t* row_kstar, float* row_aux, float* per_row,
+                    float* loss_accum, float* dE_hat, float* dC_hat, float* dwdb, void* dE, int de_dt, void* workspace,
+                    cudaStream_t st);
+// out_dt: ge2e_dtype of out (in is fp32)
+int simt_scale_grads(const float* in, void* out, int out_dt, long long n, const float* dwdb_in, float* dwdb_out,
+                     const float* g, cudaStream_t st);
 int simt_scale_bias_sgd(float* w, float* b, float* dw, float* db, float max_norm, float lr, float* total_norm,
                         bool pdl, cudaStream_t st);
 int simt_threshold_counts(const float* sim, int N, int M, const float* thresholds, int T, long long* accept_all,

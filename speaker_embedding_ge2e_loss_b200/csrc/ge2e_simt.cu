@@ -15,6 +15,7 @@
 //                    (reference s3:64-79, s3:27, s3:114-127 and their autograd)
 //   contrast_bwd     the contrast gradient has two non-zeros per row: gather/scatter kernel
 //   finalize_kernel  one CTA per speaker: diagonal term, normalisation Jacobians, fan-out
+#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <limits.h>
 
@@ -22,6 +23,7 @@
 #include <stdlib.h>
 
 #include <initializer_list>
+#include <type_traits>
 
 #include "ge2e_common.cuh"
 #include "ge2e_tc_ptx.cuh"
@@ -85,8 +87,94 @@ __device__ __forceinline__ size_t phys_row(const int32_t* __restrict__ idx, size
   return idx != nullptr ? static_cast<size_t>(__ldg(idx + r)) : r;
 }
 
-__device__ __forceinline__ bool is_vec(const void* p, int D) {
-  return ((D & 3) == 0) && ((reinterpret_cast<uintptr_t>(p) & 15) == 0);
+// four consecutive elements of T at an aligned address: 16 bytes for fp32, 8 bytes for the half types
+template <typename T>
+__device__ __forceinline__ bool is_vec(const T* p, int D) {
+  return ((D & 3) == 0) && ((reinterpret_cast<uintptr_t>(p) & (4 * sizeof(T) - 1)) == 0);
+}
+
+// ---- element types of E and dE (ge2e_dtype) ---------------------------------------------------
+// E is fp32, bf16 or fp16; a half-type element is widened to fp32 when it is loaded, and every number after that
+// load is the fp32 path's.  dE is fp32 or E's type; it is rounded to its type (nearest even) once, when it is
+// stored.  Everything between prep and finalize (e_hat, c_hat, the row statistics, dE_hat, dC_hat) stays fp32.
+__device__ __forceinline__ float to_f(__half x) { return __half2float(x); }
+__device__ __forceinline__ float to_f(__nv_bfloat16 x) { return __bfloat162float(x); }
+template <typename T> __device__ __forceinline__ T from_f(float x);
+template <> __device__ __forceinline__ float from_f<float>(float x) { return x; }
+template <> __device__ __forceinline__ __half from_f<__half>(float x) { return __float2half_rn(x); }
+template <> __device__ __forceinline__ __nv_bfloat16 from_f<__nv_bfloat16>(float x) { return __float2bfloat16_rn(x); }
+
+// four half-type elements (8 bytes) <-> a float4
+template <typename T> __device__ __forceinline__ float4 widen4(uint2 r);
+template <> __device__ __forceinline__ float4 widen4<__nv_bfloat16>(uint2 r) {
+  return make_float4(__uint_as_float(r.x << 16), __uint_as_float(r.x & 0xffff0000u), __uint_as_float(r.y << 16),
+                     __uint_as_float(r.y & 0xffff0000u));
+}
+template <> __device__ __forceinline__ float4 widen4<__half>(uint2 r) {
+  const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&r.x));
+  const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&r.y));
+  return make_float4(a.x, a.y, b.x, b.y);
+}
+template <typename T> __device__ __forceinline__ uint2 narrow4(float4 v);
+template <> __device__ __forceinline__ uint2 narrow4<__nv_bfloat16>(float4 v) {
+  const __nv_bfloat162 a = __floats2bfloat162_rn(v.x, v.y), b = __floats2bfloat162_rn(v.z, v.w);
+  return make_uint2(*reinterpret_cast<const uint32_t*>(&a), *reinterpret_cast<const uint32_t*>(&b));
+}
+template <> __device__ __forceinline__ uint2 narrow4<__half>(float4 v) {
+  const __half2 a = __floats2half2_rn(v.x, v.y), b = __floats2half2_rn(v.z, v.w);
+  return make_uint2(*reinterpret_cast<const uint32_t*>(&a), *reinterpret_cast<const uint32_t*>(&b));
+}
+
+// four elements of T as one vector: a float4 for fp32, 8 bytes for the half types
+template <typename T>
+using vec4_t = typename std::conditional<std::is_same<T, float>::value, float4, uint2>::type;
+template <typename T>
+__device__ __forceinline__ float4 ldg4v(const vec4_t<T>* p) {     // read-only path
+  if constexpr (std::is_same<T, float>::value) return __ldg(p);
+  else return widen4<T>(__ldg(p));
+}
+template <typename T>
+__device__ __forceinline__ void st4vv(vec4_t<T>* p, float4 v) {
+  if constexpr (std::is_same<T, float>::value) *p = v;
+  else *p = narrow4<T>(v);
+}
+// elements [0, 4) at p (is_vec-aligned)
+template <typename T>
+__device__ __forceinline__ float4 ldg4(const T* p) { return ldg4v<T>(reinterpret_cast<const vec4_t<T>*>(p)); }
+template <typename T>
+__device__ __forceinline__ void st4v(T* p, float4 v) { st4vv<T>(reinterpret_cast<vec4_t<T>*>(p), v); }
+// ld4 / st4 for any element type (tail-safe; vec = is_vec of the row base)
+template <typename T>
+__device__ __forceinline__ float4 ld4e(const T* __restrict__ row, int col, int D, bool vec) {
+  if constexpr (std::is_same<T, float>::value) {
+    return ld4(row, col, D, vec);
+  } else {
+    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (vec) {
+      if (col < D) v = ldg4(row + col);
+    } else {
+      if (col + 0 < D) v.x = to_f(__ldg(row + col + 0));
+      if (col + 1 < D) v.y = to_f(__ldg(row + col + 1));
+      if (col + 2 < D) v.z = to_f(__ldg(row + col + 2));
+      if (col + 3 < D) v.w = to_f(__ldg(row + col + 3));
+    }
+    return v;
+  }
+}
+template <typename T>
+__device__ __forceinline__ void st4e(T* __restrict__ row, int col, int D, bool vec, float4 v) {
+  if constexpr (std::is_same<T, float>::value) {
+    st4(row, col, D, vec, v);
+  } else {
+    if (vec) {
+      if (col < D) st4v(row + col, v);
+    } else {
+      if (col + 0 < D) row[col + 0] = from_f<T>(v.x);
+      if (col + 1 < D) row[col + 1] = from_f<T>(v.y);
+      if (col + 2 < D) row[col + 2] = from_f<T>(v.z);
+      if (col + 3 < D) row[col + 3] = from_f<T>(v.w);
+    }
+  }
 }
 
 // ------------------------------------------------------------------------------------------
@@ -94,8 +182,8 @@ __device__ __forceinline__ bool is_vec(const void* p, int D) {
 // ------------------------------------------------------------------------------------------
 // Body shared by prep_kernel and the fused small-batch kernel: speaker j, block of kThreads threads,
 // `smem` = (M + 1) * Dp floats.
-template <bool ROUND>
-__device__ __forceinline__ void prep_body(const float* __restrict__ E, const int32_t* __restrict__ idx, int j, int M,
+template <bool ROUND, typename TE = float>
+__device__ __forceinline__ void prep_body(const TE* __restrict__ E, const int32_t* __restrict__ idx, int j, int M,
                                           int D, int Dp, float* __restrict__ e_hat, float* __restrict__ c_hat,
                                           float* __restrict__ cos_diag, float* smem) {
   __shared__ float red[kWarps];
@@ -109,7 +197,7 @@ __device__ __forceinline__ void prep_body(const float* __restrict__ E, const int
   for (int v = tid; v < M * (Dp >> 2); v += kThreads) {
     const int i = v / (Dp >> 2), col = (v % (Dp >> 2)) << 2;
     *reinterpret_cast<float4*>(&sE[(size_t)i * Dp + col]) =
-        ld4(E + phys_row(idx, (size_t)j * M + i) * D, col, D, vec_in);
+        ld4e(E + phys_row(idx, (size_t)j * M + i) * D, col, D, vec_in);
   }
   __syncthreads();
   for (int d = tid; d < Dp; d += kThreads) {
@@ -161,9 +249,9 @@ __device__ __forceinline__ void prep_body(const float* __restrict__ E, const int
   }
 }
 
-template <bool ROUND>
+template <bool ROUND, typename TE>
 __global__ void __launch_bounds__(kThreads)
-prep_kernel(const float* __restrict__ E, const int32_t* __restrict__ idx, int M, int D, int Dp,
+prep_kernel(const TE* __restrict__ E, const int32_t* __restrict__ idx, int M, int D, int Dp,
             float* __restrict__ e_hat, float* __restrict__ c_hat, float* __restrict__ cos_diag,
             float* __restrict__ accum) {
   extern __shared__ __align__(16) float smem[];
@@ -211,9 +299,9 @@ constexpr int kRowBatch = 4;   // rows in flight per lane (KCH float4 loads each
 constexpr int kRegRows = 16;   // register-resident variants hold up to this many rows per speaker
 constexpr int kRegBlocksPerSM = 4;   // register-resident variants: <= 128 registers, 16 warps resident per SM
 
-template <int KCH, int PREC>
+template <int KCH, int PREC, typename TE>
 __global__ void __launch_bounds__(kPrepWarps * 32)
-prep_warp_kernel(const float* __restrict__ E, const int32_t* __restrict__ idx, int n_local, int M,
+prep_warp_kernel(const TE* __restrict__ E, const int32_t* __restrict__ idx, int n_local, int M,
                  float* __restrict__ e_hat, float* __restrict__ c_hat, float* __restrict__ cos_diag,
                  float* __restrict__ accum) {
   constexpr int D = KCH * 128;
@@ -223,8 +311,8 @@ prep_warp_kernel(const float* __restrict__ E, const int32_t* __restrict__ idx, i
   pdl_trigger();     // the forward tensor-core kernel may set itself up while this grid runs
   if (blockIdx.x == 0 && threadIdx.x < 4 && accum != nullptr) accum[threadIdx.x] = 0.f;
   if (j >= n_local) return;
-  auto rowp = [&](int i) {      // + c * 32 float4 per 128-column chunk
-    return reinterpret_cast<const float4*>(E + phys_row(idx, (size_t)j * M + i) * D) + lane;
+  auto rowp = [&](int i) {      // + c * 32 vectors per 128-column chunk
+    return reinterpret_cast<const vec4_t<TE>*>(E + phys_row(idx, (size_t)j * M + i) * D) + lane;
   };
   float4 s[KCH];
 #pragma unroll
@@ -235,7 +323,7 @@ prep_warp_kernel(const float* __restrict__ E, const int32_t* __restrict__ idx, i
     for (int r = 0; r < kRowBatch; ++r)
 #pragma unroll
       for (int c = 0; c < KCH; ++c)
-        v[r][c] = (i0 + r < M) ? __ldg(rowp(i0 + r) + c * 32) : make_float4(0.f, 0.f, 0.f, 0.f);
+        v[r][c] = (i0 + r < M) ? ldg4v<TE>(rowp(i0 + r) + c * 32) : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
     for (int r = 0; r < kRowBatch; ++r)
 #pragma unroll
@@ -263,7 +351,7 @@ prep_warp_kernel(const float* __restrict__ E, const int32_t* __restrict__ idx, i
     for (int r = 0; r < kRowBatch; ++r)
 #pragma unroll
       for (int c = 0; c < KCH; ++c)
-        v[r][c] = (i0 + r < M) ? __ldg(rowp(i0 + r) + c * 32) : make_float4(0.f, 0.f, 0.f, 0.f);
+        v[r][c] = (i0 + r < M) ? ldg4v<TE>(rowp(i0 + r) + c * 32) : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
     for (int r = 0; r < kRowBatch; ++r) {
       ne2[r] = 0.f; nd2[r] = 0.f; ed[r] = 0.f;
@@ -354,9 +442,9 @@ __device__ __forceinline__ void speaker_sum(float (&x)[Q], float (*xch)[Q][16], 
   }
 }
 
-template <int W, int RR, int PREC>
+template <int W, int RR, int PREC, typename TE>
 __global__ void __launch_bounds__(kPrepWarps * 32, kRegBlocksPerSM)
-prep_reg_kernel(const float* __restrict__ E, const int32_t* __restrict__ idx, int n_local, int M,
+prep_reg_kernel(const TE* __restrict__ E, const int32_t* __restrict__ idx, int n_local, int M,
                 float* __restrict__ e_hat, float* __restrict__ c_hat, float* __restrict__ cos_diag,
                 float* __restrict__ accum) {
   constexpr int D = W * 128, R = RR;       // rows held in registers (M <= R <= 16)
@@ -373,8 +461,7 @@ prep_reg_kernel(const float* __restrict__ E, const int32_t* __restrict__ idx, in
   float4 v[R];
 #pragma unroll
   for (int i = 0; i < R; ++i)
-    v[i] = (i < M) ? __ldg(reinterpret_cast<const float4*>(E + phys_row(idx, (size_t)j * M + i) * D + col))
-                   : make_float4(0.f, 0.f, 0.f, 0.f);
+    v[i] = (i < M) ? ldg4(E + phys_row(idx, (size_t)j * M + i) * D + col) : make_float4(0.f, 0.f, 0.f, 0.f);
   float4 s = v[0];
 #pragma unroll
   for (int i = 1; i < R; ++i) { s.x += v[i].x; s.y += v[i].y; s.z += v[i].z; s.w += v[i].w; }
@@ -721,12 +808,12 @@ contrast_bwd_kernel(const float* __restrict__ e_hat, const float* __restrict__ c
 // threads, `smem` = (2 M + 2) * Dp floats.  dE_hat / dC_hat are read with plain loads (the fused
 // kernel reads what its own block has just written).
 // REUSE_E: sE already holds the speaker's raw rows (prep_body staged them at the same place earlier in this kernel).
-template <bool REUSE_E = false>
-__device__ __forceinline__ void finalize_body(const float* __restrict__ E, const float* dE_hat, const float* dC_hat,
+template <bool REUSE_E = false, typename TE = float, typename TD = float>
+__device__ __forceinline__ void finalize_body(const TE* __restrict__ E, const float* dE_hat, const float* dC_hat,
                                               const float* cos_diag, const float* row_stat, const float* row_aux,
                                               const float* row_scale, int j, int M, int D, int Dp, float w, float b,
                                               float g, float eps,
-                                              int variant, float* __restrict__ dE, const int32_t* __restrict__ idx,
+                                              int variant, TD* __restrict__ dE, const int32_t* __restrict__ idx,
                                               float* smem) {
   __shared__ float red[kWarps];
   __shared__ float s_bc[2];
@@ -741,7 +828,7 @@ __device__ __forceinline__ void finalize_body(const float* __restrict__ E, const
     for (int v = tid; v < M * (Dp >> 2); v += kThreads) {
       const int i = v / (Dp >> 2), col = (v % (Dp >> 2)) << 2;
       *reinterpret_cast<float4*>(&sE[(size_t)i * Dp + col]) =
-          ld4(E + phys_row(idx, (size_t)j * M + i) * D, col, D, vec_e);
+          ld4e(E + phys_row(idx, (size_t)j * M + i) * D, col, D, vec_e);
     }
     __syncthreads();
   }
@@ -854,19 +941,20 @@ __device__ __forceinline__ void finalize_body(const float* __restrict__ E, const
     o.y = de.y + bc.y + (sd.y - du.y) / m1;
     o.z = de.z + bc.z + (sd.z - du.z) / m1;
     o.w = de.w + bc.w + (sd.w - du.w) / m1;
-    st4(dE + phys_row(idx, (size_t)j * M + i) * D, col, D, vec_o, o);
+    st4e(dE + phys_row(idx, (size_t)j * M + i) * D, col, D, vec_o, o);
   }
 }
 
+template <typename TE, typename TD>
 __global__ void __launch_bounds__(kThreads)
-finalize_kernel(const float* __restrict__ E, const float* __restrict__ dE_hat,
+finalize_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
                 const float* __restrict__ dC_hat, const float* __restrict__ cos_diag,
                 const float* __restrict__ row_stat, const float* __restrict__ row_aux,
                 const float* __restrict__ row_scale, int M, int D, int Dp,
                 const float* __restrict__ wp, const float* __restrict__ bp, float eps, int variant,
-                const float* __restrict__ gp, float* __restrict__ dE, const int32_t* __restrict__ idx) {
+                const float* __restrict__ gp, TD* __restrict__ dE, const int32_t* __restrict__ idx) {
   extern __shared__ __align__(16) float smem[];
-  finalize_body(E, dE_hat, dC_hat, cos_diag, row_stat, row_aux, row_scale, blockIdx.x, M, D, Dp, __ldg(wp), __ldg(bp), __ldg(gp),
+  finalize_body<false>(E, dE_hat, dC_hat, cos_diag, row_stat, row_aux, row_scale, blockIdx.x, M, D, Dp, __ldg(wp), __ldg(bp), __ldg(gp),
                 eps, variant, dE, idx, smem);
 }
 
@@ -877,13 +965,13 @@ finalize_kernel(const float* __restrict__ E, const float* __restrict__ dE_hat,
 // the speaker's rows (the 2nd and 3rd hit L1): column sums; per-row scalars + sum_i du_i;
 // outputs.  Row i's scalars live in lane i between the passes.
 // ------------------------------------------------------------------------------------------
-template <int KCH>
+template <int KCH, typename TE, typename TD>
 __global__ void __launch_bounds__(kPrepWarps * 32)
-finalize_warp_kernel(const float* __restrict__ E, const float* __restrict__ dE_hat,
+finalize_warp_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
                      const float* __restrict__ dC_hat, const float* __restrict__ cos_diag,
                      const float* __restrict__ row_aux, const float* __restrict__ row_scale, int n_local, int M,
                      const float* __restrict__ wp, const float* __restrict__ bp, float eps, int variant,
-                     const float* __restrict__ gp, float* __restrict__ dE, const int32_t* __restrict__ idx) {
+                     const float* __restrict__ gp, TD* __restrict__ dE, const int32_t* __restrict__ idx) {
   constexpr int D = KCH * 128;
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const int j = blockIdx.x * kPrepWarps + wid;
@@ -891,8 +979,8 @@ finalize_warp_kernel(const float* __restrict__ E, const float* __restrict__ dE_h
   pdl_trigger();     // the next step's prep may be scheduled (it waits for this grid before touching memory)
   if (j >= n_local) return;
   const float w = __ldg(wp), b = __ldg(bp), g = __ldg(gp);
-  auto rowp = [&](int i) {
-    return reinterpret_cast<const float4*>(E + phys_row(idx, (size_t)j * M + i) * D) + lane;
+  auto rowp = [&](int i) {      // + c * 32 vectors per 128-column chunk
+    return reinterpret_cast<const vec4_t<TE>*>(E + phys_row(idx, (size_t)j * M + i) * D) + lane;
   };
   const float4* Gj = reinterpret_cast<const float4*>(dE_hat + (size_t)j * M * D) + lane;
   float4 s[KCH];
@@ -904,7 +992,7 @@ finalize_warp_kernel(const float* __restrict__ E, const float* __restrict__ dE_h
     for (int r = 0; r < kRowBatch; ++r)
 #pragma unroll
       for (int c = 0; c < KCH; ++c)
-        v[r][c] = (i0 + r < M) ? __ldg(rowp(i0 + r) + c * 32) : make_float4(0.f, 0.f, 0.f, 0.f);
+        v[r][c] = (i0 + r < M) ? ldg4v<TE>(rowp(i0 + r) + c * 32) : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
     for (int r = 0; r < kRowBatch; ++r)
 #pragma unroll
@@ -952,7 +1040,7 @@ finalize_warp_kernel(const float* __restrict__ E, const float* __restrict__ dE_h
 #pragma unroll
       for (int c = 0; c < KCH; ++c) {
         const bool in = i0 + r < M;
-        v[r][c] = in ? __ldg(rowp(i0 + r) + c * 32) : make_float4(0.f, 0.f, 0.f, 0.f);
+        v[r][c] = in ? ldg4v<TE>(rowp(i0 + r) + c * 32) : make_float4(0.f, 0.f, 0.f, 0.f);
         const float4 gv = in ? __ldg(Gj + (size_t)(i0 + r) * (D / 4) + c * 32) : make_float4(0.f, 0.f, 0.f, 0.f);
         const float4 e = v[r][c];
         const float4 d = make_float4(s[c].x - e.x, s[c].y - e.y, s[c].z - e.z, s[c].w - e.w);
@@ -1008,13 +1096,13 @@ finalize_warp_kernel(const float* __restrict__ E, const float* __restrict__ dE_h
   }
   // pass 3: dE_i = de_i + dc_j / M + (sd - du_i) / (M - 1)
   for (int i = 0; i < M; ++i) {
-    float4* Oi = reinterpret_cast<float4*>(dE + phys_row(idx, (size_t)j * M + i) * D) + lane;
+    vec4_t<TD>* Oi = reinterpret_cast<vec4_t<TD>*>(dE + phys_row(idx, (size_t)j * M + i) * D) + lane;
     const float r_ag = __shfl_sync(0xffffffffu, a_g, i), r_ae = __shfl_sync(0xffffffffu, a_e, i);
     const float r_ad = __shfl_sync(0xffffffffu, a_d, i), r_be = __shfl_sync(0xffffffffu, b_e, i);
     const float r_bd = __shfl_sync(0xffffffffu, b_d, i);
 #pragma unroll
     for (int c = 0; c < KCH; ++c) {
-      const float4 e = __ldg(rowp(i) + c * 32);
+      const float4 e = ldg4v<TE>(rowp(i) + c * 32);
       const float4 gv = __ldg(Gj + (size_t)i * (D / 4) + c * 32);
       const float ev[4] = {e.x, e.y, e.z, e.w}, gg[4] = {gv.x, gv.y, gv.z, gv.w};
       const float sv[4] = {s[c].x, s[c].y, s[c].z, s[c].w}, sdv[4] = {sd[c].x, sd[c].y, sd[c].z, sd[c].w};
@@ -1027,7 +1115,7 @@ finalize_warp_kernel(const float* __restrict__ E, const float* __restrict__ dE_h
         const float du = r_be * ev[t] + r_bd * d;
         o[t] = de + bv[t] + (sdv[t] - du) * inv_m1;
       }
-      Oi[c * 32] = make_float4(o[0], o[1], o[2], o[3]);
+      st4vv<TD>(Oi + c * 32, make_float4(o[0], o[1], o[2], o[3]));
     }
   }
 }
@@ -1043,13 +1131,13 @@ finalize_warp_kernel(const float* __restrict__ E, const float* __restrict__ dE_h
 //   de_i = a_g gv_i + a_e e_i + a_d d_i ,  du_i = b_e e_i + b_d d_i ,  d_i = s - e_i
 //   dE_i = de_i + dc_j / M + (sum_i' du_i' - du_i) / (M - 1)
 // ------------------------------------------------------------------------------------------
-template <int W, int RR>
+template <int W, int RR, typename TE, typename TD>
 __global__ void __launch_bounds__(kPrepWarps * 32, kRegBlocksPerSM)
-finalize_reg_kernel(const float* __restrict__ E, const float* __restrict__ dE_hat,
+finalize_reg_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
                     const float* __restrict__ dC_hat, const float* __restrict__ cos_diag,
                     const float* __restrict__ row_aux, const float* __restrict__ row_scale, int n_local, int M,
                     const float* __restrict__ wp, const float* __restrict__ bp, float eps, int variant,
-                    const float* __restrict__ gp, float* __restrict__ dE, const int32_t* __restrict__ idx) {
+                    const float* __restrict__ gp, TD* __restrict__ dE, const int32_t* __restrict__ idx) {
   constexpr int D = W * 128, R = RR;       // rows held in registers (M <= R <= 16)
   static_assert(R <= 16, "reduce16_transposed handles 16 rows");
   static_assert(kPrepWarps % W == 0, "a block holds whole speakers");
@@ -1062,8 +1150,7 @@ finalize_reg_kernel(const float* __restrict__ E, const float* __restrict__ dE_ha
   // the row index is an input of the whole op as well (never written by the preceding grids)
 #pragma unroll
   for (int i = 0; i < R; ++i)
-    v[i] = (active && i < M) ? __ldg(reinterpret_cast<const float4*>(E + phys_row(idx, (size_t)j * M + i) * D + col))
-                             : make_float4(0.f, 0.f, 0.f, 0.f);
+    v[i] = (active && i < M) ? ldg4(E + phys_row(idx, (size_t)j * M + i) * D + col) : make_float4(0.f, 0.f, 0.f, 0.f);
   // what depends on E alone runs before the wait: the column sum s and the partial row sums |e|^2, |s - e|^2,
   // e.(s - e) and |s|^2 (t[1..4]); e.dE_hat and s.dC_hat (t[0], t[5]) follow it
   float4 s = v[0];
@@ -1169,7 +1256,7 @@ finalize_reg_kernel(const float* __restrict__ E, const float* __restrict__ dE_ha
       const float4 gv = __ldg(reinterpret_cast<const float4*>(Gj + (size_t)i * D));
       const float4 o = make_float4(r_g * gv.x + r_e * e.x + fmaf(r_s, s.x, base.x), r_g * gv.y + r_e * e.y + fmaf(r_s, s.y, base.y),
                                    r_g * gv.z + r_e * e.z + fmaf(r_s, s.z, base.z), r_g * gv.w + r_e * e.w + fmaf(r_s, s.w, base.w));
-      *reinterpret_cast<float4*>(dE + phys_row(idx, (size_t)j * M + i) * D + col) = o;
+      st4v(dE + phys_row(idx, (size_t)j * M + i) * D + col, o);
     }
   }
 }
@@ -1299,8 +1386,25 @@ bool warp_path_ok(int D, std::initializer_list<const void*> ptrs) {
   return true;
 }
 
-template <int KCH>
-void launch_prep_warp(const float* E, const int32_t* idx, int n_local, int M, int prec, float* e_hat, float* c_hat,
+// rows of E / dE start at multiples of four elements: 16 bytes for fp32, 8 bytes for the half types
+template <typename T>
+bool rows_vec_ok(const T* p) { return (reinterpret_cast<uintptr_t>(p) & (4 * sizeof(T) - 1)) == 0; }
+
+// f(TE{}) with the element type of E (ge2e_dtype code, checked by the C ABI)
+template <typename F>
+int with_e_type(int e_dt, F&& f) {
+  if (e_dt == GE2E_DT_BF16) return f(__nv_bfloat16{});
+  if (e_dt == GE2E_DT_F16) return f(__half{});
+  return f(float{});
+}
+// f(TE{}, TD{}) with the element types of E and dE (dE: fp32 or E's type)
+template <typename F>
+int with_e_de_types(int e_dt, int de_dt, F&& f) {
+  return with_e_type(e_dt, [&](auto te) -> int { return de_dt == GE2E_DT_F32 ? f(te, float{}) : f(te, te); });
+}
+
+template <int KCH, typename TE>
+void launch_prep_warp(const TE* E, const int32_t* idx, int n_local, int M, int prec, float* e_hat, float* c_hat,
                       float* cos_diag, float* accum, cudaStream_t st) {
   const int grid = (n_local + kPrepWarps - 1) / kPrepWarps;
   if (KCH <= 2 && M <= kRegRows) {
@@ -1308,48 +1412,49 @@ void launch_prep_warp(const float* E, const int32_t* idx, int n_local, int M, in
     constexpr int W = KCH <= 2 ? KCH : 1, spb = kPrepWarps / W;
     const dim3 g((n_local + spb - 1) / spb), bl(kPrepWarps * 32);
 #define GE2E_PREP_REG(RR)                                                                                          \
-  (prec == 3 ? launch_pdl(prep_reg_kernel<W, RR, 3>, g, bl, 0, st, true, E, idx, n_local, M, e_hat, c_hat, cos_diag, accum) \
-   : prec == 2 ? launch_pdl(prep_reg_kernel<W, RR, 2>, g, bl, 0, st, true, E, idx, n_local, M, e_hat, c_hat, cos_diag, accum) \
-   : prec == 1 ? launch_pdl(prep_reg_kernel<W, RR, 1>, g, bl, 0, st, true, E, idx, n_local, M, e_hat, c_hat, cos_diag, accum) \
-               : launch_pdl(prep_reg_kernel<W, RR, 0>, g, bl, 0, st, true, E, idx, n_local, M, e_hat, c_hat, cos_diag, accum))
+  (prec == 3 ? launch_pdl(prep_reg_kernel<W, RR, 3, TE>, g, bl, 0, st, true, E, idx, n_local, M, e_hat, c_hat, cos_diag, accum) \
+   : prec == 2 ? launch_pdl(prep_reg_kernel<W, RR, 2, TE>, g, bl, 0, st, true, E, idx, n_local, M, e_hat, c_hat, cos_diag, accum) \
+   : prec == 1 ? launch_pdl(prep_reg_kernel<W, RR, 1, TE>, g, bl, 0, st, true, E, idx, n_local, M, e_hat, c_hat, cos_diag, accum) \
+               : launch_pdl(prep_reg_kernel<W, RR, 0, TE>, g, bl, 0, st, true, E, idx, n_local, M, e_hat, c_hat, cos_diag, accum))
     if (M <= 4) GE2E_PREP_REG(4); else if (M <= 8) GE2E_PREP_REG(8); else if (M <= 12) GE2E_PREP_REG(12); else GE2E_PREP_REG(16);
 #undef GE2E_PREP_REG
     return;
   }
-  if (prec == 3) launch_pdl(prep_warp_kernel<KCH, 3>, dim3(grid), dim3(kPrepWarps * 32), 0, st, true, E, idx, n_local, M,
+  if (prec == 3) launch_pdl(prep_warp_kernel<KCH, 3, TE>, dim3(grid), dim3(kPrepWarps * 32), 0, st, true, E, idx, n_local, M,
                             e_hat, c_hat, cos_diag, accum);
-  else if (prec == 2) launch_pdl(prep_warp_kernel<KCH, 2>, dim3(grid), dim3(kPrepWarps * 32), 0, st, true, E, idx, n_local, M,
+  else if (prec == 2) launch_pdl(prep_warp_kernel<KCH, 2, TE>, dim3(grid), dim3(kPrepWarps * 32), 0, st, true, E, idx, n_local, M,
                             e_hat, c_hat, cos_diag, accum);
-  else if (prec == 1) launch_pdl(prep_warp_kernel<KCH, 1>, dim3(grid), dim3(kPrepWarps * 32), 0, st, true, E, idx, n_local,
+  else if (prec == 1) launch_pdl(prep_warp_kernel<KCH, 1, TE>, dim3(grid), dim3(kPrepWarps * 32), 0, st, true, E, idx, n_local,
                                  M, e_hat, c_hat, cos_diag, accum);
-  else launch_pdl(prep_warp_kernel<KCH, 0>, dim3(grid), dim3(kPrepWarps * 32), 0, st, true, E, idx, n_local, M,
+  else launch_pdl(prep_warp_kernel<KCH, 0, TE>, dim3(grid), dim3(kPrepWarps * 32), 0, st, true, E, idx, n_local, M,
                   e_hat, c_hat, cos_diag, accum);
 }
 
-template <int KCH>
-void launch_finalize_warp(const float* E, const float* dE_hat, const float* dC_hat, const float* cos_diag,
+template <int KCH, typename TE, typename TD>
+void launch_finalize_warp(const TE* E, const float* dE_hat, const float* dC_hat, const float* cos_diag,
                           const float* row_aux, const float* row_scale, int n_local, int M, const float* w,
                           const float* b, float eps,
-                          int variant, const float* g, float* dE, const int32_t* idx, bool pdl, cudaStream_t st) {
+                          int variant, const float* g, TD* dE, const int32_t* idx, bool pdl, cudaStream_t st) {
   const int grid = (n_local + kPrepWarps - 1) / kPrepWarps;
   if (KCH <= 2 && M <= kRegRows) {
     constexpr int W = KCH <= 2 ? KCH : 1, spb = kPrepWarps / W;
     const dim3 gr((n_local + spb - 1) / spb), bl(kPrepWarps * 32);
 #define GE2E_FIN_REG(RR)                                                                                     \
-  launch_pdl(finalize_reg_kernel<W, RR>, gr, bl, 0, st, pdl, E, dE_hat, dC_hat, cos_diag, row_aux, row_scale, n_local, M, \
+  launch_pdl(finalize_reg_kernel<W, RR, TE, TD>, gr, bl, 0, st, pdl, E, dE_hat, dC_hat, cos_diag, row_aux, row_scale, n_local, M, \
              w, b, eps, variant, g, dE, idx)
     if (M <= 4) GE2E_FIN_REG(4); else if (M <= 8) GE2E_FIN_REG(8); else if (M <= 12) GE2E_FIN_REG(12); else GE2E_FIN_REG(16);
 #undef GE2E_FIN_REG
     return;
   }
-  launch_pdl(finalize_warp_kernel<KCH>, dim3(grid), dim3(kPrepWarps * 32), 0, st, pdl, E, dE_hat, dC_hat, cos_diag,
+  launch_pdl(finalize_warp_kernel<KCH, TE, TD>, dim3(grid), dim3(kPrepWarps * 32), 0, st, pdl, E, dE_hat, dC_hat, cos_diag,
              row_aux, row_scale, n_local, M, w, b, eps, variant, g, dE, idx);
 }
 
-int simt_prep(const float* E, const int32_t* row_index, int n_local, int M, int D, int prec, float* e_hat,
-              float* c_hat_local, float* cos_diag, float* accum, cudaStream_t st) {
+template <typename TE>
+int simt_prep_t(const TE* E, const int32_t* row_index, int n_local, int M, int D, int prec, float* e_hat,
+                float* c_hat_local, float* cos_diag, float* accum, cudaStream_t st) {
   const bool round_tf32_ = prec == 1;
-  if (warp_path_ok(D, {E, e_hat, c_hat_local})) {
+  if (rows_vec_ok(E) && warp_path_ok(D, {e_hat, c_hat_local})) {
     if (D == 128) launch_prep_warp<1>(E, row_index, n_local, M, prec, e_hat, c_hat_local, cos_diag, accum, st);
     else if (D == 256) launch_prep_warp<2>(E, row_index, n_local, M, prec, e_hat, c_hat_local, cos_diag, accum, st);
     else launch_prep_warp<4>(E, row_index, n_local, M, prec, e_hat, c_hat_local, cos_diag, accum, st);
@@ -1361,16 +1466,24 @@ int simt_prep(const float* E, const int32_t* row_index, int n_local, int M, int 
   const size_t smem = (size_t)(M + 1) * Dp * sizeof(float);
   if (smem > kGenericSmemCap) return GE2E_ERR_UNSUPPORTED;
   if (round_tf32_) {
-    int rc = set_smem(prep_kernel<true>, smem);
+    int rc = set_smem(prep_kernel<true, TE>, smem);
     if (rc != GE2E_OK) return rc;
     prep_kernel<true><<<n_local, kThreads, smem, st>>>(E, row_index, M, D, Dp, e_hat, c_hat_local, cos_diag, accum);
   } else {
-    int rc = set_smem(prep_kernel<false>, smem);
+    int rc = set_smem(prep_kernel<false, TE>, smem);
     if (rc != GE2E_OK) return rc;
     prep_kernel<false><<<n_local, kThreads, smem, st>>>(E, row_index, M, D, Dp, e_hat, c_hat_local, cos_diag, accum);
   }
   GE2E_LAUNCHED();
   return GE2E_OK;
+}
+
+int simt_prep(const void* E, int e_dt, const int32_t* row_index, int n_local, int M, int D, int prec, float* e_hat,
+              float* c_hat_local, float* cos_diag, float* accum, cudaStream_t st) {
+  return with_e_type(e_dt, [&](auto te) -> int {
+    using TE = decltype(te);
+    return simt_prep_t(static_cast<const TE*>(E), row_index, n_local, M, D, prec, e_hat, c_hat_local, cos_diag, accum, st);
+  });
 }
 
 int simt_fwd_rows(const RowsArgs& a, float* row_stat, int32_t* row_kstar, float* row_aux, float* loss_accum,
@@ -1427,11 +1540,12 @@ int simt_bwd_rows(const RowsArgs& a, const float* row_stat, const int32_t* row_k
   return dispatch_strip<MODE_BWD_DC, GE2E_SOFTMAX>(p, splits, st);
 }
 
-int simt_bwd_finalize(const float* E, const int32_t* row_index, const float* dE_hat, const float* dC_hat_local,
-                      const float* cos_diag, const float* row_stat, const float* row_aux, const float* row_scale,
-                      int n_local, int M, int D, const float* w, const float* b, float eps, int variant,
-                      const float* grad_out, float* dE, bool pdl, cudaStream_t st) {
-  if (M <= 32 && warp_path_ok(D, {E, dE_hat, dC_hat_local, dE})) {
+template <typename TE, typename TD>
+int simt_bwd_finalize_t(const TE* E, const int32_t* row_index, const float* dE_hat, const float* dC_hat_local,
+                        const float* cos_diag, const float* row_stat, const float* row_aux, const float* row_scale,
+                        int n_local, int M, int D, const float* w, const float* b, float eps, int variant,
+                        const float* grad_out, TD* dE, bool pdl, cudaStream_t st) {
+  if (M <= 32 && rows_vec_ok(E) && rows_vec_ok(dE) && warp_path_ok(D, {dE_hat, dC_hat_local})) {
     if (D == 128) launch_finalize_warp<1>(E, dE_hat, dC_hat_local, cos_diag, row_aux, row_scale, n_local, M, w, b, eps, variant, grad_out, dE, row_index, pdl, st);
     else if (D == 256) launch_finalize_warp<2>(E, dE_hat, dC_hat_local, cos_diag, row_aux, row_scale, n_local, M, w, b, eps, variant, grad_out, dE, row_index, pdl, st);
     else launch_finalize_warp<4>(E, dE_hat, dC_hat_local, cos_diag, row_aux, row_scale, n_local, M, w, b, eps, variant, grad_out, dE, row_index, pdl, st);
@@ -1441,12 +1555,24 @@ int simt_bwd_finalize(const float* E, const int32_t* row_index, const float* dE_
   const int Dp = (D + 3) & ~3;
   if (M > finalize_max_rows(D)) return GE2E_ERR_UNSUPPORTED;
   const size_t smem = (size_t)(2 * M + 2) * Dp * sizeof(float);
-  int rc = set_smem(finalize_kernel, smem);
+  int rc = set_smem(finalize_kernel<TE, TD>, smem);
   if (rc != GE2E_OK) return rc;
   finalize_kernel<<<n_local, kThreads, smem, st>>>(E, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux, row_scale, M, D,
                                                    Dp, w, b, eps, variant, grad_out, dE, row_index);
   GE2E_LAUNCHED();
   return GE2E_OK;
+}
+
+int simt_bwd_finalize(const void* E, int e_dt, const int32_t* row_index, const float* dE_hat, const float* dC_hat_local,
+                      const float* cos_diag, const float* row_stat, const float* row_aux, const float* row_scale,
+                      int n_local, int M, int D, const float* w, const float* b, float eps, int variant,
+                      const float* grad_out, void* dE, int de_dt, bool pdl, cudaStream_t st) {
+  return with_e_de_types(e_dt, de_dt, [&](auto te, auto td) -> int {
+    using TE = decltype(te);
+    using TD = decltype(td);
+    return simt_bwd_finalize_t(static_cast<const TE*>(E), row_index, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux,
+                               row_scale, n_local, M, D, w, b, eps, variant, grad_out, static_cast<TD*>(dE), pdl, st);
+  });
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1473,13 +1599,13 @@ constexpr int kSmallMaxN = 128, kSmallMaxM = 16, kSmallMaxD = 256, kSmallPickN =
 constexpr size_t kSmallHeaderBytes = 256;
 
 struct SmallParams {
-  const float* E; const int32_t* idx; int M, D, Dp;
+  const void* E; const int32_t* idx; int M, D, Dp;   // E: element type TE of the kernel
   const float* w; const float* b; float eps;
   const float* grad_out;            // nullable: 1
   float* e_hat; float* c_hat; float* cos_diag; float* row_stat; int32_t* row_kstar; float* row_aux;
   float* per_row;                   // nullable
   float* loss_accum;                // [0] = loss (zeroed here)
-  float* dE_hat; float* dC_hat; float* dwdb; float* dE;
+  float* dE_hat; float* dC_hat; float* dwdb; void* dE;   // dE: element type TD of the kernel
   int stop;                         // debug, timing only: leave after stage `stop` (0 = run everything)
   int cluster;                      // the grid is ONE thread-block cluster (N <= 8): hardware barriers
   unsigned* ctr;                    // workspace header: {barrier arrivals, exits}; zero on entry, restored
@@ -1527,9 +1653,11 @@ __device__ __forceinline__ float4 ld4_cg(const float* row, int col, int D, bool 
 // MR = M rounded up to a multiple of 4: the cosine block's loops over the speaker's rows are fully
 // unrolled without predicates (rows M..MR-1 of the staged e_hat are zero), so the shared-memory loads of
 // all rows are issued together instead of one load -> use chain per row.
-template <int VARIANT, int MR>
+template <int VARIANT, int MR, typename TE, typename TD>
 __global__ void __launch_bounds__(kThreads, 1)
 small_step_kernel(const SmallParams p) {
+  const TE* E = static_cast<const TE*>(p.E);
+  TD* dE = static_cast<TD*>(p.dE);
   extern __shared__ __align__(16) float smem[];
   __shared__ float red[3 * kWarps];
   __shared__ float s_cd[32];
@@ -1571,8 +1699,8 @@ small_step_kernel(const SmallParams p) {
   // through global memory) are replaced by forms that keep the speaker's state in shared memory from here to the
   // last store: a HALF-warp per row (all M <= 16 rows at once), per-row norms computed once, e_hat rows written
   // straight into the stage-2 operand tile, dE_hat rows handed to the Jacobians in shared memory.
-  const bool fast = (Dp == D) && (D % 64 == 0) && is_vec(p.E, D) && is_vec(p.e_hat, D) && is_vec(p.c_hat, D) &&
-                    is_vec(p.dE_hat, D) && is_vec(p.dC_hat, D) && is_vec(p.dE, D);
+  const bool fast = (Dp == D) && (D % 64 == 0) && is_vec(E, D) && is_vec(p.e_hat, D) && is_vec(p.c_hat, D) &&
+                    is_vec(p.dE_hat, D) && is_vec(p.dC_hat, D) && is_vec(dE, D);
   float* fE = sA;                                     // [M][Dp] raw rows, later d e (gradient through e_hat)
   float* fS = fE + (size_t)M * Dp;                    // [Dp] column sums of the raw rows, later of d u
   float* fU = fS + Dp;                                // [M][Dp] dE_hat rows, later d u
@@ -1583,9 +1711,9 @@ small_step_kernel(const SmallParams p) {
   float c_norm2 = 0.f, c_mine = 0.f;                  // fast path: |c_j|^2 (every thread), c_j[tid]
   if (fast) {
     for (int i = wid; i < M; i += kWarps) {
-      const float4* src = reinterpret_cast<const float4*>(p.E + phys_row(p.idx, (size_t)j * M + i) * D);
+      const TE* src = E + phys_row(p.idx, (size_t)j * M + i) * D;
       float4* dst = reinterpret_cast<float4*>(fE + (size_t)i * Dp);
-      for (int c4 = lane; c4 < ncol4; c4 += 32) dst[c4] = __ldg(src + c4);
+      for (int c4 = lane; c4 < ncol4; c4 += 32) dst[c4] = ldg4(src + 4 * c4);
     }
     for (int v = tid; v < (MR - M) * Dp; v += kThreads) sEh[(size_t)M * Dp + v] = 0.f;
     __syncthreads();
@@ -1641,7 +1769,7 @@ small_step_kernel(const SmallParams p) {
       }
     }
   } else {
-    prep_body<false>(p.E, p.idx, j, M, D, Dp, p.e_hat, p.c_hat, p.cos_diag, sA);
+    prep_body<false>(E, p.idx, j, M, D, Dp, p.e_hat, p.c_hat, p.cos_diag, sA);
   }
   GE2E_SMALL_STAMP(1);
   if (p.stop == 1) return;
@@ -2034,7 +2162,7 @@ small_step_kernel(const SmallParams p) {
     }
     __syncthreads();
     for (int i = wid; i < M; i += kWarps) {           // fan-out of d c and of the leave-one-out centroids (s3:105-111)
-      float4* dst = reinterpret_cast<float4*>(p.dE + phys_row(p.idx, (size_t)j * M + i) * D);
+      TD* dst = dE + phys_row(p.idx, (size_t)j * M + i) * D;
       for (int c4 = lane; c4 < ncol4; c4 += 32) {
         const float4 de = reinterpret_cast<const float4*>(fE + (size_t)i * Dp)[c4];
         const float4 du = reinterpret_cast<const float4*>(fU + (size_t)i * Dp)[c4];
@@ -2045,12 +2173,12 @@ small_step_kernel(const SmallParams p) {
         o.y = de.y + bc.y + (sd.y - du.y) * inv_m1;
         o.z = de.z + bc.z + (sd.z - du.z) * inv_m1;
         o.w = de.w + bc.w + (sd.w - du.w) * inv_m1;
-        dst[c4] = o;
+        st4v(dst + 4 * c4, o);
       }
     }
   } else {
-    finalize_body<true>(p.E, p.dE_hat, p.dC_hat, p.cos_diag, p.row_stat, p.row_aux, nullptr, j, M, D, Dp, w, b, g, eps,
-                        VARIANT, p.dE, p.idx, sA);      // sA still holds the raw rows prep_body staged
+    finalize_body<true>(E, p.dE_hat, p.dC_hat, p.cos_diag, p.row_stat, p.row_aux, nullptr, j, M, D, Dp, w, b, g, eps,
+                        VARIANT, dE, p.idx, sA);      // sA still holds the raw rows prep_body staged
   }
   } while (0);
   __syncthreads();
@@ -2096,10 +2224,11 @@ size_t small_step_workspace_bytes(int N, int M, int D) {
   return small_step_supported(N, M, D) ? kSmallHeaderBytes + (size_t)N * N * D * sizeof(float) : 0;
 }
 
-int simt_small_step(const float* E, const int32_t* row_index, int N, int M, int D, const float* w, const float* b,
-                    float eps, int variant, const float* grad_out, float* e_hat, float* c_hat, float* cos_diag,
-                    float* row_stat, int32_t* row_kstar, float* row_aux, float* per_row, float* loss_accum,
-                    float* dE_hat, float* dC_hat, float* dwdb, float* dE, void* workspace, cudaStream_t st) {
+int simt_small_step(const void* E, int e_dt, const int32_t* row_index, int N, int M, int D, const float* w,
+                    const float* b, float eps, int variant, const float* grad_out, float* e_hat, float* c_hat,
+                    float* cos_diag, float* row_stat, int32_t* row_kstar, float* row_aux, float* per_row,
+                    float* loss_accum, float* dE_hat, float* dC_hat, float* dwdb, void* dE, int de_dt, void* workspace,
+                    cudaStream_t st) {
   SmallParams p;
   p.E = E; p.idx = row_index; p.M = M; p.D = D; p.Dp = (D + 3) & ~3;
   p.w = w; p.b = b; p.eps = eps; p.grad_out = grad_out;
@@ -2119,7 +2248,7 @@ int simt_small_step(const float* E, const int32_t* row_index, int N, int M, int 
   p.cluster = N <= 8 ? 1 : 0;
 #define GE2E_SMALL_LAUNCH(V, R)                                                                   \
   do {                                                                                            \
-    int rc = set_smem(small_step_kernel<V, R>, smem);                                             \
+    int rc = set_smem(small_step_kernel<V, R, TE, TD>, smem);                                     \
     if (rc != GE2E_OK) return rc;                                                                 \
     cudaLaunchConfig_t cfg{};                                                                     \
     cfg.gridDim = dim3(N); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = smem; cfg.stream = st; \
@@ -2129,17 +2258,23 @@ int simt_small_step(const float* E, const int32_t* row_index, int N, int M, int 
     at[1].id = cudaLaunchAttributeClusterDimension;                                               \
     at[1].val.clusterDim.x = N; at[1].val.clusterDim.y = 1; at[1].val.clusterDim.z = 1;           \
     cfg.attrs = at; cfg.numAttrs = p.cluster ? 2 : 1;                                             \
-    GE2E_CUDA_TRY(cudaLaunchKernelEx(&cfg, small_step_kernel<V, R>, p));                          \
+    GE2E_CUDA_TRY(cudaLaunchKernelEx(&cfg, small_step_kernel<V, R, TE, TD>, p));                  \
   } while (0)
   const int mr = (M + 3) & ~3;
-  if (variant == GE2E_SOFTMAX) {
-    if (mr == 4) GE2E_SMALL_LAUNCH(GE2E_SOFTMAX, 4); else if (mr == 8) GE2E_SMALL_LAUNCH(GE2E_SOFTMAX, 8);
-    else if (mr == 12) GE2E_SMALL_LAUNCH(GE2E_SOFTMAX, 12); else GE2E_SMALL_LAUNCH(GE2E_SOFTMAX, 16);
-  } else {
-    if (mr == 4) GE2E_SMALL_LAUNCH(GE2E_CONTRAST, 4); else if (mr == 8) GE2E_SMALL_LAUNCH(GE2E_CONTRAST, 8);
-    else if (mr == 12) GE2E_SMALL_LAUNCH(GE2E_CONTRAST, 12); else GE2E_SMALL_LAUNCH(GE2E_CONTRAST, 16);
-  }
+  const int rc = with_e_de_types(e_dt, de_dt, [&](auto te, auto td) -> int {
+    using TE = decltype(te);
+    using TD = decltype(td);
+    if (variant == GE2E_SOFTMAX) {
+      if (mr == 4) GE2E_SMALL_LAUNCH(GE2E_SOFTMAX, 4); else if (mr == 8) GE2E_SMALL_LAUNCH(GE2E_SOFTMAX, 8);
+      else if (mr == 12) GE2E_SMALL_LAUNCH(GE2E_SOFTMAX, 12); else GE2E_SMALL_LAUNCH(GE2E_SOFTMAX, 16);
+    } else {
+      if (mr == 4) GE2E_SMALL_LAUNCH(GE2E_CONTRAST, 4); else if (mr == 8) GE2E_SMALL_LAUNCH(GE2E_CONTRAST, 8);
+      else if (mr == 12) GE2E_SMALL_LAUNCH(GE2E_CONTRAST, 12); else GE2E_SMALL_LAUNCH(GE2E_CONTRAST, 16);
+    }
+    return GE2E_OK;
+  });
 #undef GE2E_SMALL_LAUNCH
+  if (rc != GE2E_OK) return rc;
   GE2E_LAUNCHED();
   return GE2E_OK;
 }
@@ -2165,32 +2300,40 @@ __global__ void scale_bias_sgd_kernel(float* w, float* b, float* dw, float* db, 
 
 // Gradients of a step that ran with upstream gradient 1, scaled by the real one (the loss is linear in it):
 // out = g * in, {dw, db}_out = g * {dw, db}_in.  One launch; the eager module path's backward.
+// fp32 in; out is fp32 or a half type, each element rounded once after the scaling (so a small fp16 gradient times a
+// loss scale keeps the digits it would lose if it were rounded first).
+template <typename TO>
 __global__ void __launch_bounds__(256)
-scale_grads_kernel(const float* __restrict__ in, float* __restrict__ out, long long n, const float* __restrict__ dwdb_in,
+scale_grads_kernel(const float* __restrict__ in, TO* __restrict__ out, long long n, const float* __restrict__ dwdb_in,
                    float* __restrict__ dwdb_out, const float* __restrict__ gp) {
   pdl_wait();
   const float g = __ldg(gp);
   if (blockIdx.x == 0 && threadIdx.x < 2) dwdb_out[threadIdx.x] = g * dwdb_in[threadIdx.x];
   const long long stride = (long long)gridDim.x * blockDim.x, t0 = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if ((n & 3) == 0 && ((reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(out)) & 15) == 0) {
+  if ((n & 3) == 0 && ((reinterpret_cast<uintptr_t>(in) & 15) | (reinterpret_cast<uintptr_t>(out) & (4 * sizeof(TO) - 1))) == 0) {
     const float4* i4 = reinterpret_cast<const float4*>(in);
-    float4* o4 = reinterpret_cast<float4*>(out);
     for (long long i = t0; i < (n >> 2); i += stride) {
       float4 v = __ldcs(i4 + i);
       v.x *= g; v.y *= g; v.z *= g; v.w *= g;
-      __stcs(o4 + i, v);
+      if constexpr (std::is_same<TO, float>::value) __stcs(reinterpret_cast<float4*>(out) + i, v);
+      else __stcs(reinterpret_cast<uint2*>(out) + i, narrow4<TO>(v));
     }
   } else {
-    for (long long i = t0; i < n; i += stride) out[i] = g * in[i];
+    for (long long i = t0; i < n; i += stride) out[i] = from_f<TO>(g * in[i]);
   }
 }
 
-int simt_scale_grads(const float* in, float* out, long long n, const float* dwdb_in, float* dwdb_out, const float* g,
-                     cudaStream_t st) {
+int simt_scale_grads(const float* in, void* out, int out_dt, long long n, const float* dwdb_in, float* dwdb_out,
+                     const float* g, cudaStream_t st) {
   long long blocks = (n / 4 + 255) / 256;
   if (blocks < 1) blocks = 1;
   if (blocks > 148 * 8) blocks = 148 * 8;
-  launch_pdl(scale_grads_kernel, dim3((unsigned)blocks), dim3(256), 0, st, true, in, out, n, dwdb_in, dwdb_out, g);
+  with_e_type(out_dt, [&](auto to) -> int {
+    using TO = decltype(to);
+    launch_pdl(scale_grads_kernel<TO>, dim3((unsigned)blocks), dim3(256), 0, st, true, in, static_cast<TO*>(out), n,
+               dwdb_in, dwdb_out, g);
+    return GE2E_OK;
+  });
   GE2E_LAUNCHED();
   return GE2E_OK;
 }

@@ -32,6 +32,26 @@ def _f32c(t: Tensor) -> Tensor:
     return t.contiguous()
 
 
+# element types the kernels read E in (and write dE in): ge2e_dtype codes of include/ge2e_b200.h
+_DTYPES = {torch.float32: _lib.DT_F32, torch.bfloat16: _lib.DT_BF16, torch.float16: _lib.DT_F16}
+
+
+def _emb(E: Tensor) -> Tuple[Tensor, int]:
+    """E contiguous, with its ge2e_dtype code: float32, bfloat16 or float16 embeddings."""
+    code = _DTYPES.get(E.dtype)
+    if code is None:
+        raise TypeError(f"embeddings must be float32, bfloat16 or float16, got {E.dtype}")
+    return E.contiguous(), code
+
+
+def _params(w: Tensor, b: Tensor) -> Tuple[Tensor, Tensor]:
+    """The loss parameters stay float32 whatever the embeddings are."""
+    for name, t in (("w", w), ("b", b)):
+        if t.dtype != torch.float32:
+            raise TypeError(f"{name} must be float32, got {t.dtype}")
+    return w.contiguous(), b.contiguous()
+
+
 def _same_f32c(*ts: Optional[Tensor]) -> None:
     """The staged ops hand raw pointers to fp32 kernels: a half-precision or strided tensor (autocast, a
     slice) would be read and written out of bounds, so refuse it instead of copying (outputs alias)."""
@@ -123,8 +143,8 @@ def _fwd_impl(E: Tensor, w: Tensor, b: Tensor, eps: float, variant: int, precisi
     Returns (loss, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale); the last two
     are 1-element placeholders where the path does not use them."""
     _need_cuda(E, w, b)
-    E, w, b = _f32c(E), _f32c(w), _f32c(b)
-    if _lib.planes_need_copy(E.data_ptr(), precision):
+    (E, ecode), (w, b) = _emb(E), _params(w, b)
+    if _lib.planes_need_copy(E.data_ptr(), precision, E.element_size()):
         E = E.clone()
     if row_index is None:
         N, M, D = E.shape
@@ -162,12 +182,12 @@ def _fwd_impl(E: Tensor, w: Tensor, b: Tensor, eps: float, variant: int, precisi
             dE_hat = dE_hat.view(U, D)
         row_kstar = torch.empty(U if variant == _lib.CONTRAST else 1, dtype=torch.int32, device=dev)
         ws, ws_bytes = _workspace(N, N, M, D, variant, precision, dev)
-        rc = lib().ge2e_b200_forward_indexed(E.data_ptr(), _ptr(row_index), N, M, D, w.data_ptr(), b.data_ptr(), eps,
-                                             variant, precision, e_hat.data_ptr(), c_hat.data_ptr(),
-                                             cos_diag.data_ptr(), row_stat.data_ptr(), row_kstar.data_ptr(),
-                                             row_aux.data_ptr(), accum.data_ptr(),
-                                             dE_hat.data_ptr() if fused else None,
-                                             row_scale.data_ptr() if fused else None, _ptr(ws), ws_bytes, _stream())
+        rc = lib().ge2e_b200_forward_typed(E.data_ptr(), ecode, _ptr(row_index), N, M, D, w.data_ptr(), b.data_ptr(),
+                                           eps, variant, precision, e_hat.data_ptr(), c_hat.data_ptr(),
+                                           cos_diag.data_ptr(), row_stat.data_ptr(), row_kstar.data_ptr(),
+                                           row_aux.data_ptr(), accum.data_ptr(),
+                                           dE_hat.data_ptr() if fused else None,
+                                           row_scale.data_ptr() if fused else None, _ptr(ws), ws_bytes, _stream())
     _check(rc, "ge2e_b200_forward")
     return accum[0], e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale
 
@@ -177,7 +197,7 @@ def _bwd_impl(grad_out, E, w, b, e_hat, c_hat, cos_diag, row_stat, row_kstar, ro
     """loss.backward() (s4:200) through the C ABI.  ``dE_hat`` / ``row_scale``: what the forward prepared
     (1-element placeholders where the path does not use them).  Returns (dE shaped like E, dwdb[2])."""
     _need_cuda(grad_out, E, w, b)
-    E, w, b = _f32c(E), _f32c(w), _f32c(b)
+    (E, ecode), (w, b) = _emb(E), _params(w, b)
     g = _f32c(grad_out)
     N, D = c_hat.shape
     U = e_hat.shape[0]
@@ -192,12 +212,12 @@ def _bwd_impl(grad_out, E, w, b, e_hat, c_hat, cos_diag, row_stat, row_kstar, ro
         dC_ptr = scratch.data_ptr() + 16
         dE_hat_ptr = dE_hat.data_ptr() if fused else dC_ptr + N * D * 4
         ws, ws_bytes = _workspace(N, N, M, D, variant, precision, dev)
-        rc = lib().ge2e_b200_backward_indexed(E.data_ptr(), _ptr(row_index), e_hat.data_ptr(), c_hat.data_ptr(),
-                                              cos_diag.data_ptr(), row_stat.data_ptr(), row_kstar.data_ptr(),
-                                              row_aux.data_ptr(), row_scale.data_ptr() if fused else None, N, M, D,
-                                              w.data_ptr(), b.data_ptr(), eps, variant, precision, g.data_ptr(),
-                                              dE_hat_ptr, dC_ptr, scratch.data_ptr(), dE.data_ptr(), _ptr(ws), ws_bytes,
-                                              _stream())
+        rc = lib().ge2e_b200_backward_typed(E.data_ptr(), ecode, _ptr(row_index), e_hat.data_ptr(), c_hat.data_ptr(),
+                                            cos_diag.data_ptr(), row_stat.data_ptr(), row_kstar.data_ptr(),
+                                            row_aux.data_ptr(), row_scale.data_ptr() if fused else None, N, M, D,
+                                            w.data_ptr(), b.data_ptr(), eps, variant, precision, g.data_ptr(),
+                                            dE_hat_ptr, dC_ptr, scratch.data_ptr(), dE.data_ptr(), ecode, _ptr(ws),
+                                            ws_bytes, _stream())
     _check(rc, "ge2e_b200_backward")
     return dE, scratch[1:3]
 
@@ -217,9 +237,11 @@ def _(E, w, b, eps, variant, precision):
     N, M, D = E.shape
     U = N * M
     fused = _tc_softmax(N, M, D, variant, precision)
-    return (E.new_empty(()), E.new_empty((U, D)), E.new_empty((N, D)), E.new_empty(U), E.new_empty(U),
-            E.new_empty(U if variant == _lib.CONTRAST else 1, dtype=torch.int32), E.new_empty(U),
-            E.new_empty((U, D) if fused else (1,)), E.new_empty(U if fused else 1))
+    f32 = torch.float32      # every intermediate is float32 whatever E's element type
+    return (E.new_empty((), dtype=f32), E.new_empty((U, D), dtype=f32), E.new_empty((N, D), dtype=f32),
+            E.new_empty(U, dtype=f32), E.new_empty(U, dtype=f32),
+            E.new_empty(U if variant == _lib.CONTRAST else 1, dtype=torch.int32), E.new_empty(U, dtype=f32),
+            E.new_empty((U, D) if fused else (1,), dtype=f32), E.new_empty(U if fused else 1, dtype=f32))
 
 
 @torch.library.custom_op("ge2e_b200::bwd", mutates_args=())
@@ -235,7 +257,7 @@ def ge2e_bwd(grad_out: Tensor, E: Tensor, w: Tensor, b: Tensor, e_hat: Tensor, c
 @ge2e_bwd.register_fake
 def _(grad_out, E, w, b, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale, eps, variant,
       precision):
-    return torch.empty_like(E), E.new_empty(2)
+    return torch.empty_like(E), E.new_empty(2, dtype=torch.float32)
 
 
 def _fwd_setup(ctx, inputs, output):
@@ -303,12 +325,13 @@ class _StepBufs:
 
 
 class _EagerPlan:
-    __slots__ = ("N", "M", "D", "U", "variant", "precision", "device", "dev_index", "path", "fused", "ws_bytes", "free",
-                 "one", "free_on", "planes", "bwd_ok")
+    __slots__ = ("N", "M", "D", "U", "variant", "precision", "dtype", "device", "dev_index", "path", "fused", "ws_bytes",
+                 "free", "one", "free_on", "planes", "bwd_ok")
 
-    def __init__(self, dev, N, M, D, variant, precision):
+    def __init__(self, dev, N, M, D, variant, precision, dtype):
         self.N, self.M, self.D, self.U = N, M, D, N * M
         self.variant, self.precision, self.device = variant, precision, dev
+        self.dtype = dtype                      # ge2e_dtype code of E and of the dE handed back
         self.dev_index = dev.index if dev.index is not None else torch.cuda.current_device()
         h = lib()
         self.path = h.ge2e_b200_path(N, N, M, D, variant, precision)
@@ -362,15 +385,16 @@ class _EagerPlan:
 
 
 _EAGER_PLANS: dict = {}
+_TORCH_DTYPES = {code: dt for dt, code in _DTYPES.items()}
 
 
-def _eager_plan(dev, N, M, D, variant, precision) -> _EagerPlan:
-    key = (dev.index, N, M, D, variant, precision)
+def _eager_plan(dev, N, M, D, variant, precision, dtype) -> _EagerPlan:
+    key = (dev.index, N, M, D, variant, precision, dtype)
     plan = _EAGER_PLANS.get(key)
     if plan is None:
         if len(_EAGER_PLANS) > 32:
             _EAGER_PLANS.clear()
-        plan = _EAGER_PLANS[key] = _EagerPlan(dev, N, M, D, variant, precision)
+        plan = _EAGER_PLANS[key] = _EagerPlan(dev, N, M, D, variant, precision, dtype)
     return plan
 
 
@@ -389,7 +413,7 @@ class _Lease:
 
 
 class _GE2EEager(torch.autograd.Function):
-    """ge2e_b200_forward_indexed / ge2e_b200_backward_indexed without the torch.library dispatch layers
+    """ge2e_b200_forward_typed / ge2e_b200_backward_typed without the torch.library dispatch layers
     (which cost ~0.2 ms of host time per step: more than the kernels at every size up to cfg3)."""
 
     @staticmethod
@@ -397,10 +421,7 @@ class _GE2EEager(torch.autograd.Function):
         if not (E.is_cuda and w.is_cuda and b.is_cuda):
             raise RuntimeError("speaker_embedding_ge2e_loss_b200 runs on CUDA (sm_100a) tensors only; "
                                "there is no CPU fallback")
-        if E.dtype != torch.float32 or w.dtype != torch.float32 or b.dtype != torch.float32:
-            raise TypeError(f"expected float32, got {E.dtype}")
-        if not E.is_contiguous():
-            E = E.contiguous()
+        (E, ecode), _ = _emb(E), _params(w, b)
         if row_index is None:
             N, M, D = E.shape
         else:
@@ -409,9 +430,9 @@ class _GE2EEager(torch.autograd.Function):
             if speakers <= 0 or N * M != U_:
                 raise ValueError(f"{U_} rows do not split into {speakers} speakers")
         dev = E.device
-        plan = _eager_plan(dev, N, M, D, variant, precision)
-        if plan.planes and E.data_ptr() % 16:
-            E = E.clone()           # the fp16-plane kernels read E 16 bytes at a time
+        plan = _eager_plan(dev, N, M, D, variant, precision, ecode)
+        if plan.planes and E.data_ptr() % (4 * E.element_size()):
+            E = E.clone()           # the fp16-plane kernels read E four elements at a time
         want_grad = ctx.needs_input_grad[0] or ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
         if want_grad and not plan.bwd_ok:
             _lib.check_backward_shape(M, D)
@@ -425,12 +446,14 @@ class _GE2EEager(torch.autograd.Function):
                 stream = _raw_stream(plan.dev_index)
                 bufs = plan.take_on(stream)
                 accum = torch.empty(4, dtype=torch.float32, device=dev)     # escapes as the loss tensor: never pooled
-                dE = torch.empty_like(E)
+                # the gradient for upstream gradient 1 stays float32: backward rounds g * dE to E's type once, so a
+                # loss scale reaches small fp16 gradients before the rounding does
+                dE = torch.empty_like(E, dtype=torch.float32)
                 ws = plan.workspace(stream)
-                rc = lib().ge2e_b200_forward_backward(
-                    E.data_ptr(), _ptr(row_index), N, M, D, w.data_ptr(), b.data_ptr(), eps, variant, precision,
+                rc = lib().ge2e_b200_forward_backward_typed(
+                    E.data_ptr(), ecode, _ptr(row_index), N, M, D, w.data_ptr(), b.data_ptr(), eps, variant, precision,
                     plan.one.data_ptr(), *bufs.step_ptrs, accum.data_ptr(), bufs.dE_hat.data_ptr(), bufs.dC_hat.data_ptr(),
-                    dE.data_ptr(), _ptr(ws), plan.ws_bytes, stream)
+                    dE.data_ptr(), _lib.DT_F32, _ptr(ws), plan.ws_bytes, stream)
             _check(rc, "ge2e_b200_forward_backward")
             plan.give_on(bufs, stream)  # the next step on this stream may overwrite them: stream order
             ctx.lease = None
@@ -442,8 +465,8 @@ class _GE2EEager(torch.autograd.Function):
             stream = _raw_stream(plan.dev_index)
             ws = plan.workspace(stream)
             fused = False
-            rc = lib().ge2e_b200_forward_indexed(
-                E.data_ptr(), _ptr(row_index), N, M, D, w.data_ptr(), b.data_ptr(), eps, variant, precision,
+            rc = lib().ge2e_b200_forward_typed(
+                E.data_ptr(), ecode, _ptr(row_index), N, M, D, w.data_ptr(), b.data_ptr(), eps, variant, precision,
                 *bufs.fwd_ptrs, accum.data_ptr(), bufs.dE_hat.data_ptr() if fused else None,
                 bufs.row_scale.data_ptr() if fused else None, _ptr(ws), plan.ws_bytes, stream)
         _check(rc, "ge2e_b200_forward")
@@ -459,11 +482,12 @@ class _GE2EEager(torch.autograd.Function):
             dev = dE1.device
             g = g_loss if (g_loss.dtype == torch.float32 and g_loss.is_cuda) else g_loss.to(dev, torch.float32)
             with _on_device(dev):
-                dE = torch.empty_like(dE1)
+                dE = torch.empty_like(dE1, dtype=_TORCH_DTYPES[plan.dtype])
                 dwdb = torch.empty(2, dtype=torch.float32, device=dev)      # escapes as dw / db
-                rc = lib().ge2e_b200_scale_grads(dE1.data_ptr(), dE.data_ptr(), dE1.numel(), acc1.data_ptr() + 4,
-                                                 dwdb.data_ptr(), g.data_ptr(), _raw_stream(plan.dev_index))
-            _check(rc, "ge2e_b200_scale_grads")
+                rc = lib().ge2e_b200_scale_grads_typed(dE1.data_ptr(), dE.data_ptr(), plan.dtype, dE1.numel(),
+                                                       acc1.data_ptr() + 4, dwdb.data_ptr(), g.data_ptr(),
+                                                       _raw_stream(plan.dev_index))
+            _check(rc, "ge2e_b200_scale_grads_typed")
             return dE, dwdb[0], dwdb[1], None, None, None, None, None
         E, w, b = ctx.saved_tensors
         eps, variant, precision, plan, fused, row_index, N, M, D = ctx.cfg
@@ -475,14 +499,18 @@ class _GE2EEager(torch.autograd.Function):
             accum = torch.empty(4, dtype=torch.float32, device=dev)     # escapes as dw / db: never pooled
             stream = _raw_stream(plan.dev_index)
             ws = plan.workspace(stream)
-            rc = lib().ge2e_b200_backward_indexed(
-                E.data_ptr(), _ptr(row_index), bufs.e_hat.data_ptr(), bufs.c_hat.data_ptr(), bufs.cos_diag.data_ptr(),
-                bufs.row_stat.data_ptr(), bufs.kstar.data_ptr(), bufs.row_aux.data_ptr(),
+            rc = lib().ge2e_b200_backward_typed(
+                E.data_ptr(), plan.dtype, _ptr(row_index), bufs.e_hat.data_ptr(), bufs.c_hat.data_ptr(),
+                bufs.cos_diag.data_ptr(), bufs.row_stat.data_ptr(), bufs.kstar.data_ptr(), bufs.row_aux.data_ptr(),
                 bufs.row_scale.data_ptr() if fused else None, N, M, D, w.data_ptr(), b.data_ptr(), eps, variant,
                 precision, g.data_ptr(), bufs.dE_hat.data_ptr(), bufs.dC_hat.data_ptr(), accum.data_ptr(), dE.data_ptr(),
-                _ptr(ws), plan.ws_bytes, stream)
-        _check(rc, "ge2e_b200_backward")
+                plan.dtype, _ptr(ws), plan.ws_bytes, stream)
+        _check(rc, "ge2e_b200_backward_typed")
         return dE, accum[1], accum[2], None, None, None, None, None
+
+
+# host-only query (a ctypes call): under torch.compile its answer is a constant of the traced graph
+_resolve_precision = torch.compiler.assume_constant_result(_lib.resolve_precision)
 
 
 def ge2e_loss(E: Tensor, w: Tensor, b: Tensor, eps: float = 1e-6, variant: str = "softmax",
@@ -499,7 +527,7 @@ def ge2e_loss(E: Tensor, w: Tensor, b: Tensor, eps: float = 1e-6, variant: str =
         if speakers <= 0 or E.shape[0] % speakers != 0 or E.shape[0] // speakers < 2:
             raise ValueError("speakers must divide the number of rows, with M >= 2 utterances per speaker")
         N, vcode = speakers, _lib.VARIANTS[variant]
-        pcode = _lib.resolve_precision(precision, N, N, E.shape[0] // N, E.shape[1], vcode)
+        pcode = _resolve_precision(precision, N, N, E.shape[0] // N, E.shape[1], vcode)
         if torch.compiler.is_compiling():
             return ge2e_fwd(E[unperm].reshape(N, E.shape[0] // N, E.shape[1]), w, b, float(eps), vcode, pcode)[0]
         idx = _index_ok(unperm, E.shape[0], E.device)
@@ -509,7 +537,7 @@ def ge2e_loss(E: Tensor, w: Tensor, b: Tensor, eps: float = 1e-6, variant: str =
     if E.shape[1] < 2:
         raise ValueError("GE2E needs M >= 2 utterances per speaker (the reference divides by M - 1)")
     vcode = _lib.VARIANTS[variant]
-    pcode = _lib.resolve_precision(precision, E.shape[0], E.shape[0], E.shape[1], E.shape[2], vcode)
+    pcode = _resolve_precision(precision, E.shape[0], E.shape[0], E.shape[1], E.shape[2], vcode)
     if torch.compiler.is_compiling():
         return ge2e_fwd(E, w, b, float(eps), vcode, pcode)[0]
     return _GE2EEager.apply(E, w, b, float(eps), vcode, pcode, None, 0)
@@ -520,8 +548,8 @@ def prep(E: Tensor, c_hat_local_out: Tensor, precision: int):
     """Stage 1 on the local speakers; writes c_hat into ``c_hat_local_out`` (a slice of the
     all-gather buffer).  Returns (e_hat, cos_diag, accum)."""
     _need_cuda(E, c_hat_local_out)
-    E = _f32c(E)
-    if _lib.planes_need_copy(E.data_ptr(), precision):
+    E, ecode = _emb(E)
+    if _lib.planes_need_copy(E.data_ptr(), precision, E.element_size()):
         E = E.clone()
     _same_f32c(c_hat_local_out)
     n, M, D = E.shape
@@ -530,9 +558,9 @@ def prep(E: Tensor, c_hat_local_out: Tensor, precision: int):
     cos_diag = torch.empty(n * M, dtype=torch.float32, device=dev)
     accum = torch.empty(4, dtype=torch.float32, device=dev)
     with torch.cuda.device(dev):
-        rc = lib().ge2e_b200_prep(E.data_ptr(), n, M, D, precision, e_hat.data_ptr(),
-                                  c_hat_local_out.data_ptr(), cos_diag.data_ptr(), accum.data_ptr(), _stream())
-    check(rc, "ge2e_b200_prep")
+        rc = lib().ge2e_b200_prep_typed(E.data_ptr(), ecode, None, n, M, D, precision, e_hat.data_ptr(),
+                                        c_hat_local_out.data_ptr(), cos_diag.data_ptr(), accum.data_ptr(), _stream())
+    check(rc, "ge2e_b200_prep_typed")
     return e_hat, cos_diag, accum
 
 
@@ -587,16 +615,16 @@ def bwd_rows(e_hat, c_hat_all, cos_diag, row_stat, row_kstar, row_aux, n_local, 
 
 def bwd_finalize(E, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux, w, b, eps, variant, grad_out,
                  row_scale=None):
-    E = _f32c(E)
+    """dE in E's element type (fp32, bf16 or fp16), rounded once."""
+    E, ecode = _emb(E)
     _same_f32c(dE_hat, dC_hat_local, cos_diag, row_stat, row_aux, w, b, grad_out, row_scale)
     _need_cuda(E)
     n, M, D = E.shape
     dE = torch.empty_like(E)
     with torch.cuda.device(E.device):
-        rc = lib().ge2e_b200_bwd_finalize(E.data_ptr(), dE_hat.data_ptr(), dC_hat_local.data_ptr(),
-                                          cos_diag.data_ptr(), row_stat.data_ptr(), row_aux.data_ptr(),
-                                          _ptr(row_scale), n, M, D, w.data_ptr(),
-                                          b.data_ptr(), eps, variant, grad_out.data_ptr(), dE.data_ptr(),
-                                          _stream())
-    check(rc, "ge2e_b200_bwd_finalize")
+        rc = lib().ge2e_b200_bwd_finalize_typed(E.data_ptr(), ecode, None, dE_hat.data_ptr(), dC_hat_local.data_ptr(),
+                                                cos_diag.data_ptr(), row_stat.data_ptr(), row_aux.data_ptr(),
+                                                _ptr(row_scale), n, M, D, w.data_ptr(), b.data_ptr(), eps, variant,
+                                                grad_out.data_ptr(), dE.data_ptr(), ecode, _stream())
+    check(rc, "ge2e_b200_bwd_finalize_typed")
     return dE

@@ -12,14 +12,19 @@ import torch
 
 from . import _lib
 from ._lib import check, lib
+from .ops import _DTYPES
 
 
 class GE2EPlan:
     def __init__(self, N: int, M: int, D: int, variant: str = "softmax", precision: str = "fp32",
-                 eps: float = 1e-6, device=None, sgd=None):
+                 eps: float = 1e-6, device=None, sgd=None, dtype: torch.dtype = torch.float32):
         """``sgd=(lr, max_norm)``: every step ends with the trainer's tail for the two loss parameters
         (clip_grad_norm_ on (w, b) + plain SGD, s4_train_embed_model.py:202-203) as one more kernel,
-        updating the ``w`` / ``b`` passed to ``step`` in place."""
+        updating the ``w`` / ``b`` passed to ``step`` in place.  ``dtype``: element type of the embeddings
+        ``step`` takes (float32, bfloat16 or float16); ``.dE`` has it too, everything else is float32."""
+        if dtype not in _DTYPES:
+            raise TypeError(f"dtype must be float32, bfloat16 or float16, got {dtype}")
+        self.dtype, self._dtype_code = dtype, _DTYPES[dtype]
         self.sgd = None if sgd is None else (float(sgd[0]), float(sgd[1]))
         if M < 2:
             raise ValueError("GE2E needs M >= 2 utterances per speaker")
@@ -44,7 +49,7 @@ class GE2EPlan:
         self.row_scale = torch.empty(U, dtype=f32, device=dev)   # tensor-core softmax path: factor of the dE_hat rows
         self.dC_hat = torch.empty((N, D), dtype=f32, device=dev)
         self._accum = torch.empty(4, dtype=f32, device=dev)      # {loss, dw, db, -}: zeroed by prep every step
-        self.dE = torch.empty((N, M, D), dtype=f32, device=dev)
+        self.dE = torch.empty((N, M, D), dtype=dtype, device=dev)
         self.grad_out = torch.ones((), dtype=f32, device=dev)
         nbytes = lib().ge2e_b200_step_workspace_bytes(N, M, D, self.variant, self.precision)
         self._ws = torch.zeros(max(nbytes, 1), dtype=torch.uint8, device=dev)   # zero once: the kernels restore it
@@ -57,11 +62,14 @@ class GE2EPlan:
 
     def step(self, E: torch.Tensor, w: torch.Tensor, b: torch.Tensor, backward: bool = True) -> None:
         """Enqueue fwd (+ bwd) on the current stream.  Results land in .loss/.dE/.dw/.db."""
-        assert E.is_cuda and E.dtype == torch.float32 and E.is_contiguous() and tuple(E.shape) == (self.N, self.M, self.D)
-        h, N, M, D = lib(), self.N, self.M, self.D
-        if _lib.planes_need_copy(E.data_ptr(), self.precision):
+        if E.dtype != self.dtype:
+            raise TypeError(f"GE2EPlan was built for {self.dtype} embeddings, got {E.dtype}")
+        assert E.is_cuda and E.is_contiguous() and tuple(E.shape) == (self.N, self.M, self.D)
+        h, N, M, D, dt = lib(), self.N, self.M, self.D, self._dtype_code
+        if _lib.planes_need_copy(E.data_ptr(), self.precision, E.element_size()):
             # a plan copies nothing behind the caller's back (its steps are captured into graphs)
-            raise ValueError("GE2EPlan: the fp16-plane precisions need a 16-byte-aligned E; this one sits at an "
+            raise ValueError("GE2EPlan: the fp16-plane precisions need a 16-byte-aligned E (8-byte for bfloat16 / "
+                             "float16); this one sits at an "
                              "offset of its storage -- pass E.clone(), or build the plan with precision='fp32_simt'")
         if backward and not self._bwd_ok:
             _lib.check_backward_shape(M, D)
@@ -69,25 +77,26 @@ class GE2EPlan:
         ws = self._ws.data_ptr() if self._ws_bytes else None
         if backward:
             accum_ptr = self._accum.data_ptr()
-            rc = h.ge2e_b200_forward_backward(E.data_ptr(), None, N, M, D, w.data_ptr(), b.data_ptr(), self.eps,
-                                              self.variant, self.precision, self.grad_out.data_ptr(),
-                                              self.e_hat.data_ptr(), self.c_hat.data_ptr(), self.cos_diag.data_ptr(),
-                                              self.row_stat.data_ptr(), self.row_kstar.data_ptr(),
-                                              self.row_aux.data_ptr(), self.row_scale.data_ptr(), accum_ptr,
-                                              self.dE_hat.data_ptr(), self.dC_hat.data_ptr(), self.dE.data_ptr(), ws,
-                                              self._ws_bytes, stream)
-            check(rc, "ge2e_b200_forward_backward")
+            rc = h.ge2e_b200_forward_backward_typed(E.data_ptr(), dt, None, N, M, D, w.data_ptr(), b.data_ptr(),
+                                                    self.eps, self.variant, self.precision, self.grad_out.data_ptr(),
+                                                    self.e_hat.data_ptr(), self.c_hat.data_ptr(),
+                                                    self.cos_diag.data_ptr(), self.row_stat.data_ptr(),
+                                                    self.row_kstar.data_ptr(), self.row_aux.data_ptr(),
+                                                    self.row_scale.data_ptr(), accum_ptr, self.dE_hat.data_ptr(),
+                                                    self.dC_hat.data_ptr(), self.dE.data_ptr(), dt, ws, self._ws_bytes,
+                                                    stream)
+            check(rc, "ge2e_b200_forward_backward_typed")
             if self.sgd is not None:
                 rc = h.ge2e_b200_scale_bias_sgd(w.data_ptr(), b.data_ptr(), accum_ptr + 4, accum_ptr + 8, self.sgd[1],
                                                 self.sgd[0], None, stream)
                 check(rc, "ge2e_b200_scale_bias_sgd")
             return
-        rc = h.ge2e_b200_forward(E.data_ptr(), N, M, D, w.data_ptr(), b.data_ptr(), self.eps, self.variant,
-                                 self.precision, self.e_hat.data_ptr(), self.c_hat.data_ptr(),
-                                 self.cos_diag.data_ptr(), self.row_stat.data_ptr(), self.row_kstar.data_ptr(),
-                                 self.row_aux.data_ptr(), self._accum.data_ptr(), None, None, ws, self._ws_bytes,
-                                 stream)
-        check(rc, "ge2e_b200_forward")
+        rc = h.ge2e_b200_forward_typed(E.data_ptr(), dt, None, N, M, D, w.data_ptr(), b.data_ptr(), self.eps,
+                                       self.variant, self.precision, self.e_hat.data_ptr(), self.c_hat.data_ptr(),
+                                       self.cos_diag.data_ptr(), self.row_stat.data_ptr(), self.row_kstar.data_ptr(),
+                                       self.row_aux.data_ptr(), self._accum.data_ptr(), None, None, ws, self._ws_bytes,
+                                       stream)
+        check(rc, "ge2e_b200_forward_typed")
 
     def capture(self, E, w: torch.Tensor, b: torch.Tensor, backward: bool = True, steps: int = 1):
         """Capture ``steps`` consecutive steps into one CUDA graph bound to these tensors; returns the
@@ -249,6 +258,9 @@ class ShardedGE2EPlan:
         torch.sum(self.red_all, dim=0, out=self.red_sum)
 
     def step(self, E_local: torch.Tensor, w: torch.Tensor, b: torch.Tensor) -> None:
+        if E_local.dtype != torch.float32:
+            raise TypeError(f"ShardedGE2EPlan takes float32 embeddings only, got {E_local.dtype}; bfloat16 / float16 "
+                            "embeddings run through GE2ELoss(process_group=...) or a single-device GE2EPlan(dtype=...)")
         if self.peer:
             return self._step_peer(E_local, w, b)
         h, dist = lib(), self.dist
@@ -342,7 +354,8 @@ class _HostFeed:
         for d in self.shape:
             n *= d
         if not (E_host.dtype == torch.float32 and E_host.is_contiguous() and E_host.numel() == n):
-            raise ValueError(f"submit: expected a contiguous fp32 batch of {n} values")
+            raise ValueError(f"submit: expected a contiguous fp32 batch of {n} values (the host-fed plans take float32 "
+                             f"embeddings only, got {E_host.dtype})")
         if E_host.device.type == "cpu" and not E_host.is_pinned():
             raise ValueError("submit: the host batch must be in pinned memory (an unpinned copy is synchronous)")
         i = self._k % self.depth

@@ -69,7 +69,10 @@ class ShardedGE2EFunction(torch.autograd.Function):
         n_total = n_local * world
         spk_offset = rank * n_local
         E_local = E_local.contiguous()
-        c_hat_all = torch.empty((n_total, D), dtype=E_local.dtype, device=E_local.device)
+        # the normalised centroids are float32 for half-precision embeddings (prep widens E); other dtypes keep E's,
+        # so the host-side emulation of the stages can run in float64
+        c_dtype = torch.float32 if E_local.dtype in (torch.bfloat16, torch.float16) else E_local.dtype
+        c_hat_all = torch.empty((n_total, D), dtype=c_dtype, device=E_local.device)
         mine = c_hat_all[spk_offset:spk_offset + n_local]
         e_hat, cos_diag, accum = stages.prep(E_local, mine, precision)
         # all-gather of the normalised centroids (8.4 MB at N=8192, D=256)
