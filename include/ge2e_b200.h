@@ -131,6 +131,14 @@ void ge2e_b200_debug_stamps(unsigned long long* device_buf);
 int ge2e_b200_debug_step_schedule(int u_local, int n_total, int cta_group, int max_clusters,
                                   int* de_begin_host, int* dc_begin_host, int* partial_host,
                                   int* units_host);
+/* Debug, host only: the model behind the pass-2 ranges of ge2e_b200_debug_step_schedule (same arguments).
+ * Pass 2 of a cluster waits per utterance tile for that tile's row sums, not for the whole grid.  dc_rot_host[c]:
+ * cluster c walks its pass-2 range starting that many units in, wrapping around (0 = in order).  finish_host[c]:
+ * the model's predicted finish of cluster c, in stream units of work.  model_host = {pass-1 -> pass-2 transition
+ * in units, predicted makespan of the same pass-1 cut with a grid barrier between the passes}.  Arrays need
+ * max_clusters entries (model_host 2).  Returns the cluster count. */
+int ge2e_b200_debug_step_model(int u_local, int n_total, int cta_group, int max_clusters, int* dc_rot_host,
+                               double* finish_host, double* model_host);
 /* GE2E_OK if the current CUDA device can run this library (sm_100), else GE2E_ERR_DEVICE. */
 int ge2e_b200_check_device(void);
 

@@ -81,6 +81,9 @@ def main():
         torch.cuda.synchronize()
         h.ge2e_b200_debug_trace(None, -1)
         t = tr.cpu().numpy().reshape(148, 3, ev)
+        # fixed slots of the epilogue record: [61] pass 1 done, [62] pass 2 begins, [63] ns waiting for row sums
+        fixed = t[:, 2, ev - 3:].copy()
+        t[:, 2, ev - 3:] = 0
         t0 = t[t > 0].min()
         ends = np.array([t[c][t[c] > 0].max() if (t[c] > 0).any() else 0 for c in range(148)])
         for c in (0, int(np.argmax(ends)), int(np.argmin(np.where(ends > 0, ends, ends.max())))):
@@ -88,6 +91,12 @@ def main():
                 v = t[c, role]
                 v = v[v > 0]
                 print(f"cta {c:3d} {name}: " + " ".join(f"{(x - t0) / 1e3:.1f}" for x in v))
+        print("per CTA (us from kernel start): pass-1 done, pass-2 begins, total wait for pass-2 row sums")
+        for c in range(148):
+            p1, p2, wait = fixed[c]
+            if p1 or p2 or wait:
+                f = lambda x: f"{(x - t0) / 1e3:6.1f}" if x else "     -"
+                print(f"cta {c:3d}: {f(p1)} {f(p2)} {wait / 1e3:6.2f}")
 
 
 if __name__ == "__main__":

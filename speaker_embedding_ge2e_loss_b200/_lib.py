@@ -60,6 +60,7 @@ PROTOTYPES = {
     "ge2e_b200_debug_hybrid": (None, [C.c_int]),
     "ge2e_b200_debug_step_schedule": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                                 C.c_void_p, C.c_void_p]),
+    "ge2e_b200_debug_step_model": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "ge2e_b200_check_device": (C.c_int, []),
     "ge2e_b200_workspace_bytes": (C.c_size_t, [C.c_int] * 6),
     "ge2e_b200_prep": (C.c_int, [_f32p, C.c_int, C.c_int, C.c_int, C.c_int, _f32p, _f32p, _f32p, _f32p,

@@ -58,7 +58,7 @@ bool on_tc(int n_local, int n_total, int M, int D, int variant, int precision) {
 
 extern "C" {
 
-int ge2e_b200_version(void) { return 101; }
+int ge2e_b200_version(void) { return 102; }
 
 const char* ge2e_b200_strerror(int status) {
   switch (status) {
@@ -88,6 +88,12 @@ int ge2e_b200_debug_step_schedule(int u_local, int n_total, int cta_group, int m
   if (!de_begin_host || !dc_begin_host || !partial_host || !units_host) return GE2E_ERR_ARGUMENT;
   return tc_debug_step_schedule(u_local, n_total, cta_group, max_clusters, de_begin_host, dc_begin_host,
                                 partial_host, units_host);
+}
+
+int ge2e_b200_debug_step_model(int u_local, int n_total, int cta_group, int max_clusters, int* dc_rot_host,
+                               double* finish_host, double* model_host) {
+  if (!dc_rot_host || !finish_host || !model_host) return GE2E_ERR_ARGUMENT;
+  return tc_debug_step_model(u_local, n_total, cta_group, max_clusters, dc_rot_host, finish_host, model_host);
 }
 
 int ge2e_b200_path(int n_local, int n_total, int M, int D, int variant, int precision) {

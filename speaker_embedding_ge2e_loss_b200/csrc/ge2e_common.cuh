@@ -200,6 +200,7 @@ void tc_set_trace(unsigned long long* device_buf, int mode);
 void tc_set_stamps(unsigned long long* device_buf);
 int tc_debug_step_schedule(int u_local, int n_total, int cg, int max_clusters, int* de_begin, int* dc_begin,
                            int* partial, int* units);
+int tc_debug_step_model(int u_local, int n_total, int cg, int max_clusters, int* dc_rot, double* finish, double* model);
 size_t tc_workspace_bytes(int n_local, int n_total, int M, int D, int variant);
 int tc_fwd_rows(const RowsArgs& a, float* row_stat, int32_t* row_kstar, float* row_aux,
                 float* loss_accum, float* per_row_out, void* ws, size_t ws_bytes, bool after_prep,

@@ -17,8 +17,9 @@
 //            (the forward's row loss) and P, rounded to TF32, is written back over T in TMEM;
 //            MMA2  Acc[128 x D] += P . Y_unit  (A from TMEM, B MN-major from smem) -> un-normalised
 //            dE_hat rows: the true row is g w exp(m - lse_r) times it (row_scale, applied by finalize)
-//          -- grid-wide barrier: every row sum is complete --
-//          pass 2 (DC segments: X = C_hat rows, Y = E_hat): epilogue G = w g softmax(S) with the own
+//          -- per utterance tile: the segment that completes a tile's row sums closes its 128 rows --
+//          pass 2 (DC segments: X = C_hat rows, Y = E_hat; a stream unit is one utterance tile, and its epilogue
+//            waits for that tile's rows only, not for the grid): epilogue G = w g softmax(S) with the own
 //            speaker's rows masked, written back over T; MMA2 Acc += G . Y_unit -> dC_hat = (wG)^T E_hat
 //          the accumulator leaves through shared memory and a TMA store / TMA reduce-add.
 //          Issued contraction work: 8 U N D (algorithmic 6: S is recomputed once, for pass 2).
@@ -34,11 +35,13 @@
 //   FWD   the flat pair list is cut into equal contiguous ranges over the clusters (stream-K); a
 //         cluster whose range covers only part of an owner group publishes (max, sum) per row and
 //         the last cluster to finish that tile merges.
-//   STEP  both passes in ONE launch, each cut evenly over the clusters: whole owner groups where
-//         that balances (plain store), else a flat cut whose partial accumulators are added into the
-//         zero-filled output at the L2 (cp.reduce.async.bulk).  The per-cluster ranges are computed on
-//         the host (make_step_sched) and passed by value.  The TMA and MMA warps run straight from
-//         pass 1 into pass 2 (their operands are inputs); only the epilogue waits at the barrier.
+//   STEP  both passes in ONE launch: whole owner groups where that balances (plain store), else cut
+//         groups whose partial accumulators are added into the zero-filled output at the L2
+//         (cp.reduce.async.bulk).  The per-cluster ranges are computed on the host (make_step_sched) and
+//         passed by value: pass 2 is cut against a model of when each cluster leaves pass 1 and when each
+//         utterance tile's row sums are complete, and a cluster walks its pass-2 range rotated so that
+//         the tiles completed last come last.  The TMA and MMA warps run straight from pass 1 into
+//         pass 2 (their operands are inputs); only the epilogue waits, per stream unit.
 //
 // Warp roles (384 threads): warp 0 = TMA producer, warp 1 = MMA issuer, warp 2 = TMEM allocator,
 // warps 4-11 = epilogue (TMEM lane quarter = warp % 4, column half = (warp - 4) / 4: two threads
@@ -51,6 +54,8 @@
 #include <stdlib.h>
 
 #include <algorithm>
+#include <cstring>
+#include <vector>
 
 #include "ge2e_common.cuh"
 #include "ge2e_tc_ptx.cuh"
@@ -129,10 +134,13 @@ struct TmSet {
   CUtensorMap out_peer[kMaxPeers];
 };
 
-// STEP: pair range [begin[c], begin[c + 1]) of cluster c in the dE_hat (pass 1) / dC_hat (pass 2) pair lists
+// STEP: pair range [begin[c], begin[c + 1]) of cluster c in the dE_hat (pass 1) / dC_hat (pass 2) pair lists;
+// cluster c walks its pass-2 range (one owner group whenever dc_rot[c] != 0) starting dc_rot[c] units in and
+// wrapping around, so that the utterance tiles whose row sums are completed last are visited last
 struct StepSched {
   int de[kMaxClusters + 1];
   int dc[kMaxClusters + 1];
+  unsigned char dc_rot[kMaxClusters];
 };
 
 struct TcParams {
@@ -158,7 +166,7 @@ struct TcParams {
   int32_t* kstar_out;
   float* loss_accum;
   float* per_row_out;
-  int* seg_done;              // [OT] stream units finished per owner tile (zeroed by the host)
+  int* seg_done;              // [OT] stream units finished per owner tile; STEP: per utterance tile, pass 1 (zero on entry and exit)
   float2* seg_part;           // [OT][maxseg][128] partial row state
   int maxseg;
   // BWD outputs (dE_hat / dC_hat go through the `out` tensor maps)
@@ -167,7 +175,7 @@ struct TcParams {
   long long zero_n4;          //      (float4 count; 0 = nothing to clear)
   float4* zero2_base;         // STEP: dE_hat when some owner group is cut between clusters
   long long zero2_n4;
-  int* ctr;                   // STEP: {CTAs done zero-filling, CTAs done, CTAs done with pass 1}: zero on entry and exit
+  int* ctr;                   // STEP: {CTAs done zero-filling, CTAs done, utterance tiles complete}: zero on entry and exit
   int peer_rows;              // STEP: > 0: centroid rows per rank, pass 2 flushes through tms.out_peer (see TmSet)
   unsigned long long* stamps; // STEP, nullable: [CTA]{start, end} globaltimer stamps (in-situ kernel time)
   unsigned long long* trace;  // debug: [CTA][3 roles][kTraceEvents] globaltimer stamps, or nullptr
@@ -180,12 +188,21 @@ constexpr int kTraceEvents = 64;
 template <bool DBG>
 struct Tracer {
   unsigned long long* buf;
-  int n;
-  __device__ __forceinline__ Tracer(unsigned long long* base, int role)
-      : buf(DBG && base ? base + (static_cast<size_t>(blockIdx.x) * 3 + role) * kTraceEvents : nullptr), n(0) {}
+  int n, cap;
+  // reserve: slots at the end of the record kept for put()
+  __device__ __forceinline__ Tracer(unsigned long long* base, int role, int reserve = 0)
+      : buf(DBG && base ? base + (static_cast<size_t>(blockIdx.x) * 3 + role) * kTraceEvents : nullptr), n(0),
+        cap(kTraceEvents - reserve) {}
   __device__ __forceinline__ void mark() {
     if (DBG) {
-      if (buf != nullptr && n < kTraceEvents) buf[n++] = globaltimer_ns();
+      if (buf != nullptr && n < cap) buf[n++] = globaltimer_ns();
+    }
+  }
+  // the step kernel's epilogue record reserves its last three slots: [61] pass 1 done (row sums counted),
+  // [62] first pass-2 segment begins, [63] total ns spent waiting for pass-2 row sums
+  __device__ __forceinline__ void put(int slot, unsigned long long v) {
+    if (DBG) {
+      if (buf != nullptr) buf[slot] = v;
     }
   }
 };
@@ -194,6 +211,7 @@ struct SharedTail {
   uint64_t bars[BAR_COUNT];
   uint32_t tmem_base;
   int flag;
+  int rows_all_done;                      // STEP: this CTA has seen ctr[2] == OT (every utterance tile complete)
   union {
     float red[2 * kEpiWarps];
     float red3[3 * kEpiWarps];
@@ -217,6 +235,12 @@ struct Walk {
   long long gp, end;      // remaining pair range of the current part
   long long gp2, end2;    // BWD: the other part, visited second
   int kind, kind2;        // kind of the current / of the second part (kind2 < 0: no second part left)
+  int rot;                // STEP: first unit of a pass-2 segment, relative to s0 (StepSched::dc_rot)
+  // unit visited i-th in the segment [s0, s1) returned by next()
+  __device__ __forceinline__ int unit(int i, int s0, int s1) const {
+    const int u = s0 + i + (kind == SEG_DC ? rot : 0);
+    return u < s1 ? u : u - (s1 - s0);
+  }
   __device__ __forceinline__ bool next(const TcParams& p, int& kind_out, int& og, int& s0, int& s1) {
     while (gp >= end) {
       if (kind2 < 0) return false;
@@ -354,10 +378,12 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
       wk.gp = (static_cast<long long>(cl) * p.GP) / NC;
       wk.end = (static_cast<long long>(cl + 1) * p.GP) / NC;
       wk.gp2 = wk.end2 = 0;
+      wk.rot = 0;
     } else {
       // pass 1 (dE_hat segments), then pass 2 (dC_hat segments); a pass that is not in p.phases has empty ranges
       wk.kind = SEG_DE; wk.gp = sched.de[cl]; wk.end = sched.de[cl + 1];
       wk.kind2 = SEG_DC; wk.gp2 = sched.dc[cl]; wk.end2 = sched.dc[cl + 1];
+      wk.rot = sched.dc_rot[cl];
     }
     return wk;
   };
@@ -462,17 +488,19 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
         auto load_mma1_unit = [&](int u) {       // stages of two slabs, n = 128
           for (int ks = 0; ks < oslabs; ks += 2) load_k(tm_k, u * kUnit, kUnit / CG, ks, min(2, oslabs - ks));
         };
+        const int u0 = wk.unit(0, s0, s1), nun = s1 - s0;
         if (kInterleaveFill) {
           for (int ks = 0; ks < oslabs; ks += 2) {
             const int n = min(2, oslabs - ks);
             for (int q = 0; q < n; ++q) load_own(ks + q);
-            load_k(tm_k, s0 * kUnit, kUnit / CG, ks, n);
+            load_k(tm_k, u0 * kUnit, kUnit / CG, ks, n);
           }
         } else {
-          load_mma1_unit(s0);
+          load_mma1_unit(u0);
         }
-        for (int u = s0; u < s1; ++u) {
-          if (u + 1 < s1) load_mma1_unit(u + 1);
+        for (int i = 0; i < nun; ++i) {
+          const int u = wk.unit(i, s0, s1);
+          if (i + 1 < nun) load_mma1_unit(wk.unit(i + 1, s0, s1));
           for (int kc = 0; kc < kUnit / kM2; ++kc) load_mn(tm_mn, u * kUnit + kc * kM2);
         }
       }
@@ -634,19 +662,19 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
           __syncwarp();
         } else {
           mma1_unit(it, true);
-          for (int u = s0; u < s1; ++u, ++it) {
-            if (u + 1 < s1) {
+          for (int i = 0; i < s1 - s0; ++i, ++it) {
+            if (i + 1 < s1 - s0) {
               mma1_unit(it + 1, false);
             } else {
               if (elect_one()) commit(BAR_A_EMPTY);
               __syncwarp();
             }
             tr.mark();   // MMA1(next) issued
-            if (u == s0 && sg > 0) { mbar_wait(bar(BAR_ACC_EMPTY), (sg - 1) & 1); tc_fence_after(); }
+            if (i == 0 && sg > 0) { mbar_wait(bar(BAR_ACC_EMPTY), (sg - 1) & 1); tc_fence_after(); }
             mbar_wait(bar(BAR_G_FULL + (it & 1)), (it >> 1) & 1);
             tc_fence_after();
             tr.mark();   // G landed
-            mma2_unit(it, u == s0);
+            mma2_unit(it, i == 0);
             tr.mark();   // MMA2 issued
           }
           if (elect_one()) commit(BAR_ACC_FULL);
@@ -678,7 +706,7 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
     // forward kernel in front of it (SPLIT: the probabilities must be normalised BEFORE they are cut into
     // fp16 planes, so the log-sum-exp has to be known when pass 1 starts)
     const bool close_here = kBwd && !kSplit && (p.phases & PASS_ROWS);
-    Tracer<DBG> tr((trow == 0 && half == 0) ? p.trace : nullptr, 2);
+    Tracer<DBG> tr((trow == 0 && half == 0) ? p.trace : nullptr, 2, kBwd ? 3 : 0);
     tr.mark();
     // epilogue -> MMA signals go to the leader CTA of the pair
     const uint32_t s_empty0 = lbar(BAR_S_EMPTY), g_full0 = lbar(BAR_G_FULL), acc_empty = lbar(BAR_ACC_EMPTY);
@@ -718,29 +746,41 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
       if (p.zero_n4 > 0) zfill(p.zero_base, p.zero_n4);
       if (p.zero2_n4 > 0) zfill(p.zero2_base, p.zero2_n4);
       if (close_here) zfill(reinterpret_cast<float4*>(p.rowsum), (p.n_own[SEG_DE] + 3) / 4);
+      if (et == 0) tail->rows_all_done = 0;
       __threadfence();
       named_bar_sync(1, kEpiThreads);
       if (et == 0) atomicAdd(p.ctr, 1);
     }
 
-    // STEP: between the passes.  Grid-wide barrier (every row sum complete), then each CTA closes a slice
-    // of the rows: log-sum-exp, row loss, q = 1 - p_jj, the factor of the un-normalised dE_hat row; the
-    // diagonal terms of dw and the closed-form db (SURVEY 8(a-bis) items 8, 12) ride along.
+    // STEP: closing a row -- log-sum-exp, row loss, q = 1 - p_jj, the factor of the un-normalised dE_hat row; the
+    // diagonal terms of dw and the closed-form db (SURVEY 8(a-bis) items 8, 12) ride along.  close_here: once per
+    // utterance tile, by the CTA whose pass-1 segment completes the tile's row sums (close_tile); otherwise every
+    // CTA closes a grid-strided slice of rows whose statistics an earlier launch wrote (close_rows).
     int lift2 = kSplitLift;      // SPLIT pass 2: exponent of the probability planes (set by close_rows)
-    bool arrived = false;        // this CTA's row sums are out and counted at the grid barrier
-    auto arrive_pass1 = [&]() {
-      named_bar_sync(1, kEpiThreads);      // every thread's row-sum atomics have returned
-      if (et == 0) { __threadfence(); atomicAdd(p.ctr + 2, 1); }
-      arrived = true;
-      tr.mark();   // arrived at the grid barrier
+    auto close_row = [&](int r) {
+      const float cdv = __ldg(p.cos_diag + r);
+      float stat, q;
+      if (close_here) {
+        const RowClose rc = close_softmax_row_log2(m2, __ldcg(p.rowsum + r), fmaf(cdv, w2, b2),
+                                                   fmaf(w, cdv + eps, b), eps);      // s3:120-121
+        stat = rc.stat; q = rc.q;
+        p.row_stat_out[r] = stat;
+        p.row_aux_out[r] = q;
+        p.row_scale_out[r] = w / rc.z;      // = w exp(m - lse_r)
+        if (p.per_row_out != nullptr) p.per_row_out[r] = rc.per;
+        loss_acc += rc.per;
+      } else {
+        stat = __ldg(p.row_stat + r);
+        q = __ldg(p.row_aux + r);
+        if (kSplit && (p.phases & PASS_ROWS))      // dE_hat row r was formed from p * 2^(14 + k_r)
+          p.row_scale_out[r] = w * exp2f(static_cast<float>(-(kSplitLift + split_extra_lift(q))));
+      }
+      if (p.phases & PASS_CENTROIDS) {
+        dw_acc = fmaf(-q, cdv + eps, dw_acc);     // diagonal element G_jj = -g q (uses cos_diag)
+        db_acc -= eps * expf(-stat);              // item 12: db = -g sum eps / (sum exp + eps)
+      }
     };
     auto close_rows = [&]() {
-      if (close_here) {
-        if (!arrived) arrive_pass1();      // a cluster without pass-1 work
-        if (et == 0) spin_until(p.ctr + 2, static_cast<int>(gridDim.x));
-        named_bar_sync(1, kEpiThreads);
-      }
-      tr.mark();   // grid barrier passed
       const int U = p.n_own[SEG_DE];
       if (kSplit && (p.phases & PASS_CENTROIDS)) {
         // pass 2's lift: every CTA takes the maximum of q over ALL rows (U floats out of the L2)
@@ -754,38 +794,40 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
         lift2 = kSplitLift + split_extra_lift(qm);
         named_bar_sync(1, kEpiThreads);      // red is reused by the scalar reductions
       }
-      for (int r = blockIdx.x * kEpiThreads + et; r < U; r += gridDim.x * kEpiThreads) {
-        const float cdv = __ldg(p.cos_diag + r);
-        float stat, q;
-        if (close_here) {
-          const RowClose rc = close_softmax_row_log2(m2, __ldcg(p.rowsum + r), fmaf(cdv, w2, b2),
-                                                     fmaf(w, cdv + eps, b), eps);      // s3:120-121
-          stat = rc.stat; q = rc.q;
-          p.row_stat_out[r] = stat;
-          p.row_aux_out[r] = q;
-          p.row_scale_out[r] = w / rc.z;      // = w exp(m - lse_r)
-          if (p.per_row_out != nullptr) p.per_row_out[r] = rc.per;
-          loss_acc += rc.per;
-        } else {
-          stat = __ldg(p.row_stat + r);
-          q = __ldg(p.row_aux + r);
-          if (kSplit && (p.phases & PASS_ROWS))      // dE_hat row r was formed from p * 2^(14 + k_r)
-            p.row_scale_out[r] = w * exp2f(static_cast<float>(-(kSplitLift + split_extra_lift(q))));
-        }
-        if (p.phases & PASS_CENTROIDS) {
-          dw_acc = fmaf(-q, cdv + eps, dw_acc);     // diagonal element G_jj = -g q (uses cos_diag)
-          db_acc -= eps * expf(-stat);              // item 12: db = -g sum eps / (sum exp + eps)
-        }
-      }
+      for (int r = blockIdx.x * kEpiThreads + et; r < U; r += gridDim.x * kEpiThreads) close_row(r);
       tr.mark();   // rows closed
     };
+    // close_here, pass 2: stream unit u is utterance tile u (kUnit == kTile), its row sums are final once every
+    // pass-1 segment of that tile has counted its units into seg_done[u].  No deadlock: pass-1 work never waits
+    // on pass 2 (a CTA's pass-1 segments precede its pass-2 segments, the TMA and MMA warps need no row
+    // statistics), and every CTA of the grid is co-resident (max_clusters).
+    static_assert(kUnit == kTile, "a pass-2 stream unit must be exactly one pass-1 owner tile");
+    unsigned long long ready_wait_ns = 0;      // DBG: time this thread spent waiting for row sums
+    // ctr[2] counts complete tiles: once a CTA has seen all of them, its pass-2 units need no acquire load
+    // in front of their row-sum loads (most of pass 2 at large shapes)
+    auto tile_ready = [&](int u) {
+      if (*reinterpret_cast<volatile int*>(&tail->rows_all_done) != 0) return true;
+      int v;
+      asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p.ctr + 2) : "memory");
+      if (v >= p.OT[SEG_DE]) { tail->rows_all_done = 1; return true; }
+      asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p.seg_done + u) : "memory");
+      return v >= p.ST[SEG_DE];
+    };
+    auto wait_tile = [&](int u) {
+      if (tile_ready(u)) return;
+      const unsigned long long t0 = DBG ? globaltimer_ns() : 0ull;
+      spin_until(p.seg_done + u, p.ST[SEG_DE]);
+      if (DBG) ready_wait_ns += globaltimer_ns() - t0;
+    };
     bool closed = false;
+    int sg_dc0 = -1;             // DBG: first pass-2 segment
 
     Walk wk = make_walk();
     int kind, og, s0, s1;
     for (int sg = 0; wk.next(p, kind, og, s0, s1); ++sg) {
       const bool is_dc = kBwd && kind == SEG_DC;       // CTA-uniform
-      if (kBwd && is_dc && !closed) { close_rows(); closed = true; }
+      if (kBwd && !close_here && is_dc && !closed) { close_rows(); closed = true; }
+      if (DBG && is_dc && sg_dc0 < 0) { sg_dc0 = sg; tr.put(kTraceEvents - 2, globaltimer_ns()); }   // pass 2 begins
       const int n_str = p.n_str[kind];
       const int ot = og * CG + cr;
       const bool tile_valid = ot < p.OT[kind];         // CTA-uniform
@@ -830,21 +872,32 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
         c0r = ovalid ? (b2 + static_cast<float>(kSplitLift + split_extra_lift(__ldg(p.row_aux + orow)))) -
                            __ldg(p.row_stat + orow) * kLog2e
                      : -INFINITY;
-      if (is_dc && half == 0) {
+      // lse_s[buf] of unit u, loaded when this unit's turn comes (close_here: once its row sums are final)
+      auto stage_lse = [&](int u, int buf) {
+        if (close_here) wait_tile(u);
         float raw = 0.f, cdv = 0.f;
-        const bool v0 = lse2_raw(s0 * kUnit + trow, raw, cdv);
-        tail->lse_s[it & 1][trow] = lse2_of(v0, raw, cdv);
-      }
+        const bool v = lse2_raw(u * kUnit + trow, raw, cdv);
+        tail->lse_s[buf][trow] = lse2_of(v, raw, cdv);
+      };
+      if (is_dc && half == 0) stage_lse(wk.unit(0, s0, s1), it & 1);
+      bool deferred = false;     // the next unit's row sums were not final at prefetch time: staged at its turn
 
-      for (int u = s0; u < s1; u += kStepUnits, ++it) {
-        const int nu = min(kStepUnits, s1 - u);
+      for (int i = 0; i < s1 - s0; i += kStepUnits, ++it) {
+        const int u = wk.unit(i, s0, s1);
+        const int nu = min(kStepUnits, s1 - s0 - i);
         const int buf = it & 1;
         float nraw = 0.f, ncd = 0.f;
         bool nvalid = false;
         if (is_dc) {
-          named_bar_sync(1, kEpiThreads);      // lse_s[buf] staged (by the previous unit, or above)
-          // the next unit's raw inputs travel while this unit is processed
-          if (half == 0 && u + 1 < s1) nvalid = lse2_raw((u + 1) * kUnit + trow, nraw, ncd);
+          if (half == 0 && deferred) { stage_lse(u, buf); deferred = false; }
+          named_bar_sync(1, kEpiThreads);      // lse_s[buf] staged (by the previous unit, above, or just now)
+          // the next unit's raw inputs travel while this unit is processed -- if its row sums are final already:
+          // a poll, never a wait, so that a late tile holds up its own unit only
+          if (half == 0 && i + 1 < s1 - s0) {
+            const int un = wk.unit(i + 1, s0, s1);
+            if (!close_here || tile_ready(un)) nvalid = lse2_raw(un * kUnit + trow, nraw, ncd);
+            else deferred = true;
+          }
         }
         mbar_wait(bar(BAR_S_FULL + buf), (it >> 1) & 1);
         tc_fence_after();
@@ -981,7 +1034,7 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
           __syncwarp();
           if (lane == 0) arrive_leader(s_empty0 + 8u * buf);
         } else {
-          if (is_dc && half == 0 && u + 1 < s1) tail->lse_s[buf ^ 1][trow] = lse2_of(nvalid, nraw, ncd);
+          if (is_dc && half == 0 && i + 1 < s1 - s0 && !deferred) tail->lse_s[buf ^ 1][trow] = lse2_of(nvalid, nraw, ncd);
           tmem_st_wait();
           tc_fence_before();
           __syncwarp();
@@ -1060,8 +1113,8 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
         }
       } else {
         // pass 1: the row sums are final once the last tile has been consumed -- they do not wait for the
-        // accumulator; after the cluster's last pass-1 segment the CTA arrives at the grid barrier BEFORE
-        // it flushes, so the flush runs under the barrier's skew instead of in front of it
+        // accumulator; the segment counts its units into the tile's counter and the CTA that completes the tile
+        // closes its rows, all while the last MMA2 of the segment runs
         if (!is_dc && !close_here) {
           // SPLIT (or a lone pass 1 never happens without close_here in TF32): nothing to publish
         } else if (!is_dc) {
@@ -1073,7 +1126,24 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
             const float old = atomicAdd(p.rowsum + orow, rs_acc);
             asm volatile("" ::"f"(old));
           }
-          if (wk.kind == SEG_DE && wk.gp >= wk.end) arrive_pass1();
+          // value-returning atomics: when the old value is back the add has been performed at the L2, so the
+          // release below needs one fence, not one per thread
+          named_bar_sync(1, kEpiThreads);
+          if (et == 0) {
+            bool last = false;
+            if (tile_valid) {
+              __threadfence();
+              last = atomicAdd(p.seg_done + ot, s1 - s0) + (s1 - s0) == p.ST[SEG_DE];
+              if (last) { __threadfence(); atomicAdd(p.ctr + 2, 1); }
+            }
+            tail->flag = last;
+          }
+          named_bar_sync(1, kEpiThreads);
+          if (tail->flag != 0) {      // CTA-uniform; tail->flag is rewritten after the flush's barrier only
+            __threadfence();          // acquire: every other segment's row sums of this tile are visible
+            if (et < kTile && ot * kTile + et < p.n_own[SEG_DE]) close_row(ot * kTile + et);
+          }
+          if (DBG && wk.kind == SEG_DE && wk.gp >= wk.end) tr.put(kTraceEvents - 3, globaltimer_ns());   // pass 1 out
         } else if (ovalid) {
           dw_acc += kSplit ? dw_seg * exp2f(static_cast<float>(-lift2)) : dw_seg;
         }
@@ -1140,7 +1210,8 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
       }
       tr.mark();   // segment flushed
     }
-    if (kBwd && !closed) close_rows();     // no pass-2 segment in this cluster (or pass 1 alone)
+    if (kBwd && !close_here && !closed) close_rows();     // no pass-2 segment in this cluster (or pass 1 alone)
+    if (DBG && kBwd) tr.put(kTraceEvents - 1, ready_wait_ns);
 
     // ------------------------------------------------------------ scalar reductions (once per CTA)
     if (!kBwd) {
@@ -1166,11 +1237,15 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
         if (close_here) atomicAdd(p.loss_accum, tl);
         if (p.phases & PASS_CENTROIDS) { atomicAdd(p.dwdb + 0, tw); atomicAdd(p.dwdb + 1, tb); }
         if (p.stamps != nullptr) p.stamps[2 * blockIdx.x + 1] = globaltimer_ns();
-        // last CTA out restores the counters
-        if (atomicAdd(p.ctr + 1, 1) == static_cast<int>(gridDim.x) - 1) {
-          atomicExch(p.ctr, 0); atomicExch(p.ctr + 1, 0); atomicExch(p.ctr + 2, 0);
-        }
+        // last CTA out restores the counters: every other CTA has counted its pass-1 units and read the tile
+        // counters for the last time before its own arrival here
+        const bool last_out = atomicAdd(p.ctr + 1, 1) == static_cast<int>(gridDim.x) - 1;
+        if (last_out) { atomicExch(p.ctr, 0); atomicExch(p.ctr + 1, 0); atomicExch(p.ctr + 2, 0); }
+        tail->flag = last_out;
       }
+      named_bar_sync(1, kEpiThreads);
+      if (close_here && tail->flag != 0)
+        for (int t = et; t < p.OT[SEG_DE]; t += kEpiThreads) p.seg_done[t] = 0;
     }
   }
 
@@ -1465,22 +1540,191 @@ bool cut_pass(long long GP, int OG, int ST, int NC, const double* delay, int* ou
   return true;
 }
 
-int make_step_sched(int OGe, int STe, int OGc, int STc, int phases, int max_cl, StepSched* S, bool* de_partial,
-                    bool* dc_partial) {
+// Model of one step-kernel launch whose pass 1 closes the rows (TF32 / HYB, both passes), in units of one stream
+// unit's work.  Cluster c runs its pass-1 range first; a pass-1 segment ends `len` units (plus kStraddle when it is
+// not the cluster's first) after the previous one, and the utterance tiles of its owner group are complete when
+// the last segment touching them ends.  Pass 2 starts at load1[c] + kPassSwitch (accumulator drain, pass-2 owner
+// tile load: what the MMA warp waits for before the first pass-2 tile) and a pass-2 unit cannot be consumed before
+// its utterance tile is complete.  kPassSwitch: 6.7 us from "row sums out" to the first pass-2 tile against 2.66 us
+// per stream unit at cfg3 (instrumented trace, B200 at 1000 W, profiles/r5_step_dataflow).
+constexpr double kPassSwitch = 2.5;
+
+struct StepModel {
+  int NC = 0;
+  double start2[kMaxClusters];    // pass-2 start of every cluster
+  std::vector<double> ready;      // [STc] time utterance tile t is complete
+};
+
+void model_pass1(const int* de, int NC, int OGe, int STe, int cg, int STc, StepModel* m) {
+  (void)OGe;
+  m->NC = NC;
+  m->ready.assign(STc, 0.0);
+  for (int c = 0; c < NC; ++c) {
+    double t = 0;
+    for (long long gp = de[c]; gp < de[c + 1];) {
+      const long long og = gp / STe, end = std::min<long long>(de[c + 1], (og + 1) * STe);
+      t += static_cast<double>(end - gp) + (gp > de[c] ? kStraddle : 0);
+      for (int k = 0; k < cg; ++k) {
+        const long long tile = og * cg + k;
+        if (tile < STc) m->ready[tile] = std::max(m->ready[tile], t);
+      }
+      gp = end;
+    }
+    m->start2[c] = de[c + 1] > de[c] ? t + kPassSwitch : 0.0;
+  }
+}
+
+// finish time of cluster c walking pass-2 pairs [a, b) (units visited from a + rot on, wrapping in one group)
+double model_finish(const StepModel& m, int c, long long a, long long b, int STc, int rot) {
+  double t = m.start2[c];
+  const long long n = b - a;
+  for (long long i = 0; i < n; ++i) {
+    long long gp = a + i + rot;
+    if (gp >= b) gp -= n;
+    if (i > 0 && gp / STc != (gp - 1) / STc && rot == 0) t += kStraddle;
+    t = std::max(t, m.ready[gp % STc]) + 1.0;
+  }
+  return t;
+}
+
+// rotation that visits the last-completed tile of a one-group range last (0 when the range spans groups)
+int best_rotation(const StepModel& m, long long a, long long b, int STc) {
+  if (b - a < 2 || a / STc != (b - 1) / STc) return 0;
+  long long late = a;
+  for (long long gp = a; gp < b; ++gp)
+    if (m.ready[gp % STc] >= m.ready[late % STc]) late = gp;
+  return static_cast<int>((late + 1 - a) % (b - a));
+}
+
+// Pass-2 cut for a makespan target T: clusters in order take pairs while their predicted finish stays within T --
+// in order for a range that spans groups, else with the last-completed tiles visited last (best_rotation).  A range
+// touches at most two owner groups when a group is no shorter than the level share.
+bool greedy_pass2(const StepModel& m, long long GP, int STc, double T, int* out) {
+  const int NC = m.NC;
+  const long long level = (GP + NC - 1) / NC;
+  long long gp = 0;
+  for (int c = 0; c < NC; ++c) {
+    out[c] = static_cast<int>(gp);
+    double late = -1, t_in = m.start2[c];
+    long long n = 0, nlate = 0;
+    bool crossed = false;
+    while (gp < GP) {
+      const bool cross = n > 0 && gp % STc == 0;
+      if (cross && STc >= level && crossed) break;    // a third group
+      const double r = m.ready[gp % STc];
+      const double t1 = std::max(t_in + (cross ? kStraddle : 0), r) + 1.0;
+      const double l = std::max(late, r);
+      const long long nl = (r > late) ? 1 : nlate + (r == late ? 1 : 0);
+      const double est = (crossed || cross) ? t1 : std::max(m.start2[c] + static_cast<double>(n + 1), l + nl);
+      if (est > T) break;
+      crossed = crossed || cross; t_in = t1; late = l; nlate = nl; ++n; ++gp;
+    }
+  }
+  out[NC] = static_cast<int>(GP);
+  return gp == GP;
+}
+
+double model_makespan(const StepModel& m, const int* dc, int STc, const unsigned char* rot, double* finish) {
+  double worst = 0;
+  for (int c = 0; c < m.NC; ++c) {
+    const double f = std::max(m.start2[c], model_finish(m, c, dc[c], dc[c + 1], STc, rot[c]));
+    if (finish != nullptr) finish[c] = f;
+    worst = std::max(worst, f);
+  }
+  return worst;
+}
+
+// the barrier version's schedule: pass 2 cut with `delay` for the clusters that finish pass 1 within kStraddle
+// units of the busiest one (they flushed after the barrier instead of under it)
+bool cut_pass2_barrier(const int* de, int NC, long long GPe, long long GPc, int OGc, int STc, int* dc) {
+  double delay[kMaxClusters];
+  long long busiest = 0;
+  for (int c = 0; c < NC; ++c) busiest = std::max<long long>(busiest, de[c + 1] - de[c]);
+  for (int c = 0; c < NC; ++c) {
+    const long long load = de[c + 1] - de[c];
+    delay[c] = (GPe > 0 && load > 0) ? std::max<double>(0.0, kStraddle - static_cast<double>(busiest - load)) : 0.0;
+  }
+  return cut_pass(GPc, OGc, STc, NC, GPe > 0 ? delay : nullptr, dc);
+}
+
+struct SchedKey {
+  int OGe, STe, OGc, STc, phases, max_cl, cg, rows_closed;
+  bool operator==(const SchedKey& o) const {
+    return OGe == o.OGe && STe == o.STe && OGc == o.OGc && STc == o.STc && phases == o.phases &&
+           max_cl == o.max_cl && cg == o.cg && rows_closed == o.rows_closed;
+  }
+};
+struct SchedEntry { SchedKey key; StepSched S; int NC; bool dep, dcp; };
+thread_local SchedEntry g_sched[4];
+thread_local int g_sched_used = 0, g_sched_next = 0;
+
+// rows_closed: pass 1 closes the rows in the launch (TF32 / HYB) -- pass 2 waits per utterance tile, and the
+// pass-2 cut follows the model above; otherwise (SPLIT, rows closed by the forward kernel) the cut of the
+// barrier version is kept.  model_finish (nullable): the model's per-cluster finish times of the result.
+int make_step_sched(int OGe, int STe, int OGc, int STc, int phases, int max_cl, int cg, bool rows_closed,
+                    StepSched* S, bool* de_partial, bool* dc_partial, double* model_out = nullptr,
+                    double* barrier_makespan = nullptr) {
+  const SchedKey key{OGe, STe, OGc, STc, phases, max_cl, cg, rows_closed ? 1 : 0};
+  if (model_out == nullptr && barrier_makespan == nullptr)
+    for (int i = 0; i < g_sched_used; ++i)
+      if (g_sched[i].key == key) {
+        *S = g_sched[i].S; *de_partial = g_sched[i].dep; *dc_partial = g_sched[i].dcp;
+        return g_sched[i].NC;
+      }
   const long long GPe = (phases & PASS_ROWS) ? static_cast<long long>(OGe) * STe : 0;
   const long long GPc = (phases & PASS_CENTROIDS) ? static_cast<long long>(OGc) * STc : 0;
   const int NC = static_cast<int>(std::max<long long>(1, std::min<long long>(max_cl, std::max(GPe, GPc))));
+  std::memset(S->dc_rot, 0, sizeof(S->dc_rot));
   *de_partial = cut_pass(GPe, OGe, STe, NC, nullptr, S->de);
-  // pass 2 starts at the grid barrier, i.e. when the busiest cluster of pass 1 is done; whoever finishes
-  // pass 1 within ~kStraddle units of that moment still has its own flush in front of it
-  double delay[kMaxClusters];
-  long long busiest = 0;
-  for (int c = 0; c < NC; ++c) busiest = std::max<long long>(busiest, S->de[c + 1] - S->de[c]);
-  for (int c = 0; c < NC; ++c) {
-    const long long load = S->de[c + 1] - S->de[c];
-    delay[c] = (GPe > 0 && load > 0) ? std::max<double>(0.0, kStraddle - static_cast<double>(busiest - load)) : 0.0;
+  const bool both = phases == (PASS_ROWS | PASS_CENTROIDS);
+  *dc_partial = cut_pass2_barrier(S->de, NC, both ? GPe : 0, GPc, OGc, STc, S->dc);
+  // The model cut costs ~24 greedy passes over the pair list (46 us of host time at cfg3, 4 ms at cfg4 when every
+  // cluster carries ~443 units a pass); past 64 units per cluster the transition and the readiness waits are a few
+  // percent of a pass at most, and the barrier version's cut is walked without the barrier.
+  if (both && rows_closed) {
+    StepModel m;
+    model_pass1(S->de, NC, OGe, STe, cg, STc, &m);
+    if (barrier_makespan != nullptr) {
+      // the barrier version: pass 2 of cluster c started at max(busiest pass 1, its own + kPassSwitch)
+      StepModel mb = m;
+      double p1 = 0;
+      for (int c = 0; c < NC; ++c) p1 = std::max(p1, mb.start2[c] - kPassSwitch);
+      for (int c = 0; c < NC; ++c) mb.start2[c] = std::max(p1, mb.start2[c]);
+      std::fill(mb.ready.begin(), mb.ready.end(), 0.0);
+      *barrier_makespan = model_makespan(mb, S->dc, STc, S->dc_rot, nullptr);
+    }
+    // candidate 1: the barrier version's cut, walked in order without the barrier
+    double best = model_makespan(m, S->dc, STc, S->dc_rot, nullptr);
+    // candidate 2: the smallest makespan target the greedy cut meets (bisection)
+    int cand[kMaxClusters + 1];
+    unsigned char rot[kMaxClusters];
+    double lo = 0, hi = best;
+    for (int c = 0; c < NC; ++c) lo = std::max(lo, std::min(m.start2[c], hi));
+    lo = std::max(lo, static_cast<double>(GPc) / NC);
+    const bool small = GPc <= 64LL * NC;
+    for (int iter = 0; small && iter < 24 && hi - lo > 0.02; ++iter) {
+      const double mid = 0.5 * (lo + hi);
+      if (greedy_pass2(m, GPc, STc, mid, cand)) hi = mid; else lo = mid;
+    }
+    if (small && greedy_pass2(m, GPc, STc, hi, cand)) {
+      for (int c = 0; c < NC; ++c) rot[c] = static_cast<unsigned char>(std::min(255, best_rotation(m, cand[c], cand[c + 1], STc)));
+      for (int c = 0; c < NC; ++c)
+        if (cand[c + 1] - cand[c] > 255) rot[c] = 0;
+      const double got = model_makespan(m, cand, STc, rot, nullptr);
+      if (got < best) {
+        best = got;
+        std::memcpy(S->dc, cand, sizeof(int) * (NC + 1));
+        std::memcpy(S->dc_rot, rot, sizeof(rot[0]) * NC);
+        *dc_partial = false;
+        for (int c = 0; c <= NC; ++c) *dc_partial |= (S->dc[c] % STc) != 0;
+      }
+    }
+    if (model_out != nullptr) model_makespan(m, S->dc, STc, S->dc_rot, model_out);
   }
-  *dc_partial = cut_pass(GPc, OGc, STc, NC, (phases == (PASS_ROWS | PASS_CENTROIDS)) ? delay : nullptr, S->dc);
+  SchedEntry& e = g_sched[g_sched_next];
+  e.key = key; e.S = *S; e.NC = NC; e.dep = *de_partial; e.dcp = *dc_partial;
+  g_sched_next = (g_sched_next + 1) % 4;
+  g_sched_used = std::min(g_sched_used + 1, 4);
   return NC;
 }
 
@@ -1575,10 +1819,25 @@ int tc_debug_step_schedule(int u_local, int n_total, int cg, int max_clusters, i
   StepSched S{};
   bool dep = false, dcp = false;
   const int NC = make_step_sched((OTe + cg - 1) / cg, STe, (OTc + cg - 1) / cg, STc, PASS_ROWS | PASS_CENTROIDS,
-                                 max_clusters, &S, &dep, &dcp);
+                                 max_clusters, cg, true, &S, &dep, &dcp);
   for (int c = 0; c <= NC; ++c) { de_begin[c] = S.de[c]; dc_begin[c] = S.dc[c]; }
   partial[0] = dep ? 1 : 0; partial[1] = dcp ? 1 : 0;
   units[0] = (OTe + cg - 1) / cg; units[1] = STe; units[2] = (OTc + cg - 1) / cg; units[3] = STc;
+  return NC;
+}
+
+int tc_debug_step_model(int u_local, int n_total, int cg, int max_clusters, int* dc_rot, double* finish,
+                        double* model) {
+  if (u_local <= 0 || n_total <= 0 || (cg != 1 && cg != 2) || max_clusters <= 0 || max_clusters > kMaxClusters)
+    return GE2E_ERR_ARGUMENT;
+  const int OTe = (u_local + kTile - 1) / kTile, STe = (n_total + kUnit - 1) / kUnit;
+  const int OTc = (n_total + kTile - 1) / kTile, STc = (u_local + kUnit - 1) / kUnit;
+  StepSched S{};
+  bool dep = false, dcp = false;
+  const int NC = make_step_sched((OTe + cg - 1) / cg, STe, (OTc + cg - 1) / cg, STc, PASS_ROWS | PASS_CENTROIDS,
+                                 max_clusters, cg, true, &S, &dep, &dcp, finish, &model[1]);
+  for (int c = 0; c < NC; ++c) dc_rot[c] = S.dc_rot[c];
+  model[0] = kPassSwitch;
   return NC;
 }
 
@@ -1694,7 +1953,7 @@ int tc_step(const RowsArgs& a, int phases, const float* grad_out, const float* r
   StepSched sched{};
   bool de_partial = false, dc_partial = false;
   const int NC = make_step_sched((p.OT[SEG_DE] + cg - 1) / cg, p.ST[SEG_DE], (p.OT[SEG_DC] + cg - 1) / cg, p.ST[SEG_DC],
-                                 phases, max_cl, &sched, &de_partial, &dc_partial);
+                                 phases, max_cl, cg, !split, &sched, &de_partial, &dc_partial);
   // outputs assembled from partial accumulators (TMA reduce-add) are zero-filled by the kernel itself;
   // D % 32 == 0 makes every row a whole number of float4
   if ((phases & PASS_CENTROIDS) && dc_partial && !peers) {
@@ -1708,6 +1967,9 @@ int tc_step(const RowsArgs& a, int phases, const float* grad_out, const float* r
   p.ctr = static_cast<int*>(ws);
   const Layout L = fwd_layout(U, a.n_total, a.D, a.variant);
   p.rowsum = reinterpret_cast<float*>(static_cast<uint8_t*>(ws) + kWsHeaderBytes + L.done_bytes + L.part_bytes);
+  // per-utterance-tile pass-1 counters: the forward kernel's stream-K counters (OT = the same U rows), zero on
+  // entry and exit of either kernel
+  p.seg_done = reinterpret_cast<int*>(static_cast<uint8_t*>(ws) + kWsHeaderBytes);
   // {dw, db} accumulate: zeroed by prep when the passes run in one step; a lone backward clears them here
   if (phases == PASS_CENTROIDS) GE2E_CUDA_TRY(cudaMemsetAsync(dwdb_accum, 0, 2 * sizeof(float), st));
 
