@@ -456,6 +456,31 @@ int ge2e_b200_forward_backward_typed(const void* E, int e_dtype, const int32_t* 
                                      float* accum, float* dE_hat, float* dC_hat, void* dE, int de_dtype,
                                      void* workspace, size_t workspace_bytes, ge2e_stream_t stream);
 
+/* ---- per-utterance losses (reduction "none") ---------------------------------------------
+ * L_r, the loss of utterance row r in logical [speaker][utterance] order (calc_loss's per_embedding_loss, s3:121):
+ *   softmax  log(sum_k exp S_rk + eps) - S_rj        contrast  1 - sigmoid(S_rj) + max_{k != j} sigmoid(S_rk)
+ * ge2e_b200_forward_per_row_typed: ge2e_b200_forward_typed that also writes per_row[N*M] (device, required);
+ *   accum[0] is still the sum.
+ * ge2e_b200_backward_per_row_typed: ge2e_b200_backward_typed for the upstream gradient grad_rows[N*M] (device, logical
+ *   order, required; any values, negative and zero included) in place of the scalar grad_out:
+ *   dE = sum_r grad_rows[r] dL_r / dE, accum[1] = dw, accum[2] = db likewise; dE is rounded to de_dtype once.
+ * A NULL per_row / grad_rows returns GE2E_ERR_ARGUMENT before anything is launched.  The upstream gradient is known
+ * only after the forward, so these run the staged kernels (forward, then backward) on every shape: the single-kernel
+ * step and the whole-step-in-forward scheme (ge2e_b200_forward_backward with grad_out = 1, then
+ * ge2e_b200_scale_grads) have no per-row form, nor have the speaker-sharded entry points. */
+int ge2e_b200_forward_per_row_typed(const void* E, int e_dtype, const int32_t* row_index, int N, int M, int D,
+                                    const float* w, const float* b, float eps, int variant, int precision, float* e_hat,
+                                    float* c_hat, float* cos_diag, float* row_stat, int32_t* row_kstar, float* row_aux,
+                                    float* accum, float* dE_hat, float* row_scale, float* per_row, void* workspace,
+                                    size_t workspace_bytes, ge2e_stream_t stream);
+int ge2e_b200_backward_per_row_typed(const void* E, int e_dtype, const int32_t* row_index, const float* e_hat,
+                                     const float* c_hat, const float* cos_diag, const float* row_stat,
+                                     const int32_t* row_kstar, const float* row_aux, const float* row_scale, int N,
+                                     int M, int D, const float* w, const float* b, float eps, int variant,
+                                     int precision, const float* grad_rows, float* dE_hat, float* dC_hat, float* accum,
+                                     void* dE, int de_dtype, void* workspace, size_t workspace_bytes,
+                                     ge2e_stream_t stream);
+
 /* ---- static helpers of the reference class (used by s5_eval_model.py:42-43) ----------- */
 
 /* get_centroids (s3:33-38): C[N, D] = mean over utterances. */

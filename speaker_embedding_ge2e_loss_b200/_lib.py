@@ -132,6 +132,13 @@ PROTOTYPES = {
                                                    C.c_float, C.c_int, C.c_int, _f32p, _f32p, _f32p, _f32p, _f32p,
                                                    _i32p, _f32p, _f32p, _f32p, _f32p, _f32p, C.c_void_p, C.c_int,
                                                    C.c_void_p, C.c_size_t, _stream]),
+    "ge2e_b200_forward_per_row_typed": (C.c_int, [C.c_void_p, C.c_int, _i32p, C.c_int, C.c_int, C.c_int, _f32p, _f32p,
+                                                  C.c_float, C.c_int, C.c_int, _f32p, _f32p, _f32p, _f32p, _i32p, _f32p,
+                                                  _f32p, _f32p, _f32p, _f32p, C.c_void_p, C.c_size_t, _stream]),
+    "ge2e_b200_backward_per_row_typed": (C.c_int, [C.c_void_p, C.c_int, _i32p, _f32p, _f32p, _f32p, _f32p, _i32p, _f32p,
+                                                   _f32p, C.c_int, C.c_int, C.c_int, _f32p, _f32p, C.c_float, C.c_int,
+                                                   C.c_int, _f32p, _f32p, _f32p, _f32p, C.c_void_p, C.c_int, C.c_void_p,
+                                                   C.c_size_t, _stream]),
     "ge2e_b200_centroids": (C.c_int, [_f32p, C.c_int, C.c_int, C.c_int, _f32p, _stream]),
     "ge2e_b200_utterance_centroids": (C.c_int, [_f32p, C.c_int, C.c_int, C.c_int, _f32p, _stream]),
     "ge2e_b200_normalize_rows": (C.c_int, [_f32p, C.c_int, C.c_int, _f32p, _stream]),

@@ -169,12 +169,12 @@ static int fwd_rows_impl(const float* e_hat, const float* c_hat_all, const float
       rc = tc_fwd_rows(a, row_stat, row_kstar, row_aux, loss_accum, per_row_out, workspace, workspace_bytes, after_prep,
                        (cudaStream_t)stream, tc_prec(precision));
       if (rc != GE2E_OK || dE_hat == nullptr || row_scale == nullptr) return rc;
-      return tc_step(a, 1, nullptr, row_stat, row_aux, nullptr, nullptr, row_scale, nullptr, nullptr, dE_hat, nullptr,
+      return tc_step(a, 1, nullptr, nullptr, row_stat, row_aux, nullptr, nullptr, row_scale, nullptr, nullptr, dE_hat, nullptr,
                      nullptr, workspace, workspace_bytes, (cudaStream_t)stream, nullptr, 0, tc_prec(precision));
     }
     // softmax with a backward to follow: the rows pass of the step kernel (loss + un-normalised dE_hat)
     if (variant == GE2E_SOFTMAX && dE_hat != nullptr && row_scale != nullptr)
-      return tc_step(a, 1, nullptr, nullptr, nullptr, row_stat, row_aux, row_scale, loss_accum, per_row_out, dE_hat,
+      return tc_step(a, 1, nullptr, nullptr, nullptr, nullptr, row_stat, row_aux, row_scale, loss_accum, per_row_out, dE_hat,
                      nullptr, nullptr, workspace, workspace_bytes, (cudaStream_t)stream);
     return tc_fwd_rows(a, row_stat, row_kstar, row_aux, loss_accum, per_row_out, workspace, workspace_bytes,
                        after_prep, (cudaStream_t)stream);
@@ -194,14 +194,14 @@ int ge2e_b200_fwd_rows(const float* e_hat, const float* c_hat_all, const float* 
                        workspace, workspace_bytes, false, stream);
 }
 
-int ge2e_b200_bwd_rows(const float* e_hat, const float* c_hat_all, const float* cos_diag,
-                       const float* row_stat, const int32_t* row_kstar, const float* row_aux,
-                       const float* row_scale, int n_local, int n_total, int spk_offset, int M, int D,
-                       const float* w, const float* b, float eps,
-                       int variant, int precision, const float* grad_out, float* dE_hat,
-                       float* dC_hat_partial, float* dwdb_accum, void* workspace,
-                       size_t workspace_bytes, ge2e_stream_t stream) {
-  if (!e_hat || !c_hat_all || !cos_diag || !row_stat || !w || !b || !grad_out || !dE_hat ||
+// grad_rows (nullable): the upstream gradient per local utterance row, in place of the scalar grad_out
+static int bwd_rows_impl(const float* e_hat, const float* c_hat_all, const float* cos_diag, const float* row_stat,
+                         const int32_t* row_kstar, const float* row_aux, const float* row_scale, int n_local,
+                         int n_total, int spk_offset, int M, int D, const float* w, const float* b, float eps,
+                         int variant, int precision, const float* grad_out, const float* grad_rows, float* dE_hat,
+                         float* dC_hat_partial, float* dwdb_accum, void* workspace, size_t workspace_bytes,
+                         ge2e_stream_t stream) {
+  if (!e_hat || !c_hat_all || !cos_diag || !row_stat || !w || !b || (!grad_out && !grad_rows) || !dE_hat ||
       !dC_hat_partial || !dwdb_accum)
     return GE2E_ERR_ARGUMENT;
   int rc = check_shape(n_local, n_total, spk_offset, M, D);
@@ -219,20 +219,33 @@ int ge2e_b200_bwd_rows(const float* e_hat, const float* c_hat_all, const float* 
     if (workspace_bytes < tc_workspace_bytes(n_local, n_total, M, D, variant) ||
         (workspace == nullptr && tc_workspace_bytes(n_local, n_total, M, D, variant) > 0))
       return GE2E_ERR_WORKSPACE;
-    return tc_step(a, 2, grad_out, row_stat, row_aux, nullptr, nullptr, nullptr, nullptr, nullptr, dE_hat,
+    return tc_step(a, 2, grad_out, grad_rows, row_stat, row_aux, nullptr, nullptr, nullptr, nullptr, nullptr, dE_hat,
                    dC_hat_partial, dwdb_accum, workspace, workspace_bytes, (cudaStream_t)stream, nullptr, 0,
                    tc_prec(precision));
   }
-  return simt_bwd_rows(a, row_stat, row_kstar, row_aux, grad_out, dE_hat, dC_hat_partial, dwdb_accum,
+  return simt_bwd_rows(a, row_stat, row_kstar, row_aux, grad_out, grad_rows, dE_hat, dC_hat_partial, dwdb_accum,
                        (cudaStream_t)stream);
 }
 
-int ge2e_b200_bwd_finalize_typed(const void* E, int e_dtype, const int32_t* row_index, const float* dE_hat,
-                                 const float* dC_hat_local, const float* cos_diag, const float* row_stat,
-                                 const float* row_aux, const float* row_scale, int n_local, int M, int D,
-                                 const float* w, const float* b, float eps, int variant, const float* grad_out,
-                                 void* dE, int de_dtype, ge2e_stream_t stream) {
-  if (!E || !dE_hat || !dC_hat_local || !cos_diag || !row_stat || !w || !b || !grad_out || !dE)
+int ge2e_b200_bwd_rows(const float* e_hat, const float* c_hat_all, const float* cos_diag,
+                       const float* row_stat, const int32_t* row_kstar, const float* row_aux,
+                       const float* row_scale, int n_local, int n_total, int spk_offset, int M, int D,
+                       const float* w, const float* b, float eps,
+                       int variant, int precision, const float* grad_out, float* dE_hat,
+                       float* dC_hat_partial, float* dwdb_accum, void* workspace,
+                       size_t workspace_bytes, ge2e_stream_t stream) {
+  return bwd_rows_impl(e_hat, c_hat_all, cos_diag, row_stat, row_kstar, row_aux, row_scale, n_local, n_total,
+                       spk_offset, M, D, w, b, eps, variant, precision, grad_out, nullptr, dE_hat, dC_hat_partial,
+                       dwdb_accum, workspace, workspace_bytes, stream);
+}
+
+// grad_rows (nullable): as in bwd_rows_impl, per logical utterance row
+static int bwd_finalize_impl(const void* E, int e_dtype, const int32_t* row_index, const float* dE_hat,
+                             const float* dC_hat_local, const float* cos_diag, const float* row_stat,
+                             const float* row_aux, const float* row_scale, int n_local, int M, int D, const float* w,
+                             const float* b, float eps, int variant, const float* grad_out, const float* grad_rows,
+                             void* dE, int de_dtype, ge2e_stream_t stream) {
+  if (!E || !dE_hat || !dC_hat_local || !cos_diag || !row_stat || !w || !b || (!grad_out && !grad_rows) || !dE)
     return GE2E_ERR_ARGUMENT;
   if (variant == GE2E_SOFTMAX && !row_aux) return GE2E_ERR_ARGUMENT;
   int rc = check_shape(n_local, n_local, 0, M, D);
@@ -240,7 +253,16 @@ int ge2e_b200_bwd_finalize_typed(const void* E, int e_dtype, const int32_t* row_
   if ((rc = check_enum(variant, GE2E_FP32)) != GE2E_OK) return rc;
   if ((rc = check_dtypes(e_dtype, de_dtype)) != GE2E_OK) return rc;
   return simt_bwd_finalize(E, e_dtype, row_index, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux, row_scale, n_local,
-                           M, D, w, b, eps, variant, grad_out, dE, de_dtype, true, (cudaStream_t)stream);
+                           M, D, w, b, eps, variant, grad_out, grad_rows, dE, de_dtype, true, (cudaStream_t)stream);
+}
+
+int ge2e_b200_bwd_finalize_typed(const void* E, int e_dtype, const int32_t* row_index, const float* dE_hat,
+                                 const float* dC_hat_local, const float* cos_diag, const float* row_stat,
+                                 const float* row_aux, const float* row_scale, int n_local, int M, int D,
+                                 const float* w, const float* b, float eps, int variant, const float* grad_out,
+                                 void* dE, int de_dtype, ge2e_stream_t stream) {
+  return bwd_finalize_impl(E, e_dtype, row_index, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux, row_scale, n_local,
+                           M, D, w, b, eps, variant, grad_out, nullptr, dE, de_dtype, stream);
 }
 
 int ge2e_b200_bwd_finalize_indexed(const float* E, const int32_t* row_index, const float* dE_hat,
@@ -321,11 +343,12 @@ static bool tc_softmax_step(int n_local, int n_total, int M, int D, int variant,
   return variant == GE2E_SOFTMAX && on_tc(n_local, n_total, M, D, variant, precision);
 }
 
-int ge2e_b200_forward_typed(const void* E, int e_dtype, const int32_t* row_index, int N, int M, int D, const float* w,
-                            const float* b, float eps, int variant, int precision, float* e_hat, float* c_hat,
-                            float* cos_diag, float* row_stat, int32_t* row_kstar, float* row_aux, float* accum,
-                            float* dE_hat, float* row_scale, void* workspace, size_t workspace_bytes,
-                            ge2e_stream_t stream) {
+// per_row (nullable): [N*M] row losses in logical order
+static int forward_impl(const void* E, int e_dtype, const int32_t* row_index, int N, int M, int D, const float* w,
+                        const float* b, float eps, int variant, int precision, float* e_hat, float* c_hat,
+                        float* cos_diag, float* row_stat, int32_t* row_kstar, float* row_aux, float* accum,
+                        float* dE_hat, float* row_scale, float* per_row, void* workspace, size_t workspace_bytes,
+                        ge2e_stream_t stream) {
   if (!accum) return GE2E_ERR_ARGUMENT;
   int rc = check_enum(variant, precision);
   if (rc != GE2E_OK) return rc;
@@ -336,7 +359,26 @@ int ge2e_b200_forward_typed(const void* E, int e_dtype, const int32_t* row_index
   rc = ge2e_b200_prep_typed(E, e_dtype, row_index, N, M, D, precision, e_hat, c_hat, cos_diag, accum, stream);
   if (rc != GE2E_OK) return rc;
   return fwd_rows_impl(e_hat, c_hat, cos_diag, N, N, 0, M, D, w, b, eps, variant, precision, row_stat, row_kstar,
-                       row_aux, accum, nullptr, nullptr, dE_hat, row_scale, workspace, workspace_bytes, tc, stream);
+                       row_aux, accum, per_row, nullptr, dE_hat, row_scale, workspace, workspace_bytes, tc, stream);
+}
+
+int ge2e_b200_forward_typed(const void* E, int e_dtype, const int32_t* row_index, int N, int M, int D, const float* w,
+                            const float* b, float eps, int variant, int precision, float* e_hat, float* c_hat,
+                            float* cos_diag, float* row_stat, int32_t* row_kstar, float* row_aux, float* accum,
+                            float* dE_hat, float* row_scale, void* workspace, size_t workspace_bytes,
+                            ge2e_stream_t stream) {
+  return forward_impl(E, e_dtype, row_index, N, M, D, w, b, eps, variant, precision, e_hat, c_hat, cos_diag, row_stat,
+                      row_kstar, row_aux, accum, dE_hat, row_scale, nullptr, workspace, workspace_bytes, stream);
+}
+
+int ge2e_b200_forward_per_row_typed(const void* E, int e_dtype, const int32_t* row_index, int N, int M, int D,
+                                    const float* w, const float* b, float eps, int variant, int precision, float* e_hat,
+                                    float* c_hat, float* cos_diag, float* row_stat, int32_t* row_kstar, float* row_aux,
+                                    float* accum, float* dE_hat, float* row_scale, float* per_row, void* workspace,
+                                    size_t workspace_bytes, ge2e_stream_t stream) {
+  if (!per_row) return GE2E_ERR_ARGUMENT;
+  return forward_impl(E, e_dtype, row_index, N, M, D, w, b, eps, variant, precision, e_hat, c_hat, cos_diag, row_stat,
+                      row_kstar, row_aux, accum, dE_hat, row_scale, per_row, workspace, workspace_bytes, stream);
 }
 
 int ge2e_b200_forward_indexed(const float* E, const int32_t* row_index, int N, int M, int D, const float* w,
@@ -358,24 +400,47 @@ int ge2e_b200_forward(const float* E, int N, int M, int D, const float* w, const
                                    stream);
 }
 
+static int backward_impl(const void* E, int e_dtype, const int32_t* row_index, const float* e_hat, const float* c_hat,
+                         const float* cos_diag, const float* row_stat, const int32_t* row_kstar, const float* row_aux,
+                         const float* row_scale, int N, int M, int D, const float* w, const float* b, float eps,
+                         int variant, int precision, const float* grad_out, const float* grad_rows, float* dE_hat,
+                         float* dC_hat, float* accum, void* dE, int de_dtype, void* workspace, size_t workspace_bytes,
+                         ge2e_stream_t stream) {
+  if (!accum) return GE2E_ERR_ARGUMENT;
+  if (check_dtypes(e_dtype, de_dtype) != GE2E_OK) return GE2E_ERR_ARGUMENT;
+  if (M > finalize_max_rows(D)) return GE2E_ERR_UNSUPPORTED;     // before the rows kernels run
+  // row_scale is meaningful only where the forward produced it
+  const float* scale = tc_softmax_step(N, N, M, D, variant, precision) ? row_scale : nullptr;
+  int rc = bwd_rows_impl(e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, scale, N, N, 0, M, D, w, b, eps, variant,
+                         precision, grad_out, grad_rows, dE_hat, dC_hat, accum + 1, workspace, workspace_bytes, stream);
+  if (rc != GE2E_OK) return rc;
+  // the finalize kernel directly follows the dC_hat tensor-core kernel: programmatic launch
+  return bwd_finalize_impl(E, e_dtype, row_index, dE_hat, dC_hat, cos_diag, row_stat, row_aux, scale, N, M, D, w, b, eps,
+                           variant, grad_out, grad_rows, dE, de_dtype, stream);
+}
+
 int ge2e_b200_backward_typed(const void* E, int e_dtype, const int32_t* row_index, const float* e_hat,
                              const float* c_hat, const float* cos_diag, const float* row_stat, const int32_t* row_kstar,
                              const float* row_aux, const float* row_scale, int N, int M, int D, const float* w,
                              const float* b, float eps, int variant, int precision, const float* grad_out,
                              float* dE_hat, float* dC_hat, float* accum, void* dE, int de_dtype, void* workspace,
                              size_t workspace_bytes, ge2e_stream_t stream) {
-  if (!accum) return GE2E_ERR_ARGUMENT;
-  if (check_dtypes(e_dtype, de_dtype) != GE2E_OK) return GE2E_ERR_ARGUMENT;
-  if (M > finalize_max_rows(D)) return GE2E_ERR_UNSUPPORTED;     // before the rows kernels run
-  // row_scale is meaningful only where the forward produced it
-  const float* scale = tc_softmax_step(N, N, M, D, variant, precision) ? row_scale : nullptr;
-  int rc = ge2e_b200_bwd_rows(e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, scale, N, N, 0, M, D, w, b, eps,
-                              variant, precision, grad_out, dE_hat, dC_hat, accum + 1, workspace,
-                              workspace_bytes, stream);
-  if (rc != GE2E_OK) return rc;
-  // the finalize kernel directly follows the dC_hat tensor-core kernel: programmatic launch
-  return ge2e_b200_bwd_finalize_typed(E, e_dtype, row_index, dE_hat, dC_hat, cos_diag, row_stat, row_aux, scale, N, M, D,
-                                      w, b, eps, variant, grad_out, dE, de_dtype, stream);
+  return backward_impl(E, e_dtype, row_index, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, row_scale, N, M, D,
+                       w, b, eps, variant, precision, grad_out, nullptr, dE_hat, dC_hat, accum, dE, de_dtype, workspace,
+                       workspace_bytes, stream);
+}
+
+int ge2e_b200_backward_per_row_typed(const void* E, int e_dtype, const int32_t* row_index, const float* e_hat,
+                                     const float* c_hat, const float* cos_diag, const float* row_stat,
+                                     const int32_t* row_kstar, const float* row_aux, const float* row_scale, int N,
+                                     int M, int D, const float* w, const float* b, float eps, int variant,
+                                     int precision, const float* grad_rows, float* dE_hat, float* dC_hat, float* accum,
+                                     void* dE, int de_dtype, void* workspace, size_t workspace_bytes,
+                                     ge2e_stream_t stream) {
+  if (!grad_rows) return GE2E_ERR_ARGUMENT;
+  return backward_impl(E, e_dtype, row_index, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, row_scale, N, M, D,
+                       w, b, eps, variant, precision, nullptr, grad_rows, dE_hat, dC_hat, accum, dE, de_dtype,
+                       workspace, workspace_bytes, stream);
 }
 
 int ge2e_b200_backward_indexed(const float* E, const int32_t* row_index, const float* e_hat, const float* c_hat,
@@ -420,10 +485,10 @@ int ge2e_b200_step_rows(const float* e_hat, const float* c_hat_all, const float*
       rc = tc_fwd_rows(a, row_stat, row_kstar, row_aux, accum, nullptr, workspace, workspace_bytes, true,
                        (cudaStream_t)stream, tc_prec(precision));
       if (rc != GE2E_OK) return rc;
-      return tc_step(a, 3, grad_out, row_stat, row_aux, nullptr, nullptr, row_scale, nullptr, nullptr, dE_hat,
+      return tc_step(a, 3, grad_out, nullptr, row_stat, row_aux, nullptr, nullptr, row_scale, nullptr, nullptr, dE_hat,
                      dC_hat_partial, accum + 1, workspace, workspace_bytes, (cudaStream_t)stream, nullptr, 0, tc_prec(precision));
     }
-    return tc_step(a, 3, grad_out, nullptr, nullptr, row_stat, row_aux, row_scale, accum, nullptr, dE_hat,
+    return tc_step(a, 3, grad_out, nullptr, nullptr, nullptr, row_stat, row_aux, row_scale, accum, nullptr, dE_hat,
                    dC_hat_partial, accum + 1, workspace, workspace_bytes, (cudaStream_t)stream);
   }
   if (is_planes(precision)) return GE2E_ERR_UNSUPPORTED;
@@ -469,10 +534,10 @@ int ge2e_b200_step_rows_peers(const float* e_hat, const float* c_hat_all, const 
     rc = tc_fwd_rows(a, row_stat, row_kstar, row_aux, accum, nullptr, workspace, workspace_bytes, true,
                      (cudaStream_t)stream, tc_prec(precision));
     if (rc != GE2E_OK) return rc;
-    return tc_step(a, 3, grad_out, row_stat, row_aux, nullptr, nullptr, row_scale, nullptr, nullptr, dE_hat, nullptr,
+    return tc_step(a, 3, grad_out, nullptr, row_stat, row_aux, nullptr, nullptr, row_scale, nullptr, nullptr, dE_hat, nullptr,
                    accum + 1, workspace, workspace_bytes, (cudaStream_t)stream, dC_owner_host, n_ranks, tc_prec(precision));
   }
-  return tc_step(a, 3, grad_out, nullptr, nullptr, row_stat, row_aux, row_scale, accum, nullptr, dE_hat, nullptr,
+  return tc_step(a, 3, grad_out, nullptr, nullptr, nullptr, row_stat, row_aux, row_scale, accum, nullptr, dE_hat, nullptr,
                  accum + 1, workspace, workspace_bytes, (cudaStream_t)stream, dC_owner_host, n_ranks);
 }
 

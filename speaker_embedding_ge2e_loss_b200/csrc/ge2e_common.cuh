@@ -142,9 +142,11 @@ int simt_prep(const void* E, int e_dt, const int32_t* row_index, int n_local, in
               float* c_hat_local, float* cos_diag, float* accum, cudaStream_t st);
 int simt_fwd_rows(const RowsArgs& a, float* row_stat, int32_t* row_kstar, float* row_aux,
                   float* loss_accum, float* per_row_out, float* sim_out, cudaStream_t st);
+// grad_rows (nullable): the upstream gradient per local utterance row, in place of the scalar grad_out -- selects the
+// row-gradient (RG) instantiations of the backward kernels
 int simt_bwd_rows(const RowsArgs& a, const float* row_stat, const int32_t* row_kstar,
-                  const float* row_aux, const float* grad_out, float* dE_hat, float* dC_hat_partial,
-                  float* dwdb_accum, cudaStream_t st);
+                  const float* row_aux, const float* grad_out, const float* grad_rows, float* dE_hat,
+                  float* dC_hat_partial, float* dwdb_accum, cudaStream_t st);
 // largest M whose backward finalize runs at width D (0: D unsupported); see ge2e_b200_max_utterances
 int finalize_max_rows(int D);
 int simt_bwd_finalize(const void* E, int e_dt, const int32_t* row_index, const float* dE_hat, const float* dC_hat_local,
@@ -152,7 +154,8 @@ int simt_bwd_finalize(const void* E, int e_dt, const int32_t* row_index, const f
                       const float* row_scale /* nullable: dE_hat row r is g * row_scale[r] * dE_hat[r] */,
                       int n_local, int M, int D,
                       const float* w, const float* b, float eps, int variant,
-                      const float* grad_out, void* dE, int de_dt, bool pdl, cudaStream_t st);
+                      const float* grad_out, const float* grad_rows /* nullable, as in simt_bwd_rows */, void* dE,
+                      int de_dt, bool pdl, cudaStream_t st);
 // fused single-kernel fwd+bwd step for small batches (ge2e_simt.cu)
 bool small_step_supported(int N, int M, int D);
 bool small_step_preferred(int N, int M, int D, int variant);   // supported AND faster than the pipeline
@@ -207,9 +210,11 @@ int tc_fwd_rows(const RowsArgs& a, float* row_stat, int32_t* row_kstar, float* r
                 cudaStream_t st, int prec = 0 /* 0 TF32, 1 split fp16 planes, 2 one fp16 plane */);
 // softmax step on tensor cores; phases: 1 = rows pass (loss, row statistics, un-normalised dE_hat + row_scale),
 // 2 = centroid pass (dC_hat_partial, {dw, db}), 3 = both in one launch
+// grad_rows (nullable, phases == 2 only): the upstream gradient per local utterance row in place of grad_out
 // dC_owner (nullable, HOST array of n_ranks device pointers): speaker-sharded over peer memory -- pass 2 adds its
 // accumulators straight into the owner rank's dC_local[n_total / n_ranks, D] (see ge2e_b200_step_rows_peers)
-int tc_step(const RowsArgs& a, int phases, const float* grad_out, const float* row_stat_in, const float* row_aux_in,
+int tc_step(const RowsArgs& a, int phases, const float* grad_out, const float* grad_rows, const float* row_stat_in,
+            const float* row_aux_in,
             float* row_stat, float* row_aux, float* row_scale, float* loss_accum, float* per_row_out, float* dE_hat,
             float* dC_hat_partial, float* dwdb_accum, void* ws, size_t ws_bytes, cudaStream_t st,
             float* const* dC_owner = nullptr, int n_ranks = 0, int prec = 0);

@@ -512,6 +512,7 @@ struct StripParams {
   const float* w;
   const float* b;
   const float* grad_out;
+  const float* grad_rows;  // bwd, RG instantiations: upstream gradient per local utterance row (replaces grad_out)
   float eps;
   float* row_stat_out;     // fwd
   int32_t* kstar_out;      // fwd contrast
@@ -556,7 +557,8 @@ struct RedT<5, R, KCH> {
   }
 };
 
-template <int MODE, int VARIANT, int KCH, int R>
+// RG: the upstream gradient is one value per utterance row (p.grad_rows) instead of the scalar p.grad_out
+template <int MODE, int VARIANT, int KCH, int R, bool RG = false>
 __global__ void __launch_bounds__(kThreads)
 strip_kernel(const StripParams p) {
   extern __shared__ __align__(16) float stage[];   // [32][KCH*128]
@@ -567,7 +569,7 @@ strip_kernel(const StripParams p) {
   const int D = p.D;
   const bool vec_own = is_vec(p.own, D), vec_str = is_vec(p.str, D);
   const float w = __ldg(p.w), b = __ldg(p.b), eps = p.eps;
-  const float g = (MODE == MODE_FWD) ? 1.f : __ldg(p.grad_out);
+  const float g = (MODE == MODE_FWD || RG) ? 1.f : __ldg(p.grad_out);
 
   float4 a[R][KCH];
 #pragma unroll
@@ -585,6 +587,7 @@ strip_kernel(const StripParams p) {
   float cd[R];      // cos_diag of the owner row
   float lse[R];     // BWD_DE
   float qd[R];      // BWD_DE: 1 - p_jj
+  float gr[R];      // BWD_DE: upstream gradient of the owner row
   float m_run[R], l_run[R];   // FWD softmax (per lane, merged at the end)
   float best[R]; int bestk[R];  // FWD contrast
   float4 acc[R][KCH];
@@ -593,11 +596,12 @@ strip_kernel(const StripParams p) {
   for (int q = 0; q < R; ++q) {
     const int row = own0 + q;
     // rows past the end: lse = +inf makes every G of that row exactly 0
-    jg[q] = -1; cd[q] = 0.f; lse[q] = INFINITY; qd[q] = 0.f;
+    jg[q] = -1; cd[q] = 0.f; lse[q] = INFINITY; qd[q] = 0.f; gr[q] = g;
     if (MODE != MODE_BWD_DC && row < p.n_own) {
       jg[q] = p.spk_offset + row / p.M;
       cd[q] = __ldg(p.cos_diag + row);
       if (MODE == MODE_BWD_DE) { lse[q] = __ldg(p.row_stat + row); qd[q] = __ldg(p.row_aux + row); }
+      if (MODE == MODE_BWD_DE && RG) gr[q] = __ldg(p.grad_rows + row);
     }
     m_run[q] = -INFINITY; l_run[q] = 0.f; best[q] = -INFINITY; bestk[q] = INT_MAX;
 #pragma unroll
@@ -629,13 +633,16 @@ strip_kernel(const StripParams p) {
 
     if (MODE == MODE_BWD_DC) {
       // owner = centroid (global index own0+q), stream = local utterance row k
-      float lse_r = 0.f; int jg_r = -2;
-      if (valid) { lse_r = __ldg(p.row_stat + k); jg_r = p.spk_offset + k / p.M; }
+      float lse_r = 0.f, g_r = g; int jg_r = -2;
+      if (valid) {
+        lse_r = __ldg(p.row_stat + k); jg_r = p.spk_offset + k / p.M;
+        if (RG) g_r = __ldg(p.grad_rows + k);
+      }
 #pragma unroll
       for (int q = 0; q < R; ++q) {
         const float S = fmaf(w, dot[q] + eps, b);
         const bool off = valid && (jg_r != own0 + q);
-        gq[q] = off ? w * g * expf(S - lse_r) : 0.f;
+        gq[q] = off ? w * g_r * expf(S - lse_r) : 0.f;
       }
     } else {
 #pragma unroll
@@ -657,7 +664,7 @@ strip_kernel(const StripParams p) {
           }
         } else {  // MODE_BWD_DE (softmax only)
           const float pr = valid ? expf(S - lse[q]) : 0.f;
-          const float G = g * (diag ? -qd[q] : pr);     // own speaker: p_jj - 1 = -q, no cancellation
+          const float G = gr[q] * (diag ? -qd[q] : pr);     // own speaker: p_jj - 1 = -q, no cancellation
           dw_acc = fmaf(G, cosv, dw_acc);
           gq[q] = (valid && !diag) ? w * G : 0.f;
         }
@@ -732,7 +739,7 @@ strip_kernel(const StripParams p) {
         for (int c = 0; c < KCH; ++c)
           st4(p.acc_out + (size_t)row * D, (lane << 2) + c * 128, D, vec_out, acc[q][c]);
         // db = sum_k G = -g * eps / (sum exp + eps): closed form (SURVEY 8(a-bis) item 12)
-        if (lane == 0) db_part -= g * eps * expf(-lse[q]);
+        if (lane == 0) db_part -= gr[q] * eps * expf(-lse[q]);
       }
     }
     const float dw_tot = block_sum(dw_acc, red);
@@ -760,7 +767,9 @@ strip_kernel(const StripParams p) {
 // ------------------------------------------------------------------------------------------
 // contrast backward: G has two non-zeros per row (the diagonal and k*): gather / scatter.
 // grid = ceil(U_local / 8), block = 256 (one warp per utterance row)
+// gp: the upstream gradient -- one scalar, or (RG) one per utterance row
 // ------------------------------------------------------------------------------------------
+template <bool RG = false>
 __global__ void __launch_bounds__(kThreads)
 contrast_bwd_kernel(const float* __restrict__ e_hat, const float* __restrict__ c_hat_all,
                     const float* __restrict__ cos_diag, const float* __restrict__ row_stat,
@@ -770,9 +779,10 @@ contrast_bwd_kernel(const float* __restrict__ e_hat, const float* __restrict__ c
   __shared__ float red[kWarps];
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   const int r = blockIdx.x * kWarps + wid;
-  const float w = __ldg(wp), b = __ldg(bp), g = __ldg(gp);
+  const float w = __ldg(wp), b = __ldg(bp), g0 = RG ? 0.f : __ldg(gp);
   float dw = 0.f, db = 0.f;
   if (r < U) {
+    const float g = RG ? __ldg(gp + r) : g0;
     const float cd = __ldg(cos_diag + r) + eps;
     const float sp = 1.f / (1.f + expf(-fmaf(w, cd, b)));
     const float Gp = -g * sp * (1.f - sp);
@@ -808,13 +818,15 @@ contrast_bwd_kernel(const float* __restrict__ e_hat, const float* __restrict__ c
 // threads, `smem` = (2 M + 2) * Dp floats.  dE_hat / dC_hat are read with plain loads (the fused
 // kernel reads what its own block has just written).
 // REUSE_E: sE already holds the speaker's raw rows (prep_body staged them at the same place earlier in this kernel).
-template <bool REUSE_E = false, typename TE = float, typename TD = float>
+// RG: the upstream gradient of logical row r is g_rows[r] (g unused); where bwd_rows already folded it into dE_hat
+// (row_scale == nullptr) it only enters the diagonal term.
+template <bool REUSE_E = false, typename TE = float, typename TD = float, bool RG = false>
 __device__ __forceinline__ void finalize_body(const TE* __restrict__ E, const float* dE_hat, const float* dC_hat,
                                               const float* cos_diag, const float* row_stat, const float* row_aux,
                                               const float* row_scale, int j, int M, int D, int Dp, float w, float b,
                                               float g, float eps,
                                               int variant, TD* __restrict__ dE, const int32_t* __restrict__ idx,
-                                              float* smem) {
+                                              float* smem, const float* __restrict__ g_rows = nullptr) {
   __shared__ float red[kWarps];
   __shared__ float s_bc[2];
   float* sE = smem;                          // [M][Dp] raw embeddings -> later de (gradient through e_hat)
@@ -873,8 +885,9 @@ __device__ __forceinline__ void finalize_body(const TE* __restrict__ E, const fl
     const int r = j * M + i;
     float ne2 = 0.f, nu2 = 0.f, eu = 0.f, eg = 0.f;
     const float* gh = dE_hat + (size_t)r * D;
+    const float gr = RG ? __ldg(g_rows + r) : g;
     // tensor-core softmax path: dE_hat holds un-normalised rows, the true row is g * row_scale[r] times it
-    const float gsc = row_scale != nullptr ? g * row_scale[r] : 1.f;
+    const float gsc = row_scale != nullptr ? gr * row_scale[r] : 1.f;
     for (int d = lane << 2; d < Dp; d += 128) {
       const float4 e = *reinterpret_cast<const float4*>(&sE[(size_t)i * Dp + d]);
       const float4 s = *reinterpret_cast<const float4*>(&sS[d]);
@@ -891,10 +904,10 @@ __device__ __forceinline__ void finalize_body(const TE* __restrict__ E, const fl
     const float Sd = fmaf(w, cos_diag[r] + eps, b);
     float Gd;
     if (variant == GE2E_SOFTMAX) {
-      Gd = -g * row_aux[r];                 // g (p_jj - 1), accumulated off-diagonal in fwd
+      Gd = -gr * row_aux[r];                // g (p_jj - 1), accumulated off-diagonal in fwd
     } else {
       const float sp = 1.f / (1.f + expf(-Sd));
-      Gd = -g * sp * (1.f - sp);
+      Gd = -gr * sp * (1.f - sp);
     }
     const float dd = w * Gd;
     // d e_hat = dE_hat_offdiag + dd * u_hat ;  d u_hat = dd * e_hat
@@ -945,7 +958,8 @@ __device__ __forceinline__ void finalize_body(const TE* __restrict__ E, const fl
   }
 }
 
-template <typename TE, typename TD>
+// gp: the upstream gradient -- one scalar, or (RG) one per logical utterance row
+template <typename TE, typename TD, bool RG = false>
 __global__ void __launch_bounds__(kThreads)
 finalize_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
                 const float* __restrict__ dC_hat, const float* __restrict__ cos_diag,
@@ -954,8 +968,8 @@ finalize_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
                 const float* __restrict__ wp, const float* __restrict__ bp, float eps, int variant,
                 const float* __restrict__ gp, TD* __restrict__ dE, const int32_t* __restrict__ idx) {
   extern __shared__ __align__(16) float smem[];
-  finalize_body<false>(E, dE_hat, dC_hat, cos_diag, row_stat, row_aux, row_scale, blockIdx.x, M, D, Dp, __ldg(wp), __ldg(bp), __ldg(gp),
-                eps, variant, dE, idx, smem);
+  finalize_body<false, TE, TD, RG>(E, dE_hat, dC_hat, cos_diag, row_stat, row_aux, row_scale, blockIdx.x, M, D, Dp, __ldg(wp),
+                                  __ldg(bp), RG ? 0.f : __ldg(gp), eps, variant, dE, idx, smem, gp);
 }
 
 
@@ -965,7 +979,7 @@ finalize_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
 // the speaker's rows (the 2nd and 3rd hit L1): column sums; per-row scalars + sum_i du_i;
 // outputs.  Row i's scalars live in lane i between the passes.
 // ------------------------------------------------------------------------------------------
-template <int KCH, typename TE, typename TD>
+template <int KCH, typename TE, typename TD, bool RG = false>
 __global__ void __launch_bounds__(kPrepWarps * 32)
 finalize_warp_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
                      const float* __restrict__ dC_hat, const float* __restrict__ cos_diag,
@@ -978,7 +992,7 @@ finalize_warp_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
   pdl_wait();        // launched with the PDL attribute: dE_hat / dC_hat come from the preceding grids
   pdl_trigger();     // the next step's prep may be scheduled (it waits for this grid before touching memory)
   if (j >= n_local) return;
-  const float w = __ldg(wp), b = __ldg(bp), g = __ldg(gp);
+  const float w = __ldg(wp), b = __ldg(bp), g = RG ? 0.f : __ldg(gp);
   auto rowp = [&](int i) {      // + c * 32 vectors per 128-column chunk
     return reinterpret_cast<const vec4_t<TE>*>(E + phys_row(idx, (size_t)j * M + i) * D) + lane;
   };
@@ -1063,15 +1077,16 @@ finalize_warp_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
         const float ne = sqrtf(ne2[r]), nu = sqrtf(nd2[r]) * inv_m1;
         const float inv_ne = 1.f / fmaxf(ne, kCosDelta), inv_nu = 1.f / fmaxf(nu, kCosDelta);
         const float cdv = (ed[r] * inv_m1) * inv_ne * inv_nu;       // e_hat . u_hat
+        const float gr = RG ? __ldcg(gp + row) : g;                 // upstream gradient of this row
         float Gd;                                                   // diagonal element of G
         if (variant == GE2E_SOFTMAX) {
-          Gd = -g * __ldg(row_aux + row);                           // g (p_jj - 1)
+          Gd = -gr * __ldg(row_aux + row);                          // g (p_jj - 1)
         } else {
           const float sp = 1.f / (1.f + expf(-fmaf(w, __ldg(cos_diag + row) + eps, b)));
-          Gd = -g * sp * (1.f - sp);
+          Gd = -gr * sp * (1.f - sp);
         }
         const float dd = w * Gd;
-        const float gsc = row_scale != nullptr ? g * __ldcg(row_scale + row) : 1.f;   // un-normalised dE_hat rows
+        const float gsc = row_scale != nullptr ? gr * __ldcg(row_scale + row) : 1.f;   // un-normalised dE_hat rows
         float proj_e = eg[r] * gsc * inv_ne + dd * cdv;             // e_hat . d e_hat
         float proj_u = dd * cdv;                                    // u_hat . d u_hat
         if (ne < kCosDelta) proj_e *= clamp_proj_scale(ne);         // warp-uniform, rare
@@ -1131,7 +1146,7 @@ finalize_warp_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
 //   de_i = a_g gv_i + a_e e_i + a_d d_i ,  du_i = b_e e_i + b_d d_i ,  d_i = s - e_i
 //   dE_i = de_i + dc_j / M + (sum_i' du_i' - du_i) / (M - 1)
 // ------------------------------------------------------------------------------------------
-template <int W, int RR, typename TE, typename TD>
+template <int W, int RR, typename TE, typename TD, bool RG = false>
 __global__ void __launch_bounds__(kPrepWarps * 32, kRegBlocksPerSM)
 finalize_reg_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
                     const float* __restrict__ dC_hat, const float* __restrict__ cos_diag,
@@ -1173,12 +1188,13 @@ finalize_reg_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
   pdl_wait();        // launched with the PDL attribute: dE_hat / dC_hat come from the preceding grids
   pdl_trigger();     // the next step's prep may be scheduled (it waits for this grid before touching memory)
   if (!active) return;     // all W warps of the speaker
-  const float w = __ldg(wp), b = __ldg(bp), g = __ldg(gp);
+  const float w = __ldg(wp), b = __ldg(bp), g = RG ? 0.f : __ldg(gp);
   const int my_row = rev4(lane & 15);
   const int row = j * M + min(my_row, M - 1);     // lanes past row M - 1 hold no row
   const float4 dch = __ldcg(reinterpret_cast<const float4*>(dC_hat + (size_t)j * D + col));
   const float aux = variant == GE2E_SOFTMAX ? __ldcg(row_aux + row) : __ldg(cos_diag + row);
-  const float gsc = row_scale != nullptr ? g * __ldcg(row_scale + row) : 1.f;   // un-normalised dE_hat rows
+  // un-normalised dE_hat rows (RG: g_r joins below -- loaded here it would be one more register through the sums)
+  const float gsc0 = row_scale != nullptr ? (RG ? __ldcg(row_scale + row) : g * __ldcg(row_scale + row)) : 1.f;
   const float* Gj = dE_hat + (size_t)j * M * D + col;
   {
     float eg[16];
@@ -1210,12 +1226,14 @@ finalize_reg_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
     const float ne = sqrtf(t_ne2), nu = sqrtf(t_nd2) * inv_m1;
     const float inv_ne = 1.f / fmaxf(ne, kCosDelta), inv_nu = 1.f / fmaxf(nu, kCosDelta);
     const float cdv = (t_ed * inv_m1) * inv_ne * inv_nu;          // e_hat . u_hat
+    const float gr = RG ? __ldcg(gp + row) : g;                   // upstream gradient of this lane's row
+    const float gsc = (RG && row_scale != nullptr) ? gr * gsc0 : gsc0;
     float Gd;                                                     // diagonal element of G
     if (variant == GE2E_SOFTMAX) {
-      Gd = -g * aux;                                              // g (p_jj - 1)
+      Gd = -gr * aux;                                             // g (p_jj - 1)
     } else {
       const float sp = 1.f / (1.f + expf(-fmaf(w, aux + eps, b)));
-      Gd = -g * sp * (1.f - sp);
+      Gd = -gr * sp * (1.f - sp);
     }
     const float dd = w * Gd;
     const float proj_e = t_eg * gsc * inv_ne + dd * cdv;          // e_hat . d e_hat
@@ -1339,10 +1357,10 @@ int set_smem(K kernel, size_t bytes) {
   return GE2E_OK;
 }
 
-template <int MODE, int VARIANT, int KCH, int R>
+template <int MODE, int VARIANT, int KCH, int R, bool RG>
 int launch_strip(const StripParams& p, int splits, cudaStream_t st) {
   const size_t smem = (size_t)kStreamRows * KCH * 128 * sizeof(float);
-  auto kern = strip_kernel<MODE, VARIANT, KCH, R>;
+  auto kern = strip_kernel<MODE, VARIANT, KCH, R, RG>;
   int rc = set_smem(kern, smem);
   if (rc != GE2E_OK) return rc;
   dim3 grid((p.n_own + kWarps * R - 1) / (kWarps * R), splits);
@@ -1351,13 +1369,13 @@ int launch_strip(const StripParams& p, int splits, cudaStream_t st) {
   return GE2E_OK;
 }
 
-template <int MODE, int VARIANT>
+template <int MODE, int VARIANT, bool RG = false>
 int dispatch_strip(const StripParams& p, int splits, cudaStream_t st) {
   const int D = p.D;
-  if (D <= 128) return launch_strip<MODE, VARIANT, 1, 4>(p, splits, st);
-  if (D <= 256) return launch_strip<MODE, VARIANT, 2, 4>(p, splits, st);   // R = 8 was tried: 1.65 ms vs 1.40 ms at cfg3
-  if (D <= 512) return launch_strip<MODE, VARIANT, 4, 2>(p, splits, st);
-  if (D <= 1024) return launch_strip<MODE, VARIANT, 8, 1>(p, splits, st);
+  if (D <= 128) return launch_strip<MODE, VARIANT, 1, 4, RG>(p, splits, st);
+  if (D <= 256) return launch_strip<MODE, VARIANT, 2, 4, RG>(p, splits, st);   // R = 8 was tried: 1.65 ms vs 1.40 ms at cfg3
+  if (D <= 512) return launch_strip<MODE, VARIANT, 4, 2, RG>(p, splits, st);
+  if (D <= 1024) return launch_strip<MODE, VARIANT, 8, 1, RG>(p, splits, st);
   return GE2E_ERR_UNSUPPORTED;
 }
 
@@ -1430,7 +1448,7 @@ void launch_prep_warp(const TE* E, const int32_t* idx, int n_local, int M, int p
                   e_hat, c_hat, cos_diag, accum);
 }
 
-template <int KCH, typename TE, typename TD>
+template <int KCH, bool RG, typename TE, typename TD>
 void launch_finalize_warp(const TE* E, const float* dE_hat, const float* dC_hat, const float* cos_diag,
                           const float* row_aux, const float* row_scale, int n_local, int M, const float* w,
                           const float* b, float eps,
@@ -1440,13 +1458,13 @@ void launch_finalize_warp(const TE* E, const float* dE_hat, const float* dC_hat,
     constexpr int W = KCH <= 2 ? KCH : 1, spb = kPrepWarps / W;
     const dim3 gr((n_local + spb - 1) / spb), bl(kPrepWarps * 32);
 #define GE2E_FIN_REG(RR)                                                                                     \
-  launch_pdl(finalize_reg_kernel<W, RR, TE, TD>, gr, bl, 0, st, pdl, E, dE_hat, dC_hat, cos_diag, row_aux, row_scale, n_local, M, \
+  launch_pdl(finalize_reg_kernel<W, RR, TE, TD, RG>, gr, bl, 0, st, pdl, E, dE_hat, dC_hat, cos_diag, row_aux, row_scale, n_local, M, \
              w, b, eps, variant, g, dE, idx)
     if (M <= 4) GE2E_FIN_REG(4); else if (M <= 8) GE2E_FIN_REG(8); else if (M <= 12) GE2E_FIN_REG(12); else GE2E_FIN_REG(16);
 #undef GE2E_FIN_REG
     return;
   }
-  launch_pdl(finalize_warp_kernel<KCH, TE, TD>, dim3(grid), dim3(kPrepWarps * 32), 0, st, pdl, E, dE_hat, dC_hat, cos_diag,
+  launch_pdl(finalize_warp_kernel<KCH, TE, TD, RG>, dim3(grid), dim3(kPrepWarps * 32), 0, st, pdl, E, dE_hat, dC_hat, cos_diag,
              row_aux, row_scale, n_local, M, w, b, eps, variant, g, dE, idx);
 }
 
@@ -1501,8 +1519,8 @@ int simt_fwd_rows(const RowsArgs& a, float* row_stat, int32_t* row_kstar, float*
 }
 
 int simt_bwd_rows(const RowsArgs& a, const float* row_stat, const int32_t* row_kstar, const float* row_aux,
-                  const float* grad_out, float* dE_hat, float* dC_hat_partial, float* dwdb_accum,
-                  cudaStream_t st) {
+                  const float* grad_out, const float* grad_rows, float* dE_hat, float* dC_hat_partial,
+                  float* dwdb_accum, cudaStream_t st) {
   const int U = a.n_local * a.M;
   // one memset when the caller placed {dw, db} right behind dC_hat_partial, else two
   const size_t dc_elems = (size_t)a.n_total * a.D;
@@ -1513,20 +1531,26 @@ int simt_bwd_rows(const RowsArgs& a, const float* row_stat, const int32_t* row_k
     GE2E_CUDA_TRY(cudaMemsetAsync(dwdb_accum, 0, 2 * sizeof(float), st));
   }
   if (a.variant == GE2E_CONTRAST) {
-    contrast_bwd_kernel<<<(U + kWarps - 1) / kWarps, kThreads, 0, st>>>(
-        a.e_hat, a.c_hat_all, a.cos_diag, row_stat, row_kstar, U, a.D, a.w, a.b, a.eps, grad_out,
-        dE_hat, dC_hat_partial, dwdb_accum);
+    if (grad_rows != nullptr)
+      contrast_bwd_kernel<true><<<(U + kWarps - 1) / kWarps, kThreads, 0, st>>>(
+          a.e_hat, a.c_hat_all, a.cos_diag, row_stat, row_kstar, U, a.D, a.w, a.b, a.eps, grad_rows,
+          dE_hat, dC_hat_partial, dwdb_accum);
+    else
+      contrast_bwd_kernel<<<(U + kWarps - 1) / kWarps, kThreads, 0, st>>>(
+          a.e_hat, a.c_hat_all, a.cos_diag, row_stat, row_kstar, U, a.D, a.w, a.b, a.eps, grad_out,
+          dE_hat, dC_hat_partial, dwdb_accum);
     GE2E_LAUNCHED();
     return GE2E_OK;
   }
   StripParams p{};
   p.D = a.D; p.M = a.M; p.spk_offset = a.spk_offset;
   p.cos_diag = a.cos_diag; p.row_stat = row_stat; p.row_aux = row_aux; p.w = a.w; p.b = a.b; p.grad_out = grad_out;
-  p.eps = a.eps;
+  p.grad_rows = grad_rows; p.eps = a.eps;
+  const bool rg = grad_rows != nullptr;
   // dE_hat: owner = utterances, stream = centroids
   p.own = a.e_hat; p.n_own = U; p.str = a.c_hat_all; p.n_str = a.n_total;
   p.acc_out = dE_hat; p.dwdb = dwdb_accum; p.chunks_per_split = INT_MAX / 2;
-  int rc = dispatch_strip<MODE_BWD_DE, GE2E_SOFTMAX>(p, 1, st);
+  int rc = rg ? dispatch_strip<MODE_BWD_DE, GE2E_SOFTMAX, true>(p, 1, st) : dispatch_strip<MODE_BWD_DE, GE2E_SOFTMAX>(p, 1, st);
   if (rc != GE2E_OK) return rc;
   // dC_hat: owner = centroids, stream = utterances, stream range split across blockIdx.y
   p.own = a.c_hat_all; p.n_own = a.n_total; p.str = a.e_hat; p.n_str = U;
@@ -1537,27 +1561,29 @@ int simt_bwd_rows(const RowsArgs& a, const float* row_stat, const int32_t* row_k
   splits = max(1, min(splits, nchunks));
   p.chunks_per_split = (nchunks + splits - 1) / splits;
   splits = (nchunks + p.chunks_per_split - 1) / p.chunks_per_split;
-  return dispatch_strip<MODE_BWD_DC, GE2E_SOFTMAX>(p, splits, st);
+  return rg ? dispatch_strip<MODE_BWD_DC, GE2E_SOFTMAX, true>(p, splits, st)
+            : dispatch_strip<MODE_BWD_DC, GE2E_SOFTMAX>(p, splits, st);
 }
 
-template <typename TE, typename TD>
+// RG: grad_out is the upstream gradient per logical utterance row
+template <bool RG, typename TE, typename TD>
 int simt_bwd_finalize_t(const TE* E, const int32_t* row_index, const float* dE_hat, const float* dC_hat_local,
                         const float* cos_diag, const float* row_stat, const float* row_aux, const float* row_scale,
                         int n_local, int M, int D, const float* w, const float* b, float eps, int variant,
                         const float* grad_out, TD* dE, bool pdl, cudaStream_t st) {
   if (M <= 32 && rows_vec_ok(E) && rows_vec_ok(dE) && warp_path_ok(D, {dE_hat, dC_hat_local})) {
-    if (D == 128) launch_finalize_warp<1>(E, dE_hat, dC_hat_local, cos_diag, row_aux, row_scale, n_local, M, w, b, eps, variant, grad_out, dE, row_index, pdl, st);
-    else if (D == 256) launch_finalize_warp<2>(E, dE_hat, dC_hat_local, cos_diag, row_aux, row_scale, n_local, M, w, b, eps, variant, grad_out, dE, row_index, pdl, st);
-    else launch_finalize_warp<4>(E, dE_hat, dC_hat_local, cos_diag, row_aux, row_scale, n_local, M, w, b, eps, variant, grad_out, dE, row_index, pdl, st);
+    if (D == 128) launch_finalize_warp<1, RG>(E, dE_hat, dC_hat_local, cos_diag, row_aux, row_scale, n_local, M, w, b, eps, variant, grad_out, dE, row_index, pdl, st);
+    else if (D == 256) launch_finalize_warp<2, RG>(E, dE_hat, dC_hat_local, cos_diag, row_aux, row_scale, n_local, M, w, b, eps, variant, grad_out, dE, row_index, pdl, st);
+    else launch_finalize_warp<4, RG>(E, dE_hat, dC_hat_local, cos_diag, row_aux, row_scale, n_local, M, w, b, eps, variant, grad_out, dE, row_index, pdl, st);
     GE2E_LAUNCHED();
     return GE2E_OK;
   }
   const int Dp = (D + 3) & ~3;
   if (M > finalize_max_rows(D)) return GE2E_ERR_UNSUPPORTED;
   const size_t smem = (size_t)(2 * M + 2) * Dp * sizeof(float);
-  int rc = set_smem(finalize_kernel<TE, TD>, smem);
+  int rc = set_smem(finalize_kernel<TE, TD, RG>, smem);
   if (rc != GE2E_OK) return rc;
-  finalize_kernel<<<n_local, kThreads, smem, st>>>(E, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux, row_scale, M, D,
+  finalize_kernel<TE, TD, RG><<<n_local, kThreads, smem, st>>>(E, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux, row_scale, M, D,
                                                    Dp, w, b, eps, variant, grad_out, dE, row_index);
   GE2E_LAUNCHED();
   return GE2E_OK;
@@ -1566,12 +1592,18 @@ int simt_bwd_finalize_t(const TE* E, const int32_t* row_index, const float* dE_h
 int simt_bwd_finalize(const void* E, int e_dt, const int32_t* row_index, const float* dE_hat, const float* dC_hat_local,
                       const float* cos_diag, const float* row_stat, const float* row_aux, const float* row_scale,
                       int n_local, int M, int D, const float* w, const float* b, float eps, int variant,
-                      const float* grad_out, void* dE, int de_dt, bool pdl, cudaStream_t st) {
+                      const float* grad_out, const float* grad_rows, void* dE, int de_dt, bool pdl,
+                      cudaStream_t st) {
   return with_e_de_types(e_dt, de_dt, [&](auto te, auto td) -> int {
     using TE = decltype(te);
     using TD = decltype(td);
-    return simt_bwd_finalize_t(static_cast<const TE*>(E), row_index, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux,
-                               row_scale, n_local, M, D, w, b, eps, variant, grad_out, static_cast<TD*>(dE), pdl, st);
+    if (grad_rows != nullptr)
+      return simt_bwd_finalize_t<true>(static_cast<const TE*>(E), row_index, dE_hat, dC_hat_local, cos_diag, row_stat,
+                                       row_aux, row_scale, n_local, M, D, w, b, eps, variant, grad_rows,
+                                       static_cast<TD*>(dE), pdl, st);
+    return simt_bwd_finalize_t<false>(static_cast<const TE*>(E), row_index, dE_hat, dC_hat_local, cos_diag, row_stat,
+                                      row_aux, row_scale, n_local, M, D, w, b, eps, variant, grad_out,
+                                      static_cast<TD*>(dE), pdl, st);
   });
 }
 

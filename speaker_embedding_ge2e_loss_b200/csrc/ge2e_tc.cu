@@ -55,6 +55,7 @@
 
 #include <algorithm>
 #include <cstring>
+#include <type_traits>
 #include <vector>
 
 #include "ge2e_common.cuh"
@@ -160,6 +161,7 @@ struct TcParams {
   const float* w;
   const float* b;
   const float* grad_out;
+  const float* grad_rows;     // STEP pass 2 alone, RG instantiations: upstream gradient per local utterance row
   float eps;
   // FWD outputs
   float* row_stat_out;
@@ -221,9 +223,16 @@ struct SharedTail {
     alignas(16) float2 xch[kTile];        // FWD: row state of the upper column half
   };
 };
+// RG instantiations (per-row upstream gradient): lse_s[buf][r] then holds lse2 - log2 |g_r| (/ gamma on the planes) and
+// gsign[buf] the signs of g_r, one bit per stream row, staged by the same threads at the same points
+struct SharedTailRG : SharedTail {
+  uint32_t gsign[2][kUnit / 32];
+};
 constexpr size_t kWsHeaderBytes = 256;   // workspace: [header: BWD counters][FWD seg_done][FWD seg_part]
-constexpr size_t kSmemBytes = 1024 + kMaxSlabs * kSlabBytes + kRingBytes + sizeof(SharedTail);
-static_assert(kSmemBytes <= 232448, "dynamic shared memory over the 227 KB per-CTA limit");
+template <bool RG = false>
+constexpr size_t kSmemBytesT = 1024 + kMaxSlabs * kSlabBytes + kRingBytes + (RG ? sizeof(SharedTailRG) : sizeof(SharedTail));
+constexpr size_t kSmemBytes = kSmemBytesT<false>;
+static_assert(kSmemBytesT<true> <= 232448, "dynamic shared memory over the 227 KB per-CTA limit");
 
 __device__ __forceinline__ int cluster_of_pair(long long gp, long long GP, int NC) {
   // largest c with floor(c * GP / NC) <= gp
@@ -292,7 +301,13 @@ __device__ __forceinline__ void split_pack(float p0, float p1, uint32_t& hi, uin
   lo = *reinterpret_cast<const uint32_t*>(&l);
 }
 
-template <int MODE, int VARIANT, int CG, int PREC, bool DBG>
+// RG (STEP, pass 2 alone): the upstream gradient is one value g_r per utterance row (p.grad_rows), not the scalar
+// p.grad_out.  The tail above the ring has 608 bytes left, too few for a staged fp32 copy of g_r (1 KB double
+// buffered), so |g_r| is folded into the staged log-sum-exp (exp2(S log2e - lse2 + log2 |g_r|) = p |g_r|, one more
+// fp32 rounding of an exponent that already carries one) and its sign is staged as one bit per stream row (SharedTailRG).
+// The fp16 planes carry p (g_r / gamma), gamma = max_r |g_r|, lifted by the largest q_r |g_r| / gamma; the flush
+// applies w gamma.
+template <int MODE, int VARIANT, int CG, int PREC, bool DBG, bool RG = false>
 __global__ void __launch_bounds__(kThreadsTc, 1)
 tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepSched sched, const TcParams p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -316,7 +331,8 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
   uint8_t* smem_al = smem_raw + (smem_base - smem_u32(smem_raw));
   const uint32_t a_smem = smem_base;
   const uint32_t ring_smem = smem_base + kMaxSlabs * kSlabBytes;
-  SharedTail* tail = reinterpret_cast<SharedTail*>(smem_al + kMaxSlabs * kSlabBytes + kRingBytes);
+  using Tail = std::conditional_t<RG, SharedTailRG, SharedTail>;
+  Tail* tail = reinterpret_cast<Tail*>(smem_al + kMaxSlabs * kSlabBytes + kRingBytes);
   const uint32_t bars = smem_u32(&tail->bars[0]);
   auto bar = [&](int i) { return bars + 8u * i; };
 
@@ -692,8 +708,13 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
     const float w = __ldg(p.w), b = __ldg(p.b), eps = p.eps;
     const float w2 = w * kLog2e, b2 = fmaf(w, eps, b) * kLog2e;   // log2-domain affine: S*log2e
     const float bb = fmaf(w, eps, b);
-    const float g = (kBwd && p.grad_out != nullptr) ? __ldg(p.grad_out) : 1.f;
+    const float g = (kBwd && !RG && p.grad_out != nullptr) ? __ldg(p.grad_out) : 1.f;
     const float wg = w * g;
+    float gamma = 1.f, inv_gamma = 1.f;   // RG, SPLIT pass 2: max_r |g_r| and its inverse (0 when every g_r is 0)
+    // RG: sign bits of g_r for stream rows [32 w, 32 w + 32) of the unit staged in buffer buf
+    auto gsign_of = [&](int buf, int w) -> uint32_t {
+      if constexpr (RG) return tail->gsign[buf][w]; else return 0u;
+    };
     // STEP, pass 1: every logit is bounded by |w| + (w eps + b) because |cos| <= 1, so the exponentials are
     // taken against that FIXED shift (log2 domain: m2) instead of a running row maximum: P <= 1, partial row
     // sums and partial accumulators of different clusters simply add, nothing is ever rescaled.  The
@@ -776,22 +797,48 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
           p.row_scale_out[r] = w * exp2f(static_cast<float>(-(kSplitLift + split_extra_lift(q))));
       }
       if (p.phases & PASS_CENTROIDS) {
-        dw_acc = fmaf(-q, cdv + eps, dw_acc);     // diagonal element G_jj = -g q (uses cos_diag)
-        db_acc -= eps * expf(-stat);              // item 12: db = -g sum eps / (sum exp + eps)
+        if (RG) {
+          const float gr = __ldg(p.grad_rows + r);
+          dw_acc = fmaf(-q * gr, cdv + eps, dw_acc);
+          db_acc -= gr * eps * expf(-stat);
+        } else {
+          dw_acc = fmaf(-q, cdv + eps, dw_acc);     // diagonal element G_jj = -g q (uses cos_diag)
+          db_acc -= eps * expf(-stat);              // item 12: db = -g sum eps / (sum exp + eps)
+        }
       }
     };
     auto close_rows = [&]() {
       const int U = p.n_own[SEG_DE];
       if (kSplit && (p.phases & PASS_CENTROIDS)) {
         // pass 2's lift: every CTA takes the maximum of q over ALL rows (U floats out of the L2)
-        float qm = 0.f;
-        for (int r = et; r < U; r += kEpiThreads) qm = fmaxf(qm, __ldg(p.row_aux + r));
-        qm = warp_max(qm);
-        if (lane == 0) tail->red[ew] = qm;
-        named_bar_sync(1, kEpiThreads);
-        qm = tail->red[0];
-        for (int i = 1; i < kEpiWarps; ++i) qm = fmaxf(qm, tail->red[i]);
-        lift2 = kSplitLift + split_extra_lift(qm);
+        if (RG) {
+          // the planes carry p g_r / gamma: the lift comes from max_r q_r |g_r| / gamma
+          float qm = 0.f, gm = 0.f;
+          for (int r = et; r < U; r += kEpiThreads) {
+            const float ga = fabsf(__ldg(p.grad_rows + r));
+            qm = fmaxf(qm, __ldg(p.row_aux + r) * ga);
+            gm = fmaxf(gm, ga);
+          }
+          qm = warp_max(qm);
+          gm = warp_max(gm);
+          if (lane == 0) { tail->red[ew] = qm; tail->red[kEpiWarps + ew] = gm; }
+          named_bar_sync(1, kEpiThreads);
+          qm = tail->red[0];
+          gm = tail->red[kEpiWarps];
+          for (int i = 1; i < kEpiWarps; ++i) { qm = fmaxf(qm, tail->red[i]); gm = fmaxf(gm, tail->red[kEpiWarps + i]); }
+          gamma = gm;
+          inv_gamma = gm > 0.f ? 1.f / gm : 0.f;
+          lift2 = kSplitLift + split_extra_lift(qm * inv_gamma);
+        } else {
+          float qm = 0.f;
+          for (int r = et; r < U; r += kEpiThreads) qm = fmaxf(qm, __ldg(p.row_aux + r));
+          qm = warp_max(qm);
+          if (lane == 0) tail->red[ew] = qm;
+          named_bar_sync(1, kEpiThreads);
+          qm = tail->red[0];
+          for (int i = 1; i < kEpiWarps; ++i) qm = fmaxf(qm, tail->red[i]);
+          lift2 = kSplitLift + split_extra_lift(qm);
+        }
         named_bar_sync(1, kEpiThreads);      // red is reused by the scalar reductions
       }
       for (int r = blockIdx.x * kEpiThreads + et; r < U; r += gridDim.x * kEpiThreads) close_row(r);
@@ -873,11 +920,23 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
                            __ldg(p.row_stat + orow) * kLog2e
                      : -INFINITY;
       // lse_s[buf] of unit u, loaded when this unit's turn comes (close_here: once its row sums are final)
+      // RG: g_r of stream row ur (0 past the end), loaded with the row's other inputs
+      auto grad_of = [&](int ur) -> float { return (RG && ur < n_str) ? __ldg(p.grad_rows + ur) : 0.f; };
+      // lse_s[buf][trow] (+ RG: |g_r| folded in, its sign into gsign); every lane of the warp takes part
+      auto stage_row = [&](int buf, bool valid, float raw, float cdv, float gr) {
+        float l = lse2_of(valid, raw, cdv);
+        if constexpr (RG) {
+          l -= log2f(fabsf(gr) * inv_gamma);      // exp2(. - l) = p |g_r| (/ gamma); g_r = 0: l = +inf, p = 0
+          const uint32_t neg = __ballot_sync(0xffffffffu, gr < 0.f);
+          if (lane == 0) tail->gsign[buf][quarter] = neg;
+        }
+        tail->lse_s[buf][trow] = l;
+      };
       auto stage_lse = [&](int u, int buf) {
         if (close_here) wait_tile(u);
         float raw = 0.f, cdv = 0.f;
         const bool v = lse2_raw(u * kUnit + trow, raw, cdv);
-        tail->lse_s[buf][trow] = lse2_of(v, raw, cdv);
+        stage_row(buf, v, raw, cdv, grad_of(u * kUnit + trow));
       };
       if (is_dc && half == 0) stage_lse(wk.unit(0, s0, s1), it & 1);
       bool deferred = false;     // the next unit's row sums were not final at prefetch time: staged at its turn
@@ -886,7 +945,7 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
         const int u = wk.unit(i, s0, s1);
         const int nu = min(kStepUnits, s1 - s0 - i);
         const int buf = it & 1;
-        float nraw = 0.f, ncd = 0.f;
+        float nraw = 0.f, ncd = 0.f, ngr = 0.f;
         bool nvalid = false;
         if (is_dc) {
           if (half == 0 && deferred) { stage_lse(u, buf); deferred = false; }
@@ -895,7 +954,10 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
           // a poll, never a wait, so that a late tile holds up its own unit only
           if (half == 0 && i + 1 < s1 - s0) {
             const int un = wk.unit(i + 1, s0, s1);
-            if (!close_here || tile_ready(un)) nvalid = lse2_raw(un * kUnit + trow, nraw, ncd);
+            if (!close_here || tile_ready(un)) {
+              nvalid = lse2_raw(un * kUnit + trow, nraw, ncd);
+              ngr = grad_of(un * kUnit + trow);
+            }
             else deferred = true;
           }
         }
@@ -934,6 +996,7 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
               const bool special = (cc < dhi) && (cc + 32 > dlo);
               const bool any_special = __any_sync(0xffffffffu, special);
               const float b2s = b2 + static_cast<float>(lift2);
+              const uint32_t neg = gsign_of(buf, ch);     // RG: signs of g_r (|g_r| / gamma is in ls)
 #pragma unroll
               for (int i = 0; i < 32; i += 2) {
                 const float2 l2 = *reinterpret_cast<const float2*>(ls + i);
@@ -943,6 +1006,10 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
                 if (any_special) {     // own speaker's rows
                   if (cc + i >= dlo && cc + i < dhi) p0 = 0.f;
                   if (cc + i + 1 >= dlo && cc + i + 1 < dhi) p1 = 0.f;
+                }
+                if (RG) {
+                  if ((neg >> i) & 1u) p0 = -p0;
+                  if ((neg >> (i + 1)) & 1u) p1 = -p1;
                 }
                 dw_seg = fmaf(p0, d0 + eps, dw_seg);
                 dw_seg = fmaf(p1, d1 + eps, dw_seg);
@@ -1008,6 +1075,7 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
             } else {
               // ---- pass 2: G tile = w g softmax(S), own speaker's rows masked, written back over T
               const float4* ls4 = reinterpret_cast<const float4*>(&tail->lse_s[buf][ch * 32]);
+              const uint32_t neg = gsign_of(buf, ch);     // RG: signs of g_r (|g_r| is in ls4)
               const bool special = (cc < dhi) && (cc + 32 > dlo);
               const bool any_special = __any_sync(0xffffffffu, special);
 #pragma unroll
@@ -1020,6 +1088,7 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
                   const float dot = __uint_as_float(v[i]);
                   float pr = ex2(fmaf(dot, w2, b2) - ls[q]);                     // lse = +inf past the end
                   if (any_special && cc + i >= dlo && cc + i < dhi) pr = 0.f;    // own speaker's rows
+                  if (RG && ((neg >> i) & 1u)) pr = -pr;                          // g_r p_rk
                   dw_seg = fmaf(pr, dot + eps, dw_seg);
                   gq[i] = __float_as_uint(round_tf32(wg * pr));
                 }
@@ -1034,7 +1103,7 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
           __syncwarp();
           if (lane == 0) arrive_leader(s_empty0 + 8u * buf);
         } else {
-          if (is_dc && half == 0 && i + 1 < s1 - s0 && !deferred) tail->lse_s[buf ^ 1][trow] = lse2_of(nvalid, nraw, ncd);
+          if (is_dc && half == 0 && i + 1 < s1 - s0 && !deferred) stage_row(buf ^ 1, nvalid, nraw, ncd, ngr);
           tmem_st_wait();
           tc_fence_before();
           __syncwarp();
@@ -1145,7 +1214,8 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
           }
           if (DBG && wk.kind == SEG_DE && wk.gp >= wk.end) tr.put(kTraceEvents - 3, globaltimer_ns());   // pass 1 out
         } else if (ovalid) {
-          dw_acc += kSplit ? dw_seg * exp2f(static_cast<float>(-lift2)) : dw_seg;
+          if (RG && kSplit) dw_acc += dw_seg * (exp2f(static_cast<float>(-lift2)) * gamma);
+          else dw_acc += kSplit ? dw_seg * exp2f(static_cast<float>(-lift2)) : dw_seg;
         }
         // drain the accumulator [128 x D] of this segment (columns split between the two halves)
         mbar_wait(bar(BAR_ACC_FULL), sg & 1);
@@ -1161,8 +1231,8 @@ tc_strip_kernel(const __grid_constant__ TmSet tms, const __grid_constant__ StepS
           uint32_t v[32];
           tmem_ld32(tmem + lane_addr + 2 * kUnit + ch * 32, v);
           tmem_ld_wait();
-          if (kSplit && is_dc) {       // the G planes carried p * 2^lift2: dC_hat = w g 2^-lift2 (.)
-            const float fs = wg * exp2f(static_cast<float>(-lift2));
+          if (kSplit && is_dc) {       // the G planes carried p * 2^lift2: dC_hat = w g 2^-lift2 (.)  (RG: w gamma)
+            const float fs = (RG ? wg * gamma : wg) * exp2f(static_cast<float>(-lift2));
 #pragma unroll
             for (int i = 0; i < 32; ++i) v[i] = __float_as_uint(__uint_as_float(v[i]) * fs);
           }
@@ -1728,13 +1798,13 @@ int make_step_sched(int OGe, int STe, int OGc, int STc, int phases, int max_cl, 
   return NC;
 }
 
-template <int MODE, int VARIANT, int CG, int PREC, bool DBG>
+template <int MODE, int VARIANT, int CG, int PREC, bool DBG, bool RG = false>
 int launch_tc_impl(const TmSet& tms, const StepSched& sched, const TcParams& p, int NC, bool pdl, cudaStream_t st) {
-  auto kern = tc_strip_kernel<MODE, VARIANT, CG, PREC, DBG>;
+  auto kern = tc_strip_kernel<MODE, VARIANT, CG, PREC, DBG, RG>;
   static bool attr_set[kMaxDevices] = {false};    // per instantiation and device
   const int dev = current_device();
   if (dev < 0 || dev >= kMaxDevices || !attr_set[dev]) {
-    GE2E_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes));
+    GE2E_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytesT<RG>));
     if (dev >= 0 && dev < kMaxDevices) attr_set[dev] = true;
   }
   TcParams q = p;
@@ -1744,7 +1814,7 @@ int launch_tc_impl(const TmSet& tms, const StepSched& sched, const TcParams& p, 
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(NC * CG);
   cfg.blockDim = dim3(kThreadsTc);
-  cfg.dynamicSmemBytes = kSmemBytes;
+  cfg.dynamicSmemBytes = kSmemBytesT<RG>;
   cfg.stream = st;
   cudaLaunchAttribute at[2];
   at[0].id = cudaLaunchAttributeClusterDimension;
@@ -1914,10 +1984,10 @@ int tc_fwd_rows(const RowsArgs& a, float* row_stat, int32_t* row_kstar, float* r
 // The softmax step on tensor cores.  phases = PASS_ROWS: forward rows + un-normalised dE_hat (+ row_scale);
 // PASS_CENTROIDS: dC_hat_partial, {dw, db} from the row statistics of an earlier PASS_ROWS launch;
 // both: one launch with a grid-wide barrier between the passes.
-int tc_step(const RowsArgs& a, int phases, const float* grad_out, const float* row_stat_in, const float* row_aux_in,
-            float* row_stat, float* row_aux, float* row_scale, float* loss_accum, float* per_row_out, float* dE_hat,
-            float* dC_hat_partial, float* dwdb_accum, void* ws, size_t ws_bytes, cudaStream_t st,
-            float* const* dC_owner, int n_ranks, int prec) {
+int tc_step(const RowsArgs& a, int phases, const float* grad_out, const float* grad_rows, const float* row_stat_in,
+            const float* row_aux_in, float* row_stat, float* row_aux, float* row_scale, float* loss_accum,
+            float* per_row_out, float* dE_hat, float* dC_hat_partial, float* dwdb_accum, void* ws, size_t ws_bytes,
+            cudaStream_t st, float* const* dC_owner, int n_ranks, int prec) {
   const int U = a.n_local * a.M;
   const bool peers = dC_owner != nullptr && n_ranks > 1;
   const bool split = prec != PREC_TF32;         // fp16 operand planes
@@ -1929,6 +1999,8 @@ int tc_step(const RowsArgs& a, int phases, const float* grad_out, const float* r
   if (peers && (n_ranks > kMaxPeers || a.n_total % n_ranks != 0 || (a.n_total / n_ranks) % kTile != 0 ||
                 !(phases & PASS_CENTROIDS)))
     return GE2E_ERR_UNSUPPORTED;
+  // a per-row upstream gradient is known only after the forward: the centroid pass alone, on one device
+  if (grad_rows != nullptr && (phases != PASS_CENTROIDS || peers)) return GE2E_ERR_UNSUPPORTED;
   if (ws == nullptr || ws_bytes < tc_workspace_bytes(a.n_local, a.n_total, a.M, a.D, a.variant)) return GE2E_ERR_WORKSPACE;
   if ((reinterpret_cast<uintptr_t>(ws) & 15) != 0) return GE2E_ERR_WORKSPACE;
   const int cg = pick_cg(a.D);
@@ -1941,7 +2013,7 @@ int tc_step(const RowsArgs& a, int phases, const float* grad_out, const float* r
   if (split) p.oslabs = (prec == PREC_SPLIT ? 2 : 1) * (a.D / 64);
   if (hyb) p.oslabs = a.D / 64;
   p.phases = phases;
-  p.row_stat = row_stat_in; p.row_aux = row_aux_in; p.grad_out = grad_out; p.dwdb = dwdb_accum;
+  p.row_stat = row_stat_in; p.row_aux = row_aux_in; p.grad_out = grad_out; p.grad_rows = grad_rows; p.dwdb = dwdb_accum;
   p.row_stat_out = row_stat; p.row_aux_out = row_aux; p.row_scale_out = row_scale; p.loss_accum = loss_accum;
   p.per_row_out = per_row_out;
   p.n_own[SEG_DE] = U; p.n_str[SEG_DE] = a.n_total;
@@ -2018,6 +2090,14 @@ int tc_step(const RowsArgs& a, int phases, const float* grad_out, const float* r
       if (dC_owner[r] == nullptr || (reinterpret_cast<uintptr_t>(dC_owner[r]) & 15) != 0) return GE2E_ERR_ARGUMENT;
       if ((rc = make_map_2d(&tms.out_peer[r], dC_owner[r], p.peer_rows, a.D, kTile)) != GE2E_OK) return rc;
     }
+  }
+  if (grad_rows != nullptr) {     // row-gradient instantiations (no instrumented twins); phases == PASS_CENTROIDS
+    if (split)
+      return prec == PREC_F16 ? launch_tc_impl<TC_STEP, GE2E_SOFTMAX, 2, PREC_F16, false, true>(tms, sched, p, NC, false, st)
+                              : launch_tc_impl<TC_STEP, GE2E_SOFTMAX, 2, PREC_SPLIT, false, true>(tms, sched, p, NC, false, st);
+    if (hyb) return launch_tc_impl<TC_STEP, GE2E_SOFTMAX, 2, PREC_HYB, false, true>(tms, sched, p, NC, true, st);
+    return cg == 2 ? launch_tc_impl<TC_STEP, GE2E_SOFTMAX, 2, PREC_TF32, false, true>(tms, sched, p, NC, false, st)
+                   : launch_tc_impl<TC_STEP, GE2E_SOFTMAX, 1, PREC_TF32, false, true>(tms, sched, p, NC, false, st);
   }
   if (split) return launch_tc_split<TC_STEP>(prec, tms, sched, p, NC, phases != PASS_CENTROIDS, st);
   if (hyb) {

@@ -4,12 +4,13 @@ Same constructor (``GE2ELoss(hp)`` reading ``hp.general.device`` and ``hp.genera
 same learnable 0-dim ``w`` / ``b`` parameters (10.0 / -5.0, s3:16-17), same
 ``forward(embeddings[N, M, D]) -> 0-dim loss`` and the same static helpers, so
 ``s4_train_embed_model.py`` and ``s5_eval_model.py`` can use it unchanged.  Extensions (keyword
-only): ``variant`` ("softmax" | "contrast"), ``precision`` ("fp32" | "tf32") and
-``process_group`` (speaker-sharded multi-GPU).  CUDA (sm_100a) only: CPU tensors raise.
+only): ``variant`` ("softmax" | "contrast"), ``precision`` ("fp32" | "tf32"), ``reduction`` ("sum" |
+"mean" | "none") and ``process_group`` (speaker-sharded multi-GPU).  CUDA (sm_100a) only: CPU tensors raise.
 """
 from __future__ import annotations
 
 import torch
+import torch.distributed as dist
 import torch.nn as nn
 
 from . import _lib, ops
@@ -28,8 +29,13 @@ def _hp_get(hp, name, default):
 
 class GE2ELoss(nn.Module):
     def __init__(self, hp=None, *, w: float = 10.0, b: float = -5.0, variant=None,
-                 precision=None, eps=None, device=None, process_group=None):
+                 precision=None, eps=None, device=None, process_group=None, reduction: str = "sum"):
         super().__init__()
+        # reduction="none": per-utterance losses [N, M] (calc_loss's per_embedding_loss, s3:121), differentiable
+        if reduction not in ops.REDUCTIONS:
+            raise ValueError(f"reduction must be one of {ops.REDUCTIONS}, got {reduction!r}")
+        if reduction == "none" and process_group is not None:
+            raise ValueError('reduction="none" is not supported together with a process_group')
         # the reference's trainer constructs GE2ELoss(hp) with no keywords (s4_train_embed_model.py:33):
         # the two opt-in extensions can therefore also come from hp.general (ge2e_variant / ge2e_precision);
         # absent both, the defaults reproduce the reference (softmax, fp32 arithmetic)
@@ -45,6 +51,7 @@ class GE2ELoss(nn.Module):
         self.variant = variant
         self.precision = precision
         self.process_group = process_group
+        self.reduction = reduction
         # s3:16-17
         self.w = nn.Parameter(torch.tensor(float(w)).to(self.device), requires_grad=True)
         self.b = nn.Parameter(torch.tensor(float(b)).to(self.device), requires_grad=True)
@@ -57,9 +64,13 @@ class GE2ELoss(nn.Module):
         if self.process_group is not None:
             if unperm is not None:
                 raise ValueError("unperm is not supported together with a process_group")
-            return sharded_ge2e_loss(embeddings, self.w, self.b, self.eps, self.variant, self.precision,
+            loss = sharded_ge2e_loss(embeddings, self.w, self.b, self.eps, self.variant, self.precision,
                                      self.process_group)
-        return ops.ge2e_loss(embeddings, self.w, self.b, self.eps, self.variant, self.precision, unperm, speakers)
+            if self.reduction == "mean":     # the global sum over every rank's N_local * M utterances
+                loss = loss / (embeddings.shape[0] * embeddings.shape[1] * dist.get_world_size(self.process_group))
+            return loss
+        return ops.ge2e_loss(embeddings, self.w, self.b, self.eps, self.variant, self.precision, unperm, speakers,
+                             reduction=self.reduction)
 
     @torch.no_grad()
     def clip_and_sgd_step(self, lr: float, max_norm: float = 1.0, return_norm: bool = False):

@@ -1,6 +1,7 @@
 """torch.library custom ops over the C ABI (CUDA only; raises on CPU tensors).
 
-``ge2e_b200::fwd`` / ``ge2e_b200::bwd`` are the single-device ops; the staged ops
+``ge2e_b200::fwd`` / ``ge2e_b200::bwd`` are the single-device ops (``fwd_per_row`` / ``bwd_per_row``: the
+per-utterance losses of reduction="none" and their per-row upstream gradient); the staged ops
 (``prep``, ``fwd_rows``, ``bwd_rows``, ``bwd_finalize``) are what the speaker-sharded
 autograd function in ``sharded.py`` strings together around its collectives.
 """
@@ -134,14 +135,15 @@ def _tc_softmax(N: int, M: int, D: int, variant: int, precision: int) -> bool:
 
 
 def _fwd_impl(E: Tensor, w: Tensor, b: Tensor, eps: float, variant: int, precision: int, packed: bool,
-              row_index: Optional[Tensor] = None, speakers: int = 0, want_grad: bool = True):
+              row_index: Optional[Tensor] = None, speakers: int = 0, want_grad: bool = True, per_row: bool = False):
     """GE2ELoss.forward (reference s3:19-30) through the C ABI.  ``packed``: the per-call intermediates
     come out of ONE allocation (views); the custom op needs non-aliasing outputs and passes False.
     ``row_index`` (with ``speakers``): E is [U, D] in the embedder's row order and logical row r lives
     at row_index[r] (the trainer's ``embeddings[unperm]``, s4:189-192, folded into the kernels).
     ``want_grad``: a backward will follow (tensor-core softmax path: the forward prepares dE_hat).
     Returns (loss, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale); the last two
-    are 1-element placeholders where the path does not use them."""
+    are 1-element placeholders where the path does not use them.  ``per_row``: the first element is the
+    per-utterance losses [N, M] (logical order) instead of their sum."""
     _need_cuda(E, w, b)
     (E, ecode), (w, b) = _emb(E), _params(w, b)
     if _lib.planes_need_copy(E.data_ptr(), precision, E.element_size()):
@@ -182,6 +184,15 @@ def _fwd_impl(E: Tensor, w: Tensor, b: Tensor, eps: float, variant: int, precisi
             dE_hat = dE_hat.view(U, D)
         row_kstar = torch.empty(U if variant == _lib.CONTRAST else 1, dtype=torch.int32, device=dev)
         ws, ws_bytes = _workspace(N, N, M, D, variant, precision, dev)
+        if per_row:
+            per = torch.empty((N, M), dtype=torch.float32, device=dev)
+            rc = lib().ge2e_b200_forward_per_row_typed(
+                E.data_ptr(), ecode, _ptr(row_index), N, M, D, w.data_ptr(), b.data_ptr(), eps, variant, precision,
+                e_hat.data_ptr(), c_hat.data_ptr(), cos_diag.data_ptr(), row_stat.data_ptr(), row_kstar.data_ptr(),
+                row_aux.data_ptr(), accum.data_ptr(), dE_hat.data_ptr() if fused else None,
+                row_scale.data_ptr() if fused else None, per.data_ptr(), _ptr(ws), ws_bytes, _stream())
+            _check(rc, "ge2e_b200_forward_per_row_typed")
+            return per, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale
         rc = lib().ge2e_b200_forward_typed(E.data_ptr(), ecode, _ptr(row_index), N, M, D, w.data_ptr(), b.data_ptr(),
                                            eps, variant, precision, e_hat.data_ptr(), c_hat.data_ptr(),
                                            cos_diag.data_ptr(), row_stat.data_ptr(), row_kstar.data_ptr(),
@@ -193,9 +204,10 @@ def _fwd_impl(E: Tensor, w: Tensor, b: Tensor, eps: float, variant: int, precisi
 
 
 def _bwd_impl(grad_out, E, w, b, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale, eps,
-              variant, precision, row_index: Optional[Tensor] = None):
+              variant, precision, row_index: Optional[Tensor] = None, per_row: bool = False):
     """loss.backward() (s4:200) through the C ABI.  ``dE_hat`` / ``row_scale``: what the forward prepared
-    (1-element placeholders where the path does not use them).  Returns (dE shaped like E, dwdb[2])."""
+    (1-element placeholders where the path does not use them).  ``per_row``: grad_out is the upstream gradient
+    of the per-utterance losses, [N, M].  Returns (dE shaped like E, dwdb[2])."""
     _need_cuda(grad_out, E, w, b)
     (E, ecode), (w, b) = _emb(E), _params(w, b)
     g = _f32c(grad_out)
@@ -212,13 +224,14 @@ def _bwd_impl(grad_out, E, w, b, e_hat, c_hat, cos_diag, row_stat, row_kstar, ro
         dC_ptr = scratch.data_ptr() + 16
         dE_hat_ptr = dE_hat.data_ptr() if fused else dC_ptr + N * D * 4
         ws, ws_bytes = _workspace(N, N, M, D, variant, precision, dev)
-        rc = lib().ge2e_b200_backward_typed(E.data_ptr(), ecode, _ptr(row_index), e_hat.data_ptr(), c_hat.data_ptr(),
-                                            cos_diag.data_ptr(), row_stat.data_ptr(), row_kstar.data_ptr(),
-                                            row_aux.data_ptr(), row_scale.data_ptr() if fused else None, N, M, D,
-                                            w.data_ptr(), b.data_ptr(), eps, variant, precision, g.data_ptr(),
-                                            dE_hat_ptr, dC_ptr, scratch.data_ptr(), dE.data_ptr(), ecode, _ptr(ws),
-                                            ws_bytes, _stream())
-    _check(rc, "ge2e_b200_backward")
+        if per_row and g.numel() != U:
+            raise ValueError(f"the upstream gradient of the per-utterance losses needs {U} entries, got {g.numel()}")
+        entry = lib().ge2e_b200_backward_per_row_typed if per_row else lib().ge2e_b200_backward_typed
+        rc = entry(E.data_ptr(), ecode, _ptr(row_index), e_hat.data_ptr(), c_hat.data_ptr(), cos_diag.data_ptr(),
+                   row_stat.data_ptr(), row_kstar.data_ptr(), row_aux.data_ptr(), row_scale.data_ptr() if fused else None,
+                   N, M, D, w.data_ptr(), b.data_ptr(), eps, variant, precision, g.data_ptr(), dE_hat_ptr, dC_ptr,
+                   scratch.data_ptr(), dE.data_ptr(), ecode, _ptr(ws), ws_bytes, _stream())
+    _check(rc, "ge2e_b200_backward_per_row_typed" if per_row else "ge2e_b200_backward")
     return dE, scratch[1:3]
 
 
@@ -276,6 +289,52 @@ def _fwd_backward(ctx, g_loss, *_unused):
 
 
 ge2e_fwd.register_autograd(_fwd_backward, setup_context=_fwd_setup)
+
+
+@torch.library.custom_op("ge2e_b200::fwd_per_row", mutates_args=())
+def ge2e_fwd_per_row(E: Tensor, w: Tensor, b: Tensor, eps: float, variant: int,
+                     precision: int) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """ge2e_b200::fwd with the per-utterance losses [N, M] (reduction="none") in place of their sum."""
+    return _fwd_impl(E, w, b, eps, variant, precision, packed=False, per_row=True)
+
+
+@ge2e_fwd_per_row.register_fake
+def _(E, w, b, eps, variant, precision):
+    N, M, D = E.shape
+    U = N * M
+    fused = _tc_softmax(N, M, D, variant, precision)
+    f32 = torch.float32
+    return (E.new_empty((N, M), dtype=f32), E.new_empty((U, D), dtype=f32), E.new_empty((N, D), dtype=f32),
+            E.new_empty(U, dtype=f32), E.new_empty(U, dtype=f32),
+            E.new_empty(U if variant == _lib.CONTRAST else 1, dtype=torch.int32), E.new_empty(U, dtype=f32),
+            E.new_empty((U, D) if fused else (1,), dtype=f32), E.new_empty(U if fused else 1, dtype=f32))
+
+
+@torch.library.custom_op("ge2e_b200::bwd_per_row", mutates_args=())
+def ge2e_bwd_per_row(grad_rows: Tensor, E: Tensor, w: Tensor, b: Tensor, e_hat: Tensor, c_hat: Tensor,
+                     cos_diag: Tensor, row_stat: Tensor, row_kstar: Tensor, row_aux: Tensor, dE_hat: Tensor,
+                     row_scale: Tensor, eps: float, variant: int, precision: int) -> Tuple[Tensor, Tensor]:
+    """Backward of ge2e_b200::fwd_per_row for the upstream gradient grad_rows[N, M].  Returns (dE[N,M,D], dwdb[2])."""
+    dE, dwdb = _bwd_impl(grad_rows.contiguous(), E, w, b, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat,
+                         row_scale, eps, variant, precision, per_row=True)
+    return dE, dwdb.clone()
+
+
+@ge2e_bwd_per_row.register_fake
+def _(grad_rows, E, w, b, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale, eps, variant,
+      precision):
+    return torch.empty_like(E), E.new_empty(2, dtype=torch.float32)
+
+
+def _fwd_per_row_backward(ctx, g_rows, *_unused):
+    E, w, b, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale = ctx.saved_tensors
+    eps, variant, precision = ctx.cfg
+    dE, dwdb = ge2e_bwd_per_row(g_rows.to(torch.float32), E, w, b, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux,
+                                dE_hat, row_scale, eps, variant, precision)
+    return dE, dwdb[0], dwdb[1], None, None, None
+
+
+ge2e_fwd_per_row.register_autograd(_fwd_per_row_backward, setup_context=_fwd_setup)
 
 
 # --------------------------------------------------------------------------- eager module path
@@ -509,18 +568,101 @@ class _GE2EEager(torch.autograd.Function):
         return dE, accum[1], accum[2], None, None, None, None, None
 
 
+class _GE2EPerRow(torch.autograd.Function):
+    """reduction="none": the per-utterance losses L[N, M] (logical order) through ge2e_b200_forward_per_row_typed, and
+    dE = sum_r g_r dL_r/dE through ge2e_b200_backward_per_row_typed.  The upstream gradient is unknown when the forward
+    runs, so this is always the staged pipeline: forward kernels now (the tensor-core softmax paths also prepare
+    dE_hat / row_scale when a gradient is needed), backward kernels in backward."""
+
+    @staticmethod
+    def forward(ctx, E, w, b, eps, variant, precision, row_index, speakers):
+        if not (E.is_cuda and w.is_cuda and b.is_cuda):
+            raise RuntimeError("speaker_embedding_ge2e_loss_b200 runs on CUDA (sm_100a) tensors only; "
+                               "there is no CPU fallback")
+        (E, ecode), _ = _emb(E), _params(w, b)
+        if row_index is None:
+            N, M, D = E.shape
+        else:
+            U_, D = E.shape
+            N, M = speakers, U_ // max(1, speakers)
+            if speakers <= 0 or N * M != U_:
+                raise ValueError(f"{U_} rows do not split into {speakers} speakers")
+        dev = E.device
+        plan = _eager_plan(dev, N, M, D, variant, precision, ecode)
+        if plan.planes and E.data_ptr() % (4 * E.element_size()):
+            E = E.clone()           # the fp16-plane kernels read E four elements at a time
+        want_grad = ctx.needs_input_grad[0] or ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
+        if want_grad and not plan.bwd_ok:
+            _lib.check_backward_shape(M, D)
+        fused = want_grad and plan.fused
+        with _on_device(dev):
+            bufs = plan.take()
+            accum = torch.empty(4, dtype=torch.float32, device=dev)
+            per = torch.empty((N, M), dtype=torch.float32, device=dev)     # escapes: never pooled
+            stream = _raw_stream(plan.dev_index)
+            ws = plan.workspace(stream)
+            rc = lib().ge2e_b200_forward_per_row_typed(
+                E.data_ptr(), ecode, _ptr(row_index), N, M, D, w.data_ptr(), b.data_ptr(), eps, variant, precision,
+                *bufs.fwd_ptrs, accum.data_ptr(), bufs.dE_hat.data_ptr() if fused else None,
+                bufs.row_scale.data_ptr() if fused else None, per.data_ptr(), _ptr(ws), plan.ws_bytes, stream)
+        _check(rc, "ge2e_b200_forward_per_row_typed")
+        ctx.save_for_backward(E, w, b)
+        ctx.lease = _Lease(bufs)
+        ctx.cfg = (eps, variant, precision, plan, fused, row_index, N, M, D)
+        return per
+
+    @staticmethod
+    def backward(ctx, g_per):
+        E, w, b = ctx.saved_tensors
+        eps, variant, precision, plan, fused, row_index, N, M, D = ctx.cfg
+        bufs = ctx.lease.bufs
+        dev = E.device
+        # one float32 per utterance row, contiguous: `per.sum().backward()` hands over an expanded (stride-0) ones
+        g = g_per.to(dev, torch.float32).contiguous()
+        with _on_device(dev):
+            dE = torch.empty_like(E)
+            accum = torch.empty(4, dtype=torch.float32, device=dev)     # escapes as dw / db: never pooled
+            stream = _raw_stream(plan.dev_index)
+            ws = plan.workspace(stream)
+            rc = lib().ge2e_b200_backward_per_row_typed(
+                E.data_ptr(), plan.dtype, _ptr(row_index), bufs.e_hat.data_ptr(), bufs.c_hat.data_ptr(),
+                bufs.cos_diag.data_ptr(), bufs.row_stat.data_ptr(), bufs.kstar.data_ptr(), bufs.row_aux.data_ptr(),
+                bufs.row_scale.data_ptr() if fused else None, N, M, D, w.data_ptr(), b.data_ptr(), eps, variant,
+                precision, g.data_ptr(), bufs.dE_hat.data_ptr(), bufs.dC_hat.data_ptr(), accum.data_ptr(), dE.data_ptr(),
+                plan.dtype, _ptr(ws), plan.ws_bytes, stream)
+        _check(rc, "ge2e_b200_backward_per_row_typed")
+        return dE, accum[1], accum[2], None, None, None, None, None
+
+
 # host-only query (a ctypes call): under torch.compile its answer is a constant of the traced graph
 _resolve_precision = torch.compiler.assume_constant_result(_lib.resolve_precision)
 
 
+REDUCTIONS = ("sum", "mean", "none")
+
+
 def ge2e_loss(E: Tensor, w: Tensor, b: Tensor, eps: float = 1e-6, variant: str = "softmax",
-              precision: str = "fp32", unperm: Optional[Tensor] = None, speakers: int = 0) -> Tensor:
+              precision: str = "fp32", unperm: Optional[Tensor] = None, speakers: int = 0, *,
+              reduction: str = "sum") -> Tensor:
     """Functional form: differentiable in E, w, b.  Eager calls go through a plain autograd.Function;
     under torch.compile the registered custom ops (same kernels) are used.
 
     ``unperm`` (with ``speakers`` = N): E is the embedder's output [N*M, D] in shuffled row order and
     the loss is that of ``E[unperm].reshape(N, M, D)`` (s4_train_embed_model.py:189-192); the gather and
-    the scatter of its backward happen inside the kernels, dE comes back in E's row order."""
+    the scatter of its backward happen inside the kernels, dE comes back in E's row order.
+
+    ``reduction``: "sum" (the reference's 0-dim loss), "mean" (the sum over N*M) or "none": the per-utterance
+    losses L[N, M] as float32 in logical [speaker][utterance] order (calc_loss's per_embedding_loss, s3:121),
+    differentiable for any upstream gradient g[N, M]."""
+    if reduction not in REDUCTIONS:
+        raise ValueError(f"reduction must be one of {REDUCTIONS}, got {reduction!r}")
+    loss = _ge2e_loss(E, w, b, eps, variant, precision, unperm, speakers, reduction == "none")
+    if reduction == "mean":
+        return loss / (E.shape[0] if unperm is not None else E.shape[0] * E.shape[1])
+    return loss
+
+
+def _ge2e_loss(E, w, b, eps, variant, precision, unperm, speakers, per_row: bool) -> Tensor:
     if unperm is not None:
         if E.dim() != 2:
             raise ValueError(f"with unperm the embeddings must be [N*M, D], got {tuple(E.shape)}")
@@ -529,9 +671,10 @@ def ge2e_loss(E: Tensor, w: Tensor, b: Tensor, eps: float = 1e-6, variant: str =
         N, vcode = speakers, _lib.VARIANTS[variant]
         pcode = _resolve_precision(precision, N, N, E.shape[0] // N, E.shape[1], vcode)
         if torch.compiler.is_compiling():
-            return ge2e_fwd(E[unperm].reshape(N, E.shape[0] // N, E.shape[1]), w, b, float(eps), vcode, pcode)[0]
+            op = ge2e_fwd_per_row if per_row else ge2e_fwd
+            return op(E[unperm].reshape(N, E.shape[0] // N, E.shape[1]), w, b, float(eps), vcode, pcode)[0]
         idx = _index_ok(unperm, E.shape[0], E.device)
-        return _GE2EEager.apply(E, w, b, float(eps), vcode, pcode, idx, speakers)
+        return (_GE2EPerRow if per_row else _GE2EEager).apply(E, w, b, float(eps), vcode, pcode, idx, speakers)
     if E.dim() != 3:
         raise ValueError(f"embeddings must be [N, M, D], got {tuple(E.shape)}")
     if E.shape[1] < 2:
@@ -539,8 +682,8 @@ def ge2e_loss(E: Tensor, w: Tensor, b: Tensor, eps: float = 1e-6, variant: str =
     vcode = _lib.VARIANTS[variant]
     pcode = _resolve_precision(precision, E.shape[0], E.shape[0], E.shape[1], E.shape[2], vcode)
     if torch.compiler.is_compiling():
-        return ge2e_fwd(E, w, b, float(eps), vcode, pcode)[0]
-    return _GE2EEager.apply(E, w, b, float(eps), vcode, pcode, None, 0)
+        return (ge2e_fwd_per_row if per_row else ge2e_fwd)(E, w, b, float(eps), vcode, pcode)[0]
+    return (_GE2EPerRow if per_row else _GE2EEager).apply(E, w, b, float(eps), vcode, pcode, None, 0)
 
 
 # --------------------------------------------------------------------------- staged (plain functions)
