@@ -69,7 +69,7 @@ def measure(pkg, ops, lib_codes, workload, precision, steps, rounds, dev):
 
     # saved forwards for the backward-only graphs: the tensor-core softmax paths prepare dE_hat / row_scale
     w, b = crit_none.w.detach(), crit_none.b.detach()
-    saved = [ops._fwd_impl(E.detach(), w, b, crit_none.eps, vcode, pcode, packed=False, per_row=True)
+    saved = [ops._fwd_impl(E.detach(), w, b, crit_none.eps, vcode, pcode, per_row=True)
              for E in Es]
     one = torch.ones((), device=dev)
 

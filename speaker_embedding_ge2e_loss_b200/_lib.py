@@ -34,6 +34,13 @@ def resolve_precision(name: str, n_local: int, n_total: int, M: int, D: int, var
         return TF32           # shapes the fp16-operand kernels do not cover: the TF32 permission
     return PRECISIONS[name]
 
+
+def prepares_dE_hat(n_local: int, n_total: int, M: int, D: int, variant: int, precision: int) -> bool:
+    """True where the softmax loss runs on tensor cores: there a forward with a backward to follow also leaves the
+    un-normalised dE_hat rows + row_scale (ge2e_b200_fwd_rows), the backward rows stage is the centroid pass alone,
+    and the finalize applies row_scale."""
+    return variant == SOFTMAX and lib().ge2e_b200_path(n_local, n_total, M, D, variant, precision) > 0
+
 def check_backward_shape(M: int, D: int) -> None:
     """ValueError (before anything is launched) for an M whose backward the kernels cannot run at width D."""
     m = lib().ge2e_b200_max_utterances(D)

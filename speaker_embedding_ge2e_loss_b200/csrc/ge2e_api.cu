@@ -147,7 +147,7 @@ static int fwd_rows_impl(const float* e_hat, const float* c_hat_all, const float
                        const float* b, float eps, int variant, int precision, float* row_stat,
                        int32_t* row_kstar, float* row_aux, float* loss_accum, float* per_row_out,
                        float* sim_out, float* dE_hat, float* row_scale, void* workspace, size_t workspace_bytes,
-                       bool after_prep, ge2e_stream_t stream) {
+                       ge2e_stream_t stream) {
   if (!e_hat || !c_hat_all || !cos_diag || !w || !b || !row_stat || !loss_accum)
     return GE2E_ERR_ARGUMENT;
   int rc = check_shape(n_local, n_total, spk_offset, M, D);
@@ -160,24 +160,12 @@ static int fwd_rows_impl(const float* e_hat, const float* c_hat_all, const float
   if (on_tc(n_local, n_total, M, D, variant, precision)) {
     // the tensor-core path never materialises S: sim_out is an fp32-path feature
     if (sim_out != nullptr) return GE2E_ERR_UNSUPPORTED;
-    if (workspace_bytes < tc_workspace_bytes(n_local, n_total, M, D, variant) ||
-        (workspace == nullptr && tc_workspace_bytes(n_local, n_total, M, D, variant) > 0))
-      return GE2E_ERR_WORKSPACE;
-    if (is_planes(precision)) {
-      // the forward kernel closes the rows; with a backward to follow, the rows pass of the step kernel then
-      // forms dE_hat from probabilities that are already normalised (see ge2e_tc.cu, PREC_SPLIT)
-      rc = tc_fwd_rows(a, row_stat, row_kstar, row_aux, loss_accum, per_row_out, workspace, workspace_bytes, after_prep,
-                       (cudaStream_t)stream, tc_prec(precision));
-      if (rc != GE2E_OK || dE_hat == nullptr || row_scale == nullptr) return rc;
-      return tc_step(a, 1, nullptr, nullptr, row_stat, row_aux, nullptr, nullptr, row_scale, nullptr, nullptr, dE_hat, nullptr,
-                     nullptr, workspace, workspace_bytes, (cudaStream_t)stream, nullptr, 0, tc_prec(precision));
-    }
-    // softmax with a backward to follow: the rows pass of the step kernel (loss + un-normalised dE_hat)
-    if (variant == GE2E_SOFTMAX && dE_hat != nullptr && row_scale != nullptr)
-      return tc_step(a, 1, nullptr, nullptr, nullptr, nullptr, row_stat, row_aux, row_scale, loss_accum, per_row_out, dE_hat,
-                     nullptr, nullptr, workspace, workspace_bytes, (cudaStream_t)stream);
-    return tc_fwd_rows(a, row_stat, row_kstar, row_aux, loss_accum, per_row_out, workspace, workspace_bytes,
-                       after_prep, (cudaStream_t)stream);
+    TcRowsBufs t;
+    t.row_stat = row_stat; t.row_kstar = row_kstar; t.row_aux = row_aux; t.loss_accum = loss_accum;
+    t.per_row = per_row_out; t.dE_hat = dE_hat; t.row_scale = row_scale;
+    // softmax with a backward to follow: the rows pass of the step kernel also leaves the un-normalised dE_hat
+    const int phases = (variant == GE2E_SOFTMAX && dE_hat != nullptr && row_scale != nullptr) ? 1 : 0;
+    return tc_rows(a, tc_prec(precision), phases, t, workspace, workspace_bytes, (cudaStream_t)stream);
   }
   return simt_fwd_rows(a, row_stat, row_kstar, row_aux, loss_accum, per_row_out, sim_out,
                        (cudaStream_t)stream);
@@ -191,7 +179,7 @@ int ge2e_b200_fwd_rows(const float* e_hat, const float* c_hat_all, const float* 
                        ge2e_stream_t stream) {
   return fwd_rows_impl(e_hat, c_hat_all, cos_diag, n_local, n_total, spk_offset, M, D, w, b, eps, variant,
                        precision, row_stat, row_kstar, row_aux, loss_accum, per_row_out, sim_out, dE_hat, row_scale,
-                       workspace, workspace_bytes, false, stream);
+                       workspace, workspace_bytes, stream);
 }
 
 // grad_rows (nullable): the upstream gradient per local utterance row, in place of the scalar grad_out
@@ -216,12 +204,11 @@ static int bwd_rows_impl(const float* e_hat, const float* c_hat_all, const float
   if (is_planes(precision) && (!on_tc(n_local, n_total, M, D, variant, precision) || row_scale == nullptr))
     return GE2E_ERR_UNSUPPORTED;
   if (variant == GE2E_SOFTMAX && row_scale != nullptr && on_tc(n_local, n_total, M, D, variant, precision)) {
-    if (workspace_bytes < tc_workspace_bytes(n_local, n_total, M, D, variant) ||
-        (workspace == nullptr && tc_workspace_bytes(n_local, n_total, M, D, variant) > 0))
-      return GE2E_ERR_WORKSPACE;
-    return tc_step(a, 2, grad_out, grad_rows, row_stat, row_aux, nullptr, nullptr, nullptr, nullptr, nullptr, dE_hat,
-                   dC_hat_partial, dwdb_accum, workspace, workspace_bytes, (cudaStream_t)stream, nullptr, 0,
-                   tc_prec(precision));
+    TcRowsBufs t;
+    t.grad_out = grad_out; t.grad_rows = grad_rows;
+    t.row_stat = const_cast<float*>(row_stat); t.row_aux = const_cast<float*>(row_aux);   // read by the centroid pass
+    t.dE_hat = dE_hat; t.dC_hat_partial = dC_hat_partial; t.dwdb = dwdb_accum;
+    return tc_rows(a, tc_prec(precision), 2, t, workspace, workspace_bytes, (cudaStream_t)stream);
   }
   return simt_bwd_rows(a, row_stat, row_kstar, row_aux, grad_out, grad_rows, dE_hat, dC_hat_partial, dwdb_accum,
                        (cudaStream_t)stream);
@@ -355,11 +342,10 @@ static int forward_impl(const void* E, int e_dtype, const int32_t* row_index, in
   if ((rc = check_dtypes(e_dtype, GE2E_DT_F32)) != GE2E_OK) return rc;
   // tensor-core path: prep and the rows kernel are adjacent in the stream, the second one is launched
   // programmatically under the first one's tail
-  const bool tc = on_tc(N, N, M, D, variant, precision);
   rc = ge2e_b200_prep_typed(E, e_dtype, row_index, N, M, D, precision, e_hat, c_hat, cos_diag, accum, stream);
   if (rc != GE2E_OK) return rc;
   return fwd_rows_impl(e_hat, c_hat, cos_diag, N, N, 0, M, D, w, b, eps, variant, precision, row_stat, row_kstar,
-                       row_aux, accum, per_row, nullptr, dE_hat, row_scale, workspace, workspace_bytes, tc, stream);
+                       row_aux, accum, per_row, nullptr, dE_hat, row_scale, workspace, workspace_bytes, stream);
 }
 
 int ge2e_b200_forward_typed(const void* E, int e_dtype, const int32_t* row_index, int N, int M, int D, const float* w,
@@ -478,23 +464,18 @@ int ge2e_b200_step_rows(const float* e_hat, const float* c_hat_all, const float*
   if ((rc = check_enum(variant, precision)) != GE2E_OK) return rc;
   if (variant == GE2E_CONTRAST && !row_kstar) return GE2E_ERR_ARGUMENT;
   if (tc_softmax_step(n_local, n_total, M, D, variant, precision)) {
-    // ONE launch: rows pass, grid-wide barrier, centroid pass ({loss, dw, db} += into accum: zeroed by prep)
+    // both passes of the step kernel, in which pass 2 waits per utterance tile for the row sums of pass 1
+    // ({loss, dw, db} += into accum: zeroed by prep)
     RowsArgs a{e_hat, c_hat_all, cos_diag, n_local, n_total, spk_offset, M, D, w, b, eps, variant};
-    if (is_planes(precision)) {
-      // two launches: the forward kernel closes the rows (loss, lse, q), the step kernel runs both passes on them
-      rc = tc_fwd_rows(a, row_stat, row_kstar, row_aux, accum, nullptr, workspace, workspace_bytes, true,
-                       (cudaStream_t)stream, tc_prec(precision));
-      if (rc != GE2E_OK) return rc;
-      return tc_step(a, 3, grad_out, nullptr, row_stat, row_aux, nullptr, nullptr, row_scale, nullptr, nullptr, dE_hat,
-                     dC_hat_partial, accum + 1, workspace, workspace_bytes, (cudaStream_t)stream, nullptr, 0, tc_prec(precision));
-    }
-    return tc_step(a, 3, grad_out, nullptr, nullptr, nullptr, row_stat, row_aux, row_scale, accum, nullptr, dE_hat,
-                   dC_hat_partial, accum + 1, workspace, workspace_bytes, (cudaStream_t)stream);
+    TcRowsBufs t;
+    t.grad_out = grad_out; t.row_stat = row_stat; t.row_kstar = row_kstar; t.row_aux = row_aux; t.row_scale = row_scale;
+    t.loss_accum = accum; t.dE_hat = dE_hat; t.dC_hat_partial = dC_hat_partial; t.dwdb = accum + 1;
+    return tc_rows(a, tc_prec(precision), 3, t, workspace, workspace_bytes, (cudaStream_t)stream);
   }
   if (is_planes(precision)) return GE2E_ERR_UNSUPPORTED;
   rc = fwd_rows_impl(e_hat, c_hat_all, cos_diag, n_local, n_total, spk_offset, M, D, w, b, eps, variant, precision,
                      row_stat, row_kstar, row_aux, accum, nullptr, nullptr, nullptr, nullptr, workspace, workspace_bytes,
-                     true, stream);
+                     stream);
   if (rc != GE2E_OK) return rc;
   return ge2e_b200_bwd_rows(e_hat, c_hat_all, cos_diag, row_stat, row_kstar, row_aux, nullptr, n_local, n_total,
                             spk_offset, M, D, w, b, eps, variant, precision, grad_out, dE_hat, dC_hat_partial, accum + 1,
@@ -530,15 +511,10 @@ int ge2e_b200_step_rows_peers(const float* e_hat, const float* c_hat_all, const 
   // only the tensor-core softmax step flushes through peer memory; everything else keeps the reduce-scatter
   if (!tc_softmax_step(n_local, n_total, M, D, variant, precision)) return GE2E_ERR_UNSUPPORTED;
   RowsArgs a{e_hat, c_hat_all, cos_diag, n_local, n_total, spk_offset, M, D, w, b, eps, variant};
-  if (is_planes(precision)) {
-    rc = tc_fwd_rows(a, row_stat, row_kstar, row_aux, accum, nullptr, workspace, workspace_bytes, true,
-                     (cudaStream_t)stream, tc_prec(precision));
-    if (rc != GE2E_OK) return rc;
-    return tc_step(a, 3, grad_out, nullptr, row_stat, row_aux, nullptr, nullptr, row_scale, nullptr, nullptr, dE_hat, nullptr,
-                   accum + 1, workspace, workspace_bytes, (cudaStream_t)stream, dC_owner_host, n_ranks, tc_prec(precision));
-  }
-  return tc_step(a, 3, grad_out, nullptr, nullptr, nullptr, row_stat, row_aux, row_scale, accum, nullptr, dE_hat, nullptr,
-                 accum + 1, workspace, workspace_bytes, (cudaStream_t)stream, dC_owner_host, n_ranks);
+  TcRowsBufs t;
+  t.grad_out = grad_out; t.row_stat = row_stat; t.row_kstar = row_kstar; t.row_aux = row_aux; t.row_scale = row_scale;
+  t.loss_accum = accum; t.dE_hat = dE_hat; t.dwdb = accum + 1; t.dC_owner = dC_owner_host; t.n_ranks = n_ranks;
+  return tc_rows(a, tc_prec(precision), 3, t, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 // ---- whole step in one call ---------------------------------------------------------------

@@ -205,19 +205,32 @@ int tc_debug_step_schedule(int u_local, int n_total, int cg, int max_clusters, i
                            int* partial, int* units);
 int tc_debug_step_model(int u_local, int n_total, int cg, int max_clusters, int* dc_rot, double* finish, double* model);
 size_t tc_workspace_bytes(int n_local, int n_total, int M, int D, int variant);
-int tc_fwd_rows(const RowsArgs& a, float* row_stat, int32_t* row_kstar, float* row_aux,
-                float* loss_accum, float* per_row_out, void* ws, size_t ws_bytes, bool after_prep,
-                cudaStream_t st, int prec = 0 /* 0 TF32, 1 split fp16 planes, 2 one fp16 plane */);
-// softmax step on tensor cores; phases: 1 = rows pass (loss, row statistics, un-normalised dE_hat + row_scale),
-// 2 = centroid pass (dC_hat_partial, {dw, db}), 3 = both in one launch
-// grad_rows (nullable, phases == 2 only): the upstream gradient per local utterance row in place of grad_out
-// dC_owner (nullable, HOST array of n_ranks device pointers): speaker-sharded over peer memory -- pass 2 adds its
-// accumulators straight into the owner rank's dC_local[n_total / n_ranks, D] (see ge2e_b200_step_rows_peers)
-int tc_step(const RowsArgs& a, int phases, const float* grad_out, const float* grad_rows, const float* row_stat_in,
-            const float* row_aux_in,
-            float* row_stat, float* row_aux, float* row_scale, float* loss_accum, float* per_row_out, float* dE_hat,
-            float* dC_hat_partial, float* dwdb_accum, void* ws, size_t ws_bytes, cudaStream_t st,
-            float* const* dC_owner = nullptr, int n_ranks = 0, int prec = 0);
+// Buffers of one tc_rows call; a field the call does not use stays null.
+struct TcRowsBufs {
+  const float* grad_out = nullptr;    // scalar upstream gradient (phases with the centroid pass)
+  const float* grad_rows = nullptr;   // per local utterance row, in place of grad_out (the centroid pass alone)
+  // row statistics: written where the rows are closed in this call, read where an earlier call closed them
+  float* row_stat = nullptr;
+  int32_t* row_kstar = nullptr;       // contrast
+  float* row_aux = nullptr;
+  float* row_scale = nullptr;         // factor of the un-normalised dE_hat rows (rows pass)
+  float* loss_accum = nullptr;
+  float* per_row = nullptr;           // nullable: [U_local] row losses
+  float* dE_hat = nullptr;
+  float* dC_hat_partial = nullptr;
+  float* dwdb = nullptr;
+  // speaker-sharded over peer memory (HOST array of n_ranks device pointers): pass 2 adds its accumulators straight
+  // into the owner rank's dC_local[n_total / n_ranks, D] (see ge2e_b200_step_rows_peers)
+  float* const* dC_owner = nullptr;
+  int n_ranks = 0;
+};
+// The rows kernels on tensor cores.  prec: 0 TF32, 1 split fp16 planes, 2 one fp16 plane.
+// phases = 0: the forward kernel alone (loss and row statistics, either variant).  Otherwise the softmax step:
+// 1 = rows pass (loss, row statistics, un-normalised dE_hat + row_scale), 2 = centroid pass (dC_hat_partial,
+// {dw, db}) from the row statistics of an earlier rows pass, 3 = both in one launch.  On fp16 planes the forward
+// kernel closes the rows before a step that has the rows pass; on TF32 the step closes them itself.
+int tc_rows(const RowsArgs& a, int prec, int phases, const TcRowsBufs& b, void* ws, size_t ws_bytes,
+            cudaStream_t st);
 int simt_peer_publish(const float* src, float* const* dst, int n_dst, bool multicast, long long n_floats, float* zero,
                       long long zero_floats, cudaStream_t st);
 

@@ -1504,7 +1504,7 @@ int sm_count() {
 int pick_cg(int D) { return ((D / kSlabCols) % 2 != 0) ? 1 : 2; }
 
 // How many clusters of size CG can be co-resident (1 CTA per SM: the kernel needs ~225 KB smem).
-// The step kernel's grid barrier relies on this number: every CTA of its grid must be resident.
+// The step kernel's readiness polls rely on this number: every CTA of its grid must be resident.
 template <int MODE, int VARIANT, int CG>
 int max_clusters() {
   constexpr bool DBG = false;
@@ -1625,8 +1625,7 @@ struct StepModel {
   std::vector<double> ready;      // [STc] time utterance tile t is complete
 };
 
-void model_pass1(const int* de, int NC, int OGe, int STe, int cg, int STc, StepModel* m) {
-  (void)OGe;
+void model_pass1(const int* de, int NC, int STe, int cg, int STc, StepModel* m) {
   m->NC = NC;
   m->ready.assign(STc, 0.0);
   for (int c = 0; c < NC; ++c) {
@@ -1753,7 +1752,7 @@ int make_step_sched(int OGe, int STe, int OGc, int STc, int phases, int max_cl, 
   // percent of a pass at most, and the barrier version's cut is walked without the barrier.
   if (both && rows_closed) {
     StepModel m;
-    model_pass1(S->de, NC, OGe, STe, cg, STc, &m);
+    model_pass1(S->de, NC, STe, cg, STc, &m);
     if (barrier_makespan != nullptr) {
       // the barrier version: pass 2 of cluster c started at max(busiest pass 1, its own + kPassSwitch)
       StepModel mb = m;
@@ -1945,13 +1944,13 @@ size_t tc_workspace_bytes(int n_local, int n_total, int M, int D, int variant) {
   return n;
 }
 
-int tc_fwd_rows(const RowsArgs& a, float* row_stat, int32_t* row_kstar, float* row_aux, float* loss_accum,
-                float* per_row_out, void* ws, size_t ws_bytes, bool after_prep, cudaStream_t st, int prec) {
+namespace {
+
+// The forward kernel: loss and row statistics of either variant.
+int tc_fwd_rows(const RowsArgs& a, const TcRowsBufs& b, void* ws, cudaStream_t st, int prec) {
   const int U = a.n_local * a.M;
   const bool split = prec != PREC_TF32;         // fp16 operand planes
-  if (split && !tc_split_supported(a.n_local, a.n_total, a.M, a.D, a.variant)) return GE2E_ERR_UNSUPPORTED;
   const Layout L = fwd_layout(U, a.n_total, a.D, a.variant);
-  if (ws == nullptr || ws_bytes < kWsHeaderBytes + L.done_bytes + L.part_bytes) return GE2E_ERR_WORKSPACE;
   TmSet tms{};
   int rc;
   if (split) {
@@ -1965,15 +1964,14 @@ int tc_fwd_rows(const RowsArgs& a, float* row_stat, int32_t* row_kstar, float* r
   fill_common(p, a);
   if (split) p.oslabs = (prec == PREC_SPLIT ? 2 : 1) * (a.D / 64);
   p.n_own[0] = U; p.n_str[0] = a.n_total; p.OT[0] = L.OT; p.ST[0] = L.ST; p.GP = L.GP;
-  p.row_stat_out = row_stat; p.kstar_out = row_kstar; p.row_aux_out = row_aux; p.loss_accum = loss_accum;
-  p.per_row_out = per_row_out;
+  p.row_stat_out = b.row_stat; p.kstar_out = b.row_kstar; p.row_aux_out = b.row_aux; p.loss_accum = b.loss_accum;
+  p.per_row_out = b.per_row;
   // the workspace is zero on entry (caller's contract) and the kernel leaves it zeroed
   p.seg_done = reinterpret_cast<int*>(static_cast<uint8_t*>(ws) + kWsHeaderBytes);
   p.seg_part = reinterpret_cast<float2*>(static_cast<uint8_t*>(ws) + kWsHeaderBytes + L.done_bytes);
   p.maxseg = L.maxseg;
   // programmatic dependent launch: barrier init / TMEM allocation / tensormap prefetch run under the
   // tail of whatever kernel precedes this one in the stream; the kernel waits before touching memory
-  (void)after_prep;
   static const StepSched no_sched{};
   if (split) return launch_tc_split<TC_FWD>(prec, tms, no_sched, p, L.NC, true, st);
   if (a.variant == GE2E_SOFTMAX)
@@ -1981,41 +1979,34 @@ int tc_fwd_rows(const RowsArgs& a, float* row_stat, int32_t* row_kstar, float* r
   return launch_tc_cg<TC_FWD, GE2E_CONTRAST>(L.CG, tms, no_sched, p, L.NC, true, st);
 }
 
-// The softmax step on tensor cores.  phases = PASS_ROWS: forward rows + un-normalised dE_hat (+ row_scale);
-// PASS_CENTROIDS: dC_hat_partial, {dw, db} from the row statistics of an earlier PASS_ROWS launch;
-// both: one launch with a grid-wide barrier between the passes.
-int tc_step(const RowsArgs& a, int phases, const float* grad_out, const float* grad_rows, const float* row_stat_in,
-            const float* row_aux_in, float* row_stat, float* row_aux, float* row_scale, float* loss_accum,
-            float* per_row_out, float* dE_hat, float* dC_hat_partial, float* dwdb_accum, void* ws, size_t ws_bytes,
-            cudaStream_t st, float* const* dC_owner, int n_ranks, int prec) {
+// The softmax step kernel.  phases = PASS_ROWS: forward rows + un-normalised dE_hat (+ row_scale);
+// PASS_CENTROIDS: dC_hat_partial, {dw, db} from the row statistics of an earlier rows pass; both: one launch, in
+// which pass 2 waits for the row sums of each utterance tile before it reads them.  TF32 / HYB: pass 1 closes the
+// rows (row statistics, loss); SPLIT / F16: the forward kernel closed them, and both passes read them.
+int tc_step(const RowsArgs& a, int phases, const TcRowsBufs& b, void* ws, cudaStream_t st, int prec) {
   const int U = a.n_local * a.M;
-  const bool peers = dC_owner != nullptr && n_ranks > 1;
+  const bool peers = b.dC_owner != nullptr && b.n_ranks > 1;
   const bool split = prec != PREC_TF32;         // fp16 operand planes
   const bool hyb = !split && tc_hybrid_selected(a.n_local, a.n_total, a.M, a.D, a.variant);
-  // SPLIT: the rows were closed by tc_fwd_rows(split) -- pass 1 and pass 2 both read row_stat_in / row_aux_in
-  if (split && (!tc_split_supported(a.n_local, a.n_total, a.M, a.D, a.variant) || row_stat_in == nullptr ||
-                row_aux_in == nullptr))
-    return GE2E_ERR_UNSUPPORTED;
-  if (peers && (n_ranks > kMaxPeers || a.n_total % n_ranks != 0 || (a.n_total / n_ranks) % kTile != 0 ||
-                !(phases & PASS_CENTROIDS)))
-    return GE2E_ERR_UNSUPPORTED;
-  // a per-row upstream gradient is known only after the forward: the centroid pass alone, on one device
-  if (grad_rows != nullptr && (phases != PASS_CENTROIDS || peers)) return GE2E_ERR_UNSUPPORTED;
-  if (ws == nullptr || ws_bytes < tc_workspace_bytes(a.n_local, a.n_total, a.M, a.D, a.variant)) return GE2E_ERR_WORKSPACE;
-  if ((reinterpret_cast<uintptr_t>(ws) & 15) != 0) return GE2E_ERR_WORKSPACE;
+  const bool closes_rows = !split && (phases & PASS_ROWS);
   const int cg = pick_cg(a.D);
   const int slabs = a.D / kSlabCols;
   const int max_cl = max_clusters_cg<TC_STEP, GE2E_SOFTMAX>(cg);
-  if (max_cl <= 0) return GE2E_ERR_LAUNCH;     // the grid barrier needs a known co-resident cluster count
+  // pass 2 polls for row sums that other CTAs' pass 1 produces: every CTA of the grid must be co-resident
+  if (max_cl <= 0) return GE2E_ERR_LAUNCH;
   // segment kind DE: owner = utterance tiles, stream = centroids; DC: owner = centroid tiles, stream = utterances
   TcParams p{};
   fill_common(p, a);
   if (split) p.oslabs = (prec == PREC_SPLIT ? 2 : 1) * (a.D / 64);
   if (hyb) p.oslabs = a.D / 64;
   p.phases = phases;
-  p.row_stat = row_stat_in; p.row_aux = row_aux_in; p.grad_out = grad_out; p.grad_rows = grad_rows; p.dwdb = dwdb_accum;
-  p.row_stat_out = row_stat; p.row_aux_out = row_aux; p.row_scale_out = row_scale; p.loss_accum = loss_accum;
-  p.per_row_out = per_row_out;
+  p.grad_out = b.grad_out; p.grad_rows = b.grad_rows; p.dwdb = b.dwdb;
+  if (closes_rows) {
+    p.row_stat_out = b.row_stat; p.row_aux_out = b.row_aux; p.loss_accum = b.loss_accum; p.per_row_out = b.per_row;
+  } else {
+    p.row_stat = b.row_stat; p.row_aux = b.row_aux;
+  }
+  p.row_scale_out = b.row_scale;
   p.n_own[SEG_DE] = U; p.n_str[SEG_DE] = a.n_total;
   p.n_own[SEG_DC] = a.n_total; p.n_str[SEG_DC] = U;
   for (int k = 0; k < 2; ++k) {
@@ -2029,11 +2020,11 @@ int tc_step(const RowsArgs& a, int phases, const float* grad_out, const float* g
   // outputs assembled from partial accumulators (TMA reduce-add) are zero-filled by the kernel itself;
   // D % 32 == 0 makes every row a whole number of float4
   if ((phases & PASS_CENTROIDS) && dc_partial && !peers) {
-    p.zero_base = reinterpret_cast<float4*>(dC_hat_partial);
+    p.zero_base = reinterpret_cast<float4*>(b.dC_hat_partial);
     p.zero_n4 = static_cast<long long>(a.n_total) * a.D / 4;
   }
   if ((phases & PASS_ROWS) && de_partial) {
-    p.zero2_base = reinterpret_cast<float4*>(dE_hat);
+    p.zero2_base = reinterpret_cast<float4*>(b.dE_hat);
     p.zero2_n4 = static_cast<long long>(U) * a.D / 4;
   }
   p.ctr = static_cast<int*>(ws);
@@ -2043,20 +2034,13 @@ int tc_step(const RowsArgs& a, int phases, const float* grad_out, const float* g
   // entry and exit of either kernel
   p.seg_done = reinterpret_cast<int*>(static_cast<uint8_t*>(ws) + kWsHeaderBytes);
   // {dw, db} accumulate: zeroed by prep when the passes run in one step; a lone backward clears them here
-  if (phases == PASS_CENTROIDS) GE2E_CUDA_TRY(cudaMemsetAsync(dwdb_accum, 0, 2 * sizeof(float), st));
+  if (phases == PASS_CENTROIDS) GE2E_CUDA_TRY(cudaMemsetAsync(b.dwdb, 0, 2 * sizeof(float), st));
 
-  TmSet tms{};
-  int rc;
-  if (split) {
-    const int chunks_c = a.D / 64 / cg;
-    if ((rc = make_map_h3(&tms.own[SEG_DE], a.e_hat, U, a.D, kTile)) != GE2E_OK) return rc;
-    if ((rc = make_map_h3(&tms.strk[SEG_DE], a.c_hat_all, a.n_total, a.D, kBoxRows)) != GE2E_OK) return rc;
-    const int planes = prec == PREC_SPLIT ? 2 : 1;
-    if ((rc = make_map_h4(&tms.strmn[SEG_DE], a.c_hat_all, a.n_total, a.D, chunks_c, planes)) != GE2E_OK) return rc;
-    if ((rc = make_map_h3(&tms.own[SEG_DC], a.c_hat_all, a.n_total, a.D, kTile)) != GE2E_OK) return rc;
-    if ((rc = make_map_h3(&tms.strk[SEG_DC], a.e_hat, U, a.D, kBoxRows)) != GE2E_OK) return rc;
-    if ((rc = make_map_h4(&tms.strmn[SEG_DC], a.e_hat, U, a.D, chunks_c, planes)) != GE2E_OK) return rc;
-  } else if (hyb) {
+  // the operands: [SEG_DE] utterances, [SEG_DC] centroids; segment k owns op[k] and streams op[1 - k]
+  const float* op[2] = {a.e_hat, a.c_hat_all};
+  const int op_rows[2] = {U, a.n_total};
+  const void* op_k[2] = {op[0], op[1]};         // what MMA1 reads K-major
+  if (hyb) {
     // fp16 copies behind the row sums in the workspace; MMA1 reads them (K-major), MMA2 the fp32 originals (MN-major)
     uint8_t* e16 = reinterpret_cast<uint8_t*>(p.rowsum) + rowsum_bytes(U);
     uint8_t* c16 = e16 + f16_copy_bytes(U, a.D);
@@ -2067,31 +2051,37 @@ int tc_step(const RowsArgs& a, int phases, const float* grad_out, const float* g
                              reinterpret_cast<const float4*>(a.e_hat), reinterpret_cast<uint2*>(e16), na4,
                              reinterpret_cast<const float4*>(a.c_hat_all), reinterpret_cast<uint2*>(c16), nb4));
     GE2E_LAUNCHED();
-    if ((rc = make_map_h2(&tms.own[SEG_DE], e16, U, a.D, kTile)) != GE2E_OK) return rc;
-    if ((rc = make_map_h2(&tms.strk[SEG_DE], c16, a.n_total, a.D, kBoxRows)) != GE2E_OK) return rc;
-    if ((rc = make_map_3d(&tms.strmn[SEG_DE], a.c_hat_all, a.n_total, a.D, slabs / cg)) != GE2E_OK) return rc;
-    if ((rc = make_map_h2(&tms.own[SEG_DC], c16, a.n_total, a.D, kTile)) != GE2E_OK) return rc;
-    if ((rc = make_map_h2(&tms.strk[SEG_DC], e16, U, a.D, kBoxRows)) != GE2E_OK) return rc;
-    if ((rc = make_map_3d(&tms.strmn[SEG_DC], a.e_hat, U, a.D, slabs / cg)) != GE2E_OK) return rc;
-  } else {
-    if ((rc = make_map_2d(&tms.own[SEG_DE], a.e_hat, U, a.D, kTile)) != GE2E_OK) return rc;
-    if ((rc = make_map_2d(&tms.strk[SEG_DE], a.c_hat_all, a.n_total, a.D, kBoxRows)) != GE2E_OK) return rc;
-    if ((rc = make_map_3d(&tms.strmn[SEG_DE], a.c_hat_all, a.n_total, a.D, slabs / cg)) != GE2E_OK) return rc;
-    if ((rc = make_map_2d(&tms.own[SEG_DC], a.c_hat_all, a.n_total, a.D, kTile)) != GE2E_OK) return rc;
-    if ((rc = make_map_2d(&tms.strk[SEG_DC], a.e_hat, U, a.D, kBoxRows)) != GE2E_OK) return rc;
-    if ((rc = make_map_3d(&tms.strmn[SEG_DC], a.e_hat, U, a.D, slabs / cg)) != GE2E_OK) return rc;
+    op_k[0] = e16; op_k[1] = c16;
   }
-  if ((rc = make_map_2d(&tms.out[SEG_DE], dE_hat, U, a.D, kTile)) != GE2E_OK) return rc;
-  if ((rc = make_map_2d(&tms.out[SEG_DC], dC_hat_partial != nullptr ? dC_hat_partial : dE_hat, a.n_total, a.D, kTile)) != GE2E_OK)
+  // only the map makers differ between the operand encodings (split planes / HYB copies / TF32)
+  auto map_k = [&](CUtensorMap* m, const void* base, int rows, int box_rows) {
+    if (split) return make_map_h3(m, base, rows, a.D, box_rows);
+    if (hyb) return make_map_h2(m, base, rows, a.D, box_rows);
+    return make_map_2d(m, static_cast<const float*>(base), rows, a.D, box_rows);
+  };
+  auto map_mn = [&](CUtensorMap* m, const float* base, int rows) {
+    if (split) return make_map_h4(m, base, rows, a.D, a.D / 64 / cg, prec == PREC_SPLIT ? 2 : 1);
+    return make_map_3d(m, base, rows, a.D, slabs / cg);
+  };
+  TmSet tms{};
+  int rc;
+  for (int k = 0; k < 2; ++k) {
+    if ((rc = map_k(&tms.own[k], op_k[k], op_rows[k], kTile)) != GE2E_OK) return rc;
+    if ((rc = map_k(&tms.strk[k], op_k[1 - k], op_rows[1 - k], kBoxRows)) != GE2E_OK) return rc;
+    if ((rc = map_mn(&tms.strmn[k], op[1 - k], op_rows[1 - k])) != GE2E_OK) return rc;
+  }
+  if ((rc = make_map_2d(&tms.out[SEG_DE], b.dE_hat, U, a.D, kTile)) != GE2E_OK) return rc;
+  if ((rc = make_map_2d(&tms.out[SEG_DC], b.dC_hat_partial != nullptr ? b.dC_hat_partial : b.dE_hat, a.n_total, a.D,
+                        kTile)) != GE2E_OK)
     return rc;
   if (peers) {
-    p.peer_rows = a.n_total / n_ranks;
-    for (int r = 0; r < n_ranks; ++r) {
-      if (dC_owner[r] == nullptr || (reinterpret_cast<uintptr_t>(dC_owner[r]) & 15) != 0) return GE2E_ERR_ARGUMENT;
-      if ((rc = make_map_2d(&tms.out_peer[r], dC_owner[r], p.peer_rows, a.D, kTile)) != GE2E_OK) return rc;
+    p.peer_rows = a.n_total / b.n_ranks;
+    for (int r = 0; r < b.n_ranks; ++r) {
+      if (b.dC_owner[r] == nullptr || (reinterpret_cast<uintptr_t>(b.dC_owner[r]) & 15) != 0) return GE2E_ERR_ARGUMENT;
+      if ((rc = make_map_2d(&tms.out_peer[r], b.dC_owner[r], p.peer_rows, a.D, kTile)) != GE2E_OK) return rc;
     }
   }
-  if (grad_rows != nullptr) {     // row-gradient instantiations (no instrumented twins); phases == PASS_CENTROIDS
+  if (b.grad_rows != nullptr) {     // row-gradient instantiations (no instrumented twins); phases == PASS_CENTROIDS
     if (split)
       return prec == PREC_F16 ? launch_tc_impl<TC_STEP, GE2E_SOFTMAX, 2, PREC_F16, false, true>(tms, sched, p, NC, false, st)
                               : launch_tc_impl<TC_STEP, GE2E_SOFTMAX, 2, PREC_SPLIT, false, true>(tms, sched, p, NC, false, st);
@@ -2105,6 +2095,30 @@ int tc_step(const RowsArgs& a, int phases, const float* grad_out, const float* g
     return launch_tc_impl<TC_STEP, GE2E_SOFTMAX, 2, PREC_HYB, false>(tms, sched, p, NC, true, st);
   }
   return launch_tc_cg<TC_STEP, GE2E_SOFTMAX>(cg, tms, sched, p, NC, phases != PASS_CENTROIDS, st);
+}
+
+}  // namespace
+
+int tc_rows(const RowsArgs& a, int prec, int phases, const TcRowsBufs& b, void* ws, size_t ws_bytes,
+            cudaStream_t st) {
+  const bool split = prec != PREC_TF32;         // fp16 operand planes
+  const bool peers = b.dC_owner != nullptr && b.n_ranks > 1;
+  if (split && !tc_split_supported(a.n_local, a.n_total, a.M, a.D, a.variant)) return GE2E_ERR_UNSUPPORTED;
+  if (peers && (b.n_ranks > kMaxPeers || a.n_total % b.n_ranks != 0 || (a.n_total / b.n_ranks) % kTile != 0 ||
+                !(phases & PASS_CENTROIDS)))
+    return GE2E_ERR_UNSUPPORTED;
+  // a per-row upstream gradient is known only after the forward: the centroid pass alone, on one device
+  if (b.grad_rows != nullptr && (phases != PASS_CENTROIDS || peers)) return GE2E_ERR_UNSUPPORTED;
+  if (ws == nullptr || ws_bytes < tc_workspace_bytes(a.n_local, a.n_total, a.M, a.D, a.variant))
+    return GE2E_ERR_WORKSPACE;
+  if (phases != 0 && (reinterpret_cast<uintptr_t>(ws) & 15) != 0) return GE2E_ERR_WORKSPACE;
+  // the forward kernel closes the rows: alone, or on fp16 planes ahead of a step that has the rows pass (whose
+  // pass 1 then forms dE_hat from probabilities that are already normalised)
+  if (phases == 0 || (split && (phases & PASS_ROWS))) {
+    const int rc = tc_fwd_rows(a, b, ws, st, prec);
+    if (rc != GE2E_OK || phases == 0) return rc;
+  }
+  return tc_step(a, phases, b, ws, st, prec);
 }
 
 }  // namespace ge2e

@@ -82,25 +82,30 @@ def _check(rc: int, what: str) -> None:
 _WS_CACHE: dict = {}
 
 
-def _workspace(n_local: int, n_total: int, M: int, D: int, variant: int, precision: int, device):
-    """Scratch for fwd_rows / bwd_rows.  Contract of the C ABI: zero on entry; the kernels leave it
-    zeroed again, so one buffer per (device, stream, size) is zeroed once and reused (the calls on
-    one stream are ordered; another stream gets its own buffer)."""
-    nbytes = lib().ge2e_b200_workspace_bytes(n_local, n_total, M, D, variant, precision)
+def _cached_workspace(nbytes: int, device, dev_index: int, stream: int) -> Optional[Tensor]:
+    """Scratch of the rows kernels.  Contract of the C ABI: zero on entry; the kernels leave it zeroed again, so
+    one buffer per (device, stream, size) is zeroed once and reused (the calls on one stream are ordered; another
+    stream gets its own buffer)."""
     if nbytes == 0:
-        return None, 0
+        return None
     if torch.cuda.is_current_stream_capturing():
         # inside a capture torch.zeros is only recorded: a cached buffer would be handed to later eager
         # calls without ever having been cleared, and it would pin memory of the graph's private pool
-        return torch.zeros(nbytes, dtype=torch.uint8, device=device), nbytes
-    key = (device.index if device.index is not None else torch.cuda.current_device(),
-           torch.cuda.current_stream(device).cuda_stream, nbytes)
+        return torch.zeros(nbytes, dtype=torch.uint8, device=device)
+    key = (dev_index, stream, nbytes)
     ws = _WS_CACHE.get(key)
     if ws is None:
         if len(_WS_CACHE) > 64:
             _WS_CACHE.clear()
         ws = _WS_CACHE[key] = torch.zeros(nbytes, dtype=torch.uint8, device=device)
-    return ws, nbytes
+    return ws
+
+
+def _workspace(n_local: int, n_total: int, M: int, D: int, variant: int, precision: int, device):
+    """(workspace, its size) for fwd_rows / bwd_rows and the custom ops, on the current stream."""
+    nbytes = lib().ge2e_b200_workspace_bytes(n_local, n_total, M, D, variant, precision)
+    index = device.index if device.index is not None else torch.cuda.current_device()
+    return _cached_workspace(nbytes, device, index, torch.cuda.current_stream(device).cuda_stream), nbytes
 
 
 # --------------------------------------------------------------------------- single device
@@ -128,83 +133,50 @@ def _index_ok(row_index: Optional[Tensor], U: int, dev) -> Optional[Tensor]:
     return row_index.to(torch.int32).contiguous()
 
 
-def _tc_softmax(N: int, M: int, D: int, variant: int, precision: int) -> bool:
-    """True where the softmax loss runs on tensor cores: the forward then also leaves the un-normalised
-    dE_hat rows + row_scale (include/ge2e_b200.h, ge2e_b200_fwd_rows) and the backward is one pass."""
-    return variant == _lib.SOFTMAX and lib().ge2e_b200_path(N, N, M, D, variant, precision) in (1, 2, 3)
+def _forward(per: Optional[Tensor], *args) -> None:
+    """ge2e_b200_forward_typed(*args), or with ``per`` the per-utterance losses through
+    ge2e_b200_forward_per_row_typed (whose extra pointer sits in front of workspace, size and stream)."""
+    if per is None:
+        _check(lib().ge2e_b200_forward_typed(*args), "ge2e_b200_forward")
+    else:
+        _check(lib().ge2e_b200_forward_per_row_typed(*args[:-3], per.data_ptr(), *args[-3:]),
+               "ge2e_b200_forward_per_row_typed")
 
 
-def _fwd_impl(E: Tensor, w: Tensor, b: Tensor, eps: float, variant: int, precision: int, packed: bool,
-              row_index: Optional[Tensor] = None, speakers: int = 0, want_grad: bool = True, per_row: bool = False):
-    """GE2ELoss.forward (reference s3:19-30) through the C ABI.  ``packed``: the per-call intermediates
-    come out of ONE allocation (views); the custom op needs non-aliasing outputs and passes False.
-    ``row_index`` (with ``speakers``): E is [U, D] in the embedder's row order and logical row r lives
-    at row_index[r] (the trainer's ``embeddings[unperm]``, s4:189-192, folded into the kernels).
-    ``want_grad``: a backward will follow (tensor-core softmax path: the forward prepares dE_hat).
-    Returns (loss, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale); the last two
-    are 1-element placeholders where the path does not use them.  ``per_row``: the first element is the
-    per-utterance losses [N, M] (logical order) instead of their sum."""
+def _fwd_impl(E: Tensor, w: Tensor, b: Tensor, eps: float, variant: int, precision: int, per_row: bool = False):
+    """GE2ELoss.forward (reference s3:19-30) through the C ABI, with a backward to follow.  Returns (loss, e_hat,
+    c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale); the last two are 1-element placeholders where
+    the forward does not prepare them (_lib.prepares_dE_hat).  ``per_row``: the first element is the per-utterance
+    losses [N, M] (logical order) instead of their sum."""
     _need_cuda(E, w, b)
     (E, ecode), (w, b) = _emb(E), _params(w, b)
     if _lib.planes_need_copy(E.data_ptr(), precision, E.element_size()):
         E = E.clone()
-    if row_index is None:
-        N, M, D = E.shape
-    else:
-        U_, D = E.shape
-        N, M = speakers, U_ // max(1, speakers)
-        if speakers <= 0 or N * M != U_:
-            raise ValueError(f"{U_} rows do not split into {speakers} speakers")
+    N, M, D = E.shape
     U = N * M
     dev = E.device
     with _on_device(dev):
-        fused = want_grad and _tc_softmax(N, M, D, variant, precision)
-        nh, ns = (U * D, U) if fused else (1, 1)
-        if packed:
-            flat = torch.empty(U * D + N * D + 3 * U + 4 + nh + ns, dtype=torch.float32, device=dev)
-            o = 0
-            e_hat = flat[o:o + U * D].view(U, D); o += U * D
-            c_hat = flat[o:o + N * D].view(N, D); o += N * D
-            dE_hat = flat[o:o + nh]; o += nh          # 16-byte aligned: U * D and N * D are multiples of 4 here
-            cos_diag = flat[o:o + U]; o += U
-            row_stat = flat[o:o + U]; o += U
-            row_aux = flat[o:o + U]; o += U
-            row_scale = flat[o:o + ns]; o += ns
-            accum = flat[o:o + 4]
-        else:
-            accum = torch.empty(4, dtype=torch.float32, device=dev)
-            e_hat = torch.empty((U, D), dtype=torch.float32, device=dev)
-            c_hat = torch.empty((N, D), dtype=torch.float32, device=dev)
-            cos_diag = torch.empty(U, dtype=torch.float32, device=dev)
-            row_stat = torch.empty(U, dtype=torch.float32, device=dev)
-            row_aux = torch.empty(U, dtype=torch.float32, device=dev)
-            dE_hat = torch.empty(nh, dtype=torch.float32, device=dev)
-            row_scale = torch.empty(ns, dtype=torch.float32, device=dev)
-        if fused:
-            dE_hat = dE_hat.view(U, D)
+        fused = _lib.prepares_dE_hat(N, N, M, D, variant, precision)
+        accum = torch.empty(4, dtype=torch.float32, device=dev)
+        e_hat = torch.empty((U, D), dtype=torch.float32, device=dev)
+        c_hat = torch.empty((N, D), dtype=torch.float32, device=dev)
+        cos_diag = torch.empty(U, dtype=torch.float32, device=dev)
+        row_stat = torch.empty(U, dtype=torch.float32, device=dev)
+        row_aux = torch.empty(U, dtype=torch.float32, device=dev)
+        dE_hat = torch.empty((U, D) if fused else 1, dtype=torch.float32, device=dev)
+        row_scale = torch.empty(U if fused else 1, dtype=torch.float32, device=dev)
         row_kstar = torch.empty(U if variant == _lib.CONTRAST else 1, dtype=torch.int32, device=dev)
+        per = torch.empty((N, M), dtype=torch.float32, device=dev) if per_row else None
         ws, ws_bytes = _workspace(N, N, M, D, variant, precision, dev)
-        if per_row:
-            per = torch.empty((N, M), dtype=torch.float32, device=dev)
-            rc = lib().ge2e_b200_forward_per_row_typed(
-                E.data_ptr(), ecode, _ptr(row_index), N, M, D, w.data_ptr(), b.data_ptr(), eps, variant, precision,
-                e_hat.data_ptr(), c_hat.data_ptr(), cos_diag.data_ptr(), row_stat.data_ptr(), row_kstar.data_ptr(),
-                row_aux.data_ptr(), accum.data_ptr(), dE_hat.data_ptr() if fused else None,
-                row_scale.data_ptr() if fused else None, per.data_ptr(), _ptr(ws), ws_bytes, _stream())
-            _check(rc, "ge2e_b200_forward_per_row_typed")
-            return per, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale
-        rc = lib().ge2e_b200_forward_typed(E.data_ptr(), ecode, _ptr(row_index), N, M, D, w.data_ptr(), b.data_ptr(),
-                                           eps, variant, precision, e_hat.data_ptr(), c_hat.data_ptr(),
-                                           cos_diag.data_ptr(), row_stat.data_ptr(), row_kstar.data_ptr(),
-                                           row_aux.data_ptr(), accum.data_ptr(),
-                                           dE_hat.data_ptr() if fused else None,
-                                           row_scale.data_ptr() if fused else None, _ptr(ws), ws_bytes, _stream())
-    _check(rc, "ge2e_b200_forward")
-    return accum[0], e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale
+        _forward(per, E.data_ptr(), ecode, None, N, M, D, w.data_ptr(), b.data_ptr(), eps, variant, precision,
+                 e_hat.data_ptr(), c_hat.data_ptr(), cos_diag.data_ptr(), row_stat.data_ptr(), row_kstar.data_ptr(),
+                 row_aux.data_ptr(), accum.data_ptr(), dE_hat.data_ptr() if fused else None,
+                 row_scale.data_ptr() if fused else None, _ptr(ws), ws_bytes, _stream())
+    return accum[0] if per is None else per, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale
 
 
 def _bwd_impl(grad_out, E, w, b, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale, eps,
-              variant, precision, row_index: Optional[Tensor] = None, per_row: bool = False):
+              variant, precision, per_row: bool = False):
     """loss.backward() (s4:200) through the C ABI.  ``dE_hat`` / ``row_scale``: what the forward prepared
     (1-element placeholders where the path does not use them).  ``per_row``: grad_out is the upstream gradient
     of the per-utterance losses, [N, M].  Returns (dE shaped like E, dwdb[2])."""
@@ -218,7 +190,7 @@ def _bwd_impl(grad_out, E, w, b, e_hat, c_hat, cos_diag, row_stat, row_kstar, ro
     dev = E.device
     with _on_device(dev):
         dE = torch.empty_like(E)
-        fused = dE_hat.numel() == U * D and _tc_softmax(N, M, D, variant, precision)
+        fused = dE_hat.numel() == U * D and _lib.prepares_dE_hat(N, N, M, D, variant, precision)
         # [accum (4: -, dw, db, -) | dC_hat (N*D) | dE_hat (U*D) unless the forward prepared it]
         scratch = torch.empty(4 + N * D + (0 if fused else U * D), dtype=torch.float32, device=dev)
         dC_ptr = scratch.data_ptr() + 16
@@ -227,7 +199,7 @@ def _bwd_impl(grad_out, E, w, b, e_hat, c_hat, cos_diag, row_stat, row_kstar, ro
         if per_row and g.numel() != U:
             raise ValueError(f"the upstream gradient of the per-utterance losses needs {U} entries, got {g.numel()}")
         entry = lib().ge2e_b200_backward_per_row_typed if per_row else lib().ge2e_b200_backward_typed
-        rc = entry(E.data_ptr(), ecode, _ptr(row_index), e_hat.data_ptr(), c_hat.data_ptr(), cos_diag.data_ptr(),
+        rc = entry(E.data_ptr(), ecode, None, e_hat.data_ptr(), c_hat.data_ptr(), cos_diag.data_ptr(),
                    row_stat.data_ptr(), row_kstar.data_ptr(), row_aux.data_ptr(), row_scale.data_ptr() if fused else None,
                    N, M, D, w.data_ptr(), b.data_ptr(), eps, variant, precision, g.data_ptr(), dE_hat_ptr, dC_ptr,
                    scratch.data_ptr(), dE.data_ptr(), ecode, _ptr(ws), ws_bytes, _stream())
@@ -241,20 +213,30 @@ def ge2e_fwd(E: Tensor, w: Tensor, b: Tensor, eps: float, variant: int,
     """GE2ELoss.forward as a torch.library op (what torch.compile / export see).  Returns (loss, e_hat,
     c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale); everything after loss is saved for
     the backward."""
-    out = _fwd_impl(E, w, b, eps, variant, precision, packed=False)
+    out = _fwd_impl(E, w, b, eps, variant, precision)
     return (out[0].clone(),) + out[1:]       # accum[0] is a view of accum: op outputs must not alias
+
+
+def _fake_fwd(E, variant, precision, loss_shape):
+    """Outputs of _fwd_impl, for the fakes of ge2e_b200::fwd and ge2e_b200::fwd_per_row."""
+    N, M, D = E.shape
+    U = N * M
+    fused = _lib.prepares_dE_hat(N, N, M, D, variant, precision)
+    f32 = torch.float32      # every intermediate is float32 whatever E's element type
+    return (E.new_empty(loss_shape, dtype=f32), E.new_empty((U, D), dtype=f32), E.new_empty((N, D), dtype=f32),
+            E.new_empty(U, dtype=f32), E.new_empty(U, dtype=f32),
+            E.new_empty(U if variant == _lib.CONTRAST else 1, dtype=torch.int32), E.new_empty(U, dtype=f32),
+            E.new_empty((U, D) if fused else (1,), dtype=f32), E.new_empty(U if fused else 1, dtype=f32))
+
+
+def _fake_bwd(grad, E, w, b, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale, eps, variant,
+              precision):
+    return torch.empty_like(E), E.new_empty(2, dtype=torch.float32)
 
 
 @ge2e_fwd.register_fake
 def _(E, w, b, eps, variant, precision):
-    N, M, D = E.shape
-    U = N * M
-    fused = _tc_softmax(N, M, D, variant, precision)
-    f32 = torch.float32      # every intermediate is float32 whatever E's element type
-    return (E.new_empty((), dtype=f32), E.new_empty((U, D), dtype=f32), E.new_empty((N, D), dtype=f32),
-            E.new_empty(U, dtype=f32), E.new_empty(U, dtype=f32),
-            E.new_empty(U if variant == _lib.CONTRAST else 1, dtype=torch.int32), E.new_empty(U, dtype=f32),
-            E.new_empty((U, D) if fused else (1,), dtype=f32), E.new_empty(U if fused else 1, dtype=f32))
+    return _fake_fwd(E, variant, precision, ())
 
 
 @torch.library.custom_op("ge2e_b200::bwd", mutates_args=())
@@ -267,10 +249,7 @@ def ge2e_bwd(grad_out: Tensor, E: Tensor, w: Tensor, b: Tensor, e_hat: Tensor, c
     return dE, dwdb.clone()
 
 
-@ge2e_bwd.register_fake
-def _(grad_out, E, w, b, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale, eps, variant,
-      precision):
-    return torch.empty_like(E), E.new_empty(2, dtype=torch.float32)
+ge2e_bwd.register_fake(_fake_bwd)
 
 
 def _fwd_setup(ctx, inputs, output):
@@ -295,19 +274,12 @@ ge2e_fwd.register_autograd(_fwd_backward, setup_context=_fwd_setup)
 def ge2e_fwd_per_row(E: Tensor, w: Tensor, b: Tensor, eps: float, variant: int,
                      precision: int) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
     """ge2e_b200::fwd with the per-utterance losses [N, M] (reduction="none") in place of their sum."""
-    return _fwd_impl(E, w, b, eps, variant, precision, packed=False, per_row=True)
+    return _fwd_impl(E, w, b, eps, variant, precision, per_row=True)
 
 
 @ge2e_fwd_per_row.register_fake
 def _(E, w, b, eps, variant, precision):
-    N, M, D = E.shape
-    U = N * M
-    fused = _tc_softmax(N, M, D, variant, precision)
-    f32 = torch.float32
-    return (E.new_empty((N, M), dtype=f32), E.new_empty((U, D), dtype=f32), E.new_empty((N, D), dtype=f32),
-            E.new_empty(U, dtype=f32), E.new_empty(U, dtype=f32),
-            E.new_empty(U if variant == _lib.CONTRAST else 1, dtype=torch.int32), E.new_empty(U, dtype=f32),
-            E.new_empty((U, D) if fused else (1,), dtype=f32), E.new_empty(U if fused else 1, dtype=f32))
+    return _fake_fwd(E, variant, precision, (E.shape[0], E.shape[1]))
 
 
 @torch.library.custom_op("ge2e_b200::bwd_per_row", mutates_args=())
@@ -320,10 +292,7 @@ def ge2e_bwd_per_row(grad_rows: Tensor, E: Tensor, w: Tensor, b: Tensor, e_hat: 
     return dE, dwdb.clone()
 
 
-@ge2e_bwd_per_row.register_fake
-def _(grad_rows, E, w, b, e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale, eps, variant,
-      precision):
-    return torch.empty_like(E), E.new_empty(2, dtype=torch.float32)
+ge2e_bwd_per_row.register_fake(_fake_bwd)
 
 
 def _fwd_per_row_backward(ctx, g_rows, *_unused):
@@ -384,8 +353,8 @@ class _StepBufs:
 
 
 class _EagerPlan:
-    __slots__ = ("N", "M", "D", "U", "variant", "precision", "dtype", "device", "dev_index", "path", "fused", "ws_bytes",
-                 "free", "one", "free_on", "planes", "bwd_ok")
+    __slots__ = ("N", "M", "D", "U", "variant", "precision", "dtype", "device", "dev_index", "fused", "ws_bytes",
+                 "free", "one", "free_on", "bwd_ok")
 
     def __init__(self, dev, N, M, D, variant, precision, dtype):
         self.N, self.M, self.D, self.U = N, M, D, N * M
@@ -393,9 +362,7 @@ class _EagerPlan:
         self.dtype = dtype                      # ge2e_dtype code of E and of the dE handed back
         self.dev_index = dev.index if dev.index is not None else torch.cuda.current_device()
         h = lib()
-        self.path = h.ge2e_b200_path(N, N, M, D, variant, precision)
-        self.fused = variant == _lib.SOFTMAX and self.path in (1, 2, 3)
-        self.planes = precision in (_lib.FP32_SPLIT, _lib.F16)
+        self.fused = _lib.prepares_dE_hat(N, N, M, D, variant, precision)
         self.bwd_ok = M <= h.ge2e_b200_max_utterances(D)
         # the whole-step entry point (single-kernel step for reference-sized batches) may need more than the stages
         self.ws_bytes = max(h.ge2e_b200_workspace_bytes(N, N, M, D, variant, precision),
@@ -430,17 +397,7 @@ class _EagerPlan:
                 q.append(bufs)
 
     def workspace(self, stream: int):
-        if self.ws_bytes == 0:
-            return None
-        if torch.cuda.is_current_stream_capturing():
-            return torch.zeros(self.ws_bytes, dtype=torch.uint8, device=self.device)
-        key = (self.dev_index, stream, self.ws_bytes)
-        ws = _WS_CACHE.get(key)
-        if ws is None:
-            if len(_WS_CACHE) > 64:
-                _WS_CACHE.clear()
-            ws = _WS_CACHE[key] = torch.zeros(self.ws_bytes, dtype=torch.uint8, device=self.device)
-        return ws
+        return _cached_workspace(self.ws_bytes, self.device, self.dev_index, stream)
 
 
 _EAGER_PLANS: dict = {}
@@ -471,150 +428,104 @@ class _Lease:
             b.plan.give(b)
 
 
+def _eager_setup(E, w, b, variant, precision, row_index, speakers, want_grad):
+    """The checks of an eager call and its plan.  E is [N, M, D], or [N*M, D] in the embedder's row order with
+    ``row_index`` and ``speakers`` = N.  Returns (E contiguous, its ge2e_dtype code, plan)."""
+    if not (E.is_cuda and w.is_cuda and b.is_cuda):
+        raise RuntimeError("speaker_embedding_ge2e_loss_b200 runs on CUDA (sm_100a) tensors only; "
+                           "there is no CPU fallback")
+    (E, ecode), _ = _emb(E), _params(w, b)
+    if row_index is None:
+        N, M, D = E.shape
+    else:
+        U_, D = E.shape
+        N, M = speakers, U_ // max(1, speakers)
+        if speakers <= 0 or N * M != U_:
+            raise ValueError(f"{U_} rows do not split into {speakers} speakers")
+    plan = _eager_plan(E.device, N, M, D, variant, precision, ecode)
+    if _lib.planes_need_copy(E.data_ptr(), precision, E.element_size()):
+        E = E.clone()
+    if want_grad and not plan.bwd_ok:
+        _lib.check_backward_shape(M, D)
+    return E, ecode, plan
+
+
 class _GE2EEager(torch.autograd.Function):
-    """ge2e_b200_forward_typed / ge2e_b200_backward_typed without the torch.library dispatch layers
-    (which cost ~0.2 ms of host time per step: more than the kernels at every size up to cfg3)."""
+    """The summed loss of inputs that require grad, through ge2e_b200_forward_backward_typed without the
+    torch.library dispatch layers (which cost ~0.2 ms of host time per step: more than the kernels at every size up
+    to cfg3).  A loss somebody will differentiate (s4:196 + s4:200): the WHOLE step runs in forward, with upstream
+    gradient 1 -- one C call: one kernel for reference-sized batches, prep + ONE persistent step kernel + finalize on
+    the tensor-core paths (instead of a forward and a backward that each cross the grid) -- and backward only scales
+    by the real upstream gradient.  A forward that is never differentiated (s4:103) pays for gradients it does not
+    use, under torch.no_grad() too: the choice follows requires_grad of E, w and b, not the grad mode."""
 
     @staticmethod
     def forward(ctx, E, w, b, eps, variant, precision, row_index, speakers):
-        if not (E.is_cuda and w.is_cuda and b.is_cuda):
-            raise RuntimeError("speaker_embedding_ge2e_loss_b200 runs on CUDA (sm_100a) tensors only; "
-                               "there is no CPU fallback")
-        (E, ecode), _ = _emb(E), _params(w, b)
-        if row_index is None:
-            N, M, D = E.shape
-        else:
-            U_, D = E.shape
-            N, M = speakers, U_ // max(1, speakers)
-            if speakers <= 0 or N * M != U_:
-                raise ValueError(f"{U_} rows do not split into {speakers} speakers")
+        E, ecode, plan = _eager_setup(E, w, b, variant, precision, row_index, speakers, True)
         dev = E.device
-        plan = _eager_plan(dev, N, M, D, variant, precision, ecode)
-        if plan.planes and E.data_ptr() % (4 * E.element_size()):
-            E = E.clone()           # the fp16-plane kernels read E four elements at a time
-        want_grad = ctx.needs_input_grad[0] or ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
-        if want_grad and not plan.bwd_ok:
-            _lib.check_backward_shape(M, D)
-        if want_grad:
-            # A loss somebody will differentiate (s4:196 + s4:200): the WHOLE step now, with upstream gradient 1 --
-            # one C call: one kernel for reference-sized batches, prep + ONE persistent step kernel + finalize on
-            # the tensor-core paths (instead of a forward and a backward that each cross the grid) -- and backward
-            # only scales by the real upstream gradient.  A forward under grad mode that is never differentiated
-            # (s4:103) pays for gradients it does not use; wrap it in torch.no_grad() to get the forward kernels.
-            with _on_device(dev):
-                stream = _raw_stream(plan.dev_index)
-                bufs = plan.take_on(stream)
-                accum = torch.empty(4, dtype=torch.float32, device=dev)     # escapes as the loss tensor: never pooled
-                # the gradient for upstream gradient 1 stays float32: backward rounds g * dE to E's type once, so a
-                # loss scale reaches small fp16 gradients before the rounding does
-                dE = torch.empty_like(E, dtype=torch.float32)
-                ws = plan.workspace(stream)
-                rc = lib().ge2e_b200_forward_backward_typed(
-                    E.data_ptr(), ecode, _ptr(row_index), N, M, D, w.data_ptr(), b.data_ptr(), eps, variant, precision,
-                    plan.one.data_ptr(), *bufs.step_ptrs, accum.data_ptr(), bufs.dE_hat.data_ptr(), bufs.dC_hat.data_ptr(),
-                    dE.data_ptr(), _lib.DT_F32, _ptr(ws), plan.ws_bytes, stream)
-            _check(rc, "ge2e_b200_forward_backward")
-            plan.give_on(bufs, stream)  # the next step on this stream may overwrite them: stream order
-            ctx.lease = None
-            ctx.cfg = (plan, dE, accum)
-            return accum[0]
         with _on_device(dev):
-            bufs = plan.take()
-            accum = torch.empty(4, dtype=torch.float32, device=dev)     # escapes as the loss tensor: never pooled
             stream = _raw_stream(plan.dev_index)
+            bufs = plan.take_on(stream)
+            accum = torch.empty(4, dtype=torch.float32, device=dev)     # escapes as the loss tensor: never pooled
+            # the gradient for upstream gradient 1 stays float32: backward rounds g * dE to E's type once, so a
+            # loss scale reaches small fp16 gradients before the rounding does
+            dE = torch.empty_like(E, dtype=torch.float32)
             ws = plan.workspace(stream)
-            fused = False
-            rc = lib().ge2e_b200_forward_typed(
-                E.data_ptr(), ecode, _ptr(row_index), N, M, D, w.data_ptr(), b.data_ptr(), eps, variant, precision,
-                *bufs.fwd_ptrs, accum.data_ptr(), bufs.dE_hat.data_ptr() if fused else None,
-                bufs.row_scale.data_ptr() if fused else None, _ptr(ws), plan.ws_bytes, stream)
-        _check(rc, "ge2e_b200_forward")
-        ctx.save_for_backward(E, w, b)
-        ctx.lease = _Lease(bufs)
-        ctx.cfg = (eps, variant, precision, plan, fused, row_index, N, M, D)
+            rc = lib().ge2e_b200_forward_backward_typed(
+                E.data_ptr(), ecode, _ptr(row_index), plan.N, plan.M, plan.D, w.data_ptr(), b.data_ptr(), eps, variant,
+                precision, plan.one.data_ptr(), *bufs.step_ptrs, accum.data_ptr(), bufs.dE_hat.data_ptr(),
+                bufs.dC_hat.data_ptr(), dE.data_ptr(), _lib.DT_F32, _ptr(ws), plan.ws_bytes, stream)
+        _check(rc, "ge2e_b200_forward_backward")
+        plan.give_on(bufs, stream)  # the next step on this stream may overwrite them: stream order
+        ctx.cfg = (plan, dE, accum)
         return accum[0]
 
     @staticmethod
     def backward(ctx, g_loss):
-        if len(ctx.cfg) == 3:           # the step ran in forward with upstream gradient 1: scale by the real one
-            plan, dE1, acc1 = ctx.cfg
-            dev = dE1.device
-            g = g_loss if (g_loss.dtype == torch.float32 and g_loss.is_cuda) else g_loss.to(dev, torch.float32)
-            with _on_device(dev):
-                dE = torch.empty_like(dE1, dtype=_TORCH_DTYPES[plan.dtype])
-                dwdb = torch.empty(2, dtype=torch.float32, device=dev)      # escapes as dw / db
-                rc = lib().ge2e_b200_scale_grads_typed(dE1.data_ptr(), dE.data_ptr(), plan.dtype, dE1.numel(),
-                                                       acc1.data_ptr() + 4, dwdb.data_ptr(), g.data_ptr(),
-                                                       _raw_stream(plan.dev_index))
-            _check(rc, "ge2e_b200_scale_grads_typed")
-            return dE, dwdb[0], dwdb[1], None, None, None, None, None
-        E, w, b = ctx.saved_tensors
-        eps, variant, precision, plan, fused, row_index, N, M, D = ctx.cfg
-        bufs = ctx.lease.bufs
-        g = g_loss if (g_loss.dtype == torch.float32 and g_loss.is_cuda) else g_loss.to(E.device, torch.float32)
-        dev = E.device
+        plan, dE1, acc1 = ctx.cfg
+        dev = dE1.device
+        g = g_loss if (g_loss.dtype == torch.float32 and g_loss.is_cuda) else g_loss.to(dev, torch.float32)
         with _on_device(dev):
-            dE = torch.empty_like(E)
-            accum = torch.empty(4, dtype=torch.float32, device=dev)     # escapes as dw / db: never pooled
-            stream = _raw_stream(plan.dev_index)
-            ws = plan.workspace(stream)
-            rc = lib().ge2e_b200_backward_typed(
-                E.data_ptr(), plan.dtype, _ptr(row_index), bufs.e_hat.data_ptr(), bufs.c_hat.data_ptr(),
-                bufs.cos_diag.data_ptr(), bufs.row_stat.data_ptr(), bufs.kstar.data_ptr(), bufs.row_aux.data_ptr(),
-                bufs.row_scale.data_ptr() if fused else None, N, M, D, w.data_ptr(), b.data_ptr(), eps, variant,
-                precision, g.data_ptr(), bufs.dE_hat.data_ptr(), bufs.dC_hat.data_ptr(), accum.data_ptr(), dE.data_ptr(),
-                plan.dtype, _ptr(ws), plan.ws_bytes, stream)
-        _check(rc, "ge2e_b200_backward_typed")
-        return dE, accum[1], accum[2], None, None, None, None, None
+            dE = torch.empty_like(dE1, dtype=_TORCH_DTYPES[plan.dtype])
+            dwdb = torch.empty(2, dtype=torch.float32, device=dev)      # escapes as dw / db
+            rc = lib().ge2e_b200_scale_grads_typed(dE1.data_ptr(), dE.data_ptr(), plan.dtype, dE1.numel(),
+                                                   acc1.data_ptr() + 4, dwdb.data_ptr(), g.data_ptr(),
+                                                   _raw_stream(plan.dev_index))
+        _check(rc, "ge2e_b200_scale_grads_typed")
+        return dE, dwdb[0], dwdb[1], None, None, None, None, None
 
 
-class _GE2EPerRow(torch.autograd.Function):
-    """reduction="none": the per-utterance losses L[N, M] (logical order) through ge2e_b200_forward_per_row_typed, and
-    dE = sum_r g_r dL_r/dE through ge2e_b200_backward_per_row_typed.  The upstream gradient is unknown when the forward
-    runs, so this is always the staged pipeline: forward kernels now (the tensor-core softmax paths also prepare
-    dE_hat / row_scale when a gradient is needed), backward kernels in backward."""
+class _GE2EStaged(torch.autograd.Function):
+    """The staged pipeline: forward kernels now (ge2e_b200_forward_typed, or ge2e_b200_forward_per_row_typed for the
+    per-utterance losses L[N, M] in logical order), backward kernels in backward.  It serves reduction="none", whose
+    upstream gradient is unknown when the forward runs, and the summed loss when no input requires grad.  Where a
+    gradient will follow, the tensor-core softmax paths also prepare dE_hat / row_scale in the forward."""
 
     @staticmethod
-    def forward(ctx, E, w, b, eps, variant, precision, row_index, speakers):
-        if not (E.is_cuda and w.is_cuda and b.is_cuda):
-            raise RuntimeError("speaker_embedding_ge2e_loss_b200 runs on CUDA (sm_100a) tensors only; "
-                               "there is no CPU fallback")
-        (E, ecode), _ = _emb(E), _params(w, b)
-        if row_index is None:
-            N, M, D = E.shape
-        else:
-            U_, D = E.shape
-            N, M = speakers, U_ // max(1, speakers)
-            if speakers <= 0 or N * M != U_:
-                raise ValueError(f"{U_} rows do not split into {speakers} speakers")
-        dev = E.device
-        plan = _eager_plan(dev, N, M, D, variant, precision, ecode)
-        if plan.planes and E.data_ptr() % (4 * E.element_size()):
-            E = E.clone()           # the fp16-plane kernels read E four elements at a time
+    def forward(ctx, E, w, b, eps, variant, precision, row_index, speakers, per_row):
         want_grad = ctx.needs_input_grad[0] or ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
-        if want_grad and not plan.bwd_ok:
-            _lib.check_backward_shape(M, D)
+        E, ecode, plan = _eager_setup(E, w, b, variant, precision, row_index, speakers, want_grad)
         fused = want_grad and plan.fused
+        dev = E.device
         with _on_device(dev):
             bufs = plan.take()
-            accum = torch.empty(4, dtype=torch.float32, device=dev)
-            per = torch.empty((N, M), dtype=torch.float32, device=dev)     # escapes: never pooled
+            accum = torch.empty(4, dtype=torch.float32, device=dev)     # escapes as the loss tensor: never pooled
+            per = torch.empty((plan.N, plan.M), dtype=torch.float32, device=dev) if per_row else None   # escapes
             stream = _raw_stream(plan.dev_index)
             ws = plan.workspace(stream)
-            rc = lib().ge2e_b200_forward_per_row_typed(
-                E.data_ptr(), ecode, _ptr(row_index), N, M, D, w.data_ptr(), b.data_ptr(), eps, variant, precision,
-                *bufs.fwd_ptrs, accum.data_ptr(), bufs.dE_hat.data_ptr() if fused else None,
-                bufs.row_scale.data_ptr() if fused else None, per.data_ptr(), _ptr(ws), plan.ws_bytes, stream)
-        _check(rc, "ge2e_b200_forward_per_row_typed")
+            _forward(per, E.data_ptr(), ecode, _ptr(row_index), plan.N, plan.M, plan.D, w.data_ptr(), b.data_ptr(), eps,
+                     variant, precision, *bufs.fwd_ptrs, accum.data_ptr(), bufs.dE_hat.data_ptr() if fused else None,
+                     bufs.row_scale.data_ptr() if fused else None, _ptr(ws), plan.ws_bytes, stream)
         ctx.save_for_backward(E, w, b)
         ctx.lease = _Lease(bufs)
-        ctx.cfg = (eps, variant, precision, plan, fused, row_index, N, M, D)
-        return per
+        ctx.cfg = (eps, variant, precision, plan, fused, row_index)
+        return accum[0] if per is None else per
 
     @staticmethod
     def backward(ctx, g_per):
+        # reduction="none" only: a summed loss comes here only when no input requires grad, and then has no grad_fn
         E, w, b = ctx.saved_tensors
-        eps, variant, precision, plan, fused, row_index, N, M, D = ctx.cfg
+        eps, variant, precision, plan, fused, row_index = ctx.cfg
         bufs = ctx.lease.bufs
         dev = E.device
         # one float32 per utterance row, contiguous: `per.sum().backward()` hands over an expanded (stride-0) ones
@@ -627,11 +538,18 @@ class _GE2EPerRow(torch.autograd.Function):
             rc = lib().ge2e_b200_backward_per_row_typed(
                 E.data_ptr(), plan.dtype, _ptr(row_index), bufs.e_hat.data_ptr(), bufs.c_hat.data_ptr(),
                 bufs.cos_diag.data_ptr(), bufs.row_stat.data_ptr(), bufs.kstar.data_ptr(), bufs.row_aux.data_ptr(),
-                bufs.row_scale.data_ptr() if fused else None, N, M, D, w.data_ptr(), b.data_ptr(), eps, variant,
-                precision, g.data_ptr(), bufs.dE_hat.data_ptr(), bufs.dC_hat.data_ptr(), accum.data_ptr(), dE.data_ptr(),
-                plan.dtype, _ptr(ws), plan.ws_bytes, stream)
+                bufs.row_scale.data_ptr() if fused else None, plan.N, plan.M, plan.D, w.data_ptr(), b.data_ptr(), eps,
+                variant, precision, g.data_ptr(), bufs.dE_hat.data_ptr(), bufs.dC_hat.data_ptr(), accum.data_ptr(),
+                dE.data_ptr(), plan.dtype, _ptr(ws), plan.ws_bytes, stream)
         _check(rc, "ge2e_b200_backward_per_row_typed")
-        return dE, accum[1], accum[2], None, None, None, None, None
+        return dE, accum[1], accum[2], None, None, None, None, None, None
+
+
+def _apply(E, w, b, eps, variant, precision, row_index, speakers, per_row):
+    # the test of ctx.needs_input_grad, made before apply: requires_grad, whatever the grad mode
+    if per_row or not (E.requires_grad or w.requires_grad or b.requires_grad):
+        return _GE2EStaged.apply(E, w, b, eps, variant, precision, row_index, speakers, per_row)
+    return _GE2EEager.apply(E, w, b, eps, variant, precision, row_index, speakers)
 
 
 # host-only query (a ctypes call): under torch.compile its answer is a constant of the traced graph
@@ -674,7 +592,7 @@ def _ge2e_loss(E, w, b, eps, variant, precision, unperm, speakers, per_row: bool
             op = ge2e_fwd_per_row if per_row else ge2e_fwd
             return op(E[unperm].reshape(N, E.shape[0] // N, E.shape[1]), w, b, float(eps), vcode, pcode)[0]
         idx = _index_ok(unperm, E.shape[0], E.device)
-        return (_GE2EPerRow if per_row else _GE2EEager).apply(E, w, b, float(eps), vcode, pcode, idx, speakers)
+        return _apply(E, w, b, float(eps), vcode, pcode, idx, speakers, per_row)
     if E.dim() != 3:
         raise ValueError(f"embeddings must be [N, M, D], got {tuple(E.shape)}")
     if E.shape[1] < 2:
@@ -683,7 +601,7 @@ def _ge2e_loss(E, w, b, eps, variant, precision, unperm, speakers, per_row: bool
     pcode = _resolve_precision(precision, E.shape[0], E.shape[0], E.shape[1], E.shape[2], vcode)
     if torch.compiler.is_compiling():
         return (ge2e_fwd_per_row if per_row else ge2e_fwd)(E, w, b, float(eps), vcode, pcode)[0]
-    return (_GE2EPerRow if per_row else _GE2EEager).apply(E, w, b, float(eps), vcode, pcode, None, 0)
+    return _apply(E, w, b, float(eps), vcode, pcode, None, 0, per_row)
 
 
 # --------------------------------------------------------------------------- staged (plain functions)
@@ -715,8 +633,7 @@ def fwd_rows(e_hat, c_hat_all, cos_diag, n_local, n_total, spk_offset, M, D, w, 
     _same_f32c(e_hat, c_hat_all, cos_diag, w, b, accum)
     dev = e_hat.device
     U = n_local * M
-    fused = (want_grad and variant == _lib.SOFTMAX and not sim
-             and lib().ge2e_b200_path(n_local, n_total, M, D, variant, precision) in (1, 2, 3))
+    fused = want_grad and not sim and _lib.prepares_dE_hat(n_local, n_total, M, D, variant, precision)
     dE_hat = torch.empty((U, D), dtype=torch.float32, device=dev) if fused else None
     row_scale = torch.empty(U, dtype=torch.float32, device=dev) if fused else None
     row_stat = torch.empty(U, dtype=torch.float32, device=dev)

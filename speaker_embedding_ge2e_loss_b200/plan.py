@@ -160,7 +160,7 @@ class ShardedGE2EPlan:
         self.row_scale = torch.empty(U, dtype=f32, device=dev)
         self.path = lib().ge2e_b200_path(n_local, n_total, M, D, self.variant, self.precision)
         # finalize applies row_scale only where the forward produced it (softmax on tensor cores)
-        self._scaled = self.path in (1, 2, 3) and self.variant == _lib.SOFTMAX
+        self._scaled = _lib.prepares_dE_hat(n_local, n_total, M, D, self.variant, self.precision)
         self.peer, self.peer_error = False, None
         world = dist.get_world_size(self.group)
         if peer_memory and world > 1:
