@@ -178,6 +178,80 @@ __device__ __forceinline__ void st4e(T* __restrict__ row, int col, int D, bool v
 }
 
 // ------------------------------------------------------------------------------------------
+// Row arithmetic of prep and finalize, shared by every body (generic, warp, register, single-kernel step).
+// Speaker j has rows e_i, column sum s = sum_i e_i, centroid c = s / M (s3:37) and leave-one-out centroids
+// u_i = d_i / (M - 1) with d_i = s - e_i (s3:105-111).  The bodies reduce the raw sums |e|^2, |d|^2, e.d, |s|^2,
+// e.dE_hat and s.dC_hat however their threads map to rows and columns; the helpers below take those sums.
+// ------------------------------------------------------------------------------------------
+struct RowNorms {
+  float ne, nu;           // |e|, |u|
+  float inv_ne, inv_nu;   // 1 / max(|e|, delta), 1 / max(|u|, delta)
+  float cos;              // e_hat . u_hat (s3:57)
+};
+__device__ __forceinline__ RowNorms row_norms(float ne2, float nd2, float ed, float inv_m1) {
+  RowNorms n;
+  n.ne = sqrtf(ne2);
+  n.nu = sqrtf(nd2) * inv_m1;
+  n.inv_ne = 1.f / fmaxf(n.ne, kCosDelta);
+  n.inv_nu = 1.f / fmaxf(n.nu, kCosDelta);
+  n.cos = (ed * inv_m1) * n.inv_ne * n.inv_nu;
+  return n;
+}
+
+// c_hat = s * centroid_scale(|s|^2, 1 / M)
+__device__ __forceinline__ float centroid_scale(float ss, float inv_m) {
+  return inv_m / fmaxf(sqrtf(ss) * inv_m, kCosDelta);
+}
+
+// dd = w G_jj, the diagonal element of w G of a row with upstream gradient g_r.  aux is the row's row_aux for
+// softmax (q = 1 - p_jj: G_jj = g_r (p_jj - 1)) and its cos_diag for contrast (G_jj = -g_r sigma'(S_jj)).
+__device__ __forceinline__ float diag_term(int variant, float g_r, float aux, float w, float b, float eps) {
+  float Gd;
+  if (variant == GE2E_SOFTMAX) {
+    Gd = -g_r * aux;
+  } else {
+    const float sp = 1.f / (1.f + expf(-fmaf(w, aux + eps, b)));
+    Gd = -g_r * sp * (1.f - sp);
+  }
+  return w * Gd;
+}
+
+// Gradient of one row through e_hat and u_hat.  The row's gradients are d e_hat = gsc dE_hat + dd u_hat and
+// d u_hat = dd e_hat (its diagonal cosine); through the two normalisations (clamp_proj_scale)
+//   de = (d e_hat - e_hat (e_hat . d e_hat) s_e) inv_ne,   du = (d u_hat - u_hat (u_hat . d u_hat) s_u) inv_nu.
+// With e_hat = e inv_ne and u_hat = d inv_nu / (M - 1) both are linear in dE_hat, e and d:
+//   de = a_g dE_hat + a_e e + a_d d,   du = b_e e + b_d d.
+// gsc: factor of un-normalised dE_hat rows (else 1); eg = (e . dE_hat) gsc.
+struct RowJacobian {
+  float a_g, a_e, a_d, b_e, b_d;
+  __device__ __forceinline__ float de(float e, float d, float g) const { return a_g * g + a_e * e + a_d * d; }
+  __device__ __forceinline__ float du(float e, float d) const { return b_e * e + b_d * d; }
+};
+__device__ __forceinline__ RowJacobian row_jacobian(const RowNorms& n, float eg, float gsc, float dd, float inv_m1) {
+  float proj_e = eg * n.inv_ne + dd * n.cos;   // e_hat . d e_hat
+  float proj_u = dd * n.cos;                   // u_hat . d u_hat
+  if (n.ne < kCosDelta) proj_e *= clamp_proj_scale(n.ne);
+  if (n.nu < kCosDelta) proj_u *= clamp_proj_scale(n.nu);
+  RowJacobian J;
+  J.a_g = n.inv_ne * gsc;
+  J.a_e = -proj_e * n.inv_ne * n.inv_ne;
+  J.a_d = dd * n.inv_nu * inv_m1 * n.inv_ne;
+  J.b_e = dd * n.inv_ne * n.inv_nu;
+  J.b_d = -proj_u * n.inv_nu * n.inv_nu * inv_m1;
+  return J;
+}
+
+// Gradient of the centroid through c_hat = s inv / M (clamp_proj_scale), divided by M for the fan-out to the rows:
+//   dc / M = (dC_hat - c_hat (c_hat . dC_hat) s_c) inv / M = k.x dC_hat - k.y s,   sdc = s . dC_hat
+__device__ __forceinline__ float2 centroid_jacobian(float ss, float sdc, float inv_m) {
+  const float nc = sqrtf(ss) * inv_m;
+  const float inv = 1.f / fmaxf(nc, kCosDelta);
+  float proj = (sdc * inv_m) * inv;            // c_hat . dC_hat
+  if (nc < kCosDelta) proj *= clamp_proj_scale(nc);
+  return make_float2(inv * inv_m, proj * inv * inv * inv_m * inv_m);
+}
+
+// ------------------------------------------------------------------------------------------
 // K1: prep.  grid = n_local, block = 256, dynamic smem = (M + 1) * Dp floats.
 // ------------------------------------------------------------------------------------------
 // Body shared by prep_kernel and the fused small-batch kernel: speaker j, block of kThreads threads,
@@ -187,7 +261,7 @@ __device__ __forceinline__ void prep_body(const TE* __restrict__ E, const int32_
                                           int D, int Dp, float* __restrict__ e_hat, float* __restrict__ c_hat,
                                           float* __restrict__ cos_diag, float* smem) {
   __shared__ float red[kWarps];
-  __shared__ float s_inv_nc;
+  __shared__ float s_sc;
   float* sE = smem;                    // [M][Dp]
   float* sS = smem + (size_t)M * Dp;   // [Dp] column sums
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
@@ -207,43 +281,34 @@ __device__ __forceinline__ void prep_body(const TE* __restrict__ E, const int32_
   }
   __syncthreads();
 
-  const float m1 = (float)(M - 1);
+  const float inv_m = 1.f / (float)M, inv_m1 = 1.f / (float)(M - 1);
   for (int i = wid; i < M; i += kWarps) {
-    float ne2 = 0.f, nu2 = 0.f, eu = 0.f;
+    float ne2 = 0.f, nd2 = 0.f, ed = 0.f;
     for (int d = lane << 2; d < Dp; d += 128) {
       const float4 e = *reinterpret_cast<const float4*>(&sE[(size_t)i * Dp + d]);
       const float4 s = *reinterpret_cast<const float4*>(&sS[d]);
-      float4 u;                                               // s3:111
-      u.x = (s.x - e.x) / m1; u.y = (s.y - e.y) / m1; u.z = (s.z - e.z) / m1; u.w = (s.w - e.w) / m1;
-      ne2 += dot4(e, e);
-      nu2 += dot4(u, u);
-      eu += dot4(e, u);
+      const float4 dv = make_float4(s.x - e.x, s.y - e.y, s.z - e.z, s.w - e.w);
+      ne2 += dot4(e, e); nd2 += dot4(dv, dv); ed += dot4(e, dv);
     }
-    ne2 = warp_sum(ne2); nu2 = warp_sum(nu2); eu = warp_sum(eu);
-    const float inv_ne = 1.f / fmaxf(sqrtf(ne2), kCosDelta);
-    const float inv_nu = 1.f / fmaxf(sqrtf(nu2), kCosDelta);
+    const RowNorms n = row_norms(warp_sum(ne2), warp_sum(nd2), warp_sum(ed), inv_m1);
     float* out = e_hat + ((size_t)j * M + i) * D;
     for (int d = lane << 2; d < Dp; d += 128) {
       float4 e = *reinterpret_cast<const float4*>(&sE[(size_t)i * Dp + d]);
-      e.x *= inv_ne; e.y *= inv_ne; e.z *= inv_ne; e.w *= inv_ne;
+      e.x *= n.inv_ne; e.y *= n.inv_ne; e.z *= n.inv_ne; e.w *= n.inv_ne;
       if (ROUND) { e.x = round_tf32(e.x); e.y = round_tf32(e.y); e.z = round_tf32(e.z); e.w = round_tf32(e.w); }
       st4(out, d, D, vec_out, e);
     }
-    if (lane == 0) cos_diag[(size_t)j * M + i] = eu * inv_ne * inv_nu;   // s3:57
+    if (lane == 0) cos_diag[(size_t)j * M + i] = n.cos;
   }
 
   float part = 0.f;
-  const float fm = (float)M;
-  for (int d = tid; d < Dp; d += kThreads) {
-    const float c = sS[d] / fm;                                // s3:37
-    part += c * c;
-  }
+  for (int d = tid; d < Dp; d += kThreads) part += sS[d] * sS[d];
   const float tot = block_sum(part, red);
-  if (tid == 0) s_inv_nc = 1.f / fmaxf(sqrtf(tot), kCosDelta);
+  if (tid == 0) s_sc = centroid_scale(tot, inv_m);
   __syncthreads();
-  const float inv_nc = s_inv_nc;
+  const float sc = s_sc;
   for (int d = tid; d < D; d += kThreads) {
-    float c = (sS[d] / fm) * inv_nc;
+    float c = sS[d] * sc;
     if (ROUND) c = round_tf32(c);
     c_hat[(size_t)j * D + d] = c;
   }
@@ -331,18 +396,15 @@ prep_warp_kernel(const TE* __restrict__ E, const int32_t* __restrict__ idx, int 
         s[c].x += v[r][c].x; s[c].y += v[r][c].y; s[c].z += v[r][c].z; s[c].w += v[r][c].w;
       }
   }
-  // centroid (s3:37): c = s / M, c_hat = c / max(|c|, delta)
   const float inv_m = 1.f / (float)M, inv_m1 = 1.f / (float)(M - 1);
   float ss = 0.f;
 #pragma unroll
   for (int c = 0; c < KCH; ++c) ss += dot4(s[c], s[c]);
-  ss = warp_sum(ss);
-  const float sc = inv_m / fmaxf(sqrtf(ss) * inv_m, kCosDelta);
+  const float sc = centroid_scale(warp_sum(ss), inv_m);
 #pragma unroll
   for (int c = 0; c < KCH; ++c)
     put4<PREC>(c_hat, j, D, 4 * lane + 128 * c,
                make_float4(s[c].x * sc, s[c].y * sc, s[c].z * sc, s[c].w * sc));
-  // rows: |e|, |u| and e.u with u = (s - e) / (M - 1)   (s3:105-111, s3:57)
   float my_cos = 0.f;
   for (int i0 = 0; i0 < M; i0 += kRowBatch) {
     float4 v[kRowBatch][KCH];
@@ -373,13 +435,12 @@ prep_warp_kernel(const TE* __restrict__ E, const int32_t* __restrict__ idx, int 
 #pragma unroll
     for (int r = 0; r < kRowBatch; ++r) {
       if (i0 + r < M) {
-        const float inv_ne = 1.f / fmaxf(sqrtf(ne2[r]), kCosDelta);
-        const float inv_nu = 1.f / fmaxf(sqrtf(nd2[r]) * inv_m1, kCosDelta);
-        if (lane == ((i0 + r) & 31)) my_cos = (ed[r] * inv_m1) * inv_ne * inv_nu;
+        const RowNorms n = row_norms(ne2[r], nd2[r], ed[r], inv_m1);
+        if (lane == ((i0 + r) & 31)) my_cos = n.cos;
 #pragma unroll
         for (int c = 0; c < KCH; ++c) {
           float4 e = v[r][c];
-          e.x *= inv_ne; e.y *= inv_ne; e.z *= inv_ne; e.w *= inv_ne;
+          e.x *= n.inv_ne; e.y *= n.inv_ne; e.z *= n.inv_ne; e.w *= n.inv_ne;
           put4<PREC>(e_hat, (size_t)j * M + i0 + r, D, 4 * lane + 128 * c, e);
         }
       }
@@ -466,7 +527,6 @@ prep_reg_kernel(const TE* __restrict__ E, const int32_t* __restrict__ idx, int n
 #pragma unroll
   for (int i = 1; i < R; ++i) { s.x += v[i].x; s.y += v[i].y; s.z += v[i].z; s.w += v[i].w; }
   const float inv_m = 1.f / (float)M, inv_m1 = 1.f / (float)(M - 1);
-  // |e|^2, |s - e|^2, e.(s - e) of every row (u = (s - e) / (M - 1): s3:105-111), and |s|^2
   float ne2[16], nd2[16], ed[16];
 #pragma unroll
   for (int i = R; i < 16; ++i) { ne2[i] = 0.f; nd2[i] = 0.f; ed[i] = 0.f; }
@@ -479,13 +539,12 @@ prep_reg_kernel(const TE* __restrict__ E, const int32_t* __restrict__ idx, int n
   float t[4] = {reduce16_transposed(ne2, lane), reduce16_transposed(nd2, lane), reduce16_transposed(ed, lane),
                 warp_sum(dot4(s, s))};
   speaker_sum<W>(t, xch, wid, lane);
-  const float sc = inv_m / fmaxf(sqrtf(t[3]) * inv_m, kCosDelta);       // s3:37 + normalisation
+  const float sc = centroid_scale(t[3], inv_m);
   put4<PREC>(c_hat, j, D, col, make_float4(s.x * sc, s.y * sc, s.z * sc, s.w * sc));
   const int my_row = rev4(lane & 15);
-  const float inv_ne = 1.f / fmaxf(sqrtf(t[0]), kCosDelta);
-  const float inv_nu = 1.f / fmaxf(sqrtf(t[1]) * inv_m1, kCosDelta);
-  if (wid % W == 0 && lane < 16 && my_row < M)
-    cos_diag[(size_t)j * M + my_row] = (t[2] * inv_m1) * inv_ne * inv_nu;   // s3:57
+  const float inv_ne = row_norms(t[0], t[1], t[2], inv_m1).inv_ne;
+  if (wid % W == 0 && lane < 16 && my_row < M)     // the cosine in the storing lanes only
+    cos_diag[(size_t)j * M + my_row] = row_norms(t[0], t[1], t[2], inv_m1).cos;
 #pragma unroll
   for (int i = 0; i < R; ++i) {
     if (i < M) {      // warp-uniform
@@ -851,39 +910,29 @@ __device__ __forceinline__ void finalize_body(const TE* __restrict__ E, const fl
   }
   __syncthreads();
 
-  // centroid Jacobian: dc = (dC_hat - c_hat (c_hat . dC_hat) s) / max(|c|, delta)   (clamp_proj_scale)
-  const float fm = (float)M;
+  const float inv_m = 1.f / (float)M, inv_m1 = 1.f / (float)(M - 1);
   {
-    float n2 = 0.f, pr = 0.f;
+    float ss = 0.f, pr = 0.f;
     for (int d = tid; d < D; d += kThreads) {
-      const float c = sS[d] / fm;
-      n2 = fmaf(c, c, n2);
-      pr = fmaf(c, REUSE_E ? __ldcg(dC_hat + (size_t)j * D + d) : dC_hat[(size_t)j * D + d], pr);
+      ss = fmaf(sS[d], sS[d], ss);
+      pr = fmaf(sS[d], REUSE_E ? __ldcg(dC_hat + (size_t)j * D + d) : dC_hat[(size_t)j * D + d], pr);
     }
-    const float n2t = block_sum(n2, red);
+    const float sst = block_sum(ss, red);
     const float prt = block_sum(pr, red);
-    if (tid == 0) { s_bc[0] = n2t; s_bc[1] = prt; }
+    if (tid == 0) { s_bc[0] = sst; s_bc[1] = prt; }
     __syncthreads();
-    const float nc = sqrtf(s_bc[0]);
-    const float inv = 1.f / fmaxf(nc, kCosDelta);
-    float proj = s_bc[1] * inv;                  // c_hat . dC_hat
-    if (nc < kCosDelta) proj *= clamp_proj_scale(nc);
+    const float2 k = centroid_jacobian(s_bc[0], s_bc[1], inv_m);
     for (int d = tid; d < Dp; d += kThreads) {
       float v = 0.f;
-      if (d < D) {
-        const float dch = REUSE_E ? __ldcg(dC_hat + (size_t)j * D + d) : dC_hat[(size_t)j * D + d];
-        const float ch = (sS[d] / fm) * inv;
-        v = (dch - ch * proj) * inv / fm;
-      }
+      if (d < D) v = (REUSE_E ? __ldcg(dC_hat + (size_t)j * D + d) : dC_hat[(size_t)j * D + d]) * k.x - sS[d] * k.y;
       sB[d] = v;
     }
   }
   __syncthreads();
 
-  const float m1 = (float)(M - 1);
   for (int i = wid; i < M; i += kWarps) {
     const int r = j * M + i;
-    float ne2 = 0.f, nu2 = 0.f, eu = 0.f, eg = 0.f;
+    float ne2 = 0.f, nd2 = 0.f, ed = 0.f, eg = 0.f;
     const float* gh = dE_hat + (size_t)r * D;
     const float gr = RG ? __ldg(g_rows + r) : g;
     // tensor-core softmax path: dE_hat holds un-normalised rows, the true row is g * row_scale[r] times it
@@ -892,43 +941,22 @@ __device__ __forceinline__ void finalize_body(const TE* __restrict__ E, const fl
       const float4 e = *reinterpret_cast<const float4*>(&sE[(size_t)i * Dp + d]);
       const float4 s = *reinterpret_cast<const float4*>(&sS[d]);
       const float4 gv = ld4_plain(gh, d, D, vec_g);
-      float4 u;
-      u.x = (s.x - e.x) / m1; u.y = (s.y - e.y) / m1; u.z = (s.z - e.z) / m1; u.w = (s.w - e.w) / m1;
-      ne2 += dot4(e, e); nu2 += dot4(u, u); eu += dot4(e, u); eg += dot4(e, gv);
+      const float4 dv = make_float4(s.x - e.x, s.y - e.y, s.z - e.z, s.w - e.w);
+      ne2 += dot4(e, e); nd2 += dot4(dv, dv); ed += dot4(e, dv); eg += dot4(e, gv);
     }
-    ne2 = warp_sum(ne2); nu2 = warp_sum(nu2); eu = warp_sum(eu); eg = warp_sum(eg) * gsc;
-    const float ne = sqrtf(ne2), nu = sqrtf(nu2);
-    const float inv_ne = 1.f / fmaxf(ne, kCosDelta), inv_nu = 1.f / fmaxf(nu, kCosDelta);
-    const float cdv = eu * inv_ne * inv_nu;       // e_hat . u_hat (== cos_diag)
-    // diagonal element of w*G
-    const float Sd = fmaf(w, cos_diag[r] + eps, b);
-    float Gd;
-    if (variant == GE2E_SOFTMAX) {
-      Gd = -gr * row_aux[r];                // g (p_jj - 1), accumulated off-diagonal in fwd
-    } else {
-      const float sp = 1.f / (1.f + expf(-Sd));
-      Gd = -gr * sp * (1.f - sp);
-    }
-    const float dd = w * Gd;
-    // d e_hat = dE_hat_offdiag + dd * u_hat ;  d u_hat = dd * e_hat
-    float proj_e = eg * inv_ne + dd * cdv;        // e_hat . d e_hat
-    float proj_u = dd * cdv;                      // u_hat . d u_hat
-    if (ne < kCosDelta) proj_e *= clamp_proj_scale(ne);   // warp-uniform, rare
-    if (nu < kCosDelta) proj_u *= clamp_proj_scale(nu);
+    const RowNorms n = row_norms(warp_sum(ne2), warp_sum(nd2), warp_sum(ed), inv_m1);
+    const float dd = diag_term(variant, gr, variant == GE2E_SOFTMAX ? row_aux[r] : cos_diag[r], w, b, eps);
+    const RowJacobian J = row_jacobian(n, warp_sum(eg) * gsc, gsc, dd, inv_m1);
     for (int d = lane << 2; d < Dp; d += 128) {
       const float4 e = *reinterpret_cast<const float4*>(&sE[(size_t)i * Dp + d]);
       const float4 s = *reinterpret_cast<const float4*>(&sS[d]);
       const float4 gv = ld4_plain(gh, d, D, vec_g);
-      float ev[4] = {e.x, e.y, e.z, e.w}, sv[4] = {s.x, s.y, s.z, s.w}, gg[4] = {gv.x, gv.y, gv.z, gv.w};
+      const float ev[4] = {e.x, e.y, e.z, e.w}, sv[4] = {s.x, s.y, s.z, s.w}, gg[4] = {gv.x, gv.y, gv.z, gv.w};
       float de[4], du[4];
 #pragma unroll
       for (int t = 0; t < 4; ++t) {
-        const float eh = ev[t] * inv_ne;
-        const float uh = ((sv[t] - ev[t]) / m1) * inv_nu;
-        const float deh = gg[t] * gsc + dd * uh;
-        const float duh = dd * eh;
-        de[t] = (deh - eh * proj_e) * inv_ne;
-        du[t] = (duh - uh * proj_u) * inv_nu;
+        de[t] = J.de(ev[t], sv[t] - ev[t], gg[t]);
+        du[t] = J.du(ev[t], sv[t] - ev[t]);
       }
       // each (i, d) slot is read and then overwritten by the same single lane: no cross-lane hazard
       // (and no __syncwarp here: for D < 128 only some lanes enter this loop)
@@ -950,10 +978,10 @@ __device__ __forceinline__ void finalize_body(const TE* __restrict__ E, const fl
     const float4 sd = *reinterpret_cast<const float4*>(&sS[col]);
     const float4 bc = *reinterpret_cast<const float4*>(&sB[col]);
     float4 o;
-    o.x = de.x + bc.x + (sd.x - du.x) / m1;
-    o.y = de.y + bc.y + (sd.y - du.y) / m1;
-    o.z = de.z + bc.z + (sd.z - du.z) / m1;
-    o.w = de.w + bc.w + (sd.w - du.w) / m1;
+    o.x = de.x + bc.x + (sd.x - du.x) * inv_m1;
+    o.y = de.y + bc.y + (sd.y - du.y) * inv_m1;
+    o.z = de.z + bc.z + (sd.z - du.z) * inv_m1;
+    o.w = de.w + bc.w + (sd.w - du.w) * inv_m1;
     st4e(dE + phys_row(idx, (size_t)j * M + i) * D, col, D, vec_o, o);
   }
 }
@@ -1015,8 +1043,7 @@ finalize_warp_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
       }
   }
   const float inv_m = 1.f / (float)M, inv_m1 = 1.f / (float)(M - 1);
-  // centroid Jacobian: bc = dc_j / M with dc = (dC_hat - c_hat (c_hat . dC_hat) s) / max(|c|, delta)  (clamp_proj_scale)
-  float4 bc[KCH];
+  float4 bc[KCH];     // dc_j / M
   {
     float4 dch[KCH];
     float ss = 0.f, pr = 0.f;
@@ -1026,22 +1053,15 @@ finalize_warp_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
       ss += dot4(s[c], s[c]);
       pr += dot4(s[c], dch[c]);
     }
-    ss = warp_sum(ss); pr = warp_sum(pr);
-    const float nc = sqrtf(ss) * inv_m;
-    const float inv = 1.f / fmaxf(nc, kCosDelta);
-    float proj = (pr * inv_m) * inv;                // c_hat . dC_hat
-    if (nc < kCosDelta) proj *= clamp_proj_scale(nc);   // warp-uniform, rare
-    const float k1 = inv * inv_m;                   // dC_hat coefficient
-    const float k2 = proj * inv * inv * inv_m * inv_m;              // coefficient of s (c_hat = s inv / M)
+    const float2 k = centroid_jacobian(warp_sum(ss), warp_sum(pr), inv_m);
 #pragma unroll
     for (int c = 0; c < KCH; ++c) {
-      bc[c].x = dch[c].x * k1 - s[c].x * k2; bc[c].y = dch[c].y * k1 - s[c].y * k2;
-      bc[c].z = dch[c].z * k1 - s[c].z * k2; bc[c].w = dch[c].w * k1 - s[c].w * k2;
+      bc[c].x = dch[c].x * k.x - s[c].x * k.y; bc[c].y = dch[c].y * k.x - s[c].y * k.y;
+      bc[c].z = dch[c].z * k.x - s[c].z * k.y; bc[c].w = dch[c].w * k.x - s[c].w * k.y;
     }
   }
-  // pass 2: per-row scalars (kept in lane i) and sd = sum_i du_i
-  // de = a_g gv + a_e e + a_d d ,  du = b_e e + b_d d   with d = s - e (u = d / (M-1))
-  float a_g = 0.f, a_e = 0.f, a_d = 0.f, b_e = 0.f, b_d = 0.f;     // this lane's row (row index == lane)
+  // pass 2: the Jacobian of every row (kept in lane i) and sd = sum_i du_i
+  RowJacobian Jl = {0.f, 0.f, 0.f, 0.f, 0.f};     // this lane's row (row index == lane)
   float4 sd[KCH];
 #pragma unroll
   for (int c = 0; c < KCH; ++c) sd[c] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -1074,37 +1094,18 @@ finalize_warp_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
     for (int r = 0; r < kRowBatch; ++r) {
       if (i0 + r < M) {
         const int row = j * M + i0 + r;
-        const float ne = sqrtf(ne2[r]), nu = sqrtf(nd2[r]) * inv_m1;
-        const float inv_ne = 1.f / fmaxf(ne, kCosDelta), inv_nu = 1.f / fmaxf(nu, kCosDelta);
-        const float cdv = (ed[r] * inv_m1) * inv_ne * inv_nu;       // e_hat . u_hat
+        const RowNorms n = row_norms(ne2[r], nd2[r], ed[r], inv_m1);
         const float gr = RG ? __ldcg(gp + row) : g;                 // upstream gradient of this row
-        float Gd;                                                   // diagonal element of G
-        if (variant == GE2E_SOFTMAX) {
-          Gd = -gr * __ldg(row_aux + row);                          // g (p_jj - 1)
-        } else {
-          const float sp = 1.f / (1.f + expf(-fmaf(w, __ldg(cos_diag + row) + eps, b)));
-          Gd = -gr * sp * (1.f - sp);
-        }
-        const float dd = w * Gd;
+        const float dd = diag_term(variant, gr, variant == GE2E_SOFTMAX ? __ldg(row_aux + row) : __ldg(cos_diag + row),
+                                   w, b, eps);
         const float gsc = row_scale != nullptr ? gr * __ldcg(row_scale + row) : 1.f;   // un-normalised dE_hat rows
-        float proj_e = eg[r] * gsc * inv_ne + dd * cdv;             // e_hat . d e_hat
-        float proj_u = dd * cdv;                                    // u_hat . d u_hat
-        if (ne < kCosDelta) proj_e *= clamp_proj_scale(ne);         // warp-uniform, rare
-        if (nu < kCosDelta) proj_u *= clamp_proj_scale(nu);
-        // d e_hat = gv + dd u_hat, d u_hat = dd e_hat; Jacobians of the two normalisations (inv_x = 1 / max(|x|, delta)):
-        //   de = (deh - e_hat proj_e) inv_ne  ->  gv inv_ne + d (dd inv_nu inv_m1 inv_ne) - e (proj_e inv_ne^2)
-        //   du = (duh - u_hat proj_u) inv_nu  ->  e (dd inv_ne inv_nu) - d (proj_u inv_nu^2 inv_m1)
-        const float r_ag = inv_ne * gsc;
-        const float r_ad = dd * inv_nu * inv_m1 * inv_ne;
-        const float r_ae = -proj_e * inv_ne * inv_ne;
-        const float r_be = dd * inv_ne * inv_nu;
-        const float r_bd = -proj_u * inv_nu * inv_nu * inv_m1;
-        if (lane == i0 + r) { a_g = r_ag; a_e = r_ae; a_d = r_ad; b_e = r_be; b_d = r_bd; }
+        const RowJacobian J = row_jacobian(n, eg[r] * gsc, gsc, dd, inv_m1);
+        if (lane == i0 + r) Jl = J;
 #pragma unroll
         for (int c = 0; c < KCH; ++c) {
           const float4 e = v[r][c];
-          sd[c].x += r_be * e.x + r_bd * (s[c].x - e.x); sd[c].y += r_be * e.y + r_bd * (s[c].y - e.y);
-          sd[c].z += r_be * e.z + r_bd * (s[c].z - e.z); sd[c].w += r_be * e.w + r_bd * (s[c].w - e.w);
+          sd[c].x += J.du(e.x, s[c].x - e.x); sd[c].y += J.du(e.y, s[c].y - e.y);
+          sd[c].z += J.du(e.z, s[c].z - e.z); sd[c].w += J.du(e.w, s[c].w - e.w);
         }
       }
     }
@@ -1112,9 +1113,10 @@ finalize_warp_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
   // pass 3: dE_i = de_i + dc_j / M + (sd - du_i) / (M - 1)
   for (int i = 0; i < M; ++i) {
     vec4_t<TD>* Oi = reinterpret_cast<vec4_t<TD>*>(dE + phys_row(idx, (size_t)j * M + i) * D) + lane;
-    const float r_ag = __shfl_sync(0xffffffffu, a_g, i), r_ae = __shfl_sync(0xffffffffu, a_e, i);
-    const float r_ad = __shfl_sync(0xffffffffu, a_d, i), r_be = __shfl_sync(0xffffffffu, b_e, i);
-    const float r_bd = __shfl_sync(0xffffffffu, b_d, i);
+    RowJacobian J;
+    J.a_g = __shfl_sync(0xffffffffu, Jl.a_g, i); J.a_e = __shfl_sync(0xffffffffu, Jl.a_e, i);
+    J.a_d = __shfl_sync(0xffffffffu, Jl.a_d, i); J.b_e = __shfl_sync(0xffffffffu, Jl.b_e, i);
+    J.b_d = __shfl_sync(0xffffffffu, Jl.b_d, i);
 #pragma unroll
     for (int c = 0; c < KCH; ++c) {
       const float4 e = ldg4v<TE>(rowp(i) + c * 32);
@@ -1126,9 +1128,7 @@ finalize_warp_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
 #pragma unroll
       for (int t = 0; t < 4; ++t) {
         const float d = sv[t] - ev[t];
-        const float de = r_ag * gg[t] + r_ae * ev[t] + r_ad * d;
-        const float du = r_be * ev[t] + r_bd * d;
-        o[t] = de + bv[t] + (sdv[t] - du) * inv_m1;
+        o[t] = J.de(ev[t], d, gg[t]) + bv[t] + (sdv[t] - J.du(ev[t], d)) * inv_m1;
       }
       st4vv<TD>(Oi + c * 32, make_float4(o[0], o[1], o[2], o[3]));
     }
@@ -1143,7 +1143,6 @@ finalize_warp_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
 // batch; dE_hat rows are read twice (L2 / L1 hits).  Row sums through reduce16_transposed and
 // speaker_sum, the per-row Jacobian coefficients are computed lane-parallel (lane l owns row
 // rev4(l & 15)) and broadcast; the column sums (s, sum_i du_i) never leave the warp.
-//   de_i = a_g gv_i + a_e e_i + a_d d_i ,  du_i = b_e e_i + b_d d_i ,  d_i = s - e_i
 //   dE_i = de_i + dc_j / M + (sum_i' du_i' - du_i) / (M - 1)
 // ------------------------------------------------------------------------------------------
 template <int W, int RR, typename TE, typename TD, bool RG = false>
@@ -1207,68 +1206,37 @@ finalize_reg_kernel(const TE* __restrict__ E, const float* __restrict__ dE_hat,
     t[5] = warp_sum(dot4(s, dch));
   }
   speaker_sum<W>(t, xch, wid, lane);
-  const float t_eg = t[0], t_ne2 = t[1], t_nd2 = t[2], t_ed = t[3];
   const float inv_m = 1.f / (float)M, inv_m1 = 1.f / (float)(M - 1);
-  // centroid Jacobian: bc = dc_j / M with dc = (dC_hat - c_hat (c_hat . dC_hat) s) / max(|c|, delta)  (clamp_proj_scale)
-  float4 bc;
+  const float2 k = centroid_jacobian(t[4], t[5], inv_m);
+  const float4 bc = make_float4(dch.x * k.x - s.x * k.y, dch.y * k.x - s.y * k.y, dch.z * k.x - s.z * k.y,
+                                dch.w * k.x - s.w * k.y);     // dc_j / M
+  RowJacobian J;     // this lane's row
   {
-    const float nc = sqrtf(t[4]) * inv_m;
-    const float inv = 1.f / fmaxf(nc, kCosDelta);
-    float proj = (t[5] * inv_m) * inv;              // c_hat . dC_hat
-    if (nc < kCosDelta) proj *= clamp_proj_scale(nc);   // warp-uniform, rare
-    const float k1 = inv * inv_m;
-    const float k2 = proj * inv * inv * inv_m * inv_m;
-    bc = make_float4(dch.x * k1 - s.x * k2, dch.y * k1 - s.y * k2, dch.z * k1 - s.z * k2, dch.w * k1 - s.w * k2);
-  }
-  // this lane's row
-  float a_g, a_e, a_d, b_e, b_d;
-  {
-    const float ne = sqrtf(t_ne2), nu = sqrtf(t_nd2) * inv_m1;
-    const float inv_ne = 1.f / fmaxf(ne, kCosDelta), inv_nu = 1.f / fmaxf(nu, kCosDelta);
-    const float cdv = (t_ed * inv_m1) * inv_ne * inv_nu;          // e_hat . u_hat
     const float gr = RG ? __ldcg(gp + row) : g;                   // upstream gradient of this lane's row
     const float gsc = (RG && row_scale != nullptr) ? gr * gsc0 : gsc0;
-    float Gd;                                                     // diagonal element of G
-    if (variant == GE2E_SOFTMAX) {
-      Gd = -gr * aux;                                             // g (p_jj - 1)
-    } else {
-      const float sp = 1.f / (1.f + expf(-fmaf(w, aux + eps, b)));
-      Gd = -gr * sp * (1.f - sp);
-    }
-    const float dd = w * Gd;
-    const float proj_e = t_eg * gsc * inv_ne + dd * cdv;          // e_hat . d e_hat
-    const float proj_u = dd * cdv;                                // u_hat . d u_hat
-    a_g = inv_ne * gsc;
-    a_d = dd * inv_nu * inv_m1 * inv_ne;
-    a_e = -proj_e * inv_ne * inv_ne;
-    b_e = dd * inv_ne * inv_nu;
-    b_d = -proj_u * inv_nu * inv_nu * inv_m1;
-    // rows at or below the clamp (rare; lanes past row M - 1 hold no row): projections scaled by clamp_proj_scale
-    if (__any_sync(0xffffffffu, my_row < M && (ne < kCosDelta || nu < kCosDelta))) {
-      a_e *= clamp_proj_scale(ne);
-      b_d *= clamp_proj_scale(nu);
-    }
+    J = row_jacobian(row_norms(t[1], t[2], t[3], inv_m1), t[0] * gsc, gsc, diag_term(variant, gr, aux, w, b, eps),
+                     inv_m1);
   }
   float4 sd = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
   for (int i = 0; i < R; ++i) {
     if (i < M) {
-      const float r_be = __shfl_sync(0xffffffffu, b_e, rev4(i)), r_bd = __shfl_sync(0xffffffffu, b_d, rev4(i));
+      const float r_be = __shfl_sync(0xffffffffu, J.b_e, rev4(i)), r_bd = __shfl_sync(0xffffffffu, J.b_d, rev4(i));
       const float4 e = v[i];
       sd.x += r_be * e.x + r_bd * (s.x - e.x); sd.y += r_be * e.y + r_bd * (s.y - e.y);
       sd.z += r_be * e.z + r_bd * (s.z - e.z); sd.w += r_be * e.w + r_bd * (s.w - e.w);
     }
   }
-  // dE_i = a_g gv_i + a_e e_i + a_d d_i + bc + (sd - b_e e_i - b_d d_i) / (M - 1), with d_i = s - e_i, is
-  //   k_g gv_i + k_e e_i + k_s s + base:  three coefficients per row instead of five
-  const float k_s = a_d - b_d * inv_m1;
-  const float k_e = a_e - b_e * inv_m1 - k_s;
+  // dE_i = de_i + bc + (sd - du_i) / (M - 1), with d_i = s - e_i, is k_g gv_i + k_e e_i + k_s s + base:
+  // three coefficients per row instead of five
+  const float k_s = J.a_d - J.b_d * inv_m1;
+  const float k_e = J.a_e - J.b_e * inv_m1 - k_s;
   const float4 base = make_float4(fmaf(sd.x, inv_m1, bc.x), fmaf(sd.y, inv_m1, bc.y), fmaf(sd.z, inv_m1, bc.z),
                                   fmaf(sd.w, inv_m1, bc.w));
 #pragma unroll
   for (int i = 0; i < R; ++i) {
     if (i < M) {
-      const float r_g = __shfl_sync(0xffffffffu, a_g, rev4(i)), r_e = __shfl_sync(0xffffffffu, k_e, rev4(i));
+      const float r_g = __shfl_sync(0xffffffffu, J.a_g, rev4(i)), r_e = __shfl_sync(0xffffffffu, k_e, rev4(i));
       const float r_s = __shfl_sync(0xffffffffu, k_s, rev4(i));
       const float4 e = v[i];
       const float4 gv = __ldg(reinterpret_cast<const float4*>(Gj + (size_t)i * D));
@@ -1694,8 +1662,8 @@ small_step_kernel(const SmallParams p) {
   __shared__ float red[3 * kWarps];
   __shared__ float s_cd[32];
   __shared__ __align__(8) unsigned long long s_bar;   // bulk-copy completion (stage 2 operands)
-  __shared__ float s_ine[16], s_inu[16], s_aux[16];   // fast path: 1/|e|, 1/|u|, 1 - p_jj per row of the speaker
-  __shared__ float s_pe[16], s_pu[16];                // fast path: clamp_proj_scale of |e|, |u|
+  __shared__ float3 s_rsum[16];                       // fast path: |e|^2, |s - e|^2, e.(s - e) per row of the speaker
+  __shared__ float s_aux[16];                         // fast path: 1 - p_jj per row
   constexpr int R4 = MR / 4;                          // rows per thread where the block splits into 4 row groups
   const int j = blockIdx.x, N = gridDim.x, M = p.M, D = p.D, Dp = p.Dp;
   const int Np = (N + 3) & ~3;
@@ -1739,8 +1707,8 @@ small_step_kernel(const SmallParams p) {
   float* fB = fU + (size_t)M * Dp;                    // [Dp] dC_hat row, then d c / M
   const int ncol4 = Dp >> 2;
   const int hw = tid >> 4, hl = tid & 15;             // half-warp <-> row
-  const float fm = (float)M, inv_m1 = 1.f / (float)(M - 1);
-  float c_norm2 = 0.f, c_mine = 0.f;                  // fast path: |c_j|^2 (every thread), c_j[tid]
+  const float inv_m = 1.f / (float)M, inv_m1 = 1.f / (float)(M - 1);
+  float s_norm2 = 0.f, s_mine = 0.f;                  // fast path: |s_j|^2 (every thread), s_j[tid]
   if (fast) {
     for (int i = wid; i < M; i += kWarps) {
       const TE* src = E + phys_row(p.idx, (size_t)j * M + i) * D;
@@ -1749,25 +1717,22 @@ small_step_kernel(const SmallParams p) {
     }
     for (int v = tid; v < (MR - M) * Dp; v += kThreads) sEh[(size_t)M * Dp + v] = 0.f;
     __syncthreads();
-    float cpart = 0.f;
+    float spart = 0.f;
     for (int d = tid; d < Dp; d += kThreads) {
       float sum = 0.f;
       for (int i = 0; i < M; ++i) sum += fE[(size_t)i * Dp + d];                 // s3:105
       fS[d] = sum;
-      const float c = sum / fm;                                                  // s3:37
-      cpart = fmaf(c, c, cpart);
+      spart = fmaf(sum, sum, spart);
     }
-    cpart = warp_sum(cpart);
-    if (lane == 0) red[wid] = cpart;
+    spart = warp_sum(spart);
+    if (lane == 0) red[wid] = spart;
     __syncthreads();
 #pragma unroll
-    for (int q = 0; q < kWarps; ++q) c_norm2 += red[q];
-    const float inv_nc = 1.f / fmaxf(sqrtf(c_norm2), kCosDelta);
+    for (int q = 0; q < kWarps; ++q) s_norm2 += red[q];
     if (tid < D) {                                     // D <= 256 = block size: one centroid entry per thread
-      c_mine = fS[tid] / fm;
-      p.c_hat[(size_t)j * D + tid] = c_mine * inv_nc;
+      s_mine = fS[tid];
+      p.c_hat[(size_t)j * D + tid] = s_mine * centroid_scale(s_norm2, inv_m);
     }
-    // rows: |e|, |u| and e.u with u = (s - e) / (M - 1)   (s3:105-111, s3:57)
     const bool act = hw < M;
     float ne2 = 0.f, nd2 = 0.f, ed = 0.f;
     if (act)
@@ -1784,21 +1749,15 @@ small_step_kernel(const SmallParams p) {
       ed += __shfl_xor_sync(0xffffffffu, ed, o);
     }
     if (act) {
-      const float ne = sqrtf(ne2), nu = sqrtf(nd2) * inv_m1;
-      const float inv_ne = 1.f / fmaxf(ne, kCosDelta), inv_nu = 1.f / fmaxf(nu, kCosDelta);
-      const float cosd = (ed * inv_m1) * inv_ne * inv_nu;
+      const RowNorms n = row_norms(ne2, nd2, ed, inv_m1);
       float4* gdst = reinterpret_cast<float4*>(p.e_hat + ((size_t)j * M + hw) * D);
       for (int c4 = hl; c4 < ncol4; c4 += 16) {
         float4 e = reinterpret_cast<const float4*>(fE + (size_t)hw * Dp)[c4];
-        e.x *= inv_ne; e.y *= inv_ne; e.z *= inv_ne; e.w *= inv_ne;
+        e.x *= n.inv_ne; e.y *= n.inv_ne; e.z *= n.inv_ne; e.w *= n.inv_ne;
         reinterpret_cast<float4*>(sEh + (size_t)hw * Dp)[c4] = e;
         gdst[c4] = e;
       }
-      if (hl == 0) {
-        s_cd[hw] = cosd; p.cos_diag[(size_t)j * M + hw] = cosd;
-        s_ine[hw] = inv_ne; s_inu[hw] = inv_nu;
-        s_pe[hw] = clamp_proj_scale(ne); s_pu[hw] = clamp_proj_scale(nu);
-      }
+      if (hl == 0) { s_cd[hw] = n.cos; p.cos_diag[(size_t)j * M + hw] = n.cos; s_rsum[hw] = make_float3(ne2, nd2, ed); }
     }
   } else {
     prep_body<false>(E, p.idx, j, M, D, Dp, p.e_hat, p.c_hat, p.cos_diag, sA);
@@ -2093,17 +2052,9 @@ small_step_kernel(const SmallParams p) {
 #pragma unroll
         for (int o = 8; o > 0; o >>= 1) eg += __shfl_xor_sync(0xffffffffu, eg, o);
         if (act) {
-          const float inv_ne = s_ine[hw], inv_nu = s_inu[hw], cdv = s_cd[hw];
-          float Gd;                                      // diagonal element of G
-          if (VARIANT == GE2E_SOFTMAX) {
-            Gd = -g * s_aux[hw];                         // g (p_jj - 1), accumulated off-diagonal in stage 2
-          } else {
-            const float sp = 1.f / (1.f + expf(-fmaf(w, cdv + eps, b)));
-            Gd = -g * sp * (1.f - sp);
-          }
-          const float dd = w * Gd;
-          const float proj_e = (eg * inv_ne + dd * cdv) * s_pe[hw];   // (e_hat . d e_hat) s_e
-          const float proj_u = (dd * cdv) * s_pu[hw];                 // (u_hat . d u_hat) s_u
+          const float dd = diag_term(VARIANT, g, VARIANT == GE2E_SOFTMAX ? s_aux[hw] : s_cd[hw], w, b, eps);
+          const float3 rs = s_rsum[hw];
+          const RowJacobian J = row_jacobian(row_norms(rs.x, rs.y, rs.z, inv_m1), eg, 1.f, dd, inv_m1);
           for (int c4 = hl; c4 < ncol4; c4 += 16) {
             const float4 e = reinterpret_cast<const float4*>(fE + (size_t)hw * Dp)[c4];
             const float4 sv = reinterpret_cast<const float4*>(fS)[c4];
@@ -2112,12 +2063,8 @@ small_step_kernel(const SmallParams p) {
             float de[4], du[4];
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
-              const float eh = ev[t] * inv_ne;
-              const float uh = ((ss[t] - ev[t]) * inv_m1) * inv_nu;
-              const float deh = gg[t] + dd * uh;
-              const float duh = dd * eh;
-              de[t] = (deh - eh * proj_e) * inv_ne;
-              du[t] = (duh - uh * proj_u) * inv_nu;
+              de[t] = J.de(ev[t], ss[t] - ev[t], gg[t]);
+              du[t] = J.du(ev[t], ss[t] - ev[t]);
             }
             // each slot is read and then overwritten by the same lane
             reinterpret_cast<float4*>(fU + (size_t)hw * Dp)[c4] = make_float4(du[0], du[1], du[2], du[3]);
@@ -2178,19 +2125,16 @@ small_step_kernel(const SmallParams p) {
   GE2E_SMALL_STAMP(9);
   if (p.stop == 7) break;
   if (fast) {
-    // centroid Jacobian: d c = (dC_hat - c_hat (c_hat . dC_hat) s) / max(|c|, delta)  (clamp_proj_scale), kept as d c / M
     const float dch = tid < D ? __ldcg(p.dC_hat + (size_t)j * D + tid) : 0.f;      // assembled at the L2 by all CTAs
-    float prp = warp_sum(c_mine * dch);
+    float prp = warp_sum(s_mine * dch);
     if (lane == 0) red[wid] = prp;
     __syncthreads();
     float pr = 0.f;
 #pragma unroll
     for (int q = 0; q < kWarps; ++q) pr += red[q];
     if (tid < D) {
-      const float nc = sqrtf(c_norm2);
-      const float inv = 1.f / fmaxf(nc, kCosDelta);
-      const float proj = pr * inv * clamp_proj_scale(nc);   // (c_hat . dC_hat) s
-      fB[tid] = (dch - (c_mine * inv) * proj) * inv / fm;
+      const float2 k = centroid_jacobian(s_norm2, pr, inv_m);
+      fB[tid] = dch * k.x - s_mine * k.y;     // dc_j / M
     }
     __syncthreads();
     for (int i = wid; i < M; i += kWarps) {           // fan-out of d c and of the leave-one-out centroids (s3:105-111)
