@@ -465,9 +465,15 @@ int ge2e_b200_forward_backward_typed(const void* E, int e_dtype, const int32_t* 
  *   order, required; any values, negative and zero included) in place of the scalar grad_out:
  *   dE = sum_r grad_rows[r] dL_r / dE, accum[1] = dw, accum[2] = db likewise; dE is rounded to de_dtype once.
  * A NULL per_row / grad_rows returns GE2E_ERR_ARGUMENT before anything is launched.  The upstream gradient is known
- * only after the forward, so these run the staged kernels (forward, then backward) on every shape: the single-kernel
- * step and the whole-step-in-forward scheme (ge2e_b200_forward_backward with grad_out = 1, then
- * ge2e_b200_scale_grads) have no per-row form, nor have the speaker-sharded entry points. */
+ * only after the forward, so the forward and the backward are separate launches.  On the shapes where
+ * ge2e_b200_forward_backward runs the single-kernel step (ge2e_b200_step_launches() == 1, same
+ * ge2e_b200_debug_small_step rule) and the workspace has at least ge2e_b200_step_workspace_bytes() bytes, each is
+ * ONE kernel -- that step cut after the row losses: the forward runs prep and the losses; the backward re-reads E,
+ * recomputes the cosines from e_hat / c_hat, forms w G from grad_rows and the row statistics and runs the rest of
+ * the step.  Otherwise (a workspace of ge2e_b200_workspace_bytes(), every other shape) they run the staged kernels.
+ * Both forms leave and read the same forward outputs, so either forward pairs with either backward.  The
+ * whole-step-in-forward scheme (ge2e_b200_forward_backward with grad_out = 1, then ge2e_b200_scale_grads) has no
+ * per-row form, nor have the speaker-sharded entry points. */
 int ge2e_b200_forward_per_row_typed(const void* E, int e_dtype, const int32_t* row_index, int N, int M, int D,
                                     const float* w, const float* b, float eps, int variant, int precision, float* e_hat,
                                     float* c_hat, float* cos_diag, float* row_stat, int32_t* row_kstar, float* row_aux,

@@ -1,18 +1,24 @@
 """What reduction="none" costs a training step, against the summed loss, and what the per-row backward costs against
 the scalar one.
 
-    python scripts/per_row_cost.py --out DIR [--workloads cfg2,cfg3] [--precisions fp32,tf32] [--steps 20] [--rounds 9]
+    python scripts/per_row_cost.py --out DIR [--workloads cfg2,cfg3,128x10x256] [--precisions fp32,tf32] [--steps 20]
+                                   [--rounds 9]
 
-Per (workload, precision), four CUDA graphs of ``--steps`` steps each, captured over rotating batches (more than the
-126 MB L2 together, so every step reads its inputs from HBM), replayed alternately ``--rounds`` times in one process:
+A workload is a bench.py name or NxMxD.  Per (workload, precision), five CUDA graphs of ``--steps`` steps each,
+captured over up to ``--steps`` rotating batches, replayed alternately ``--rounds`` times in one process.  At cfg3 the
+batches together exceed the 126 MB L2, so every step reads its inputs from HBM; at the small workloads (cfg1, cfg2,
+128x10x256) they fit in the L2 and the numbers are those of L2-resident inputs, as in a training loop at these sizes.
+
 
   sum          loss = GE2ELoss(reduction="sum")(E); loss.backward(): the whole step in the forward call (the
                single-kernel step at cfg2, prep + step kernel + finalize at cfg3), the upstream gradient applied by
                one scaling launch in backward
-  none         L = GE2ELoss(reduction="none")(E); L.backward(g), g[N, M] random: the staged pipeline (forward kernels,
-               then the per-row backward kernels)
+  none         L = GE2ELoss(reduction="none")(E); L.backward(g), g[N, M] random: the forward kernels, then the
+               per-row backward kernels (on the single-kernel step's shapes one launch each, else the staged pipeline)
   bwd_scalar   ge2e_b200_backward_typed alone, on saved forwards (one per rotating batch)
   bwd_per_row  ge2e_b200_backward_per_row_typed alone, on the same saved forwards
+  plan_none    GE2EPlan(reduction="none").step(E, w, b): the per-row forward and backward as bare C-ABI calls
+               (grad_rows = g of the first batch); skipped on a build whose GE2EPlan has no reduction argument
 
 It prints (and writes to DIR/per_row_cost.json) the median time per step of each, the spread over the rounds, and
 the GPU's name and power limit read in the same run.
@@ -50,11 +56,18 @@ def capture(step, steps):
     return g
 
 
+def shape_of(workload):
+    if workload in WORKLOADS:
+        return WORKLOADS[workload]
+    N, M, D = (int(x) for x in workload.split("x"))
+    return N, M, D
+
+
 def measure(pkg, ops, lib_codes, workload, precision, steps, rounds, dev):
-    N, M, D = WORKLOADS[workload]
+    N, M, D = shape_of(workload)
     U = N * M
     vcode, pcode = lib_codes(precision, N, M, D)
-    n_rot = max(2, int(np.ceil(1.5 * 126e6 / (U * D * 4))))
+    n_rot = min(steps, max(2, int(np.ceil(1.5 * 126e6 / (U * D * 4)))))   # a graph uses `steps` batches at most
     Es = [make_batch(N, M, D, seed=i).to(dev).requires_grad_(True) for i in range(n_rot)]
     gen = torch.Generator().manual_seed(0)
     gs = [torch.randn(N, M, generator=gen).to(dev) for _ in range(n_rot)]
@@ -83,6 +96,15 @@ def measure(pkg, ops, lib_codes, workload, precision, steps, rounds, dev):
     graphs = {"sum": capture(step_sum, steps), "none": capture(step_none, steps),
               "bwd_scalar": capture(lambda k: bwd(k, False), steps),
               "bwd_per_row": capture(lambda k: bwd(k, True), steps)}
+    try:
+        plan = pkg.GE2EPlan(N, M, D, precision=precision, device=dev, reduction="none")
+    except TypeError:
+        plan = None
+    if plan is not None:
+        plan.grad_rows.copy_(gs[0])
+        wp, bp = w.clone(), b.clone()
+        graphs["plan_none"] = plan.capture([E.detach() for E in Es], wp, bp, steps=steps)
+        plan_launches = plan.launches_per_step
     for g in graphs.values():
         g.replay()
     torch.cuda.synchronize()
@@ -102,9 +124,11 @@ def measure(pkg, ops, lib_codes, workload, precision, steps, rounds, dev):
         "step_us_median": med,
         "step_us_min_max": {k: [round(min(v), 2), round(max(v), 2)] for k, v in times.items()},
         "none_over_sum": med["none"] / med["sum"],
+        "plan_none_over_sum": med["plan_none"] / med["sum"] if plan is not None else None,
+        "plan_none_launches_per_step": plan_launches if plan is not None else None,
         "bwd_per_row_over_scalar": med["bwd_per_row"] / med["bwd_scalar"],
         "how": (f"{steps} captured steps per graph over {n_rot} rotating batches ({n_rot * U * D * 4 / 1e6:.0f} MB of "
-                f"fp32 E), the four graphs replayed alternately {rounds} times; CUDA-event time per replay / steps, "
+                f"fp32 E), the graphs replayed alternately {rounds} times; CUDA-event time per replay / steps, "
                 "median and range over the rounds"),
     }
 
@@ -112,7 +136,7 @@ def measure(pkg, ops, lib_codes, workload, precision, steps, rounds, dev):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", required=True)
-    ap.add_argument("--workloads", default="cfg2,cfg3")
+    ap.add_argument("--workloads", default="cfg1,cfg2,128x10x256,cfg3")
     ap.add_argument("--precisions", default="fp32,tf32")
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--rounds", type=int, default=9)

@@ -330,6 +330,16 @@ static bool tc_softmax_step(int n_local, int n_total, int M, int D, int variant,
   return variant == GE2E_SOFTMAX && on_tc(n_local, n_total, M, D, variant, precision);
 }
 
+static bool use_small_step(int N, int M, int D, int variant, int precision);
+
+// Per-utterance losses on a shape of the single-kernel step: its two halves (kSmallFwd / kSmallBwd), where the caller's
+// workspace has room for them.  A workspace sized by ge2e_b200_workspace_bytes() keeps the staged kernels.
+static bool use_small_halves(int N, int M, int D, int variant, int precision, const void* workspace,
+                             size_t workspace_bytes) {
+  return use_small_step(N, M, D, variant, precision) && workspace != nullptr &&
+         workspace_bytes >= small_step_workspace_bytes(N, M, D);
+}
+
 // per_row (nullable): [N*M] row losses in logical order
 static int forward_impl(const void* E, int e_dtype, const int32_t* row_index, int N, int M, int D, const float* w,
                         const float* b, float eps, int variant, int precision, float* e_hat, float* c_hat,
@@ -340,6 +350,15 @@ static int forward_impl(const void* E, int e_dtype, const int32_t* row_index, in
   int rc = check_enum(variant, precision);
   if (rc != GE2E_OK) return rc;
   if ((rc = check_dtypes(e_dtype, GE2E_DT_F32)) != GE2E_OK) return rc;
+  if (per_row != nullptr && use_small_halves(N, M, D, variant, precision, workspace, workspace_bytes)) {
+    if (!E || !w || !b || !e_hat || !c_hat || !cos_diag || !row_stat) return GE2E_ERR_ARGUMENT;
+    if ((rc = check_shape(N, N, 0, M, D)) != GE2E_OK) return rc;
+    if (variant == GE2E_CONTRAST && !row_kstar) return GE2E_ERR_ARGUMENT;
+    if (variant == GE2E_SOFTMAX && !row_aux) return GE2E_ERR_ARGUMENT;
+    return simt_small_step(kSmallFwd, E, e_dtype, row_index, N, M, D, w, b, eps, variant, nullptr, nullptr, e_hat, c_hat,
+                           cos_diag, row_stat, row_kstar, row_aux, per_row, accum, nullptr, nullptr, nullptr, nullptr,
+                           GE2E_DT_F32, workspace, (cudaStream_t)stream);
+  }
   // tensor-core path: prep and the rows kernel are adjacent in the stream, the second one is launched
   // programmatically under the first one's tail
   rc = ge2e_b200_prep_typed(E, e_dtype, row_index, N, M, D, precision, e_hat, c_hat, cos_diag, accum, stream);
@@ -395,6 +414,19 @@ static int backward_impl(const void* E, int e_dtype, const int32_t* row_index, c
   if (!accum) return GE2E_ERR_ARGUMENT;
   if (check_dtypes(e_dtype, de_dtype) != GE2E_OK) return GE2E_ERR_ARGUMENT;
   if (M > finalize_max_rows(D)) return GE2E_ERR_UNSUPPORTED;     // before the rows kernels run
+  if (grad_rows != nullptr && use_small_halves(N, M, D, variant, precision, workspace, workspace_bytes)) {
+    if (!E || !e_hat || !c_hat || !cos_diag || !row_stat || !w || !b || !dE_hat || !dC_hat || !dE)
+      return GE2E_ERR_ARGUMENT;
+    int rc = check_shape(N, N, 0, M, D);
+    if (rc != GE2E_OK) return rc;
+    if ((rc = check_enum(variant, precision)) != GE2E_OK) return rc;
+    if (variant == GE2E_CONTRAST && !row_kstar) return GE2E_ERR_ARGUMENT;
+    if (variant == GE2E_SOFTMAX && !row_aux) return GE2E_ERR_ARGUMENT;
+    return simt_small_step(kSmallBwd, E, e_dtype, row_index, N, M, D, w, b, eps, variant, nullptr, grad_rows,
+                           const_cast<float*>(e_hat), const_cast<float*>(c_hat), const_cast<float*>(cos_diag),
+                           const_cast<float*>(row_stat), const_cast<int32_t*>(row_kstar), const_cast<float*>(row_aux),
+                           nullptr, nullptr, dE_hat, dC_hat, accum + 1, dE, de_dtype, workspace, (cudaStream_t)stream);
+  }
   // row_scale is meaningful only where the forward produced it
   const float* scale = tc_softmax_step(N, N, M, D, variant, precision) ? row_scale : nullptr;
   int rc = bwd_rows_impl(e_hat, c_hat, cos_diag, row_stat, row_kstar, row_aux, scale, N, N, 0, M, D, w, b, eps, variant,
@@ -558,9 +590,9 @@ int ge2e_b200_forward_backward_typed(const void* E, int e_dtype, const int32_t* 
   if (use_small_step(N, M, D, variant, precision)) {
     if (!workspace || workspace_bytes < small_step_workspace_bytes(N, M, D)) return GE2E_ERR_WORKSPACE;
     if (variant == GE2E_CONTRAST && !row_kstar) return GE2E_ERR_ARGUMENT;
-    return simt_small_step(E, e_dtype, row_index, N, M, D, w, b, eps, variant, grad_out, e_hat, c_hat, cos_diag,
-                           row_stat, row_kstar, row_aux, nullptr, accum, dE_hat, dC_hat, accum + 1, dE, de_dtype,
-                           workspace, (cudaStream_t)stream);
+    return simt_small_step(kSmallWhole, E, e_dtype, row_index, N, M, D, w, b, eps, variant, grad_out, nullptr, e_hat,
+                           c_hat, cos_diag, row_stat, row_kstar, row_aux, nullptr, accum, dE_hat, dC_hat, accum + 1, dE,
+                           de_dtype, workspace, (cudaStream_t)stream);
   }
   // prep (zeroes accum) -> rows: every kernel is launched programmatically under its predecessor's tail
   rc = ge2e_b200_prep_typed(E, e_dtype, row_index, N, M, D, precision, e_hat, c_hat, cos_diag, accum, stream);

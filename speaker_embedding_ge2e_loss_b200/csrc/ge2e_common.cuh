@@ -160,9 +160,12 @@ int simt_bwd_finalize(const void* E, int e_dt, const int32_t* row_index, const f
 bool small_step_supported(int N, int M, int D);
 bool small_step_preferred(int N, int M, int D, int variant);   // supported AND faster than the pipeline
 size_t small_step_workspace_bytes(int N, int M, int D);
-int simt_small_step(const void* E, int e_dt, const int32_t* row_index, int N, int M, int D, const float* w,
-                    const float* b, float eps, int variant, const float* grad_out, float* e_hat, float* c_hat,
-                    float* cos_diag, float* row_stat, int32_t* row_kstar, float* row_aux, float* per_row,
+// part: the whole step, or its forward half (through the row losses) / backward half (upstream gradient grad_rows
+// per logical row; e_hat, c_hat, cos_diag and the row statistics are inputs) -- reduction "none"
+enum { kSmallWhole = 0, kSmallFwd = 1, kSmallBwd = 2 };
+int simt_small_step(int part, const void* E, int e_dt, const int32_t* row_index, int N, int M, int D, const float* w,
+                    const float* b, float eps, int variant, const float* grad_out, const float* grad_rows, float* e_hat,
+                    float* c_hat, float* cos_diag, float* row_stat, int32_t* row_kstar, float* row_aux, float* per_row,
                     float* loss_accum, float* dE_hat, float* dC_hat, float* dwdb, void* dE, int de_dt, void* workspace,
                     cudaStream_t st);
 // out_dt: ge2e_dtype of out (in is fp32)

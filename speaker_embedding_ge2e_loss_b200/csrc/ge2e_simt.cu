@@ -254,6 +254,19 @@ __device__ __forceinline__ float2 centroid_jacobian(float ss, float sdc, float i
 // ------------------------------------------------------------------------------------------
 // K1: prep.  grid = n_local, block = 256, dynamic smem = (M + 1) * Dp floats.
 // ------------------------------------------------------------------------------------------
+// The M raw rows of speaker j, widened to fp32, into sE[M][Dp] (columns D..Dp-1 zero); ends with a __syncthreads.
+template <typename TE>
+__device__ __forceinline__ void stage_rows(const TE* __restrict__ E, const int32_t* __restrict__ idx, int j, int M,
+                                           int D, int Dp, float* sE) {
+  const bool vec_in = is_vec(E, D);
+  for (int v = threadIdx.x; v < M * (Dp >> 2); v += kThreads) {
+    const int i = v / (Dp >> 2), col = (v % (Dp >> 2)) << 2;
+    *reinterpret_cast<float4*>(&sE[(size_t)i * Dp + col]) =
+        ld4e(E + phys_row(idx, (size_t)j * M + i) * D, col, D, vec_in);
+  }
+  __syncthreads();
+}
+
 // Body shared by prep_kernel and the fused small-batch kernel: speaker j, block of kThreads threads,
 // `smem` = (M + 1) * Dp floats.
 template <bool ROUND, typename TE = float>
@@ -265,15 +278,9 @@ __device__ __forceinline__ void prep_body(const TE* __restrict__ E, const int32_
   float* sE = smem;                    // [M][Dp]
   float* sS = smem + (size_t)M * Dp;   // [Dp] column sums
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-  const bool vec_in = is_vec(E, D);
   const bool vec_out = is_vec(e_hat, D);
 
-  for (int v = tid; v < M * (Dp >> 2); v += kThreads) {
-    const int i = v / (Dp >> 2), col = (v % (Dp >> 2)) << 2;
-    *reinterpret_cast<float4*>(&sE[(size_t)i * Dp + col]) =
-        ld4e(E + phys_row(idx, (size_t)j * M + i) * D, col, D, vec_in);
-  }
-  __syncthreads();
+  stage_rows(E, idx, j, M, D, Dp, sE);
   for (int d = tid; d < Dp; d += kThreads) {
     float s = 0.f;
     for (int i = 0; i < M; ++i) s += sE[(size_t)i * Dp + d];   // s3:105
@@ -893,16 +900,9 @@ __device__ __forceinline__ void finalize_body(const TE* __restrict__ E, const fl
   float* sS = sU + (size_t)M * Dp;           // [Dp] column sums of E, later sum_i du
   float* sB = sS + Dp;                       // [Dp] dc_j / M
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-  const bool vec_e = is_vec(E, D), vec_g = is_vec(dE_hat, D), vec_o = is_vec(dE, D);
+  const bool vec_g = is_vec(dE_hat, D), vec_o = is_vec(dE, D);
 
-  if (!REUSE_E) {
-    for (int v = tid; v < M * (Dp >> 2); v += kThreads) {
-      const int i = v / (Dp >> 2), col = (v % (Dp >> 2)) << 2;
-      *reinterpret_cast<float4*>(&sE[(size_t)i * Dp + col]) =
-          ld4e(E + phys_row(idx, (size_t)j * M + i) * D, col, D, vec_e);
-    }
-    __syncthreads();
-  }
+  if (!REUSE_E) stage_rows(E, idx, j, M, D, Dp, sE);
   for (int d = tid; d < Dp; d += kThreads) {
     float s = 0.f;
     for (int i = 0; i < M; ++i) s += sE[(size_t)i * Dp + d];
@@ -1587,6 +1587,15 @@ int simt_bwd_finalize(const void* E, int e_dt, const int32_t* row_index, const f
 //   3  dC_hat_j = sum over speakers of their contribution to centroid j (fixed order:
 //      deterministic); finalize_body: diagonal term, Jacobians, fan-out -> dE
 // Same arithmetic as the pipeline's kernels (shared bodies / helpers), fp32 throughout.
+//
+// Per-utterance losses (reduction "none") learn their upstream gradient g_r only after the forward, so the same
+// kernel also runs cut at the seam between the row losses and w G, as two launches (PART):
+//   kSmallFwd  1, barrier, 2 up to the row losses: row_stat / row_aux / row_kstar, per_row, loss
+//   kSmallBwd  the raw rows re-read; e_hat, c_hat, cos_diag loaded; the cosine block recomputed with the
+//              forward's arithmetic (the staged forward stores no cosines either, so both forwards pair with this
+//              backward); w G from g_r and the stored row statistics, as the staged kernels form it; rest of 2,
+//              barrier, 3.  Its dC_hat rows and {dw, db} are cleared at entry and first added to after the cosine
+//              block: one arrival there, its wait in front of the first add.
 // ------------------------------------------------------------------------------------------
 namespace {
 
@@ -1610,6 +1619,7 @@ struct SmallParams {
   int cluster;                      // the grid is ONE thread-block cluster (N <= 8): hardware barriers
   unsigned* ctr;                    // workspace header: {barrier arrivals, exits}; zero on entry, restored
   float* part;                      // workspace: [N][N][D] centroid contributions
+  const float* grad_rows;           // kSmallBwd: upstream gradient per logical utterance row (grad_out unused)
 };
 
 __device__ __forceinline__ unsigned ld_acquire_u32(const unsigned* p) {
@@ -1618,12 +1628,14 @@ __device__ __forceinline__ unsigned ld_acquire_u32(const unsigned* p) {
   return v;
 }
 
-// every CTA of the grid arrives; `target` = arrivals expected so far (monotonic counter)
-__device__ __forceinline__ void small_grid_barrier(unsigned* ctr, unsigned target) {
-  __syncthreads();
+// small_grid_barrier in two halves: after a __syncthreads, thread 0 arrives; release: the block's writes (ordered
+// before this thread by the bar.sync) become visible with the arrival
+__device__ __forceinline__ void small_grid_arrive(unsigned* ctr) {
+  if (threadIdx.x == 0) asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(ctr) : "memory");
+}
+// `target` = arrivals expected so far (monotonic counter)
+__device__ __forceinline__ void small_grid_wait(const unsigned* ctr, unsigned target) {
   if (threadIdx.x == 0) {
-    // release: the block's writes (ordered before this thread by the bar.sync) become visible with the arrival
-    asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(ctr) : "memory");
     unsigned long long t0 = 0;
     for (unsigned spins = 0; ld_acquire_u32(ctr) < target; ++spins) {
       if ((spins & 1023u) == 1023u) {               // a missing CTA is a bug: trap instead of hanging the GPU
@@ -1635,6 +1647,13 @@ __device__ __forceinline__ void small_grid_barrier(unsigned* ctr, unsigned targe
     }
   }
   __syncthreads();
+}
+
+// every CTA of the grid arrives
+__device__ __forceinline__ void small_grid_barrier(unsigned* ctr, unsigned target) {
+  __syncthreads();
+  small_grid_arrive(ctr);
+  small_grid_wait(ctr, target);
 }
 
 // 4 floats of a row that another CTA wrote earlier in this kernel: L2 load (never the L1), tail-safe
@@ -1653,7 +1672,8 @@ __device__ __forceinline__ float4 ld4_cg(const float* row, int col, int D, bool 
 // MR = M rounded up to a multiple of 4: the cosine block's loops over the speaker's rows are fully
 // unrolled without predicates (rows M..MR-1 of the staged e_hat are zero), so the shared-memory loads of
 // all rows are issued together instead of one load -> use chain per row.
-template <int VARIANT, int MR, typename TE, typename TD>
+// PART: kSmallWhole, or one half of the step (kSmallFwd / kSmallBwd, see above)
+template <int VARIANT, int MR, typename TE, typename TD, int PART>
 __global__ void __launch_bounds__(kThreads, 1)
 small_step_kernel(const SmallParams p) {
   const TE* E = static_cast<const TE*>(p.E);
@@ -1664,6 +1684,7 @@ small_step_kernel(const SmallParams p) {
   __shared__ __align__(8) unsigned long long s_bar;   // bulk-copy completion (stage 2 operands)
   __shared__ float3 s_rsum[16];                       // fast path: |e|^2, |s - e|^2, e.(s - e) per row of the speaker
   __shared__ float s_aux[16];                         // fast path: 1 - p_jj per row
+  __shared__ float s_gr[16];                          // kSmallBwd, fast path: g_r per row
   constexpr int R4 = MR / 4;                          // rows per thread where the block splits into 4 row groups
   const int j = blockIdx.x, N = gridDim.x, M = p.M, D = p.D, Dp = p.Dp;
   const int Np = (N + 3) & ~3;
@@ -1684,13 +1705,13 @@ small_step_kernel(const SmallParams p) {
   const float w = __ldg(p.w), b = __ldg(p.b), eps = p.eps;
   const float g = p.grad_out != nullptr ? __ldg(p.grad_out) : 1.f;
   if (j == 0 && tid < 4) {
-    p.loss_accum[tid] = 0.f;                          // {loss, -, -, -} as prep does
-    if (tid < 2) p.dwdb[tid] = 0.f;
+    if (PART != kSmallBwd) p.loss_accum[tid] = 0.f;   // {loss, -, -, -} as prep does
+    if (PART != kSmallFwd && tid < 2) p.dwdb[tid] = 0.f;
   }
   // 16-byte rows: the centroid gradient is assembled at the L2 -- every CTA adds its [N][D] share with ONE bulk
   // reduce-add, into rows their owners cleared before the first grid barrier (otherwise: workspace + gather)
   const bool dc_at_l2 = (Dp == D) && is_vec(p.dC_hat, D);
-  if (dc_at_l2)
+  if (PART != kSmallFwd && dc_at_l2)
     for (int d = tid; d < D; d += kThreads) p.dC_hat[(size_t)j * D + d] = 0.f;
 
   // ---- 1: this speaker's rows
@@ -1731,7 +1752,7 @@ small_step_kernel(const SmallParams p) {
     for (int q = 0; q < kWarps; ++q) s_norm2 += red[q];
     if (tid < D) {                                     // D <= 256 = block size: one centroid entry per thread
       s_mine = fS[tid];
-      p.c_hat[(size_t)j * D + tid] = s_mine * centroid_scale(s_norm2, inv_m);
+      if (PART != kSmallBwd) p.c_hat[(size_t)j * D + tid] = s_mine * centroid_scale(s_norm2, inv_m);
     }
     const bool act = hw < M;
     float ne2 = 0.f, nd2 = 0.f, ed = 0.f;
@@ -1748,7 +1769,8 @@ small_step_kernel(const SmallParams p) {
       nd2 += __shfl_xor_sync(0xffffffffu, nd2, o);
       ed += __shfl_xor_sync(0xffffffffu, ed, o);
     }
-    if (act) {
+    if (PART == kSmallBwd && act && hl == 0) s_rsum[hw] = make_float3(ne2, nd2, ed);   // for the Jacobians only
+    if (PART != kSmallBwd && act) {
       const RowNorms n = row_norms(ne2, nd2, ed, inv_m1);
       float4* gdst = reinterpret_cast<float4*>(p.e_hat + ((size_t)j * M + hw) * D);
       for (int c4 = hl; c4 < ncol4; c4 += 16) {
@@ -1759,6 +1781,8 @@ small_step_kernel(const SmallParams p) {
       }
       if (hl == 0) { s_cd[hw] = n.cos; p.cos_diag[(size_t)j * M + hw] = n.cos; s_rsum[hw] = make_float3(ne2, nd2, ed); }
     }
+  } else if (PART == kSmallBwd) {
+    stage_rows(E, p.idx, j, M, D, Dp, sA);            // the raw rows for finalize_body (stage 3)
   } else {
     prep_body<false>(E, p.idx, j, M, D, Dp, p.e_hat, p.c_hat, p.cos_diag, sA);
   }
@@ -1769,14 +1793,17 @@ small_step_kernel(const SmallParams p) {
   asm volatile("fence.proxy.async;" ::: "memory");
   // up to 8 speakers the whole grid is one thread-block cluster: barrier.cluster (release / acquire at cluster
   // scope) instead of an arrival counter polled through the L2
-  if (p.cluster) { __syncthreads(); ptx::cluster_sync_all(); } else small_grid_barrier(p.ctr, (unsigned)N);
+  if (PART == kSmallBwd) {                            // cleared dC_hat rows / {dw, db}: waited for before the adds
+    __syncthreads();
+    if (p.cluster) ptx::cluster_arrive(); else small_grid_arrive(p.ctr);
+  } else if (p.cluster) { __syncthreads(); ptx::cluster_sync_all(); } else small_grid_barrier(p.ctr, (unsigned)N);
   GE2E_SMALL_STAMP(2);
   if (p.stop == 2) break;
 
   // ---- 2: M x N block of the similarity matrix
   const bool vec_c = is_vec(p.c_hat, D), vec_e = is_vec(p.e_hat, D);
   for (int v = tid; v < (MR - M) * Np; v += kThreads) sG[M * Np + v] = 0.f;    // padding rows of w G: read, never NaN
-  if (fast) {
+  if (fast && PART != kSmallBwd) {
     // 16 bytes per cp.async, all of a thread's copies in flight together (a warp takes rows wid, wid + 8, ...):
     // one L2 round trip for the whole centroid matrix; stage 1 left e_hat in sEh and the cosines in s_cd
     for (int k = wid; k < N; k += kWarps) {
@@ -1873,6 +1900,7 @@ small_step_kernel(const SmallParams p) {
     const int r = j * M + i;
     const float cd = sCos[i * Np + j];
     const float Sd = fmaf(w, cd, b);                                                  // s3:27
+    const float gr = PART == kSmallBwd ? __ldg(p.grad_rows + r) : g;                 // upstream gradient of the row
     float per, stat, aux = 0.f, dw_i = 0.f, db_i = 0.f;
     int ks = -1;
     if (VARIANT == GE2E_SOFTMAX) {
@@ -1893,60 +1921,75 @@ small_step_kernel(const SmallParams p) {
 #pragma unroll
       for (int q = 0; q < kPer; ++q) { ex[q] = expf(ex[q] - mx); l += ex[q]; }      // exp(-inf) = 0 off the row
       const float loff = warp_sum(l);
-      close_softmax_row(mx, loff, Sd, eps, stat, aux, per);                          // s3:120-121
-      const float sc = g * expf(mx - stat);             // G_k = g exp(S_k - stat) = sc exp(S_k - mx)
-      float dwl = 0.f;
+      if (PART == kSmallBwd) { stat = __ldg(p.row_stat + r); aux = __ldg(p.row_aux + r); per = 0.f; }   // the forward's
+      else close_softmax_row(mx, loff, Sd, eps, stat, aux, per);                     // s3:120-121
+      if (PART != kSmallFwd) {
+        const float sc = gr * expf(mx - stat);          // G_k = g exp(S_k - stat) = sc exp(S_k - mx)
+        float dwl = 0.f;
 #pragma unroll
-      for (int q = 0; q < kPer; ++q) {
-        const int k = lane + 32 * q;
-        const float G = sc * ex[q];
-        dwl = fmaf(G, cosv[q], dwl);
-        if (k < N) sG[i * Np + k] = w * G;              // zero on the own-speaker column
+        for (int q = 0; q < kPer; ++q) {
+          const int k = lane + 32 * q;
+          const float G = sc * ex[q];
+          dwl = fmaf(G, cosv[q], dwl);
+          if (k < N) sG[i * Np + k] = w * G;            // zero on the own-speaker column
+        }
+        dw_i = warp_sum(dwl) - gr * aux * cd;           // own speaker: G = g (p_jj - 1) = -g aux
+        db_i = -gr * eps * expf(-stat);                 // closed form (SURVEY 8(a-bis) item 12)
       }
-      dw_i = warp_sum(dwl) - g * aux * cd;            // own speaker: G = g (p_jj - 1) = -g aux
-      db_i = -g * eps * expf(-stat);                  // closed form (SURVEY 8(a-bis) item 12)
     } else {
       float bv = -INFINITY; int bk = INT_MAX;
-      for (int k = lane; k < N; k += 32)
-        if (k != j) {
-          const float S = fmaf(w, sCos[i * Np + k], b);
-          if (S > bv) { bv = S; bk = k; }
-        }
+      if (PART == kSmallBwd) {                          // the forward's arg-max and its logit
+        bv = __ldg(p.row_stat + r);
+        const int k = __ldg(p.row_kstar + r);
+        if (k >= 0) bk = k;
+      } else {
+        for (int k = lane; k < N; k += 32)
+          if (k != j) {
+            const float S = fmaf(w, sCos[i * Np + k], b);
+            if (S > bv) { bv = S; bk = k; }
+          }
 #pragma unroll
-      for (int o = 16; o > 0; o >>= 1) {
-        const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
-        const int ok = __shfl_xor_sync(0xffffffffu, bk, o);
-        if (ov > bv || (ov == bv && ok < bk)) { bv = ov; bk = ok; }
+        for (int o = 16; o > 0; o >>= 1) {
+          const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+          const int ok = __shfl_xor_sync(0xffffffffu, bk, o);
+          if (ov > bv || (ov == bv && ok < bk)) { bv = ov; bk = ok; }
+        }
       }
       const float sp = 1.f / (1.f + expf(-Sd));
       per = 1.f - sp;
       stat = bv;
-      const float Gp = -g * sp * (1.f - sp);
+      const float Gp = -gr * sp * (1.f - sp);
       float Gn = 0.f, cn = 0.f;
       if (bk != INT_MAX) {
         ks = bk;
         const float sn = 1.f / (1.f + expf(-bv));
         per += sn;
-        Gn = g * sn * (1.f - sn);
+        Gn = gr * sn * (1.f - sn);
         cn = sCos[i * Np + bk];
       }
-      for (int k = lane; k < N; k += 32) sG[i * Np + k] = (k == ks) ? w * Gn : 0.f;
-      dw_i = Gp * cd + Gn * cn;
-      db_i = Gp + Gn;
+      if (PART != kSmallFwd) {
+        for (int k = lane; k < N; k += 32) sG[i * Np + k] = (k == ks) ? w * Gn : 0.f;
+        dw_i = Gp * cd + Gn * cn;
+        db_i = Gp + Gn;
+      }
     }
     if (lane == 0) {
-      p.row_stat[r] = stat;
-      p.row_aux[r] = aux;
+      if (PART != kSmallBwd) p.row_stat[r] = stat;
+      if (PART == kSmallWhole || (PART == kSmallFwd && p.row_aux != nullptr)) p.row_aux[r] = aux;
       s_aux[i] = aux;
-      if (VARIANT == GE2E_CONTRAST && p.row_kstar != nullptr) p.row_kstar[r] = ks;
-      if (p.per_row != nullptr) p.per_row[r] = per;
+      if (PART == kSmallBwd) s_gr[i] = gr;
+      if (PART != kSmallBwd && VARIANT == GE2E_CONTRAST && p.row_kstar != nullptr) p.row_kstar[r] = ks;
+      if (PART != kSmallBwd && p.per_row != nullptr) p.per_row[r] = per;
       loss_part += per; dw_part += dw_i; db_part += db_i;
     }
+  }
+  if (PART == kSmallBwd) {                             // every CTA has cleared its dC_hat row, CTA 0 {dw, db}
+    if (p.cluster) ptx::cluster_wait(); else small_grid_wait(p.ctr, (unsigned)N);
   }
   // lane 0 of every warp holds its rows' {loss, dw, db}: one round through shared memory
   if (lane == 0) { red[wid] = loss_part; red[kWarps + wid] = dw_part; red[2 * kWarps + wid] = db_part; }
   __syncthreads();                                     // sG complete, partial sums staged
-  if (tid < 3) {
+  if (tid < 3 && (PART == kSmallWhole || (PART == kSmallFwd) == (tid == 0))) {
     float t = 0.f;
 #pragma unroll
     for (int q = 0; q < kWarps; ++q) t += red[tid * kWarps + q];
@@ -1954,6 +1997,7 @@ small_step_kernel(const SmallParams p) {
   }
   GE2E_SMALL_STAMP(5);
   if (p.stop == 4) break;
+  if (PART == kSmallFwd) break;
   const bool vec_g = is_vec(p.dE_hat, D), vec_p = is_vec(p.part, D);
   {
     // thread <-> (float4 column c4 of 64, group of 4): dE_hat rows rg, rg + 4, ... = (wG) C_hat, then this speaker's
@@ -2052,7 +2096,8 @@ small_step_kernel(const SmallParams p) {
 #pragma unroll
         for (int o = 8; o > 0; o >>= 1) eg += __shfl_xor_sync(0xffffffffu, eg, o);
         if (act) {
-          const float dd = diag_term(VARIANT, g, VARIANT == GE2E_SOFTMAX ? s_aux[hw] : s_cd[hw], w, b, eps);
+          const float dd = diag_term(VARIANT, PART == kSmallBwd ? s_gr[hw] : g,
+                                     VARIANT == GE2E_SOFTMAX ? s_aux[hw] : s_cd[hw], w, b, eps);
           const float3 rs = s_rsum[hw];
           const RowJacobian J = row_jacobian(row_norms(rs.x, rs.y, rs.z, inv_m1), eg, 1.f, dd, inv_m1);
           for (int c4 = hl; c4 < ncol4; c4 += 16) {
@@ -2152,6 +2197,9 @@ small_step_kernel(const SmallParams p) {
         st4v(dst + 4 * c4, o);
       }
     }
+  } else if (PART == kSmallBwd) {
+    finalize_body<true, TE, TD, true>(E, p.dE_hat, p.dC_hat, p.cos_diag, p.row_stat, p.row_aux, nullptr, j, M, D, Dp,
+                                      w, b, 0.f, eps, VARIANT, dE, p.idx, sA, p.grad_rows);   // sA: stage_rows
   } else {
     finalize_body<true>(E, p.dE_hat, p.dC_hat, p.cos_diag, p.row_stat, p.row_aux, nullptr, j, M, D, Dp, w, b, g, eps,
                         VARIANT, dE, p.idx, sA);      // sA still holds the raw rows prep_body staged
@@ -2200,20 +2248,20 @@ size_t small_step_workspace_bytes(int N, int M, int D) {
   return small_step_supported(N, M, D) ? kSmallHeaderBytes + (size_t)N * N * D * sizeof(float) : 0;
 }
 
-int simt_small_step(const void* E, int e_dt, const int32_t* row_index, int N, int M, int D, const float* w,
-                    const float* b, float eps, int variant, const float* grad_out, float* e_hat, float* c_hat,
-                    float* cos_diag, float* row_stat, int32_t* row_kstar, float* row_aux, float* per_row,
+int simt_small_step(int part, const void* E, int e_dt, const int32_t* row_index, int N, int M, int D, const float* w,
+                    const float* b, float eps, int variant, const float* grad_out, const float* grad_rows, float* e_hat,
+                    float* c_hat, float* cos_diag, float* row_stat, int32_t* row_kstar, float* row_aux, float* per_row,
                     float* loss_accum, float* dE_hat, float* dC_hat, float* dwdb, void* dE, int de_dt, void* workspace,
                     cudaStream_t st) {
   SmallParams p;
   p.E = E; p.idx = row_index; p.M = M; p.D = D; p.Dp = (D + 3) & ~3;
-  p.w = w; p.b = b; p.eps = eps; p.grad_out = grad_out;
+  p.w = w; p.b = b; p.eps = eps; p.grad_out = grad_out; p.grad_rows = grad_rows;
   p.e_hat = e_hat; p.c_hat = c_hat; p.cos_diag = cos_diag; p.row_stat = row_stat; p.row_kstar = row_kstar;
   p.row_aux = row_aux; p.per_row = per_row; p.loss_accum = loss_accum;
   p.dE_hat = dE_hat; p.dC_hat = dC_hat; p.dwdb = dwdb; p.dE = dE;
 #ifdef GE2E_DEBUG_BUILD      // scripts/small_step_trace.py builds its own library with -DGE2E_DEBUG_BUILD
   static const int stop = [] { const char* e = getenv("GE2E_SMALL_STOP"); return e ? atoi(e) : 0; }();
-  p.stop = stop;
+  p.stop = part == kSmallWhole ? stop : 0;
 #else
   p.stop = 0;
 #endif
@@ -2222,9 +2270,13 @@ int simt_small_step(const void* E, int e_dt, const int32_t* row_index, int N, in
   const size_t smem = small_smem_bytes(N, M, D);
   // N <= 8 (the portable cluster size): the N CTAs form one cluster
   p.cluster = N <= 8 ? 1 : 0;
+  // the forward half stores no dE: one instantiation per E type
 #define GE2E_SMALL_LAUNCH(V, R)                                                                   \
   do {                                                                                            \
-    int rc = set_smem(small_step_kernel<V, R, TE, TD>, smem);                                     \
+    auto kern = part == kSmallFwd ? small_step_kernel<V, R, TE, float, kSmallFwd>                 \
+              : part == kSmallBwd ? small_step_kernel<V, R, TE, TD, kSmallBwd>                    \
+                                  : small_step_kernel<V, R, TE, TD, kSmallWhole>;                 \
+    int rc = set_smem(kern, smem);                                                                \
     if (rc != GE2E_OK) return rc;                                                                 \
     cudaLaunchConfig_t cfg{};                                                                     \
     cfg.gridDim = dim3(N); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = smem; cfg.stream = st; \
@@ -2234,7 +2286,7 @@ int simt_small_step(const void* E, int e_dt, const int32_t* row_index, int N, in
     at[1].id = cudaLaunchAttributeClusterDimension;                                               \
     at[1].val.clusterDim.x = N; at[1].val.clusterDim.y = 1; at[1].val.clusterDim.z = 1;           \
     cfg.attrs = at; cfg.numAttrs = p.cluster ? 2 : 1;                                             \
-    GE2E_CUDA_TRY(cudaLaunchKernelEx(&cfg, small_step_kernel<V, R, TE, TD>, p));                  \
+    GE2E_CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, p));                                             \
   } while (0)
   const int mr = (M + 3) & ~3;
   const int rc = with_e_de_types(e_dt, de_dt, [&](auto te, auto td) -> int {

@@ -101,9 +101,12 @@ def _cached_workspace(nbytes: int, device, dev_index: int, stream: int) -> Optio
     return ws
 
 
-def _workspace(n_local: int, n_total: int, M: int, D: int, variant: int, precision: int, device):
-    """(workspace, its size) for fwd_rows / bwd_rows and the custom ops, on the current stream."""
+def _workspace(n_local: int, n_total: int, M: int, D: int, variant: int, precision: int, device, per_row: bool = False):
+    """(workspace, its size) for fwd_rows / bwd_rows and the custom ops, on the current stream.  ``per_row``: also
+    large enough for the per-utterance halves of the single-kernel step (what the eager module runs)."""
     nbytes = lib().ge2e_b200_workspace_bytes(n_local, n_total, M, D, variant, precision)
+    if per_row:
+        nbytes = max(nbytes, lib().ge2e_b200_step_workspace_bytes(n_total, M, D, variant, precision))
     index = device.index if device.index is not None else torch.cuda.current_device()
     return _cached_workspace(nbytes, device, index, torch.cuda.current_stream(device).cuda_stream), nbytes
 
@@ -167,7 +170,7 @@ def _fwd_impl(E: Tensor, w: Tensor, b: Tensor, eps: float, variant: int, precisi
         row_scale = torch.empty(U if fused else 1, dtype=torch.float32, device=dev)
         row_kstar = torch.empty(U if variant == _lib.CONTRAST else 1, dtype=torch.int32, device=dev)
         per = torch.empty((N, M), dtype=torch.float32, device=dev) if per_row else None
-        ws, ws_bytes = _workspace(N, N, M, D, variant, precision, dev)
+        ws, ws_bytes = _workspace(N, N, M, D, variant, precision, dev, per_row)
         _forward(per, E.data_ptr(), ecode, None, N, M, D, w.data_ptr(), b.data_ptr(), eps, variant, precision,
                  e_hat.data_ptr(), c_hat.data_ptr(), cos_diag.data_ptr(), row_stat.data_ptr(), row_kstar.data_ptr(),
                  row_aux.data_ptr(), accum.data_ptr(), dE_hat.data_ptr() if fused else None,
@@ -195,7 +198,7 @@ def _bwd_impl(grad_out, E, w, b, e_hat, c_hat, cos_diag, row_stat, row_kstar, ro
         scratch = torch.empty(4 + N * D + (0 if fused else U * D), dtype=torch.float32, device=dev)
         dC_ptr = scratch.data_ptr() + 16
         dE_hat_ptr = dE_hat.data_ptr() if fused else dC_ptr + N * D * 4
-        ws, ws_bytes = _workspace(N, N, M, D, variant, precision, dev)
+        ws, ws_bytes = _workspace(N, N, M, D, variant, precision, dev, per_row)
         if per_row and g.numel() != U:
             raise ValueError(f"the upstream gradient of the per-utterance losses needs {U} entries, got {g.numel()}")
         entry = lib().ge2e_b200_backward_per_row_typed if per_row else lib().ge2e_b200_backward_typed

@@ -17,13 +17,22 @@ from .ops import _DTYPES
 
 class GE2EPlan:
     def __init__(self, N: int, M: int, D: int, variant: str = "softmax", precision: str = "fp32",
-                 eps: float = 1e-6, device=None, sgd=None, dtype: torch.dtype = torch.float32):
+                 eps: float = 1e-6, device=None, sgd=None, dtype: torch.dtype = torch.float32, reduction: str = "sum"):
         """``sgd=(lr, max_norm)``: every step ends with the trainer's tail for the two loss parameters
         (clip_grad_norm_ on (w, b) + plain SGD, s4_train_embed_model.py:202-203) as one more kernel,
         updating the ``w`` / ``b`` passed to ``step`` in place.  ``dtype``: element type of the embeddings
-        ``step`` takes (float32, bfloat16 or float16); ``.dE`` has it too, everything else is float32."""
+        ``step`` takes (float32, bfloat16 or float16); ``.dE`` has it too, everything else is float32.
+
+        ``reduction="none"``: per-utterance losses.  The forward writes ``.per_row`` ([N, M] float32, logical
+        order; ``.loss`` is their sum) and the backward (``backward()``) differentiates sum_r grad_rows[r] L_r with
+        ``.grad_rows`` ([N, M] float32, initialised to ones), read when the backward runs -- so a caller can
+        weight or mask utterances from ``per_row`` on the device between a captured forward and a captured
+        backward.  On the single-kernel step's shapes each half is one kernel."""
         if dtype not in _DTYPES:
             raise TypeError(f"dtype must be float32, bfloat16 or float16, got {dtype}")
+        if reduction not in ("sum", "none"):
+            raise ValueError(f"GE2EPlan reduction must be 'sum' or 'none', got {reduction!r}")
+        self.reduction = reduction
         self.dtype, self._dtype_code = dtype, _DTYPES[dtype]
         self.sgd = None if sgd is None else (float(sgd[0]), float(sgd[1]))
         if M < 2:
@@ -59,9 +68,16 @@ class GE2EPlan:
         self._ws_bytes = nbytes
         self.loss, self.dw, self.db = self._accum[0], self._accum[1], self._accum[2]
         self._graph = None
+        if reduction == "none":
+            self.per_row = torch.empty((N, M), dtype=f32, device=dev)
+            self.grad_rows = torch.ones((N, M), dtype=f32, device=dev)
+            # tensor-core softmax: the forward also leaves the un-normalised dE_hat rows + row_scale
+            self._scaled = _lib.prepares_dE_hat(N, N, M, D, self.variant, self.precision)
+        self._fwd_E = None      # data_ptr of the last forward's E (reduction="none": what backward() differentiates)
 
     def step(self, E: torch.Tensor, w: torch.Tensor, b: torch.Tensor, backward: bool = True) -> None:
-        """Enqueue fwd (+ bwd) on the current stream.  Results land in .loss/.dE/.dw/.db."""
+        """Enqueue fwd (+ bwd) on the current stream.  Results land in .loss/.dE/.dw/.db (and .per_row with
+        reduction="none", whose backward is ``backward()``)."""
         if E.dtype != self.dtype:
             raise TypeError(f"GE2EPlan was built for {self.dtype} embeddings, got {E.dtype}")
         assert E.is_cuda and E.is_contiguous() and tuple(E.shape) == (self.N, self.M, self.D)
@@ -75,6 +91,18 @@ class GE2EPlan:
             _lib.check_backward_shape(M, D)
         stream = torch.cuda.current_stream(self.device).cuda_stream
         ws = self._ws.data_ptr() if self._ws_bytes else None
+        if self.reduction == "none":
+            rc = h.ge2e_b200_forward_per_row_typed(
+                E.data_ptr(), dt, None, N, M, D, w.data_ptr(), b.data_ptr(), self.eps, self.variant, self.precision,
+                self.e_hat.data_ptr(), self.c_hat.data_ptr(), self.cos_diag.data_ptr(), self.row_stat.data_ptr(),
+                self.row_kstar.data_ptr(), self.row_aux.data_ptr(), self._accum.data_ptr(),
+                self.dE_hat.data_ptr() if self._scaled else None, self.row_scale.data_ptr() if self._scaled else None,
+                self.per_row.data_ptr(), ws, self._ws_bytes, stream)
+            check(rc, "ge2e_b200_forward_per_row_typed")
+            self._fwd_E = E.data_ptr()
+            if backward:
+                self.backward(E, w, b)
+            return
         if backward:
             accum_ptr = self._accum.data_ptr()
             rc = h.ge2e_b200_forward_backward_typed(E.data_ptr(), dt, None, N, M, D, w.data_ptr(), b.data_ptr(),
@@ -86,10 +114,7 @@ class GE2EPlan:
                                                     self.dC_hat.data_ptr(), self.dE.data_ptr(), dt, ws, self._ws_bytes,
                                                     stream)
             check(rc, "ge2e_b200_forward_backward_typed")
-            if self.sgd is not None:
-                rc = h.ge2e_b200_scale_bias_sgd(w.data_ptr(), b.data_ptr(), accum_ptr + 4, accum_ptr + 8, self.sgd[1],
-                                                self.sgd[0], None, stream)
-                check(rc, "ge2e_b200_scale_bias_sgd")
+            self._sgd_tail(w, b, stream)
             return
         rc = h.ge2e_b200_forward_typed(E.data_ptr(), dt, None, N, M, D, w.data_ptr(), b.data_ptr(), self.eps,
                                        self.variant, self.precision, self.e_hat.data_ptr(), self.c_hat.data_ptr(),
@@ -98,24 +123,67 @@ class GE2EPlan:
                                        stream)
         check(rc, "ge2e_b200_forward_typed")
 
-    def capture(self, E, w: torch.Tensor, b: torch.Tensor, backward: bool = True, steps: int = 1):
-        """Capture ``steps`` consecutive steps into one CUDA graph bound to these tensors; returns the
-        graph (``.replay()``).  ``E`` is one batch or a list of batches the steps rotate over.  Also
-        records how many of the library's kernels one step launches."""
-        batches = list(E) if isinstance(E, (list, tuple)) else [E]
+    def _sgd_tail(self, w: torch.Tensor, b: torch.Tensor, stream: int) -> None:
+        if self.sgd is not None:
+            accum_ptr = self._accum.data_ptr()
+            rc = lib().ge2e_b200_scale_bias_sgd(w.data_ptr(), b.data_ptr(), accum_ptr + 4, accum_ptr + 8, self.sgd[1],
+                                                self.sgd[0], None, stream)
+            check(rc, "ge2e_b200_scale_bias_sgd")
+
+    def backward(self, E: torch.Tensor, w: torch.Tensor, b: torch.Tensor) -> None:
+        """reduction="none": enqueue the backward of the last forward (``step(E, w, b, backward=False)``) for the
+        upstream gradient ``.grad_rows`` on the current stream, then the ``sgd=`` tail.  ``E`` is that forward's
+        batch.  Results land in .dE/.dw/.db."""
+        if self.reduction != "none":
+            raise RuntimeError("GE2EPlan.backward() is the per-utterance backward of a reduction='none' plan; "
+                               "a 'sum' plan runs its backward inside step()")
+        if self._fwd_E is None:
+            raise RuntimeError("GE2EPlan.backward() before any forward: call step(E, w, b, backward=False) first")
+        if E.data_ptr() != self._fwd_E:
+            raise ValueError("GE2EPlan.backward() takes the E of the last forward")
+        if not self._bwd_ok:
+            _lib.check_backward_shape(self.M, self.D)
+        N, M, D, dt = self.N, self.M, self.D, self._dtype_code
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        ws = self._ws.data_ptr() if self._ws_bytes else None
+        rc = lib().ge2e_b200_backward_per_row_typed(
+            E.data_ptr(), dt, None, self.e_hat.data_ptr(), self.c_hat.data_ptr(), self.cos_diag.data_ptr(),
+            self.row_stat.data_ptr(), self.row_kstar.data_ptr(), self.row_aux.data_ptr(),
+            self.row_scale.data_ptr() if self._scaled else None, N, M, D, w.data_ptr(), b.data_ptr(), self.eps,
+            self.variant, self.precision, self.grad_rows.data_ptr(), self.dE_hat.data_ptr(), self.dC_hat.data_ptr(),
+            self._accum.data_ptr(), self.dE.data_ptr(), dt, ws, self._ws_bytes, stream)
+        check(rc, "ge2e_b200_backward_per_row_typed")
+        self._sgd_tail(w, b, stream)
+
+    def _capture(self, enqueue, steps: int):
+        """(graph of ``steps`` calls enqueue(k), library launches per call); one eager call first as warm-up."""
         with torch.cuda.device(self.device):
             side = torch.cuda.Stream()
             side.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(side):
-                self.step(batches[0], w, b, backward)   # warm-up: lazy func attributes, module load
+                enqueue(0)                              # warm-up: lazy func attributes, module load
             torch.cuda.current_stream().wait_stream(side)
             torch.cuda.synchronize()
             g = torch.cuda.CUDAGraph()
             before = lib().ge2e_b200_launch_count()
             with torch.cuda.graph(g):
                 for k in range(steps):
-                    self.step(batches[k % len(batches)], w, b, backward)
-            self.launches_per_step = (lib().ge2e_b200_launch_count() - before) // max(1, steps)
+                    enqueue(k)
+            return g, (lib().ge2e_b200_launch_count() - before) // max(1, steps)
+
+    def capture_backward(self, E: torch.Tensor, w: torch.Tensor, b: torch.Tensor):
+        """reduction="none": ``backward(E, w, b)`` as a CUDA graph of its own (``.replay()``), to replay after a
+        forward graph (``capture(E, w, b, backward=False)``) with ``grad_rows`` set in between.  Records the
+        library kernels it launches in ``backward_launches``."""
+        g, self.backward_launches = self._capture(lambda k: self.backward(E, w, b), 1)
+        return g
+
+    def capture(self, E, w: torch.Tensor, b: torch.Tensor, backward: bool = True, steps: int = 1):
+        """Capture ``steps`` consecutive steps into one CUDA graph bound to these tensors; returns the
+        graph (``.replay()``).  ``E`` is one batch or a list of batches the steps rotate over.  Also
+        records how many of the library's kernels one step launches."""
+        batches = list(E) if isinstance(E, (list, tuple)) else [E]
+        g, self.launches_per_step = self._capture(lambda k: self.step(batches[k % len(batches)], w, b, backward), steps)
         self._graph = g
         return g
 
