@@ -2040,19 +2040,11 @@ int tc_step(const RowsArgs& a, int phases, const TcRowsBufs& b, void* ws, cudaSt
   const float* op[2] = {a.e_hat, a.c_hat_all};
   const int op_rows[2] = {U, a.n_total};
   const void* op_k[2] = {op[0], op[1]};         // what MMA1 reads K-major
-  if (hyb) {
-    // fp16 copies behind the row sums in the workspace; MMA1 reads them (K-major), MMA2 the fp32 originals (MN-major)
-    uint8_t* e16 = reinterpret_cast<uint8_t*>(p.rowsum) + rowsum_bytes(U);
-    uint8_t* c16 = e16 + f16_copy_bytes(U, a.D);
-    const long long na4 = static_cast<long long>(U) * a.D / 4, nb4 = static_cast<long long>(a.n_total) * a.D / 4;
-    const long long want = (na4 + nb4 + 255) / 256;
-    const unsigned blocks = static_cast<unsigned>(std::min<long long>(want, static_cast<long long>(sm_count()) * 8));
-    GE2E_CUDA_TRY(launch_pdl(to_f16_kernel, dim3(blocks), dim3(256), 0, st, phases != PASS_CENTROIDS,
-                             reinterpret_cast<const float4*>(a.e_hat), reinterpret_cast<uint2*>(e16), na4,
-                             reinterpret_cast<const float4*>(a.c_hat_all), reinterpret_cast<uint2*>(c16), nb4));
-    GE2E_LAUNCHED();
-    op_k[0] = e16; op_k[1] = c16;
-  }
+  // fp16 copies behind the row sums in the workspace; MMA1 reads them (K-major), MMA2 the fp32 originals (MN-major).
+  // The conversion is launched once every tensor map below has been made: a call that fails launches nothing.
+  uint8_t* e16 = reinterpret_cast<uint8_t*>(p.rowsum) + rowsum_bytes(U);
+  uint8_t* c16 = e16 + f16_copy_bytes(U, a.D);
+  if (hyb) { op_k[0] = e16; op_k[1] = c16; }
   // only the map makers differ between the operand encodings (split planes / HYB copies / TF32)
   auto map_k = [&](CUtensorMap* m, const void* base, int rows, int box_rows) {
     if (split) return make_map_h3(m, base, rows, a.D, box_rows);
@@ -2076,10 +2068,17 @@ int tc_step(const RowsArgs& a, int phases, const TcRowsBufs& b, void* ws, cudaSt
     return rc;
   if (peers) {
     p.peer_rows = a.n_total / b.n_ranks;
-    for (int r = 0; r < b.n_ranks; ++r) {
-      if (b.dC_owner[r] == nullptr || (reinterpret_cast<uintptr_t>(b.dC_owner[r]) & 15) != 0) return GE2E_ERR_ARGUMENT;
+    for (int r = 0; r < b.n_ranks; ++r)       // the owner pointers were checked by tc_rows
       if ((rc = make_map_2d(&tms.out_peer[r], b.dC_owner[r], p.peer_rows, a.D, kTile)) != GE2E_OK) return rc;
-    }
+  }
+  if (hyb) {
+    const long long na4 = static_cast<long long>(U) * a.D / 4, nb4 = static_cast<long long>(a.n_total) * a.D / 4;
+    const long long want = (na4 + nb4 + 255) / 256;
+    const unsigned blocks = static_cast<unsigned>(std::min<long long>(want, static_cast<long long>(sm_count()) * 8));
+    GE2E_CUDA_TRY(launch_pdl(to_f16_kernel, dim3(blocks), dim3(256), 0, st, phases != PASS_CENTROIDS,
+                             reinterpret_cast<const float4*>(a.e_hat), reinterpret_cast<uint2*>(e16), na4,
+                             reinterpret_cast<const float4*>(a.c_hat_all), reinterpret_cast<uint2*>(c16), nb4));
+    GE2E_LAUNCHED();
   }
   if (b.grad_rows != nullptr) {     // row-gradient instantiations (no instrumented twins); phases == PASS_CENTROIDS
     if (split)
@@ -2107,6 +2106,9 @@ int tc_rows(const RowsArgs& a, int prec, int phases, const TcRowsBufs& b, void* 
   if (peers && (b.n_ranks > kMaxPeers || a.n_total % b.n_ranks != 0 || (a.n_total / b.n_ranks) % kTile != 0 ||
                 !(phases & PASS_CENTROIDS)))
     return GE2E_ERR_UNSUPPORTED;
+  // every owner block is a TMA destination; checked ahead of the first launch (the split forward, the HYB conversion)
+  for (int r = 0; peers && r < b.n_ranks; ++r)
+    if (b.dC_owner[r] == nullptr || (reinterpret_cast<uintptr_t>(b.dC_owner[r]) & 15) != 0) return GE2E_ERR_ARGUMENT;
   // a per-row upstream gradient is known only after the forward: the centroid pass alone, on one device
   if (b.grad_rows != nullptr && (phases != PASS_CENTROIDS || peers)) return GE2E_ERR_UNSUPPORTED;
   if (ws == nullptr || ws_bytes < tc_workspace_bytes(a.n_local, a.n_total, a.M, a.D, a.variant))
