@@ -473,7 +473,7 @@ int ge2e_b200_forward_backward_typed(const void* E, int e_dtype, const int32_t* 
  * the step.  Otherwise (a workspace of ge2e_b200_workspace_bytes(), every other shape) they run the staged kernels.
  * Both forms leave and read the same forward outputs, so either forward pairs with either backward.  The
  * whole-step-in-forward scheme (ge2e_b200_forward_backward with grad_out = 1, then ge2e_b200_scale_grads) has no
- * per-row form, nor have the speaker-sharded entry points. */
+ * per-row form.  The speaker-sharded forward writes per_row through ge2e_b200_fwd_rows; its backward stages follow. */
 int ge2e_b200_forward_per_row_typed(const void* E, int e_dtype, const int32_t* row_index, int N, int M, int D,
                                     const float* w, const float* b, float eps, int variant, int precision, float* e_hat,
                                     float* c_hat, float* cos_diag, float* row_stat, int32_t* row_kstar, float* row_aux,
@@ -486,6 +486,46 @@ int ge2e_b200_backward_per_row_typed(const void* E, int e_dtype, const int32_t* 
                                      int precision, const float* grad_rows, float* dE_hat, float* dC_hat, float* accum,
                                      void* dE, int de_dtype, void* workspace, size_t workspace_bytes,
                                      ge2e_stream_t stream);
+
+/* Per-utterance losses over speaker shards.  Rank q's objective term is sum_r grad_rows_q[r] L_r over its own rows;
+ * the sum over ranks is differentiated, so dE_local also carries what the other ranks' rows send through this rank's
+ * centroids, and dw / db are global once the ranks' partials are summed.  grad_rows: device, [n_local * M], this
+ * rank's rows in logical [speaker][utterance] order, any values.  NULL grad_rows returns GE2E_ERR_ARGUMENT before
+ * anything is launched.
+ *   ge2e_b200_bwd_rows_per_row             ge2e_b200_bwd_rows with grad_rows in place of grad_out: on the tensor-core
+ *                                          softmax path with the forward's row_scale the lone centroid pass (dC_hat
+ *                                          partial [n_total, D] and this rank's {dw, db}), else the SIMT kernels.
+ *                                          The caller then reduce-scatters dC_hat and all-reduces {dw, db}.
+ *   ge2e_b200_bwd_finalize_per_row_typed   ge2e_b200_bwd_finalize_typed with grad_rows: row r of an un-normalised
+ *                                          dE_hat counts grad_rows[r] * row_scale[r] times; dE in de_dtype.
+ *   ge2e_b200_bwd_rows_peers_per_row       the centroid pass of ge2e_b200_step_rows_peers alone, for grad_rows: every
+ *                                          dC_hat accumulator tile is reduce-added into the owner rank's dC_local
+ *                                          (dC_owner_host, n_ranks as there; the owners cleared their rows before the
+ *                                          cross-rank barrier in front of this call), dwdb_accum[2] receives this
+ *                                          rank's {dw, db} (overwritten).  row_scale (required) says that the
+ *                                          forward (ge2e_b200_fwd_rows with dE_hat + row_scale) prepared dE_hat.
+ *                                          GE2E_ERR_SHAPE for n_ranks outside 2..GE2E_MAX_PEERS or n_local * n_ranks
+ *                                          != n_total; GE2E_ERR_UNSUPPORTED where ge2e_b200_step_rows_peers refuses
+ *                                          (contrast, GE2E_FP32, owner rows not whole 128-row tiles);
+ *                                          GE2E_ERR_ARGUMENT for a NULL or misaligned owner pointer.  Every refusal
+ *                                          returns before anything is launched or written. */
+int ge2e_b200_bwd_rows_per_row(const float* e_hat, const float* c_hat_all, const float* cos_diag,
+                               const float* row_stat, const int32_t* row_kstar, const float* row_aux,
+                               const float* row_scale, int n_local, int n_total, int spk_offset, int M, int D,
+                               const float* w, const float* b, float eps, int variant, int precision,
+                               const float* grad_rows, float* dE_hat, float* dC_hat_partial, float* dwdb_accum,
+                               void* workspace, size_t workspace_bytes, ge2e_stream_t stream);
+int ge2e_b200_bwd_finalize_per_row_typed(const void* E, int e_dtype, const int32_t* row_index, const float* dE_hat,
+                                         const float* dC_hat_local, const float* cos_diag, const float* row_stat,
+                                         const float* row_aux, const float* row_scale, int n_local, int M, int D,
+                                         const float* w, const float* b, float eps, int variant,
+                                         const float* grad_rows, void* dE, int de_dtype, ge2e_stream_t stream);
+int ge2e_b200_bwd_rows_peers_per_row(const float* e_hat, const float* c_hat_all, const float* cos_diag,
+                                     const float* row_stat, const float* row_aux, const float* row_scale, int n_local,
+                                     int n_total, int spk_offset, int M, int D, const float* w, const float* b,
+                                     float eps, int variant, int precision, const float* grad_rows, float* dE_hat,
+                                     float* dwdb_accum, float* const* dC_owner_host, int n_ranks, void* workspace,
+                                     size_t workspace_bytes, ge2e_stream_t stream);
 
 /* ---- static helpers of the reference class (used by s5_eval_model.py:42-43) ----------- */
 

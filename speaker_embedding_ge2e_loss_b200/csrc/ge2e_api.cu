@@ -226,6 +226,18 @@ int ge2e_b200_bwd_rows(const float* e_hat, const float* c_hat_all, const float* 
                        dwdb_accum, workspace, workspace_bytes, stream);
 }
 
+int ge2e_b200_bwd_rows_per_row(const float* e_hat, const float* c_hat_all, const float* cos_diag,
+                               const float* row_stat, const int32_t* row_kstar, const float* row_aux,
+                               const float* row_scale, int n_local, int n_total, int spk_offset, int M, int D,
+                               const float* w, const float* b, float eps, int variant, int precision,
+                               const float* grad_rows, float* dE_hat, float* dC_hat_partial, float* dwdb_accum,
+                               void* workspace, size_t workspace_bytes, ge2e_stream_t stream) {
+  if (!grad_rows) return GE2E_ERR_ARGUMENT;
+  return bwd_rows_impl(e_hat, c_hat_all, cos_diag, row_stat, row_kstar, row_aux, row_scale, n_local, n_total,
+                       spk_offset, M, D, w, b, eps, variant, precision, nullptr, grad_rows, dE_hat, dC_hat_partial,
+                       dwdb_accum, workspace, workspace_bytes, stream);
+}
+
 // grad_rows (nullable): as in bwd_rows_impl, per logical utterance row
 static int bwd_finalize_impl(const void* E, int e_dtype, const int32_t* row_index, const float* dE_hat,
                              const float* dC_hat_local, const float* cos_diag, const float* row_stat,
@@ -250,6 +262,16 @@ int ge2e_b200_bwd_finalize_typed(const void* E, int e_dtype, const int32_t* row_
                                  void* dE, int de_dtype, ge2e_stream_t stream) {
   return bwd_finalize_impl(E, e_dtype, row_index, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux, row_scale, n_local,
                            M, D, w, b, eps, variant, grad_out, nullptr, dE, de_dtype, stream);
+}
+
+int ge2e_b200_bwd_finalize_per_row_typed(const void* E, int e_dtype, const int32_t* row_index, const float* dE_hat,
+                                         const float* dC_hat_local, const float* cos_diag, const float* row_stat,
+                                         const float* row_aux, const float* row_scale, int n_local, int M, int D,
+                                         const float* w, const float* b, float eps, int variant,
+                                         const float* grad_rows, void* dE, int de_dtype, ge2e_stream_t stream) {
+  if (!grad_rows) return GE2E_ERR_ARGUMENT;
+  return bwd_finalize_impl(E, e_dtype, row_index, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux, row_scale, n_local,
+                           M, D, w, b, eps, variant, nullptr, grad_rows, dE, de_dtype, stream);
 }
 
 int ge2e_b200_bwd_finalize_indexed(const float* E, const int32_t* row_index, const float* dE_hat,
@@ -547,6 +569,29 @@ int ge2e_b200_step_rows_peers(const float* e_hat, const float* c_hat_all, const 
   t.grad_out = grad_out; t.row_stat = row_stat; t.row_kstar = row_kstar; t.row_aux = row_aux; t.row_scale = row_scale;
   t.loss_accum = accum; t.dE_hat = dE_hat; t.dwdb = accum + 1; t.dC_owner = dC_owner_host; t.n_ranks = n_ranks;
   return tc_rows(a, tc_prec(precision), 3, t, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+int ge2e_b200_bwd_rows_peers_per_row(const float* e_hat, const float* c_hat_all, const float* cos_diag,
+                                     const float* row_stat, const float* row_aux, const float* row_scale, int n_local,
+                                     int n_total, int spk_offset, int M, int D, const float* w, const float* b,
+                                     float eps, int variant, int precision, const float* grad_rows, float* dE_hat,
+                                     float* dwdb_accum, float* const* dC_owner_host, int n_ranks, void* workspace,
+                                     size_t workspace_bytes, ge2e_stream_t stream) {
+  // row_scale: the forward's rows pass prepared dE_hat, so only the centroid pass remains
+  if (!e_hat || !c_hat_all || !cos_diag || !row_stat || !row_aux || !row_scale || !w || !b || !grad_rows || !dE_hat ||
+      !dwdb_accum || !dC_owner_host)
+    return GE2E_ERR_ARGUMENT;
+  int rc = check_shape(n_local, n_total, spk_offset, M, D);
+  if (rc != GE2E_OK) return rc;
+  if ((rc = check_enum(variant, precision)) != GE2E_OK) return rc;
+  if (n_ranks < 2 || n_ranks > GE2E_MAX_PEERS || n_local * n_ranks != n_total) return GE2E_ERR_SHAPE;
+  if (!tc_softmax_step(n_local, n_total, M, D, variant, precision)) return GE2E_ERR_UNSUPPORTED;
+  RowsArgs a{e_hat, c_hat_all, cos_diag, n_local, n_total, spk_offset, M, D, w, b, eps, variant};
+  TcRowsBufs t;
+  t.grad_rows = grad_rows;
+  t.row_stat = const_cast<float*>(row_stat); t.row_aux = const_cast<float*>(row_aux);   // read by the centroid pass
+  t.dE_hat = dE_hat; t.dwdb = dwdb_accum; t.dC_owner = dC_owner_host; t.n_ranks = n_ranks;
+  return tc_rows(a, tc_prec(precision), 2, t, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 // ---- whole step in one call ---------------------------------------------------------------

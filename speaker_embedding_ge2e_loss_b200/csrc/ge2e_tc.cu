@@ -2033,7 +2033,8 @@ int tc_step(const RowsArgs& a, int phases, const TcRowsBufs& b, void* ws, cudaSt
   // per-utterance-tile pass-1 counters: the forward kernel's stream-K counters (OT = the same U rows), zero on
   // entry and exit of either kernel
   p.seg_done = reinterpret_cast<int*>(static_cast<uint8_t*>(ws) + kWsHeaderBytes);
-  // {dw, db} accumulate: zeroed by prep when the passes run in one step; a lone backward clears them here
+  // {dw, db} accumulate: zeroed by prep when the passes run in one step; a lone backward clears them here (this
+  // rank's partials over peer memory too: the caller exchanges them)
   if (phases == PASS_CENTROIDS) GE2E_CUDA_TRY(cudaMemsetAsync(b.dwdb, 0, 2 * sizeof(float), st));
 
   // the operands: [SEG_DE] utterances, [SEG_DC] centroids; segment k owns op[k] and streams op[1 - k]
@@ -2109,8 +2110,9 @@ int tc_rows(const RowsArgs& a, int prec, int phases, const TcRowsBufs& b, void* 
   // every owner block is a TMA destination; checked ahead of the first launch (the split forward, the HYB conversion)
   for (int r = 0; peers && r < b.n_ranks; ++r)
     if (b.dC_owner[r] == nullptr || (reinterpret_cast<uintptr_t>(b.dC_owner[r]) & 15) != 0) return GE2E_ERR_ARGUMENT;
-  // a per-row upstream gradient is known only after the forward: the centroid pass alone, on one device
-  if (b.grad_rows != nullptr && (phases != PASS_CENTROIDS || peers)) return GE2E_ERR_UNSUPPORTED;
+  // a per-row upstream gradient is known only after the forward: the centroid pass alone.  Over peer memory it
+  // flushes like the summed step (no local partial to zero-fill: the owners cleared their rows before the barrier)
+  if (b.grad_rows != nullptr && phases != PASS_CENTROIDS) return GE2E_ERR_UNSUPPORTED;
   if (ws == nullptr || ws_bytes < tc_workspace_bytes(a.n_local, a.n_total, a.M, a.D, a.variant))
     return GE2E_ERR_WORKSPACE;
   if (phases != 0 && (reinterpret_cast<uintptr_t>(ws) & 15) != 0) return GE2E_ERR_WORKSPACE;

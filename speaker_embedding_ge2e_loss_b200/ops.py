@@ -658,36 +658,49 @@ def fwd_rows(e_hat, c_hat_all, cos_diag, n_local, n_total, spk_offset, M, D, w, 
 def bwd_rows(e_hat, c_hat_all, cos_diag, row_stat, row_kstar, row_aux, n_local, n_total, spk_offset, M, D, w, b,
              eps, variant, precision, grad_out, dE_hat=None, row_scale=None):
     """Returns (dE_hat[U_local, D], dC_hat_partial[n_total, D], dwdb[2]).  ``dE_hat`` / ``row_scale``: what
-    fwd_rows(want_grad=True) returned (None: dE_hat is computed here)."""
+    fwd_rows(want_grad=True) returned (None: dE_hat is computed here).  ``grad_out``: the scalar upstream gradient,
+    or one per local utterance row (U_local elements, logical order: the per-utterance losses)."""
     _same_f32c(e_hat, c_hat_all, cos_diag, row_stat, row_aux, w, b, grad_out, dE_hat, row_scale)
     dev = e_hat.device
+    per_row = _per_row_grad(grad_out, n_local * M)
     if dE_hat is None or row_scale is None:
         dE_hat, row_scale = torch.empty((n_local * M, D), dtype=torch.float32, device=dev), None
     scratch = torch.empty(n_total * D + 2, dtype=torch.float32, device=dev)
+    entry = "ge2e_b200_bwd_rows_per_row" if per_row else "ge2e_b200_bwd_rows"
     with torch.cuda.device(dev):
         ws, ws_bytes = _workspace(n_local, n_total, M, D, variant, precision, dev)
-        rc = lib().ge2e_b200_bwd_rows(e_hat.data_ptr(), c_hat_all.data_ptr(), cos_diag.data_ptr(),
-                                      row_stat.data_ptr(), row_kstar.data_ptr(), row_aux.data_ptr(),
-                                      _ptr(row_scale), n_local,
-                                      n_total, spk_offset, M, D, w.data_ptr(), b.data_ptr(), eps, variant, precision,
-                                      grad_out.data_ptr(), dE_hat.data_ptr(), scratch.data_ptr(),
-                                      scratch.data_ptr() + n_total * D * 4, _ptr(ws), ws_bytes, _stream())
-    _check(rc, "ge2e_b200_bwd_rows")
+        rc = getattr(lib(), entry)(e_hat.data_ptr(), c_hat_all.data_ptr(), cos_diag.data_ptr(),
+                                   row_stat.data_ptr(), row_kstar.data_ptr(), row_aux.data_ptr(),
+                                   _ptr(row_scale), n_local,
+                                   n_total, spk_offset, M, D, w.data_ptr(), b.data_ptr(), eps, variant, precision,
+                                   grad_out.data_ptr(), dE_hat.data_ptr(), scratch.data_ptr(),
+                                   scratch.data_ptr() + n_total * D * 4, _ptr(ws), ws_bytes, _stream())
+    _check(rc, entry)
     return dE_hat, scratch[:n_total * D].view(n_total, D), scratch[n_total * D:]
+
+
+def _per_row_grad(grad_out: Tensor, U: int) -> bool:
+    """True for an upstream gradient with one entry per utterance row, False for a scalar (M >= 2: U > 1)."""
+    if grad_out.numel() == 1:
+        return False
+    if grad_out.numel() != U:
+        raise ValueError(f"the upstream gradient needs 1 or {U} entries (one per utterance row), got {grad_out.numel()}")
+    return True
 
 
 def bwd_finalize(E, dE_hat, dC_hat_local, cos_diag, row_stat, row_aux, w, b, eps, variant, grad_out,
                  row_scale=None):
-    """dE in E's element type (fp32, bf16 or fp16), rounded once."""
+    """dE in E's element type (fp32, bf16 or fp16), rounded once.  ``grad_out``: scalar or per row, as in bwd_rows."""
     E, ecode = _emb(E)
     _same_f32c(dE_hat, dC_hat_local, cos_diag, row_stat, row_aux, w, b, grad_out, row_scale)
     _need_cuda(E)
     n, M, D = E.shape
+    entry = "ge2e_b200_bwd_finalize_per_row_typed" if _per_row_grad(grad_out, n * M) else "ge2e_b200_bwd_finalize_typed"
     dE = torch.empty_like(E)
     with torch.cuda.device(E.device):
-        rc = lib().ge2e_b200_bwd_finalize_typed(E.data_ptr(), ecode, None, dE_hat.data_ptr(), dC_hat_local.data_ptr(),
-                                                cos_diag.data_ptr(), row_stat.data_ptr(), row_aux.data_ptr(),
-                                                _ptr(row_scale), n, M, D, w.data_ptr(), b.data_ptr(), eps, variant,
-                                                grad_out.data_ptr(), dE.data_ptr(), ecode, _stream())
-    check(rc, "ge2e_b200_bwd_finalize_typed")
+        rc = getattr(lib(), entry)(E.data_ptr(), ecode, None, dE_hat.data_ptr(), dC_hat_local.data_ptr(),
+                                   cos_diag.data_ptr(), row_stat.data_ptr(), row_aux.data_ptr(),
+                                   _ptr(row_scale), n, M, D, w.data_ptr(), b.data_ptr(), eps, variant,
+                                   grad_out.data_ptr(), dE.data_ptr(), ecode, _stream())
+    check(rc, entry)
     return dE

@@ -196,7 +196,8 @@ class ShardedGE2EPlan:
     Results: ``.loss`` (global), ``.dE`` (this rank's rows), ``.dw`` / ``.db`` (global)."""
 
     def __init__(self, n_local: int, n_total: int, spk_offset: int, M: int, D: int, variant: str = "softmax",
-                 precision: str = "tf32", eps: float = 1e-6, group=None, device=None, peer_memory="auto"):
+                 precision: str = "tf32", eps: float = 1e-6, group=None, device=None, peer_memory="auto", *,
+                 reduction: str = "sum"):
         """``peer_memory``: "auto" (default) / True / False.  Where the softmax loss runs on tensor cores and the
         ranks of ``group`` can map each other's memory (one NVLink / NVSwitch domain, <= 8 ranks, n_local a
         multiple of 128), the two exchange steps are done by the kernels themselves over peer memory
@@ -205,8 +206,17 @@ class ShardedGE2EPlan:
         kernel's centroid pass adding its accumulator tiles straight into the owner rank's rows
         (``ge2e_b200_step_rows_peers``); two cross-rank barriers replace the two NCCL collectives.  Otherwise
         (or with ``peer_memory=False``) the step uses all_gather_into_tensor / reduce_scatter_tensor.
-        All ranks must construct the plan collectively (the buffers are rendezvoused)."""
+        All ranks must construct the plan collectively (the buffers are rendezvoused).
+
+        ``reduction="none"``: per-utterance losses, as ``GE2EPlan(reduction="none")``.  The forward
+        (``step(E, w, b, backward=False)``) writes this rank's ``.per_row`` ([n_local, M] float32, logical order)
+        and the global ``.loss``; ``backward(E, w, b)`` differentiates sum over ranks of <grad_rows_q, L_q> with
+        this rank's ``.grad_rows`` ([n_local, M] float32, initialised to ones, read when the backward runs):
+        ``.dE`` is this rank's rows, ``.dw`` / ``.db`` are global."""
+        if reduction not in ("sum", "none"):
+            raise ValueError(f"ShardedGE2EPlan reduction must be 'sum' or 'none', got {reduction!r}")
         import torch.distributed as dist
+        self.reduction = reduction
         self.dist = dist
         self.group = group if group is not None else dist.group.WORLD
         self.n_local, self.n_total, self.spk_offset, self.M, self.D = n_local, n_total, spk_offset, M, D
@@ -255,6 +265,10 @@ class ShardedGE2EPlan:
         self.results = self.red_sum if self.peer else self.red
         self.loss, self.dw, self.db = self.results[0], self.results[1], self.results[2]
         self._side = torch.cuda.Stream(device=dev)
+        if reduction == "none":
+            self.per_row = torch.empty((n_local, M), dtype=f32, device=dev)
+            self.grad_rows = torch.ones((n_local, M), dtype=f32, device=dev)
+        self._fwd_E = None      # data_ptr of the last forward's E (reduction="none": what backward() differentiates)
 
     def _setup_peer_memory(self, world: int, rank: int) -> None:
         import ctypes as C
@@ -325,10 +339,19 @@ class ShardedGE2EPlan:
               "ge2e_b200_bwd_finalize")
         torch.sum(self.red_all, dim=0, out=self.red_sum)
 
-    def step(self, E_local: torch.Tensor, w: torch.Tensor, b: torch.Tensor) -> None:
+    def step(self, E_local: torch.Tensor, w: torch.Tensor, b: torch.Tensor, backward: bool = True) -> None:
+        """Enqueue the sharded step on the current stream.  reduction="none": the forward, then ``backward()`` unless
+        ``backward=False``; a "sum" plan always runs forward and backward together."""
         if E_local.dtype != torch.float32:
             raise TypeError(f"ShardedGE2EPlan takes float32 embeddings only, got {E_local.dtype}; bfloat16 / float16 "
                             "embeddings run through GE2ELoss(process_group=...) or a single-device GE2EPlan(dtype=...)")
+        if self.reduction == "none":
+            self._forward_rows(E_local, w, b)
+            if backward:
+                self.backward(E_local, w, b)
+            return
+        if not backward:
+            raise ValueError("a reduction='sum' ShardedGE2EPlan runs its forward and backward in one step()")
         if self.peer:
             return self._step_peer(E_local, w, b)
         h, dist = lib(), self.dist
@@ -361,23 +384,124 @@ class ShardedGE2EPlan:
                                        self.grad_out.data_ptr(), self.dE.data_ptr(), s), "ge2e_b200_bwd_finalize")
         cur.wait_stream(self._side)
 
-    def capture(self, E_local, w: torch.Tensor, b: torch.Tensor, steps: int = 1):
-        """``steps`` consecutive sharded steps in one CUDA graph (NCCL collectives included).
-        ``E_local`` is one batch or a list of batches the steps rotate over."""
-        batches = list(E_local) if isinstance(E_local, (list, tuple)) else [E_local]
+    def _forward_rows(self, E_local, w, b) -> None:
+        """reduction="none", forward: prep -> all-gather of c_hat (NCCL, or publish + barrier) -> rows pass writing
+        per_row (and the un-normalised dE_hat + row_scale where scaled) -> global loss (all-reduce of the loss, or
+        publish + barrier + sum of the table)."""
+        h, dist = lib(), self.dist
+        nl, nt, off, M, D = self.n_local, self.n_total, self.spk_offset, self.M, self.D
+        s = torch.cuda.current_stream(self.device).cuda_stream
+        ws = self._ws.data_ptr() if self._ws_bytes else None
+        check(h.ge2e_b200_prep(E_local.data_ptr(), nl, M, D, self.precision, self.e_hat.data_ptr(),
+                               self.c_hat_mine.data_ptr(), self.cos_diag.data_ptr(), self.red.data_ptr(), s),
+              "ge2e_b200_prep")
+        if self.peer:
+            check(h.ge2e_b200_peer_publish(self.c_hat_mine.data_ptr(), self._peer_slices, self._n_peers, self._mcast,
+                                           nl * D, None, 0, s), "ge2e_b200_peer_publish")
+            self._hc.barrier(channel=0)      # every slice of c_hat_all has landed
+        else:
+            dist.all_gather_into_tensor(self.c_hat_all, self.c_hat_mine, group=self.group)
+            s = torch.cuda.current_stream(self.device).cuda_stream
+        check(h.ge2e_b200_fwd_rows(self.e_hat.data_ptr(), self.c_hat_all.data_ptr(), self.cos_diag.data_ptr(), nl, nt,
+                                   off, M, D, w.data_ptr(), b.data_ptr(), self.eps, self.variant, self.precision,
+                                   self.row_stat.data_ptr(), self.row_kstar.data_ptr(), self.row_aux.data_ptr(),
+                                   self.red.data_ptr(), self.per_row.data_ptr(), None,
+                                   self.dE_hat.data_ptr() if self._scaled else None,
+                                   self.row_scale.data_ptr() if self._scaled else None, ws, self._ws_bytes, s),
+              "ge2e_b200_fwd_rows")
+        if self.peer:
+            check(h.ge2e_b200_peer_publish(self.red.data_ptr(), self._red_rows, self._world, 0, 4, None, 0, s),
+                  "ge2e_b200_peer_publish")   # my {loss, 0, 0} into row `rank` of every rank's table
+            self._hd.barrier(channel=0)
+            torch.sum(self.red_all, dim=0, out=self.red_sum)
+        else:
+            dist.all_reduce(self.red[0:1], op=dist.ReduceOp.SUM, group=self.group)
+        self._fwd_E = E_local.data_ptr()
+
+    def backward(self, E_local: torch.Tensor, w: torch.Tensor, b: torch.Tensor) -> None:
+        """reduction="none": enqueue the backward of the last forward (``step(E, w, b, backward=False)``) for the
+        upstream gradient ``.grad_rows`` on the current stream.  ``E_local`` is that forward's batch.  Results land in
+        .dE (this rank's rows) and .dw / .db (global); .loss keeps the forward's global loss.  Repeatable: a second
+        backward (or a replayed backward graph) recomputes the same gradients."""
+        if self.reduction != "none":
+            raise RuntimeError("ShardedGE2EPlan.backward() is the per-utterance backward of a reduction='none' plan; "
+                               "a 'sum' plan runs its backward inside step()")
+        if self._fwd_E is None:
+            raise RuntimeError("ShardedGE2EPlan.backward() before any forward: call step(E, w, b, backward=False) first")
+        if E_local.data_ptr() != self._fwd_E:
+            raise ValueError("ShardedGE2EPlan.backward() takes the E of the last forward")
+        h, dist = lib(), self.dist
+        nl, nt, off, M, D = self.n_local, self.n_total, self.spk_offset, self.M, self.D
+        cur = torch.cuda.current_stream(self.device)
+        s = cur.cuda_stream
+        ws = self._ws.data_ptr() if self._ws_bytes else None
+        scale = self.row_scale.data_ptr() if self._scaled else None
+        dwdb = self.red.data_ptr() + 4           # red[1:3]; red[0] keeps this rank's loss (NCCL: the global loss)
+        if self.peer:
+            # cleared here, not in the forward: a second backward must not add onto the first one's rows
+            self.dC_local.zero_()
+            self._hc.barrier(channel=0)          # every owner's rows are cleared
+            check(h.ge2e_b200_bwd_rows_peers_per_row(
+                self.e_hat.data_ptr(), self.c_hat_all.data_ptr(), self.cos_diag.data_ptr(), self.row_stat.data_ptr(),
+                self.row_aux.data_ptr(), scale, nl, nt, off, M, D, w.data_ptr(), b.data_ptr(), self.eps, self.variant,
+                self.precision, self.grad_rows.data_ptr(), self.dE_hat.data_ptr(), dwdb, self._dC_owner, self._world,
+                ws, self._ws_bytes, s), "ge2e_b200_bwd_rows_peers_per_row")
+            check(h.ge2e_b200_peer_publish(self.red.data_ptr(), self._red_rows, self._world, 0, 4, None, 0, s),
+                  "ge2e_b200_peer_publish")   # my {loss, dw, db} into row `rank` of every rank's table
+            self._hd.barrier(channel=0)          # every rank's contributions to my dC rows (and its scalars) have landed
+            self._finalize_rows(E_local, w, b, s)
+            torch.sum(self.red_all, dim=0, out=self.red_sum)
+            return
+        check(h.ge2e_b200_bwd_rows_per_row(self.e_hat.data_ptr(), self.c_hat_all.data_ptr(), self.cos_diag.data_ptr(),
+                                           self.row_stat.data_ptr(), self.row_kstar.data_ptr(), self.row_aux.data_ptr(),
+                                           scale, nl, nt, off, M, D, w.data_ptr(), b.data_ptr(), self.eps, self.variant,
+                                           self.precision, self.grad_rows.data_ptr(), self.dE_hat.data_ptr(),
+                                           self.dC_partial.data_ptr(), dwdb, ws, self._ws_bytes, s),
+              "ge2e_b200_bwd_rows_per_row")
+        dist.reduce_scatter_tensor(self.dC_local, self.dC_partial, op=dist.ReduceOp.SUM, group=self.group)
+        # {dw, db} only: red[0] was all-reduced by the forward (reducing it again would scale the loss by the world)
+        self._side.wait_stream(cur)
+        with torch.cuda.stream(self._side):
+            dist.all_reduce(self.red[1:3], op=dist.ReduceOp.SUM, group=self.group)
+        self._finalize_rows(E_local, w, b, cur.cuda_stream)
+        cur.wait_stream(self._side)
+
+    def _finalize_rows(self, E_local, w, b, s: int) -> None:
+        check(lib().ge2e_b200_bwd_finalize_per_row_typed(
+            E_local.data_ptr(), _lib.DT_F32, None, self.dE_hat.data_ptr(), self.dC_local.data_ptr(),
+            self.cos_diag.data_ptr(), self.row_stat.data_ptr(), self.row_aux.data_ptr(),
+            self.row_scale.data_ptr() if self._scaled else None, self.n_local, self.M, self.D, w.data_ptr(),
+            b.data_ptr(), self.eps, self.variant, self.grad_rows.data_ptr(), self.dE.data_ptr(), _lib.DT_F32, s),
+            "ge2e_b200_bwd_finalize_per_row_typed")
+
+    def _capture(self, enqueue, steps: int):
+        """Graph of ``steps`` calls enqueue(k); two eager calls first as warm-up (communicator set-up, lazy
+        attributes)."""
         with torch.cuda.device(self.device):
             side = torch.cuda.Stream()
             side.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(side):
                 for _ in range(2):
-                    self.step(batches[0], w, b)          # warm-up: communicator set-up, lazy attributes
+                    enqueue(0)
             torch.cuda.current_stream().wait_stream(side)
             torch.cuda.synchronize()
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g):
                 for k in range(steps):
-                    self.step(batches[k % len(batches)], w, b)
+                    enqueue(k)
         return g
+
+    def capture(self, E_local, w: torch.Tensor, b: torch.Tensor, steps: int = 1, backward: bool = True):
+        """``steps`` consecutive sharded steps in one CUDA graph (NCCL collectives included).
+        ``E_local`` is one batch or a list of batches the steps rotate over.  reduction="none" with
+        ``backward=False``: the forwards alone (see ``capture_backward``)."""
+        batches = list(E_local) if isinstance(E_local, (list, tuple)) else [E_local]
+        return self._capture(lambda k: self.step(batches[k % len(batches)], w, b, backward), steps)
+
+    def capture_backward(self, E_local: torch.Tensor, w: torch.Tensor, b: torch.Tensor):
+        """reduction="none": ``backward(E_local, w, b)`` as a CUDA graph of its own, to replay after a forward graph
+        (``capture(E_local, w, b, backward=False)``) with ``grad_rows`` set in between."""
+        return self._capture(lambda k: self.backward(E_local, w, b), 1)
 
 
 class _HostFeed:

@@ -7,7 +7,10 @@ Exchange steps (SURVEY.md section 8(e); the reference has no distributed code):
             all-reduce of {dw, db}
 Every rank returns the same global loss; ``backward`` yields d(global loss)/d(E_local) and the
 *global* dw, db on every rank (do not wrap the loss module in DDP: its two scalars are already
-reduced here).
+reduced here).  With ``reduction="none"`` every rank returns the losses of its own utterance rows
+instead (no loss all-reduce); rank q's upstream gradient g_q weights its rows, and the backward
+differentiates sum over ranks of <g_q, L_q> with the same exchanges: dE_local includes what the
+other ranks' rows send through this rank's centroids, dw / db are global.
 
 The four compute stages are injectable (``stages=``) so the collective plumbing can be tested on
 CPU under gloo with a test double; the default is the CUDA C-ABI stages of ``ops.py``.
@@ -62,7 +65,7 @@ def _inplace_ok(group) -> bool:
 
 class ShardedGE2EFunction(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, E_local, w, b, eps, variant, precision, group, stages):
+    def forward(ctx, E_local, w, b, eps, variant, precision, group, stages, per_row):
         world = dist.get_world_size(group)
         rank = dist.get_rank(group)
         n_local, M, D = E_local.shape
@@ -79,11 +82,14 @@ class ShardedGE2EFunction(torch.autograd.Function):
         dist.all_gather_into_tensor(c_hat_all, mine if _inplace_ok(group) else mine.clone(), group=group)
         # want_grad: where the softmax loss runs on tensor cores the forward also leaves the un-normalised
         # dE_hat rows + row_scale (None on every other path) and the backward is the centroid pass alone
-        row_stat, row_kstar, row_aux, _, _, dE_hat, row_scale = stages.fwd_rows(
+        row_stat, row_kstar, row_aux, per, _, dE_hat, row_scale = stages.fwd_rows(
             e_hat, c_hat_all, cos_diag, n_local, n_total, spk_offset, M, D, w, b, eps, variant, precision, accum,
-            want_grad=any(ctx.needs_input_grad[:3]))
-        loss = accum[0].clone()
-        dist.all_reduce(loss, op=dist.ReduceOp.SUM, group=group)
+            per_row=per_row, want_grad=any(ctx.needs_input_grad[:3]))
+        if per_row:
+            loss = per.view(n_local, M)                 # this rank's rows: the objective is summed by the caller
+        else:
+            loss = accum[0].clone()
+            dist.all_reduce(loss, op=dist.ReduceOp.SUM, group=group)
         ctx.save_for_backward(E_local, w, b, e_hat, c_hat_all, cos_diag, row_stat, row_kstar, row_aux, dE_hat,
                               row_scale)
         ctx.cfg = (eps, variant, precision, group, stages, n_local, n_total, spk_offset, M, D)
@@ -93,7 +99,7 @@ class ShardedGE2EFunction(torch.autograd.Function):
     def backward(ctx, g):
         E_local, w, b, e_hat, c_hat_all, cos_diag, row_stat, row_kstar, row_aux, dE_hat, row_scale = ctx.saved_tensors
         eps, variant, precision, group, stages, n_local, n_total, spk_offset, M, D = ctx.cfg
-        g = g.contiguous()
+        g = g.contiguous().reshape(-1)                  # the scalar, or one entry per local utterance row
         dE_hat, dC_partial, dwdb = stages.bwd_rows(e_hat, c_hat_all, cos_diag, row_stat, row_kstar, row_aux,
                                                    n_local, n_total, spk_offset, M, D, w, b, eps, variant,
                                                    precision, g, dE_hat=dE_hat, row_scale=row_scale)
@@ -103,13 +109,22 @@ class ShardedGE2EFunction(torch.autograd.Function):
         dist.all_reduce(dwdb, op=dist.ReduceOp.SUM, group=group)
         dE = stages.bwd_finalize(E_local, dE_hat, dC_local, cos_diag, row_stat, row_aux, w, b, eps, variant, g,
                                  row_scale=row_scale)
-        return dE, dwdb[0], dwdb[1], None, None, None, None, None
+        return dE, dwdb[0], dwdb[1], None, None, None, None, None, None
+
+
+REDUCTIONS = ("sum", "none")
 
 
 def sharded_ge2e_loss(E_local, w, b, eps=1e-6, variant="softmax", precision="fp32", group=None,
-                      stages=None):
+                      stages=None, *, reduction="sum"):
     """Global GE2E loss over the speakers of all ranks in ``group`` (E_local = this rank's
-    [n_local, M, D] block, ranks ordered by speaker index)."""
+    [n_local, M, D] block, ranks ordered by speaker index).
+
+    ``reduction``: "sum" (the global loss, the same on every rank) or "none": this rank's per-utterance
+    losses L_local[n_local, M] (float32, logical [speaker][utterance] order), differentiable for any upstream
+    gradient; the backward gives d(sum over ranks of <g_q, L_q>)/dE_local and the global dw, db."""
+    if reduction not in REDUCTIONS:
+        raise ValueError(f"reduction must be one of {REDUCTIONS}, got {reduction!r}")
     if E_local.dim() != 3 or E_local.shape[1] < 2:
         raise ValueError(f"embeddings must be [n_local, M>=2, D], got {tuple(E_local.shape)}")
     group = group if group is not None else dist.group.WORLD
@@ -120,4 +135,5 @@ def sharded_ge2e_loss(E_local, w, b, eps=1e-6, variant="softmax", precision="fp3
             pcode = _lib.resolve_precision(precision, n_local, n_local * dist.get_world_size(group), M, D, vcode)
     else:       # host-side emulation of the stages (tests): no tensor-core path to resolve to
         pcode = _lib.PRECISIONS[precision]
-    return ShardedGE2EFunction.apply(E_local, w, b, float(eps), vcode, pcode, group, stages or CudaStages)
+    return ShardedGE2EFunction.apply(E_local, w, b, float(eps), vcode, pcode, group, stages or CudaStages,
+                                     reduction == "none")
