@@ -264,7 +264,9 @@ int ge2e_b200_step_rows(const float* e_hat, const float* c_hat_all, const float*
  *   -- cross-rank barrier --, then ge2e_b200_bwd_finalize on dC_local as usual.
  * Tensor-core softmax shapes with (n_total / n_ranks) % 128 == 0 only (GE2E_ERR_UNSUPPORTED otherwise: use
  * ge2e_b200_step_rows + a reduce-scatter).  The {loss, dw, db} partials of accum[] are exchanged by the
- * caller (ShardedGE2EPlan publishes them into a [ranks, 4] table in front of the second barrier). */
+ * caller (ShardedGE2EPlan publishes them into a [ranks, 4] table in front of the second barrier).
+ * The contrast loss takes ge2e_b200_fwd_rows, then ge2e_b200_contrast_bwd_rows_peers (below, with the per-utterance
+ * entry points) in place of ge2e_b200_step_rows_peers. */
 int ge2e_b200_peer_publish(const float* src, float* const* dst_host, int n_dst, int multicast,
                            long long n_floats, float* zero, long long zero_floats, ge2e_stream_t stream);
 int ge2e_b200_step_rows_peers(const float* e_hat, const float* c_hat_all, const float* cos_diag, int n_local,
@@ -526,6 +528,33 @@ int ge2e_b200_bwd_rows_peers_per_row(const float* e_hat, const float* c_hat_all,
                                      float eps, int variant, int precision, const float* grad_rows, float* dE_hat,
                                      float* dwdb_accum, float* const* dC_owner_host, int n_ranks, void* workspace,
                                      size_t workspace_bytes, ge2e_stream_t stream);
+
+/* The contrast loss over peer memory (ge2e_b200_step_rows_peers keeps refusing it: its backward is no contraction).
+ * After ge2e_b200_fwd_rows has written row_stat / row_kstar, the backward rows stage is one gather / scatter kernel:
+ * dE_hat row r = w G_n c_hat[k*] (zero where k* < 0), and w G_n e_hat_r is added straight into centroid k*'s row of
+ * its owner rank, row k* % (n_total / n_ranks) of dC_owner_host[k* / (n_total / n_ranks)] (a HOST array of n_ranks
+ * device pointers, every rank's dC_local, this rank's own included; the owners cleared their rows before the
+ * cross-rank barrier in front of this call).  The adds are reductions at the owner's memory: red.global.add.v4.f32
+ * where D % 4 == 0, scalar ones otherwise.  dwdb_accum[2] receives this rank's {dw, db} (overwritten); the caller
+ * exchanges them (ShardedGE2EPlan: its scalar table).  GE2E_FP32 and GE2E_TF32 run the same kernel (it reads
+ * c_hat_all in fp32 either way); n_local need not be a multiple of 128.
+ *   ge2e_b200_contrast_bwd_rows_peers          the scalar upstream gradient grad_out (device, one float)
+ *   ge2e_b200_contrast_bwd_rows_peers_per_row  grad_rows[n_local * M] in its place (reduction="none")
+ * Refusals, every one before anything is launched or written: GE2E_ERR_ARGUMENT for a NULL pointer (grad_rows on the
+ * per-row form included) or a NULL owner pointer, or one not 16-byte aligned where D % 4 == 0 (4-byte otherwise);
+ * GE2E_ERR_SHAPE for n_ranks outside 2..GE2E_MAX_PEERS or n_local * n_ranks != n_total; GE2E_ERR_UNSUPPORTED for
+ * GE2E_FP32_SPLIT / GE2E_F16 (contrast has no fp16-plane path); a bad shape as ge2e_b200_bwd_rows. */
+int ge2e_b200_contrast_bwd_rows_peers(const float* e_hat, const float* c_hat_all, const float* cos_diag,
+                                      const float* row_stat, const int32_t* row_kstar, int n_local, int n_total,
+                                      int spk_offset, int M, int D, const float* w, const float* b, float eps,
+                                      int precision, const float* grad_out, float* dE_hat, float* dwdb_accum,
+                                      float* const* dC_owner_host, int n_ranks, ge2e_stream_t stream);
+int ge2e_b200_contrast_bwd_rows_peers_per_row(const float* e_hat, const float* c_hat_all, const float* cos_diag,
+                                              const float* row_stat, const int32_t* row_kstar, int n_local,
+                                              int n_total, int spk_offset, int M, int D, const float* w,
+                                              const float* b, float eps, int precision, const float* grad_rows,
+                                              float* dE_hat, float* dwdb_accum, float* const* dC_owner_host,
+                                              int n_ranks, ge2e_stream_t stream);
 
 /* ---- static helpers of the reference class (used by s5_eval_model.py:42-43) ----------- */
 

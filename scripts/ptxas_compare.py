@@ -45,6 +45,8 @@ def main():
     rules = [r.split("=", 1) for r in args.rename]
 
     def norm(name):
+        if name in old:         # a parent that already has the name: nothing to map
+            return name
         for pat, rep in rules:
             name = re.sub(pat, rep, name)
         return name

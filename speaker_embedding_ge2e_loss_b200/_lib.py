@@ -156,6 +156,12 @@ PROTOTYPES = {
                                                    C.c_int, C.c_int, _f32p, _f32p, C.c_float, C.c_int, C.c_int, _f32p,
                                                    _f32p, _f32p, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t,
                                                    _stream]),
+    "ge2e_b200_contrast_bwd_rows_peers": (C.c_int, [_f32p, _f32p, _f32p, _f32p, _i32p, C.c_int, C.c_int, C.c_int,
+                                                    C.c_int, C.c_int, _f32p, _f32p, C.c_float, C.c_int, _f32p, _f32p,
+                                                    _f32p, C.c_void_p, C.c_int, _stream]),
+    "ge2e_b200_contrast_bwd_rows_peers_per_row": (C.c_int, [_f32p, _f32p, _f32p, _f32p, _i32p, C.c_int, C.c_int,
+                                                            C.c_int, C.c_int, C.c_int, _f32p, _f32p, C.c_float, C.c_int,
+                                                            _f32p, _f32p, _f32p, C.c_void_p, C.c_int, _stream]),
     "ge2e_b200_centroids": (C.c_int, [_f32p, C.c_int, C.c_int, C.c_int, _f32p, _stream]),
     "ge2e_b200_utterance_centroids": (C.c_int, [_f32p, C.c_int, C.c_int, C.c_int, _f32p, _stream]),
     "ge2e_b200_normalize_rows": (C.c_int, [_f32p, C.c_int, C.c_int, _f32p, _stream]),

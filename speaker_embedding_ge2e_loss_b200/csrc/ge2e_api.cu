@@ -594,6 +594,53 @@ int ge2e_b200_bwd_rows_peers_per_row(const float* e_hat, const float* c_hat_all,
   return tc_rows(a, tc_prec(precision), 2, t, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
+// grad_rows (nullable): per local utterance row, in place of grad_out
+static int contrast_bwd_rows_peers_impl(const float* e_hat, const float* c_hat_all, const float* cos_diag,
+                                        const float* row_stat, const int32_t* row_kstar, int n_local, int n_total,
+                                        int spk_offset, int M, int D, const float* w, const float* b, float eps,
+                                        int precision, const float* grad_out, const float* grad_rows, float* dE_hat,
+                                        float* dwdb_accum, float* const* dC_owner_host, int n_ranks,
+                                        ge2e_stream_t stream) {
+  if (!e_hat || !c_hat_all || !cos_diag || !row_stat || !row_kstar || !w || !b || (!grad_out && !grad_rows) ||
+      !dE_hat || !dwdb_accum || !dC_owner_host)
+    return GE2E_ERR_ARGUMENT;
+  int rc = check_shape(n_local, n_total, spk_offset, M, D);
+  if (rc != GE2E_OK) return rc;
+  if ((rc = check_enum(GE2E_CONTRAST, precision)) != GE2E_OK) return rc;
+  if (n_ranks < 2 || n_ranks > GE2E_MAX_PEERS || n_local * n_ranks != n_total) return GE2E_ERR_SHAPE;
+  if (is_planes(precision)) return GE2E_ERR_UNSUPPORTED;     // contrast has no fp16-plane path
+  // the vector reductions need every owner row 16-byte aligned wherever D allows them
+  const uintptr_t align = D % 4 == 0 ? 15 : 3;
+  for (int r = 0; r < n_ranks; ++r)
+    if (!dC_owner_host[r] || (reinterpret_cast<uintptr_t>(dC_owner_host[r]) & align) != 0) return GE2E_ERR_ARGUMENT;
+  RowsArgs a{e_hat, c_hat_all, cos_diag, n_local, n_total, spk_offset, M, D, w, b, eps, GE2E_CONTRAST};
+  return simt_contrast_bwd_rows_peers(a, row_stat, row_kstar, grad_out, grad_rows, dE_hat, dwdb_accum, dC_owner_host,
+                                      n_ranks, (cudaStream_t)stream);
+}
+
+int ge2e_b200_contrast_bwd_rows_peers(const float* e_hat, const float* c_hat_all, const float* cos_diag,
+                                      const float* row_stat, const int32_t* row_kstar, int n_local, int n_total,
+                                      int spk_offset, int M, int D, const float* w, const float* b, float eps,
+                                      int precision, const float* grad_out, float* dE_hat, float* dwdb_accum,
+                                      float* const* dC_owner_host, int n_ranks, ge2e_stream_t stream) {
+  if (!grad_out) return GE2E_ERR_ARGUMENT;
+  return contrast_bwd_rows_peers_impl(e_hat, c_hat_all, cos_diag, row_stat, row_kstar, n_local, n_total, spk_offset,
+                                      M, D, w, b, eps, precision, grad_out, nullptr, dE_hat, dwdb_accum,
+                                      dC_owner_host, n_ranks, stream);
+}
+
+int ge2e_b200_contrast_bwd_rows_peers_per_row(const float* e_hat, const float* c_hat_all, const float* cos_diag,
+                                              const float* row_stat, const int32_t* row_kstar, int n_local,
+                                              int n_total, int spk_offset, int M, int D, const float* w,
+                                              const float* b, float eps, int precision, const float* grad_rows,
+                                              float* dE_hat, float* dwdb_accum, float* const* dC_owner_host,
+                                              int n_ranks, ge2e_stream_t stream) {
+  if (!grad_rows) return GE2E_ERR_ARGUMENT;
+  return contrast_bwd_rows_peers_impl(e_hat, c_hat_all, cos_diag, row_stat, row_kstar, n_local, n_total, spk_offset,
+                                      M, D, w, b, eps, precision, nullptr, grad_rows, dE_hat, dwdb_accum,
+                                      dC_owner_host, n_ranks, stream);
+}
+
 // ---- whole step in one call ---------------------------------------------------------------
 // 0 = never (A/B timing), 1 = where it is faster than the pipeline (default), 2 = every supported shape (tests)
 static std::atomic<int> g_small_mode{1};

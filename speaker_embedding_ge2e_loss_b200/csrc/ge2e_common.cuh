@@ -147,6 +147,11 @@ int simt_fwd_rows(const RowsArgs& a, float* row_stat, int32_t* row_kstar, float*
 int simt_bwd_rows(const RowsArgs& a, const float* row_stat, const int32_t* row_kstar,
                   const float* row_aux, const float* grad_out, const float* grad_rows, float* dE_hat,
                   float* dC_hat_partial, float* dwdb_accum, cudaStream_t st);
+// the contrast backward rows over peer memory: the k* scatter adds into dC_owner[n_ranks] (HOST array of device
+// pointers, rank q's dC_local[n_total / n_ranks, D]); {dw, db} into dwdb_accum (cleared first)
+int simt_contrast_bwd_rows_peers(const RowsArgs& a, const float* row_stat, const int32_t* row_kstar,
+                                 const float* grad_out, const float* grad_rows, float* dE_hat, float* dwdb_accum,
+                                 float* const* dC_owner, int n_ranks, cudaStream_t st);
 // largest M whose backward finalize runs at width D (0: D unsupported); see ge2e_b200_max_utterances
 int finalize_max_rows(int D);
 int simt_bwd_finalize(const void* E, int e_dt, const int32_t* row_index, const float* dE_hat, const float* dC_hat_local,

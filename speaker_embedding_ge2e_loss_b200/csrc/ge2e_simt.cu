@@ -877,6 +877,75 @@ contrast_bwd_kernel(const float* __restrict__ e_hat, const float* __restrict__ c
   if (tid == 0) { atomicAdd(dwdb + 0, dwt); atomicAdd(dwdb + 1, dbt); }
 }
 
+// contrast_bwd_kernel, speaker-sharded over peer memory: row r's w G_n e_hat_r is added straight into the owner
+// rank's dC_local row (centroid k* lives at row k* % peer_rows of rank k* / peer_rows) instead of a full-height
+// dC_hat partial.  The adds are system-scope reductions performed at the owner's memory, since every rank adds into
+// the same rows at once.  VEC (D % 4 == 0, every row 16-byte aligned): red.global.add.v4.f32, one float4 a lane per
+// 128 columns.  dE_hat and {dw, db} as in contrast_bwd_kernel.
+struct PeerRows { float* p[GE2E_MAX_PEERS]; };
+
+template <bool RG, bool VEC>
+__global__ void __launch_bounds__(kThreads)
+contrast_bwd_peers_kernel(const float* __restrict__ e_hat, const float* __restrict__ c_hat_all,
+                          const float* __restrict__ cos_diag, const float* __restrict__ row_stat,
+                          const int32_t* __restrict__ kstar, int U, int D, const float* __restrict__ wp,
+                          const float* __restrict__ bp, float eps, const float* __restrict__ gp,
+                          float* __restrict__ dE_hat, PeerRows owner, int peer_rows, float* __restrict__ dwdb) {
+  __shared__ float red[kWarps];
+  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+  const int r = blockIdx.x * kWarps + wid;
+  const float w = __ldg(wp), b = __ldg(bp), g0 = RG ? 0.f : __ldg(gp);
+  float dw = 0.f, db = 0.f;
+  if (r < U) {
+    const float g = RG ? __ldg(gp + r) : g0;
+    const float cd = __ldg(cos_diag + r) + eps;
+    const float sp = 1.f / (1.f + expf(-fmaf(w, cd, b)));
+    const float Gp = -g * sp * (1.f - sp);
+    const int ks = __ldg(kstar + r);
+    float Gn = 0.f, cn = 0.f;
+    const float* er = e_hat + (size_t)r * D;
+    float* de = dE_hat + (size_t)r * D;
+    if (ks >= 0) {
+      const float* ck = c_hat_all + (size_t)ks * D;
+      const int o = ks / peer_rows;
+      float* dst = owner.p[0];          // owner.p[o] by selects: a dynamic index would copy the array to local memory
+#pragma unroll
+      for (int q = 1; q < GE2E_MAX_PEERS; ++q)
+        if (q == o) dst = owner.p[q];
+      dst += (size_t)(ks - o * peer_rows) * D;
+      const float sn = 1.f / (1.f + expf(-__ldg(row_stat + r)));
+      Gn = g * sn * (1.f - sn);
+      const float wg = w * Gn;
+      float d = 0.f;
+      if (VEC) {
+        const float4* er4 = reinterpret_cast<const float4*>(er);
+        const float4* ck4 = reinterpret_cast<const float4*>(ck);
+        for (int c = lane; c < (D >> 2); c += 32) {
+          const float4 e = __ldg(er4 + c), k = __ldg(ck4 + c);
+          d = fmaf(e.x, k.x, fmaf(e.y, k.y, fmaf(e.z, k.z, fmaf(e.w, k.w, d))));
+          reinterpret_cast<float4*>(de)[c] = make_float4(wg * k.x, wg * k.y, wg * k.z, wg * k.w);
+          asm volatile("red.relaxed.sys.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + 4 * c),
+                       "f"(wg * e.x), "f"(wg * e.y), "f"(wg * e.z), "f"(wg * e.w)
+                       : "memory");
+        }
+      } else {
+        for (int c = lane; c < D; c += 32) {
+          d = fmaf(__ldg(er + c), __ldg(ck + c), d);
+          de[c] = wg * __ldg(ck + c);
+          asm volatile("red.relaxed.sys.global.add.f32 [%0], %1;" ::"l"(dst + c), "f"(wg * __ldg(er + c)) : "memory");
+        }
+      }
+      cn = warp_sum(d) + eps;
+    } else {
+      for (int c = lane; c < D; c += 32) de[c] = 0.f;
+    }
+    if (lane == 0) { dw = Gp * cd + Gn * cn; db = Gp + Gn; }
+  }
+  const float dwt = block_sum(dw, red);
+  const float dbt = block_sum(db, red);
+  if (tid == 0) { atomicAdd(dwdb + 0, dwt); atomicAdd(dwdb + 1, dbt); }
+}
+
 // ------------------------------------------------------------------------------------------
 // K4: finalize.  grid = n_local, block = 256, dynamic smem = (2*M + 2) * Dp floats.
 // ------------------------------------------------------------------------------------------
@@ -1531,6 +1600,29 @@ int simt_bwd_rows(const RowsArgs& a, const float* row_stat, const int32_t* row_k
   splits = (nchunks + p.chunks_per_split - 1) / p.chunks_per_split;
   return rg ? dispatch_strip<MODE_BWD_DC, GE2E_SOFTMAX, true>(p, splits, st)
             : dispatch_strip<MODE_BWD_DC, GE2E_SOFTMAX>(p, splits, st);
+}
+
+int simt_contrast_bwd_rows_peers(const RowsArgs& a, const float* row_stat, const int32_t* row_kstar,
+                                 const float* grad_out, const float* grad_rows, float* dE_hat, float* dwdb_accum,
+                                 float* const* dC_owner, int n_ranks, cudaStream_t st) {
+  const int U = a.n_local * a.M, grid = (U + kWarps - 1) / kWarps, peer_rows = a.n_total / n_ranks;
+  PeerRows o{};
+  for (int r = 0; r < n_ranks; ++r) o.p[r] = dC_owner[r];
+  const bool vec = a.D % 4 == 0 && rows_vec_ok(a.e_hat) && rows_vec_ok(a.c_hat_all) && rows_vec_ok(dE_hat);
+  const float* g = grad_rows != nullptr ? grad_rows : grad_out;
+  GE2E_CUDA_TRY(cudaMemsetAsync(dwdb_accum, 0, 2 * sizeof(float), st));
+#define GE2E_CONTRAST_PEERS(RG, VEC)                                                                              \
+  contrast_bwd_peers_kernel<RG, VEC><<<grid, kThreads, 0, st>>>(a.e_hat, a.c_hat_all, a.cos_diag, row_stat, row_kstar, \
+                                                                U, a.D, a.w, a.b, a.eps, g, dE_hat, o, peer_rows,     \
+                                                                dwdb_accum)
+  if (grad_rows != nullptr) {
+    if (vec) GE2E_CONTRAST_PEERS(true, true); else GE2E_CONTRAST_PEERS(true, false);
+  } else {
+    if (vec) GE2E_CONTRAST_PEERS(false, true); else GE2E_CONTRAST_PEERS(false, false);
+  }
+#undef GE2E_CONTRAST_PEERS
+  GE2E_LAUNCHED();
+  return GE2E_OK;
 }
 
 // RG: grad_out is the upstream gradient per logical utterance row

@@ -198,14 +198,16 @@ class ShardedGE2EPlan:
     def __init__(self, n_local: int, n_total: int, spk_offset: int, M: int, D: int, variant: str = "softmax",
                  precision: str = "tf32", eps: float = 1e-6, group=None, device=None, peer_memory="auto", *,
                  reduction: str = "sum"):
-        """``peer_memory``: "auto" (default) / True / False.  Where the softmax loss runs on tensor cores and the
-        ranks of ``group`` can map each other's memory (one NVLink / NVSwitch domain, <= 8 ranks, n_local a
-        multiple of 128), the two exchange steps are done by the kernels themselves over peer memory
-        (``torch.distributed._symmetric_memory`` buffers): the all-gather of ``c_hat`` is a store of this rank's
-        slice into every peer (``ge2e_b200_peer_publish``), the reduce-scatter of ``dC_hat`` is the step
-        kernel's centroid pass adding its accumulator tiles straight into the owner rank's rows
-        (``ge2e_b200_step_rows_peers``); two cross-rank barriers replace the two NCCL collectives.  Otherwise
-        (or with ``peer_memory=False``) the step uses all_gather_into_tensor / reduce_scatter_tensor.
+        """``peer_memory``: "auto" (default) / True / False.  Where the ranks of ``group`` can map each other's
+        memory (one NVLink / NVSwitch domain, <= 8 ranks, n_local * world == n_total) and the loss is either the
+        softmax loss on tensor cores with n_local a multiple of 128 or the contrast loss (fp32 or tf32), the two
+        exchange steps are done by the kernels themselves over peer memory (``torch.distributed._symmetric_memory``
+        buffers): the all-gather of ``c_hat`` is a store of this rank's slice into every peer
+        (``ge2e_b200_peer_publish``), the reduce-scatter of ``dC_hat`` is the backward adding straight into the
+        owner rank's rows -- the softmax step kernel's centroid pass its accumulator tiles
+        (``ge2e_b200_step_rows_peers``), the contrast gather / scatter kernel each row's add into centroid k*
+        (``ge2e_b200_contrast_bwd_rows_peers``); two cross-rank barriers replace the two NCCL collectives.
+        Otherwise (or with ``peer_memory=False``) the step uses all_gather_into_tensor / reduce_scatter_tensor.
         All ranks must construct the plan collectively (the buffers are rendezvoused).
 
         ``reduction="none"``: per-utterance losses, as ``GE2EPlan(reduction="none")``.  The forward
@@ -242,7 +244,12 @@ class ShardedGE2EPlan:
         self.peer, self.peer_error = False, None
         world = dist.get_world_size(self.group)
         if peer_memory and world > 1:
-            ok = self._scaled and world <= 8 and n_local % 128 == 0 and n_local * world == n_total
+            # softmax: the tensor-core step's owner flush moves whole 128-row tiles; contrast: one row per add
+            if self.variant == _lib.CONTRAST:
+                kernel_ok = self.precision in (_lib.FP32, _lib.TF32)
+            else:
+                kernel_ok = self._scaled and n_local % 128 == 0
+            ok = kernel_ok and world <= 8 and n_local * world == n_total
             if ok:
                 try:
                     self._setup_peer_memory(world, dist.get_rank(self.group))
@@ -251,7 +258,8 @@ class ShardedGE2EPlan:
                     if peer_memory is True:
                         raise
             elif peer_memory is True:
-                raise ValueError("peer_memory=True needs the tensor-core softmax path, <= 8 ranks and n_local % 128 == 0")
+                raise ValueError("peer_memory=True needs <= 8 ranks and n_local * world == n_total, and for the softmax "
+                                 "loss the tensor-core path and n_local % 128 == 0 (contrast: fp32 or tf32)")
         if not self.peer:
             self.dC_partial = torch.empty((n_total, D), dtype=f32, device=dev)
             self.dC_local = torch.empty((n_local, D), dtype=f32, device=dev)
@@ -311,7 +319,8 @@ class ShardedGE2EPlan:
 
     def _step_peer(self, E_local, w, b) -> None:
         """prep -> publish c_hat slice to the peers, clear my dC rows -> barrier -> step kernel (centroid pass adds
-        into the owners' rows over NVLink) -> barrier -> all-reduce {loss, dw, db} || finalize."""
+        into the owners' rows over NVLink; contrast: forward rows, then the gather / scatter adding into them) ->
+        publish {loss, dw, db} -> barrier -> finalize."""
         h, dist = lib(), self.dist
         nl, nt, off, M, D = self.n_local, self.n_total, self.spk_offset, self.M, self.D
         cur = torch.cuda.current_stream(self.device)
@@ -323,20 +332,34 @@ class ShardedGE2EPlan:
         check(h.ge2e_b200_peer_publish(self.c_hat_mine.data_ptr(), self._peer_slices, self._n_peers, self._mcast, nl * D,
                                        self.dC_local.data_ptr(), nl * D, s), "ge2e_b200_peer_publish")
         self._hc.barrier(channel=0)          # every slice of c_hat_all has landed, every dC_local is cleared
-        check(h.ge2e_b200_step_rows_peers(self.e_hat.data_ptr(), self.c_hat_all.data_ptr(), self.cos_diag.data_ptr(), nl,
-                                          nt, off, M, D, w.data_ptr(), b.data_ptr(), self.eps, self.variant,
-                                          self.precision, self.grad_out.data_ptr(), self.row_stat.data_ptr(),
-                                          self.row_kstar.data_ptr(), self.row_aux.data_ptr(), self.row_scale.data_ptr(),
-                                          self.red.data_ptr(), self.dE_hat.data_ptr(), self._dC_owner, self._world, ws,
-                                          self._ws_bytes, s), "ge2e_b200_step_rows_peers")
+        if self.variant == _lib.CONTRAST:
+            # forward rows (row_stat, row_kstar, loss), then the gather / scatter adding into the owners' rows
+            check(h.ge2e_b200_fwd_rows(self.e_hat.data_ptr(), self.c_hat_all.data_ptr(), self.cos_diag.data_ptr(), nl,
+                                       nt, off, M, D, w.data_ptr(), b.data_ptr(), self.eps, self.variant,
+                                       self.precision, self.row_stat.data_ptr(), self.row_kstar.data_ptr(),
+                                       self.row_aux.data_ptr(), self.red.data_ptr(), None, None, None, None, ws,
+                                       self._ws_bytes, s), "ge2e_b200_fwd_rows")
+            check(h.ge2e_b200_contrast_bwd_rows_peers(
+                self.e_hat.data_ptr(), self.c_hat_all.data_ptr(), self.cos_diag.data_ptr(), self.row_stat.data_ptr(),
+                self.row_kstar.data_ptr(), nl, nt, off, M, D, w.data_ptr(), b.data_ptr(), self.eps, self.precision,
+                self.grad_out.data_ptr(), self.dE_hat.data_ptr(), self.red.data_ptr() + 4, self._dC_owner,
+                self._world, s), "ge2e_b200_contrast_bwd_rows_peers")
+        else:
+            check(h.ge2e_b200_step_rows_peers(self.e_hat.data_ptr(), self.c_hat_all.data_ptr(), self.cos_diag.data_ptr(),
+                                              nl, nt, off, M, D, w.data_ptr(), b.data_ptr(), self.eps, self.variant,
+                                              self.precision, self.grad_out.data_ptr(), self.row_stat.data_ptr(),
+                                              self.row_kstar.data_ptr(), self.row_aux.data_ptr(),
+                                              self.row_scale.data_ptr(), self.red.data_ptr(), self.dE_hat.data_ptr(),
+                                              self._dC_owner, self._world, ws, self._ws_bytes, s),
+                  "ge2e_b200_step_rows_peers")
         check(h.ge2e_b200_peer_publish(self.red.data_ptr(), self._red_rows, self._world, 0, 4, None, 0, s),
               "ge2e_b200_peer_publish")   # my {loss, dw, db} into row `rank` of every rank's table
         self._hd.barrier(channel=0)          # every rank's contributions to my dC rows (and its scalars) have landed
         check(h.ge2e_b200_bwd_finalize(E_local.data_ptr(), self.dE_hat.data_ptr(), self.dC_local.data_ptr(),
                                        self.cos_diag.data_ptr(), self.row_stat.data_ptr(), self.row_aux.data_ptr(),
-                                       self.row_scale.data_ptr(), nl, M, D, w.data_ptr(), b.data_ptr(), self.eps,
-                                       self.variant, self.grad_out.data_ptr(), self.dE.data_ptr(), s),
-              "ge2e_b200_bwd_finalize")
+                                       self.row_scale.data_ptr() if self._scaled else None, nl, M, D, w.data_ptr(),
+                                       b.data_ptr(), self.eps, self.variant, self.grad_out.data_ptr(),
+                                       self.dE.data_ptr(), s), "ge2e_b200_bwd_finalize")
         torch.sum(self.red_all, dim=0, out=self.red_sum)
 
     def step(self, E_local: torch.Tensor, w: torch.Tensor, b: torch.Tensor, backward: bool = True) -> None:
@@ -441,11 +464,19 @@ class ShardedGE2EPlan:
             # cleared here, not in the forward: a second backward must not add onto the first one's rows
             self.dC_local.zero_()
             self._hc.barrier(channel=0)          # every owner's rows are cleared
-            check(h.ge2e_b200_bwd_rows_peers_per_row(
-                self.e_hat.data_ptr(), self.c_hat_all.data_ptr(), self.cos_diag.data_ptr(), self.row_stat.data_ptr(),
-                self.row_aux.data_ptr(), scale, nl, nt, off, M, D, w.data_ptr(), b.data_ptr(), self.eps, self.variant,
-                self.precision, self.grad_rows.data_ptr(), self.dE_hat.data_ptr(), dwdb, self._dC_owner, self._world,
-                ws, self._ws_bytes, s), "ge2e_b200_bwd_rows_peers_per_row")
+            if self.variant == _lib.CONTRAST:
+                check(h.ge2e_b200_contrast_bwd_rows_peers_per_row(
+                    self.e_hat.data_ptr(), self.c_hat_all.data_ptr(), self.cos_diag.data_ptr(),
+                    self.row_stat.data_ptr(), self.row_kstar.data_ptr(), nl, nt, off, M, D, w.data_ptr(), b.data_ptr(),
+                    self.eps, self.precision, self.grad_rows.data_ptr(), self.dE_hat.data_ptr(), dwdb, self._dC_owner,
+                    self._world, s), "ge2e_b200_contrast_bwd_rows_peers_per_row")
+            else:
+                check(h.ge2e_b200_bwd_rows_peers_per_row(
+                    self.e_hat.data_ptr(), self.c_hat_all.data_ptr(), self.cos_diag.data_ptr(),
+                    self.row_stat.data_ptr(), self.row_aux.data_ptr(), scale, nl, nt, off, M, D, w.data_ptr(),
+                    b.data_ptr(), self.eps, self.variant, self.precision, self.grad_rows.data_ptr(),
+                    self.dE_hat.data_ptr(), dwdb, self._dC_owner, self._world, ws, self._ws_bytes, s),
+                    "ge2e_b200_bwd_rows_peers_per_row")
             check(h.ge2e_b200_peer_publish(self.red.data_ptr(), self._red_rows, self._world, 0, 4, None, 0, s),
                   "ge2e_b200_peer_publish")   # my {loss, dw, db} into row `rank` of every rank's table
             self._hd.barrier(channel=0)          # every rank's contributions to my dC rows (and its scalars) have landed
